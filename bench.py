@@ -28,6 +28,12 @@ brings every shard's results to rank 0 for the oracle comparison.  One "step" = 
            no text verification = every LF step of the reference runs), device-resident and end to end.
 `single_process` (N > 1) rank 0 alone drives all N GPUs through ONE gdx_count_many_sharded call.
 `cpu_baseline` (N = 1) the oracle's port of the reference's 64-query batched search on the host cores.
+
+--dump-outputs DIR  after the run, writes what the timed paths computed in their last step to DIR as float64 .npy files,
+           for a fixed, seeded sample of the batch (count_query.npy: the batch positions of the sample): count.npy, the
+           counts a caller of gdx_count_many_device receives (`value`), and locate_first_position.npy, the text
+           position of each sampled query's first hit from the last `locate` step (not with --no-locate).  The inputs
+           are seeded, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import ctypes as C
@@ -42,12 +48,15 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the tree may be read-only: the benchmark writes nothing into it
 os.environ.setdefault("GDX_ORACLE_NATIVE", "1")  # CPU baseline: oracle rebuilt with -march=native on this box
 
 TEXT_SEED = 0x5EED0001
 QUERY_SEED = 0x5EED0002
 N_CODE = ord("N")
 QCHUNK = 1 << 21  # queries are generated in chunks of this many, each from its own seed
+DUMP_SEED = 0x5EED0003
+DUMP_SAMPLE = 1 << 21  # --dump-outputs: this many queries (16 MiB of float64 per file, 48 MiB in all)
 
 
 def parse_args():
@@ -68,7 +77,14 @@ def parse_args():
     ap.add_argument("--cpu-seconds", type=float, default=12.0, help="target CPU work of the cpu_baseline sample")
     ap.add_argument("--multi-hit-queries", type=int, default=2_000_000)
     ap.add_argument("--multi-hit-len", type=int, default=14)
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write a seeded sample of the last timed step's counts and hits to DIR as .npy (see the docstring)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs dumps the outputs of this repo's CUDA path (--impl ours)")
+    return args
 
 
 # ---- synthetic data (torch on the GPU is plumbing here: RNG + gathers, nothing of the search path) ---
@@ -236,6 +252,20 @@ def measured_peaks():
     except Exception:
         peaks["random_lines_per_s"] = None
     return peaks
+
+
+def dump_pick(nq):
+    """The batch positions --dump-outputs writes: every query up to DUMP_SAMPLE, else a fixed seeded sample (sorted)."""
+    if nq <= DUMP_SAMPLE:
+        return np.arange(nq)
+    return np.sort(np.random.default_rng(DUMP_SEED).choice(nq, DUMP_SAMPLE, replace=False))
+
+
+def dump_outputs(dirname, arrays):
+    """name -> DIR/name.npy as float64 (counts, batch and text positions are integers below 2^53: exact)."""
+    os.makedirs(dirname, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(dirname, name + ".npy"), np.asarray(a).astype(np.float64))
 
 
 def workload_name(args, world):
@@ -534,7 +564,7 @@ def run_ours(args, rank, world, local_rank):
     locate = None
     peaks = measured_peaks()
     R = int(info.rank_record_bytes)
-    locate_sample = None
+    locate_sample, locate_first = None, None
     if not args.no_locate:
         hit_off = torch.zeros(nq + 1, dtype=torch.int64).pin_memory().numpy().view(np.uint64)
         state = {}
@@ -552,6 +582,9 @@ def run_ours(args, rank, world, local_rank):
         first = hits[(hit_off[b:e] - np.uint64(state["first"][0])).astype(np.int64), 1].astype(np.int64)
         single = width == 1
         assert np.array_equal(first[single], origins[b:e][single]), "locate: a unique hit is not at its origin"
+        if args.dump_outputs:  # this shard's part of the sample (every query has a hit: counts >= 1 above)
+            pick = dump_pick(nq)
+            locate_first = first[pick[(pick >= b) & (pick < e)] - b]
         ns_ = min(snq, 20_000)  # this shard's sample for the oracle comparison on rank 0
         o0 = int(hit_off[b])
         locate_sample = (hit_off[b:b + ns_ + 1] - np.uint64(o0), hits[: int(hit_off[b + ns_]) - o0].copy())
@@ -665,6 +698,10 @@ def run_ours(args, rank, world, local_rank):
         del mine, parts
         loc_samples = [None] * world
         dist.all_gather_object(loc_samples, locate_sample)
+        if locate_first is not None:  # shards in rank order = the sorted sample in order
+            firsts = [None] * world
+            dist.all_gather_object(firsts, locate_first)
+            locate_first = np.concatenate(firsts)
 
     # ---- single process, all GPUs: ONE gdx_count_many_sharded call from rank 0 (the other ranks idle) -------
     single = None
@@ -749,6 +786,14 @@ def run_ours(args, rank, world, local_rank):
     cpu_barrier()  # everyone leaves together (rank 0 was busy with the oracle meanwhile)
     if rank != 0:
         return
+    if args.dump_outputs:
+        # N > 1: the other shards' counts as gathered above (every rank checked its range of counts_all against its
+        # device-path counts)
+        pick = dump_pick(nq)
+        dumped = {"count": (counts_device_path if world == 1 else counts_all)[pick], "count_query": pick}
+        if locate_first is not None:
+            dumped["locate_first_position"] = locate_first
+        dump_outputs(args.dump_outputs, dumped)
     out = assemble(args, world, info, st, kernel_ms, step_ms, e2e, locate, no_accel, single, cpu, parity, peaks, clock_info,
                    {"data": round(t_data, 2), "index_build": round(t_build, 2), "replicate": round(t_bcast, 2),
                     "replicate_transport": transport}, steps, warm)

@@ -8,8 +8,10 @@ from __future__ import annotations
 
 import ctypes as C
 import os
+import shutil
 import subprocess
 import sys
+import tempfile
 from typing import Iterable, Sequence
 
 import numpy as np
@@ -38,16 +40,17 @@ class OraclePanic(RuntimeError):
 
 def build_library(force: bool = False) -> str:
     """Portable build by default (the .so travels between machines).  With GDX_ORACLE_NATIVE=1 (set by
-    bench.py for the CPU-baseline legs) a -march=native library is built on the machine it runs on."""
+    bench.py for the CPU-baseline legs) a -march=native library is built on the machine it runs on, into a
+    fresh temporary directory: the tree may be read-only, and a native build must not travel."""
     src = os.path.join(_HERE, "gdx_oracle.c")
     newest = max(os.path.getmtime(src), os.path.getmtime(os.path.join(_HERE, "gdx_oracle.h")))
     if os.environ.get("GDX_ORACLE_NATIVE") == "1":
-        native = os.path.join(_HERE, "_build", "libgdx_oracle_native.so")
+        out = tempfile.mkdtemp(prefix="gdx_oracle_native_")
         try:
-            subprocess.check_call(["make", "-C", _HERE, "-s", "-B", "native"], stdout=sys.stderr)
-            return native
+            subprocess.check_call(["make", "-C", _HERE, "-s", "native", "OUT=" + out], stdout=sys.stderr)
+            return os.path.join(out, "libgdx_oracle_native.so")
         except Exception:
-            pass  # no compiler on this machine: fall back to the portable build
+            shutil.rmtree(out, ignore_errors=True)  # no compiler on this machine: fall back to the portable build
     if force or not os.path.exists(_LIB_PATH) or os.path.getmtime(_LIB_PATH) < newest:
         subprocess.check_call(["make", "-C", _HERE, "-s"], stdout=sys.stderr)
     return _LIB_PATH
@@ -59,7 +62,10 @@ _lib = None
 def lib() -> C.CDLL:
     global _lib
     if _lib is None:
-        L = C.CDLL(build_library())
+        path = build_library()
+        L = C.CDLL(path)
+        if path != _LIB_PATH:  # a native build in its temporary directory: loaded, nothing left to keep
+            shutil.rmtree(os.path.dirname(path), ignore_errors=True)
         u8p, u16p, u64p, i64p = (C.POINTER(t) for t in (C.c_uint8, C.c_uint16, C.c_uint64, C.c_int64))
         vp = C.c_void_p
         L.gdxo_build.argtypes = [vp, vp, C.c_uint64, vp, C.c_uint32, C.c_uint32, C.c_uint32, C.c_uint32,

@@ -54,13 +54,20 @@ def test_struct_sizes_match_the_header(gdx, tmp_path):
     assert got == want
 
 
-def test_no_cpu_fallback(gdx):
-    import torch
-    if torch.cuda.is_available():
-        pytest.skip("a GPU is present")
-    with pytest.raises(gdx.GenedexError) as e:
-        gdx.FmIndexConfig("i32").construct_index([b"ACGT"], gdx.alphabet.ascii_dna())
-    assert "no CPU fallback" in str(e.value)
+def test_no_cpu_fallback():
+    # in a process that sees no CUDA device (CUDA_VISIBLE_DEVICES=""), so the check also runs where a GPU is present
+    code = ("import sys; sys.path.insert(0, %r)\n"
+            "import genedex_b200 as gdx\n"
+            "try:\n"
+            "    gdx.FmIndexConfig('i32').construct_index([b'ACGT'], gdx.alphabet.ascii_dna())\n"
+            "except gdx.GenedexError as e:\n"
+            "    print(e)\n"
+            "else:\n"
+            "    sys.exit('an index was built without a CUDA device')\n" % ROOT)
+    out = subprocess.run([sys.executable, "-c", code], env=dict(os.environ, CUDA_VISIBLE_DEVICES=""),
+                         capture_output=True, text=True)
+    assert out.returncode == 0, out.stdout + out.stderr
+    assert "no CPU fallback" in out.stdout
 
 
 def _host_sa(gdx, dense, sigma):
