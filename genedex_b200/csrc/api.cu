@@ -84,10 +84,9 @@ gdx_status guarded(F &&f) noexcept {
 uint64_t align_up(uint64_t v, uint64_t a) { return (v + a - 1) / a * a; }
 uint64_t div_up(uint64_t a, uint64_t b) { return (a + b - 1) / b; }
 
-// Random 32 B record reads: ask the L2 to fetch single sectors from DRAM instead of sector pairs
-// (cudaLimitMaxL2FetchGranularity is a per-context hint).  GDX_L2_FETCH_GRANULARITY=0 leaves the
-// driver default, 32/64/128 sets it (measured: no effect on B200, profiles/r1_ab_l2_fetch_granularity.txt).
-// Applied once per device, with that device current.
+// The device-resident entry points take their scratch from the stream-ordered pool: keep freed blocks
+// cached across synchronisation points instead of returning them to the driver.  Applied once per
+// device, with that device current.
 void apply_device_settings(int dev) {
     static std::mutex mu;
     static bool done[64] = {};
@@ -95,13 +94,6 @@ void apply_device_settings(int dev) {
     std::lock_guard<std::mutex> lk(mu);
     if (done[dev]) return;
     done[dev] = true;
-    const char *env = getenv("GDX_L2_FETCH_GRANULARITY");
-    const int want = env ? atoi(env) : 32;
-    if (want > 0) cudaDeviceSetLimit(cudaLimitMaxL2FetchGranularity, (size_t)want);
-    // the device-resident entry points take their scratch from the stream-ordered pool: keep freed
-    // blocks cached across synchronisation points instead of returning them to the driver
-    cudaDeviceSetLimit(cudaLimitPersistingL2CacheSize, 16ull << 20);  // room for the superblock tables
-    cudaGetLastError();
     cudaMemPool_t pool;
     if (cudaDeviceGetDefaultMemPool(&pool, dev) == cudaSuccess) {
         uint64_t keep = ~0ull;
@@ -203,6 +195,8 @@ const uint64_t kChunkFirst = env_mb("GDX_CHUNK_FIRST_MB", 4);
 const uint64_t kChunkMax = env_mb("GDX_CHUNK_MAX_MB", 32);
 const uint64_t kChunkTail = env_mb("GDX_CHUNK_TAIL_MB", 4);
 constexpr uint64_t kChunkMaxQueries = 64ull << 20;
+// first guess of the host-to-device link rate for the hybrid upload of pinned IO bytes (search_host)
+constexpr double kLinkGuessBytesPerMs = 50e6;  // 50 GB/s
 
 struct Slot {
     cudaStream_t stream = nullptr;
@@ -343,21 +337,6 @@ Workspace *acquire_ws(const gdx_index *idx) {
         w->destroy();
         delete w;
         return nullptr;
-    }
-    // The superblock table (count[c] + per-superblock ranks, ~1.5 MB for a 3.1 Gbp text) is read by
-    // every LF step: keep it in the persisting part of L2 for the kernels on the workspace's streams.
-    // Best effort (GDX_L2_PERSIST=0 disables it).
-    static const bool persist = !(getenv("GDX_L2_PERSIST") && atoi(getenv("GDX_L2_PERSIST")) == 0);
-    const uint64_t sbc_bytes = idx->h.n_superblocks * idx->h.layout.noff * 8;
-    if (persist && sbc_bytes && sbc_bytes <= (16ull << 20)) {
-        cudaStreamAttrValue attr = {};
-        attr.accessPolicyWindow.base_ptr = const_cast<uint64_t *>(idx->dev.sbc);
-        attr.accessPolicyWindow.num_bytes = sbc_bytes;
-        attr.accessPolicyWindow.hitRatio = 1.0f;
-        attr.accessPolicyWindow.hitProp = cudaAccessPropertyPersisting;
-        attr.accessPolicyWindow.missProp = cudaAccessPropertyStreaming;
-        for (auto &sl : w->slot) cudaStreamSetAttribute(sl.stream, cudaStreamAttributeAccessPolicyWindow, &attr);
-        cudaGetLastError();
     }
     return w;
 }
@@ -547,9 +526,6 @@ gdx_status init_policies(gdx_index *idx) {
     idx->verify = verify_enabled();
     if (const char *vm = getenv("GDX_VERIFY_MIN"))
         if (atoi(vm) > 0) idx->dev.verify_min_remaining = (uint32_t)atoi(vm);
-    // count: also finish intervals of up to this many rows by text comparisons (A/B: profiles/README.md)
-    if (const char *vr = getenv("GDX_VERIFY_ROWS"))
-        if (atoi(vr) > 0) idx->dev.verify_max_rows = (uint32_t)std::min(atoi(vr), 64);
     return GDX_OK;
 }
 
@@ -1841,16 +1817,7 @@ struct SortPlan {
     size_t tmp_bytes = 0;
     uint64_t total_bytes = 0;  // keys a/b + idx a/b + cub temp, 256 B aligned pieces
     bool use = false;
-    bool bucket = false;       // one-pass bucket grouping instead of the radix sort
 };
-
-bool bucket_mode() {
-    static const bool on = [] {
-        const char *e = getenv("GDX_SORT_MODE");
-        return e && strcmp(e, "bucket") == 0;
-    }();
-    return on;
-}
 
 // fixed_len: length of every query of the batch, 0 = variable
 SortPlan plan_sort(const gdx_index *idx, uint64_t nq, uint64_t fixed_len) {
@@ -1870,13 +1837,6 @@ SortPlan plan_sort(const gdx_index *idx, uint64_t nq, uint64_t fixed_len) {
     uint32_t bits = 1;
     while ((1u << bits) < idx->h.ns) ++bits;
     p.key_bits = bits;
-    if (bucket_mode() && bits <= kBucketBits) {
-        p.key_syms = kBucketBits / bits;
-        p.bucket = true;
-        p.total_bytes = 2 * align_up(nq * 4, 256) + align_up(kNumBuckets * 4, 256);  // keys, perm, histogram
-        p.use = true;
-        return p;
-    }
     p.key_syms = std::min<uint32_t>(32 / bits, 12);  // DNA: 24-bit keys = 3 radix passes, 4^12 > any batch
     cub::DoubleBuffer<uint32_t> dk(nullptr, nullptr), dv(nullptr, nullptr);
     if (cub::DeviceRadixSort::SortPairs(nullptr, p.tmp_bytes, dk, dv, (int64_t)nq, 0, (int)(p.key_bits * p.key_syms)) !=
@@ -1892,17 +1852,6 @@ gdx_status sort_queries(const gdx_index *idx, const DevQueries &dq, const SortPl
                         cudaStream_t stream, const uint32_t **perm) {
     uint8_t *base = (uint8_t *)scratch;
     const uint64_t piece = align_up(dq.nq * 4, 256);
-    if (p.bucket) {
-        uint32_t *keys = (uint32_t *)base, *out = (uint32_t *)(base + piece), *hist = (uint32_t *)(base + 2 * piece);
-        const unsigned grid = (unsigned)div_up(dq.nq, 256);
-        CUDA_TRY(cudaMemsetAsync(hist, 0, kNumBuckets * 4, stream));
-        k_bucket_count<<<grid, 256, 0, stream>>>(idx->dev, dq, p.key_bits, p.key_syms, keys, hist);
-        k_bucket_scan<<<1, 1024, 0, stream>>>(hist);
-        k_bucket_scatter<<<grid, 256, 0, stream>>>(keys, dq.nq, hist, out);
-        CUDA_TRY(cudaGetLastError());
-        *perm = out;
-        return GDX_OK;
-    }
     uint32_t *ka = (uint32_t *)base, *kb = (uint32_t *)(base + piece), *ia = (uint32_t *)(base + 2 * piece),
              *ib = (uint32_t *)(base + 3 * piece);
     void *tmp = base + 4 * piece;
@@ -1953,13 +1902,11 @@ void release_pinned_hits(const gdx_index *idx, void *p);
 
 // K3 + K4 over `n_hits` rows.  With a sampled suffix array (walks of geometric length) the compacting kernel
 // keeps every lane busy; with the dense array (one load per row) the plain one-thread-per-hit kernel is the
-// shorter program.  GDX_LOCATE_COMPACT=0/1 forces either for A/B runs.
+// shorter program.
 template <class L>
 void launch_locate_walk(const gdx_index *idx, const uint64_t *rows, uint64_t n_hits, ulonglong2 *hits,
                         unsigned long long *d_walk, cudaStream_t stream, bool hit32 = false) {
-    static const int forced = getenv("GDX_LOCATE_COMPACT") ? atoi(getenv("GDX_LOCATE_COMPACT")) : -1;
-    const bool compacting = forced >= 0 ? forced != 0 : idx->dev.sampling_rate > 1;
-    if (compacting)
+    if (idx->dev.sampling_rate > 1)
         k_locate_walk_compact<L><<<(unsigned)div_up(n_hits, kWalkSlice), 256, 0, stream>>>(idx->dev, rows, n_hits, hits, d_walk,
                                                                                            hit32 ? 1 : 0);
     else
@@ -2111,10 +2058,10 @@ struct LocatePipe {
 };
 
 // Chunked pipeline over kSlots streams: stage / pack -> H2D(queries) -> k_search -> D2H(results) per chunk.
-// If dev_a/dev_b are given the results stay on the device (locate path) and nothing is copied back.
+// With lp (locate, mode 2) the results stay on the device and every chunk continues in the LocatePipe.
 // out_elem: bytes per element of the caller's result arrays (8, or 4 for the *_u32 entry points).
 gdx_status search_host(const gdx_index *idx, Workspace *ws, const gdx_queries *qs, void *out_a_v, void *out_b_v,
-                       uint32_t out_elem, int mode, uint64_t *dev_a, uint64_t *dev_b, LocatePipe *lp = nullptr) {
+                       uint32_t out_elem, int mode, LocatePipe *lp = nullptr) {
     const uint64_t nq = qs->nq;
     uint8_t *out_a = (uint8_t *)out_a_v, *out_b = (uint8_t *)out_b_v;
     for (int s = 0; s < kSlots; ++s) ws->slot[s].ev_used = ws->slot[s].ev_loc_used = 0;
@@ -2150,10 +2097,7 @@ gdx_status search_host(const gdx_index *idx, Workspace *ws, const gdx_queries *q
     // t_pack), a raw chunk is put on the link that is just large enough to keep it busy for that long on top of
     // what is still queued there.  The queue is observed (events behind every upload), so a wrong guess of
     // either rate corrects itself: too much raw data -> the backlog grows -> the next raw chunks shrink.
-    // GDX_PACK_HYBRID=0: every chunk is packed.  GDX_LINK_GBS: initial guess of the link rate (default 50).
-    static const bool hybrid_enabled = env_flag("GDX_PACK_HYBRID", true);
-    static const double link_guess = (double)env_bytes("GDX_LINK_GBS", 50) * 1e6;  // bytes per ms
-    const bool hybrid = pack_on && src_pinned && hybrid_enabled;
+    const bool hybrid = pack_on && src_pinned;
     struct Upload {
         int slot;
         uint64_t bytes;
@@ -2172,7 +2116,7 @@ gdx_status search_host(const gdx_index *idx, Workspace *ws, const gdx_queries *q
     uint64_t raw_want = kChunkFirst;
 
     const bool stage_off = nq && qs->offsets && nq * 8 >= kStageMinBytes && !is_pinned(qs->offsets);
-    const bool to_host = nq && !dev_a && !lp;
+    const bool to_host = nq && !lp;
     const bool large_out = nq * 8 >= kStageMinBytes;
     // results as uint32 on the device: always for the u32 entry points, for large batches of the u64 ones
     // (widened by the pool while they are handed to the caller)
@@ -2213,7 +2157,7 @@ gdx_status search_host(const gdx_index *idx, Workspace *ws, const gdx_queries *q
             CUDA_TRY(sl.bytes.reserve(max_sym));
             if (pack_on) CUDA_TRY(sl.h_in.reserve(max_sym / 4 + 8));
             else if (stage_in) CUDA_TRY(sl.h_in.reserve(std::min<uint64_t>(total_in, kChunkMax) + 64));
-            if (max_q && !dev_a) {
+            if (max_q) {
                 CUDA_TRY(sl.out_a.reserve(max_q * 8));
                 if (mode == 0 || lp) CUDA_TRY(sl.out_b.reserve(max_q * 8));
                 if (stage_out) {
@@ -2261,7 +2205,7 @@ gdx_status search_host(const gdx_index *idx, Workspace *ws, const gdx_queries *q
         // growing a slot buffer frees the old one: only safe once the slot's stream has drained
         const uint64_t in_cap = nsym + 64;  // enough for either representation of the chunk
         if (sl.bytes.cap < in_cap || (qs->offsets && sl.offsets.cap < (cq + 1) * 8) ||
-            (!dev_a && (sl.out_a.cap < cq * 8 || ((mode == 0 || lp) && sl.out_b.cap < cq * 8))) ||
+            sl.out_a.cap < cq * 8 || ((mode == 0 || lp) && sl.out_b.cap < cq * 8) ||
             (sp.use && sl.sort.cap < sp.total_bytes))
             CUDA_TRY(cudaStreamSynchronize(sl.stream));
         CUDA_TRY(sl.bytes.reserve(in_cap));
@@ -2431,7 +2375,7 @@ gdx_status search_host(const gdx_index *idx, Workspace *ws, const gdx_queries *q
                 // how long will the pool need for the next packed chunk, and will the link last that long?
                 const double t_pack = (double)(budget * 4) / pack_rate;
                 const double have = (double)link_backlog();
-                const double need = t_pack * link_guess;
+                const double need = t_pack * kLinkGuessBytesPerMs;
                 raw_next = pack_on && need - have >= (double)(2ull << 20);
                 raw_want = raw_next ? std::min<uint64_t>((uint64_t)(need - have), 4 * kChunkMax) : 0;
             } else {
@@ -2439,18 +2383,11 @@ gdx_status search_host(const gdx_index *idx, Workspace *ws, const gdx_queries *q
             }
         }
 
-        uint64_t *a, *b;
-        if (dev_a) {
-            a = dev_a + q0;
-            b = dev_b ? dev_b + q0 : nullptr;
-        } else {
-            CUDA_TRY(sl.out_a.reserve(cq * 8));
-            a = sl.out_a.as<uint64_t>();
-            b = nullptr;
-            if (mode == 0 || lp) {
-                CUDA_TRY(sl.out_b.reserve(cq * 8));
-                b = sl.out_b.as<uint64_t>();
-            }
+        CUDA_TRY(sl.out_a.reserve(cq * 8));
+        uint64_t *a = sl.out_a.as<uint64_t>(), *b = nullptr;
+        if (mode == 0 || lp) {
+            CUDA_TRY(sl.out_b.reserve(cq * 8));
+            b = sl.out_b.as<uint64_t>();
         }
         if (used_staging) {
             CUDA_TRY(cudaEventRecord(sl.ev_h2d, sl.stream));
@@ -2493,7 +2430,7 @@ gdx_status search_host(const gdx_index *idx, Workspace *ws, const gdx_queries *q
             pend_out = PendingOut{k % kSlots, q0, cq, true};
             d2h_bytes += cq * dev_elem * (mode == 0 ? 2 : 1);
             GDX_TRY(finish_out(prev));
-        } else if (!dev_a) {
+        } else {
             d2h_bytes += cq * out_elem * (mode == 0 ? 2 : 1);
             CUDA_TRY(cudaMemcpyAsync(out_a + q0 * out_elem, a, cq * out_elem, cudaMemcpyDeviceToHost, sl.stream));
             if (mode == 0) CUDA_TRY(cudaMemcpyAsync(out_b + q0 * out_elem, b, cq * out_elem, cudaMemcpyDeviceToHost, sl.stream));
@@ -2673,13 +2610,13 @@ gdx_status acquire_pinned_hits(const gdx_index *idx, uint64_t bytes, void **out,
 }
 
 gdx_status finish_locate(const gdx_index *idx, Workspace *ws, uint64_t n, uint64_t total, uint64_t *hit_offsets,
-                         gdx_hit **hits, uint64_t *num_hits, bool write_last = true) {
+                         gdx_hit **hits, uint64_t *num_hits) {
     cudaStream_t st = ws->slot[0].stream;
     void *h = nullptr;
     GDX_TRY(acquire_pinned_hits(idx, total * sizeof(gdx_hit), &h));
     const gdx_status copied = [&]() -> gdx_status {
         if (total) CUDA_TRY(cudaMemcpyAsync(h, ws->hits.p, total * sizeof(gdx_hit), cudaMemcpyDeviceToHost, st));
-        CUDA_TRY(cudaMemcpyAsync(hit_offsets, ws->hit_offsets.p, (n + (write_last ? 1 : 0)) * 8, cudaMemcpyDeviceToHost, st));
+        CUDA_TRY(cudaMemcpyAsync(hit_offsets, ws->hit_offsets.p, (n + 1) * 8, cudaMemcpyDeviceToHost, st));
         CUDA_TRY(cudaMemcpyAsync(ws->small.h, ws->small.d, 16 * sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
         CUDA_TRY(cudaStreamSynchronize(st));
         return GDX_OK;
@@ -2722,7 +2659,7 @@ gdx_status search_many_impl(const gdx_index *idx, const gdx_queries *queries, vo
     DeviceGuard guard(idx->device);
     WsLease lease(idx);
     if (!lease.w) return fail(GDX_ERR_CUDA, "could not create a CUDA workspace: %s", cudaGetErrorString(cudaGetLastError()));
-    const gdx_status st = search_host(idx, lease.w, queries, a, b, elem, mode, nullptr, nullptr);
+    const gdx_status st = search_host(idx, lease.w, queries, a, b, elem, mode);
     if (st != GDX_OK) drain(lease.w);  // copies into the caller's arrays may still be in flight
     return st;
 }
@@ -2744,36 +2681,23 @@ gdx_status locate_many_impl(const gdx_index *idx, const gdx_queries *queries, ui
     Workspace *ws = lease.w;
     if (!ws) return fail(GDX_ERR_CUDA, "could not create a CUDA workspace: %s", cudaGetErrorString(cudaGetLastError()));
     const uint64_t n = queries->nq;
-    static const bool pipelined_env = !(getenv("GDX_LOCATE_PIPELINE") && atoi(getenv("GDX_LOCATE_PIPELINE")) == 0);
-    const bool pipelined = pipelined_env || hit_counts;  // (the compact form exists in the pipelined path only)
-    if (pipelined) {
-        // every chunk of the search pipeline carries on with counts -> scan -> expand -> walk -> D2H
-        LocatePipe lp{idx, ws, hit_offsets};
-        lp.hit_counts = hit_counts;
-        lp.hit_bytes = hit_counts ? 8 : sizeof(gdx_hit);
-        lp.stage_offsets = n * 8 >= kStageMinBytes && !is_pinned(hit_counts ? (const void *)hit_counts : (const void *)hit_offsets);
-        GDX_TRY(acquire_pinned_hits(idx, std::max<uint64_t>(n, 4096) * lp.hit_bytes, &lp.pinned, &lp.pinned_cap));
-        gdx_status st = search_host(idx, ws, queries, nullptr, nullptr, 8, 2, nullptr, nullptr, &lp);
-        if (st != GDX_OK) {
-            drain(ws);
-            release_pinned_hits(idx, lp.pinned);
-            return st;
-        }
-        if (write_last && hit_offsets) hit_offsets[n] = lp.total;
-        t_stats.hits = lp.total;
-        *hits = (gdx_hit *)lp.pinned;
-        *num_hits = lp.total;
-        return GDX_OK;
+    // every chunk of the search pipeline carries on with counts -> scan -> expand -> walk -> D2H
+    LocatePipe lp{idx, ws, hit_offsets};
+    lp.hit_counts = hit_counts;
+    lp.hit_bytes = hit_counts ? 8 : sizeof(gdx_hit);
+    lp.stage_offsets = n * 8 >= kStageMinBytes && !is_pinned(hit_counts ? (const void *)hit_counts : (const void *)hit_offsets);
+    GDX_TRY(acquire_pinned_hits(idx, std::max<uint64_t>(n, 4096) * lp.hit_bytes, &lp.pinned, &lp.pinned_cap));
+    gdx_status st = search_host(idx, ws, queries, nullptr, nullptr, 8, 2, &lp);
+    if (st != GDX_OK) {
+        drain(ws);
+        release_pinned_hits(idx, lp.pinned);
+        return st;
     }
-    // a buffer may only be replaced once nothing in flight uses it: every call ends synchronized
-    CUDA_TRY(ws->starts.reserve((n + 1) * 8));
-    CUDA_TRY(ws->ends.reserve((n + 1) * 8));
-    gdx_status st = search_host(idx, ws, queries, nullptr, nullptr, 8, 2, ws->starts.as<uint64_t>(), ws->ends.as<uint64_t>());
-    uint64_t total = 0;
-    if (st == GDX_OK) st = locate_device_intervals(idx, ws, ws->starts.as<uint64_t>(), ws->ends.as<uint64_t>(), n, &total);
-    if (st == GDX_OK) st = finish_locate(idx, ws, n, total, hit_offsets, hits, num_hits, write_last);
-    if (st != GDX_OK) drain(ws);
-    return st;
+    if (write_last && hit_offsets) hit_offsets[n] = lp.total;
+    t_stats.hits = lp.total;
+    *hits = (gdx_hit *)lp.pinned;
+    *num_hits = lp.total;
+    return GDX_OK;
 }
 
 }  // namespace

@@ -77,7 +77,6 @@ struct DevIndex {
     uint32_t verify_min_remaining;  // text verification needs at least this many symbols left (8; 4 with the dense suffix array)
     uint32_t isa_rate;              // sampling rate of the inverse samples (= the configured rate)
     uint32_t seed_depth;
-    uint32_t verify_max_rows;       // count: intervals of up to this many rows are finished by text comparisons (1 = one row only)
     uint64_t lut_level_off[kMaxLookupDepth + 1];
     uint64_t lut_pow[kMaxLookupDepth + 1];
     uint8_t io_to_dense[256];
@@ -114,7 +113,6 @@ inline DevIndex make_dev_index(const ImageHeader &h, const void *image) {
     d.seed_lookup = nullptr;
     d.seed_depth = 0;
     d.row_context = nullptr;
-    d.verify_max_rows = 1;
     if ((h.sampling_rate & (h.sampling_rate - 1)) == 0) {
         uint32_t s = 0;
         while ((1u << s) < h.sampling_rate) ++s;

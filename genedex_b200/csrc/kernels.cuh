@@ -42,16 +42,6 @@
 #include "device_index.h"
 #include "row_context.h"
 
-#ifndef GDX_MULTIROW
-#define GDX_MULTIROW 0
-#endif
-#ifndef GDX_KG5_VERIFY_MIN_BLOCKS
-#define GDX_KG5_VERIFY_MIN_BLOCKS 5
-#endif
-#ifndef GDX_K32_VERIFY_MIN_BLOCKS
-#define GDX_K32_VERIFY_MIN_BLOCKS 6
-#endif
-
 namespace gdx {
 
 struct DevQueries {
@@ -156,7 +146,7 @@ __device__ __forceinline__ void ldg128_na(const void *p, uint64_t &lo, uint64_t 
 struct K32 {
     static constexpr uint32_t kLog2P = 6;
     static constexpr int kSearchMinBlocks = 6;  // 40 registers: 1536 threads per SM
-    static constexpr int kVerifyMinBlocks = GDX_K32_VERIFY_MIN_BLOCKS;
+    static constexpr int kVerifyMinBlocks = 6;
     struct Planes {
         uint64_t w[4];
     };
@@ -216,7 +206,7 @@ struct KG {
     static constexpr uint32_t kLog2P = 7;
     static constexpr int kPlanes = B;
     static constexpr int kSearchMinBlocks = B <= 3 ? 5 : (B <= 5 ? 5 : 3);
-    static constexpr int kVerifyMinBlocks = B <= 3 ? 5 : (B <= 5 ? GDX_KG5_VERIFY_MIN_BLOCKS : 3);
+    static constexpr int kVerifyMinBlocks = B <= 5 ? 5 : 3;
     // The record is fetched as whole 32 B sectors: kSectors 256-bit loads cover the B planes (16 B each) and the
     // first u16 offsets behind them; an offset further back costs one more 2-byte load from the same line.
     // (Protein, B = 5: 3 sector requests instead of five 128-bit ones + the offset -- the random-access ceiling
@@ -296,9 +286,6 @@ struct KG {
 };
 
 __device__ __forceinline__ uint64_t sbc_load(const DevIndex &ix, uint64_t i, uint32_t c) {
-#ifdef GDX_EXP_FAKE_SBC  // experiment only (wrong results): same access pattern without the superblock load
-    return (i >> kSuperblockLog2) << kSuperblockLog2;
-#endif
     return __ldg(ix.sbc + (i >> kSuperblockLog2) * ix.noff + (c - 1));
 }
 
@@ -569,51 +556,6 @@ k_query_keys(const __grid_constant__ DevIndex ix, const DevQueries qs, uint32_t 
     idx[q] = (uint32_t)q;
 }
 
-// ---- one-pass bucket grouping (alternative to the full radix sort) -----------------------------------
-// For L2 sharing it is enough that queries with the same suffix are searched at about the same time:
-// group the batch by a 16-bit key (the last 8 symbols of a DNA query) with one counting-sort pass --
-// histogram, scan over the 65 536 buckets, unordered scatter -- instead of three radix passes.
-constexpr uint32_t kBucketBits = 16;
-constexpr uint32_t kNumBuckets = 1u << kBucketBits;
-
-__global__ void __launch_bounds__(256)
-k_bucket_count(const __grid_constant__ DevIndex ix, const DevQueries qs, uint32_t key_bits, uint32_t key_syms,
-               uint32_t *__restrict__ keys, uint32_t *__restrict__ hist) {
-    const uint64_t q = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (q >= qs.nq) return;
-    const uint32_t key = query_sort_key(ix, qs, q, key_bits, key_syms);
-    keys[q] = key;
-    atomicAdd(hist + key, 1u);
-}
-
-// exclusive scan of the 65 536 bucket counts: one CTA of 1024 threads, 64 buckets per thread
-__global__ void __launch_bounds__(1024) k_bucket_scan(uint32_t *__restrict__ hist) {
-    using Scan = cub::BlockScan<uint32_t, 1024>;
-    __shared__ typename Scan::TempStorage tmp;
-    constexpr uint32_t per = kNumBuckets / 1024;
-    uint32_t local[per], sum = 0;
-#pragma unroll
-    for (uint32_t j = 0; j < per; ++j) {
-        local[j] = hist[threadIdx.x * per + j];
-        sum += local[j];
-    }
-    uint32_t base;
-    Scan(tmp).ExclusiveSum(sum, base);
-#pragma unroll
-    for (uint32_t j = 0; j < per; ++j) {
-        hist[threadIdx.x * per + j] = base;
-        base += local[j];
-    }
-}
-
-__global__ void __launch_bounds__(256)
-k_bucket_scatter(const uint32_t *__restrict__ keys, uint64_t nq, uint32_t *__restrict__ cursor,
-                 uint32_t *__restrict__ perm) {
-    const uint64_t q = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (q >= nq) return;
-    perm[atomicAdd(cursor + keys[q], 1u)] = (uint32_t)q;
-}
-
 // ---- K1 + K2: seed + backward search ----------------------------------------------------------------
 // mode 0: out_a = starts, out_b = ends; mode 1: out_a = counts.
 // Follows the batched path of the reference: a symbol is translated only when the search reaches
@@ -772,37 +714,6 @@ k_search(const __grid_constant__ DevIndex ix, const DevQueries qs, uint64_t *__r
         while (!bad && pos > 0 && s != e) {
             // mode 0 (cursors) must also produce the interval: possible with the sampled inverse suffix
             // array once at least sampling_rate symbols have matched (the ISA walk stays inside them)
-#if GDX_MULTIROW
-            // (A/B variant, tools/build_variant.sh multirow -DGDX_MULTIROW=1; measured in profiles/README.md)
-            // count only (mode 1): an interval of a few rows is finished the same way, one text comparison per
-            // candidate row (adjacent SA entries share a line); the count is the number of candidates that match,
-            // and an invalid symbol is reached exactly when some candidate matches up to it (cursor.rs:40-51)
-            if (VERIFY && !CURSORS && mode == 1 && e - s > 1 && e - s <= ix.verify_max_rows &&
-                pos >= (uint64_t)ix.verify_min_remaining * (e - s)) {
-                uint32_t matches = 0;
-                for (uint64_t r = s; r < e; ++r) {
-                    const uint64_t at = resolve_row<L>(ix, r, vsteps);
-                    uint64_t jm = 0;
-                    uint32_t cm = 0;
-                    int cmp;
-                    if constexpr (PACKED) {
-                        cmp = ix.text_bits == 4
-                                  ? compare_with_text<4, false>(ix, PackedQueryWords<4>{ptail, qs.packed, begin, tail_begin}, pos, at, jm, cm)
-                                  : compare_with_text<8, false>(ix, PackedQueryWords<8>{ptail, qs.packed, begin, tail_begin}, pos, at, jm, cm);
-                    } else {
-                        cmp = ix.text_bits == 4
-                                  ? compare_with_text<4, true>(ix, ByteQueryWords<4>{tab, sbytes, p, tail_begin}, pos, at, jm, cm)
-                                  : compare_with_text<8, true>(ix, ByteQueryWords<8>{tab, sbytes, p, tail_begin}, pos, at, jm, cm);
-                    }
-                    matches += cmp == 0;
-                    bad |= cmp == 2;
-                }
-                vrows = (uint32_t)(e - s);
-                s = 0;
-                e = matches;
-                break;
-            }
-#endif
             if (VERIFY && e - s == 1 && pos >= ix.verify_min_remaining &&
                 (!CURSORS || len - pos >= ix.isa_rate)) {
                 // one candidate row: SA[s] is where query[pos..len) occurs; compare query[0..pos)

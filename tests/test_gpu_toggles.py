@@ -12,10 +12,9 @@ pytestmark = pytest.mark.gpu
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 TOGGLES = [
-    {"GDX_SORT_MODE": "bucket", "GDX_LOCATE_PIPELINE": "0", "GDX_L2_PERSIST": "0"},
     {"GDX_VERIFY": "0", "GDX_SORT_QUERIES": "0", "GDX_DENSE_SA": "0", "GDX_SEED_TABLE": "0", "GDX_CHUNK_FIRST_MB": "1", "GDX_CHUNK_MAX_MB": "2",
      "GDX_CHUNK_TAIL_MB": "1"},
-    {"GDX_FORCE_WIDE": "1", "GDX_VERIFY_MIN": "2", "GDX_CHUNK_MAX_MB": "256", "GDX_L2_FETCH_GRANULARITY": "0"},
+    {"GDX_FORCE_WIDE": "1", "GDX_VERIFY_MIN": "2", "GDX_CHUNK_MAX_MB": "256"},
     # every batch, however small, takes the host packer + packed kernel + staged uint32 results
     {"GDX_PACK_MIN_BYTES": "0", "GDX_STAGE_MIN_BYTES": "0", "GDX_CHUNK_FIRST_MB": "1", "GDX_CHUNK_MAX_MB": "1"},
     {"GDX_PACK_MIN_BYTES": "0", "GDX_STAGE_MIN_BYTES": "0", "GDX_VERIFY": "0", "GDX_SEED_TABLE": "0", "GDX_HOST_THREADS": "3",
@@ -25,7 +24,7 @@ TOGGLES = [
 ]
 
 
-@pytest.mark.parametrize("env", TOGGLES, ids=["bucket-nopipe-nohints", "lfonly-nosort-smallchunks", "wide-verifymin2", "pack-everything",
+@pytest.mark.parametrize("env", TOGGLES, ids=["lfonly-nosort-smallchunks", "wide-verifymin2", "pack-everything",
                               "pack-everything-lfonly-scalar", "no-pack-no-narrow"])
 def test_parity_under_toggles(env):
     e = dict(os.environ)
