@@ -54,8 +54,9 @@ struct DevQueries {
     uint64_t shift;           // added to the start of every query (a packed chunk need not start on a byte boundary)
     // 2-bit packed form (alphabets with <= 4 searchable symbols): symbol i of the batch (the same index
     // that addresses `bytes`) sits at bits [2i, 2i+2) of this little-endian word stream, code = dense - 1.
-    // Every symbol of a packed batch is searchable by construction (the host packer routes queries with
-    // any other byte to the IO-byte kernel), so the packed kernel has no invalid-symbol path.
+    // The host packer routes queries with any other byte to the IO-byte kernel, so its batches hold searchable
+    // symbols only.  A caller's pre-packed batch of an alphabet with fewer than 4 searchable symbols can hold
+    // codes >= ns: k_search checks those queries in full before it searches them (packed_query_unsearchable).
     const uint32_t *packed;
     // number of symbols the stream holds (host pipeline: the chunk that was uploaded; ~0 = unknown): a query whose
     // offsets point outside is reported instead of read -- offsets are caller data and not checked on the host
@@ -112,6 +113,17 @@ __device__ __forceinline__ uint64_t tail_bits(const PackedTail &t, uint32_t sym,
 }
 __device__ __forceinline__ uint32_t tail_code(const PackedTail &t, uint32_t sym) {
     return (uint32_t)((sym < 32 ? t.lo : t.hi) >> ((sym & 31u) * 2)) & 3u;
+}
+// true if a symbol of the packed query [begin, begin + tail_begin + tail) is not searchable; `t` holds its last `tail`
+// symbols.  Looks at the whole query, whatever part of it the search would reach.
+__device__ __noinline__ bool packed_query_unsearchable(const uint32_t *pk, uint64_t begin, uint64_t tail_begin,
+                                                       PackedTail t, uint32_t tail, uint32_t ns) {
+    if (packed_codes_unsearchable(t, tail, ns)) return true;
+    for (uint64_t j0 = 0; j0 < tail_begin; j0 += 64) {
+        const uint32_t nsym = tail_begin - j0 < 64 ? (uint32_t)(tail_begin - j0) : 64u;
+        if (packed_codes_unsearchable(load_packed_tail(pk, begin + j0, nsym), nsym, ns)) return true;
+    }
+    return false;
 }
 // 16 2-bit codes -> 16 nibbles holding dense symbols (code + 1); 8 codes -> 8 bytes
 __device__ __forceinline__ uint64_t expand_codes_4(uint64_t x) {
@@ -577,7 +589,7 @@ constexpr uint32_t kQuerySlotWords = kQueryStage / 4 + 1;  // 17: odd stride, co
 // CURSORS (mode 0 with VERIFY): compile the inverse-sample path only into the variant that needs it
 // PACKED: the batch is a 2-bit packed stream (DevQueries::packed); the last 64 symbols of a query are held
 // in two registers (no shared-memory staging, no translate table), lookup indices are bit-field extracts
-// when ns == 4, and there is no invalid-symbol path.
+// when ns == 4, and the only invalid symbols are codes >= ns (ns < 4), refused before the search starts.
 // slot_map (optional): the result of query q goes to slot slot_map[q] (queries re-run through the IO-byte
 // kernel because they hold a byte the packer cannot encode); errors are reported for that slot.
 // out_bits: 64 or 32 (narrow results for texts shorter than 2^32: half the D2H bytes).
@@ -626,8 +638,13 @@ k_search(const __grid_constant__ DevIndex ix, const DevQueries qs, uint64_t *__r
         PackedTail ptail = {0, 0};
         const uint8_t *sbytes = nullptr;
         bool coded = PACKED;  // the staged symbols are held as 2-bit codes in ptail
+        bool bad = false;
         if constexpr (PACKED) {
             if (tail) ptail = load_packed_tail(qs.packed, begin + tail_begin, tail);
+            // With fewer than 4 searchable symbols a caller's pre-packed batch can hold a code that is none: it would
+            // index the lookup / seed tables and the rank tables out of range.  Refused as an invalid symbol, whether or
+            // not the search would reach it (a packed batch has no lazy reference behaviour to keep).
+            if (ix.ns < 4 && tail) bad = packed_query_unsearchable(qs.packed, begin, tail_begin, ptail, tail, ix.ns);
         } else {
             // aligned words covering bytes [len - tail, len), global -> shared without a register round
             // trip: all words of the query are in flight at once
@@ -676,7 +693,6 @@ k_search(const __grid_constant__ DevIndex ix, const DevQueries qs, uint64_t *__r
             }
             return li;
         };
-        bool bad = false;
 
         // K1: lookup_table.rs:68-161
         const uint32_t depth = len < ix.lookup_depth ? (uint32_t)len : ix.lookup_depth;
@@ -688,7 +704,7 @@ k_search(const __grid_constant__ DevIndex ix, const DevQueries qs, uint64_t *__r
         // symbols are searchable; anything else (invalid byte, `N`, short query) takes the configured path,
         // which keeps the reference's lazy panic and the documented deviation where they were.
         bool seeded = false;
-        if (ix.seed_lookup && len >= ix.seed_depth) {
+        if (!bad && ix.seed_lookup && len >= ix.seed_depth) {
             const uint64_t p0 = len - ix.seed_depth;
             bool ok = true;
             const uint64_t li = lookup_index(p0, ix.seed_depth, ok);
@@ -703,7 +719,7 @@ k_search(const __grid_constant__ DevIndex ix, const DevQueries qs, uint64_t *__r
             // reference mis-indexes its table here (lookup_table.rs:154-157) -- documented deviation.
             bool ok = true;
             const uint64_t li = lookup_index(pos, depth, ok);
-            bad = !ok || broken;
+            bad = bad || !ok || broken;
             if (!bad) lut_load(ix, ix.lut_level_off[depth] + li, s, e);
         }
 

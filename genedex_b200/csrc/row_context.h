@@ -113,6 +113,21 @@ GDX_HD bool codes_from_staged(const uint16_t *tab2, const uint32_t *slot, uint32
     return (flags >> 8) == 0;
 }
 
+// true if one of the first nsym (<= 64) codes of t is >= ns, i.e. not a searchable symbol (dense = code + 1 > ns).
+// A caller's pre-packed batch can hold such codes when the alphabet has fewer than 4 searchable symbols; every code
+// is searchable when ns >= 4.  Codes past nsym are ignored.
+GDX_HD bool packed_codes_unsearchable(const PackedTail &t, uint32_t nsym, uint32_t ns) {
+    if (ns >= 4 || nsym == 0) return false;
+    const uint64_t ml = nsym >= 32 ? ~0ull : (1ull << (2 * nsym)) - 1ull;
+    const uint64_t mh = nsym >= 64 ? ~0ull : (nsym > 32 ? (1ull << (2 * (nsym - 32))) - 1ull : 0ull);
+    // bit 2j of a word is set if code j of it is out of range: ns 1 -> code != 0, 2 -> high bit, 3 -> both bits
+    auto out = [ns](uint64_t x) {
+        const uint64_t lo = x & 0x5555555555555555ull, hi = (x >> 1) & 0x5555555555555555ull;
+        return ns == 1 ? (lo | hi) : (ns == 2 ? hi : (lo & hi));
+    };
+    return ((out(t.lo) & ml) | (out(t.hi) & mh)) != 0;
+}
+
 // tab2 of codes_from_staged from the alphabet's translation table
 GDX_HD uint16_t ctx_tab2_entry(uint32_t dense, uint32_t ns) { return (uint16_t)((dense >= 1 && dense <= ns) ? dense - 1 : 0x100u); }
 

@@ -111,7 +111,9 @@ typedef enum gdx_query_encoding {
     GDX_QUERIES_IO_BYTES = 0,
     /* 2 bits per symbol, code = dense symbol - 1, symbol k of the batch at bits [2(k%4), 2(k%4)+2) of byte k/4.
      * Only for alphabets with at most 4 searchable symbols (every DNA alphabet, alphabet.rs:251-300) and only
-     * for batches made of searchable symbols (gdx_pack_queries checks that).  A quarter of the PCIe bytes:
+     * for batches made of searchable symbols (gdx_pack_queries checks that).  With fewer than 4 searchable
+     * symbols, a query holding a code >= the number of searchable symbols fails the call with
+     * GDX_ERR_INVALID_SYMBOL, wherever in the query the code sits.  A quarter of the PCIe bytes:
      * for callers that keep their reads packed.  IO-byte batches are packed by the library itself while it
      * stages them (see gdx_count_many). */
     GDX_QUERIES_PACKED_2BIT = 1

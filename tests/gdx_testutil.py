@@ -6,16 +6,41 @@ import numpy as np
 from oracle import oracle as O
 
 
+def _pairs(letters: bytes):
+    return [bytes([c, c + 32]) for c in letters]
+
+
+# Alphabets built from groups of IO symbols (searchable groups first) and the number of groups that are not
+# searchable.  They reach the rank layouts and text widths the library's predefined alphabets leave out: at most
+# 4 searchable symbols with more than 6 dense ones (generic layout, packed kernel and row context table all on),
+# fewer than 4 searchable symbols on the 32-byte layout, and a searchable symbol whose rank is derived.
+SHAPES = {
+    # name: (groups, not searchable, rank_layout, rank_record_bytes, text bits)
+    "dna_rny": (_pairs(b"ACGTNRY"), 3, 1, 64, 4),                          # sigma 8, KG<3>
+    "dna_iupac_kept": (_pairs(b"ACGTNRYKMSWBDHV"), 11, 1, 96, 4),          # sigma 16, KG<4>
+    "dna_iupac_gaps": (_pairs(b"ACGTNRYKMSWBDHV") + [b"-", b"*", b"."], 14, 1, 128, 8),  # sigma 19, KG<5>
+    "u8_ns4": ([bytes([b]) for b in range(255)], 251, 1, 640, 8),         # sigma 256, KG<8>; byte 255 is invalid
+    "acg_n": (_pairs(b"ACGN"), 1, 0, 32, 4),                               # sigma 5, ns 3, K32
+    "dna_n_searchable": (_pairs(b"ACGTN"), 0, 0, 32, 4),                   # sigma 6, ns 5: K32 derives the rank of N
+}
+
+
 def product_alphabet(gdx, name):
     A = gdx.alphabet
     if name == "protein20":
         return gdx.Alphabet.from_io_symbols(b"ACDEFGHIKLMNPQRSTVWY", 0)
+    if name in SHAPES:
+        groups, k = SHAPES[name][:2]
+        return gdx.Alphabet.from_ambiguous_io_symbols(groups, k)
     if name.startswith("u8_until_"):
         return A.u8_until(int(name.split("_")[-1]))
     return getattr(A, name)()
 
 
 def oracle_alphabet(name):
+    if name in SHAPES:
+        groups, k = SHAPES[name][:2]
+        return O.OracleAlphabet(groups, k)
     if name.startswith("u8_until_"):
         return O.u8_until(int(name.split("_")[-1]))
     return O.ALPHABETS[name]()

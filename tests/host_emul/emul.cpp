@@ -189,3 +189,8 @@ extern "C" uint32_t emul_ctx_valid_len(const uint32_t *entry) {
     const CtxEntry en = {entry[0], entry[1], entry[2], entry[3]};
     return ctx_valid_len(en);
 }
+
+// the packed kernel's check of a caller's 2-bit codes: 1 if one of the first nsym codes of hi:lo is >= ns
+extern "C" int emul_packed_unsearchable(uint64_t lo, uint64_t hi, uint32_t nsym, uint32_t ns) {
+    return packed_codes_unsearchable(PackedTail{lo, hi}, nsym, ns) ? 1 : 0;
+}

@@ -443,6 +443,74 @@ def _ctx_lib(emul):
     return emul
 
 
+def _check_row_context_entries(lib, io_to_dense, ns, dense_to_io, text, rng):
+    """emul_ctx_entry / emul_code_query / emul_ctx_matches at every SA value of the first 120 and at 400 random ones,
+    against a symbol-by-symbol model.  dense_to_io[d] = an IO byte of searchable symbol d."""
+    entry = (C.c_uint32 * 4)()
+    lo, hi = C.c_uint64(), C.c_uint64()
+    searchable_io = [dense_to_io[d] for d in range(1, ns + 1)]
+    checked = 0
+    for at in list(range(0, 120)) + rng.integers(0, text.size, 400).tolist():
+        lib.emul_ctx_entry(text.ctypes.data, at, ns, entry)
+        assert entry[0] == at
+        # model of vl: searchable symbols directly in front of `at`, capped at 45
+        vl = 0
+        while vl < 45 and at - vl - 1 >= 0 and 1 <= text[at - vl - 1] <= ns:
+            vl += 1
+        assert lib.emul_ctx_valid_len(entry) == vl, at
+        for pos in range(1, vl + 1):
+            want = text[at - pos:at]
+            for variant in range(3):
+                q = want.copy()
+                if variant == 1:
+                    j = int(rng.integers(0, pos))
+                    q[j] = (q[j] % ns) + 1         # a different searchable symbol at one place (none if ns == 1)
+                elif variant == 2 and pos > 1:
+                    q[0] = (q[0] % ns) + 1         # the leftmost compared symbol (the last one the search reaches)
+                io = bytes(dense_to_io[int(c)] for c in q)
+                # the query may be longer than pos: the symbols right of pos were matched by the search already
+                extra = bytes(rng.choice(searchable_io) for _ in range(int(rng.integers(0, 64 - pos + 1))))
+                whole = np.frombuffer(io + extra, dtype=np.uint8)
+                mis = int(rng.integers(0, 4))
+                ok = lib.emul_code_query(io_to_dense.ctypes.data, ns, whole.ctypes.data, whole.size, mis,
+                                         int(rng.integers(0, 2 ** 31)), C.byref(lo), C.byref(hi))
+                assert ok == 1
+                got = lib.emul_ctx_matches(entry, pos, lo.value, hi.value)
+                assert got == int(np.array_equal(q, want)), (at, pos, variant)
+                checked += 1
+    return checked
+
+
+def _check_staged_coding(lib, io_to_dense, ns, letters, bad_bytes, rng):
+    """codes_from_staged for every length 1..64 and misalignment; letters = IO bytes of searchable symbols"""
+    lo, hi = C.c_uint64(), C.c_uint64()
+    for tail in range(1, 65):
+        for mis in range(4):
+            q = letters[rng.integers(0, letters.size, tail)].copy()
+            ok = lib.emul_code_query(io_to_dense.ctypes.data, ns, q.ctypes.data, tail, mis, int(rng.integers(0, 2 ** 31)),
+                                     C.byref(lo), C.byref(hi))
+            assert ok == 1
+            value = lo.value | (hi.value << 64)
+            want = sum((int(io_to_dense[b]) - 1) << (2 * j) for j, b in enumerate(q.tolist()))
+            assert value == want, (tail, mis)          # also: nothing set above the last symbol
+            for bad in bad_bytes:
+                q2 = q.copy()
+                q2[int(rng.integers(0, tail))] = bad
+                assert lib.emul_code_query(io_to_dense.ctypes.data, ns, q2.ctypes.data, tail, mis, 7,
+                                           C.byref(lo), C.byref(hi)) == 0, (tail, mis, bad)
+
+
+def _wide_io_table(rng, ns):
+    """IO byte -> dense symbol of a 256-symbol alphabet with ns searchable symbols: three IO bytes per searchable
+    symbol, eight invalid bytes, every other byte a symbol above ns.  -> (io_to_dense, dense_to_io)"""
+    perm = rng.permutation(256)
+    io_to_dense = rng.integers(ns + 1, 256, 256).astype(np.uint8)
+    for k, b in enumerate(perm[: 3 * ns]):
+        io_to_dense[b] = k % ns + 1
+    io_to_dense[perm[3 * ns: 3 * ns + 8]] = 0
+    return io_to_dense, {d: int(perm[d - 1]) for d in range(1, ns + 1)}
+
+
 def test_row_context_entry_and_comparison_equal_a_plain_model(emul):
     """The verification the kernel does from one 16-byte entry must say exactly what a symbol-by-symbol comparison of
     query[0..pos) with the text in front of SA[row] says, whenever the entry claims to cover pos symbols."""
@@ -461,38 +529,25 @@ def test_row_context_entry_and_comparison_equal_a_plain_model(emul):
         pieces += [t, np.zeros(1, np.uint8)]
     text = np.concatenate(pieces)
     dense_to_io = {1: ord("A"), 2: ord("C"), 3: ord("G"), 4: ord("T"), 5: ord("N")}
-    entry = (C.c_uint32 * 4)()
-    lo, hi = C.c_uint64(), C.c_uint64()
-    checked = 0
-    for at in list(range(0, 120)) + rng.integers(0, text.size, 400).tolist():
-        lib.emul_ctx_entry(text.ctypes.data, at, ns, entry)
-        assert entry[0] == at
-        # model of vl: searchable symbols directly in front of `at`, capped at 45
-        vl = 0
-        while vl < 45 and at - vl - 1 >= 0 and 1 <= text[at - vl - 1] <= ns:
-            vl += 1
-        assert lib.emul_ctx_valid_len(entry) == vl, at
-        for pos in range(1, vl + 1):
-            want = text[at - pos:at]
-            for variant in range(3):
-                q = want.copy()
-                if variant == 1:
-                    j = int(rng.integers(0, pos))
-                    q[j] = (q[j] % 4) + 1          # a different searchable symbol at one place
-                elif variant == 2 and pos > 1:
-                    q[0] = (q[0] % 4) + 1          # the leftmost compared symbol (the last one the search reaches)
-                io = bytes(dense_to_io[int(c)] for c in q)
-                # the query may be longer than pos: the symbols right of pos were matched by the search already
-                extra = bytes(rng.choice(list(b"ACGT")) for _ in range(int(rng.integers(0, 64 - pos + 1))))
-                whole = np.frombuffer(io + extra, dtype=np.uint8)
-                mis = int(rng.integers(0, 4))
-                ok = lib.emul_code_query(io_to_dense.ctypes.data, ns, whole.ctypes.data, whole.size, mis,
-                                         int(rng.integers(0, 2 ** 31)), C.byref(lo), C.byref(hi))
-                assert ok == 1
-                got = lib.emul_ctx_matches(entry, pos, lo.value, hi.value)
-                assert got == int(np.array_equal(q, want)), (at, pos, variant)
-                checked += 1
-    assert checked > 20_000
+    assert _check_row_context_entries(lib, io_to_dense, ns, dense_to_io, text, rng) > 20_000
+
+
+@pytest.mark.parametrize("ns", [1, 2, 3, 4])
+def test_row_context_entries_over_wide_dense_texts(emul, ns):
+    """The same for alphabets with 1..4 searchable symbols among 256 dense ones (the generic rank layout with 8-bit
+    text keeps the table on): every symbol above ns, whatever its value, must end the entry's context."""
+    lib = _ctx_lib(emul)
+    rng = np.random.default_rng(40 + ns)
+    io_to_dense, dense_to_io = _wide_io_table(rng, ns)
+    pieces = []
+    for m in (1, 2, 3, 44, 45, 46, 47, 90, 200, 1000):
+        t = rng.integers(1, ns + 1, m, dtype=np.uint8)
+        if m >= 44:
+            for s in rng.integers(0, m - 3, 1 + m // 60):
+                t[s:s + int(rng.integers(1, 4))] = rng.choice([ns + 1, 127, 128, 250, 255])  # also: the top bit set
+        pieces += [t, np.zeros(1, np.uint8)]
+    text = np.concatenate(pieces)
+    assert _check_row_context_entries(lib, io_to_dense, ns, dense_to_io, text, rng) > 5_000
 
 
 def test_coding_of_staged_byte_queries(emul):
@@ -502,20 +557,37 @@ def test_coding_of_staged_byte_queries(emul):
     rng = np.random.default_rng(4)
     oa = O.ALPHABETS["ascii_dna_with_n"]()
     io_to_dense = np.array(oa.io_to_dense, dtype=np.uint8)
-    ns = oa.num_searchable
-    lo, hi = C.c_uint64(), C.c_uint64()
-    letters = np.frombuffer(b"ACGTacgt", dtype=np.uint8)
-    for tail in range(1, 65):
-        for mis in range(4):
-            q = letters[rng.integers(0, 8, tail)].copy()
-            ok = lib.emul_code_query(io_to_dense.ctypes.data, ns, q.ctypes.data, tail, mis, int(rng.integers(0, 2 ** 31)),
-                                     C.byref(lo), C.byref(hi))
-            assert ok == 1
-            value = lo.value | (hi.value << 64)
-            want = sum((int(io_to_dense[b]) - 1) << (2 * j) for j, b in enumerate(q.tolist()))
-            assert value == want, (tail, mis)          # also: nothing set above the last symbol
-            for bad in (ord("N"), ord("n"), ord("x"), 0, 255):
-                q2 = q.copy()
-                q2[int(rng.integers(0, tail))] = bad
-                assert lib.emul_code_query(io_to_dense.ctypes.data, ns, q2.ctypes.data, tail, mis, 7,
-                                           C.byref(lo), C.byref(hi)) == 0
+    _check_staged_coding(lib, io_to_dense, oa.num_searchable, np.frombuffer(b"ACGTacgt", dtype=np.uint8),
+                         (ord("N"), ord("n"), ord("x"), 0, 255), rng)
+
+
+@pytest.mark.parametrize("ns", [1, 2, 3, 4])
+def test_coding_of_staged_byte_queries_for_every_small_ns(emul, ns):
+    """The same with 1..4 searchable symbols, where most IO bytes are valid symbols that are not searchable"""
+    lib = _ctx_lib(emul)
+    rng = np.random.default_rng(70 + ns)
+    io_to_dense, _ = _wide_io_table(rng, ns)
+    letters = np.flatnonzero((io_to_dense >= 1) & (io_to_dense <= ns)).astype(np.uint8)
+    others = np.flatnonzero((io_to_dense == 0) | (io_to_dense > ns))
+    assert letters.size == 3 * ns and others.size == 256 - 3 * ns
+    bad = [int(b) for b in np.flatnonzero(io_to_dense == 0)[:2]] + [int(b) for b in rng.choice(others, 6, replace=False)]
+    _check_staged_coding(lib, io_to_dense, ns, letters, bad, rng)
+
+
+def test_check_of_prepacked_codes_equals_a_plain_model(emul):
+    """packed_codes_unsearchable (k_search with a caller's 2-bit batch): true iff one of the first nsym codes is >= ns;
+    codes past nsym (the next query of the stream) are never looked at; always false with 4 searchable symbols."""
+    emul.emul_packed_unsearchable.restype = C.c_int
+    emul.emul_packed_unsearchable.argtypes = [C.c_uint64, C.c_uint64, C.c_uint32, C.c_uint32]
+    rng = np.random.default_rng(5)
+    for ns in (1, 2, 3, 4):
+        for nsym in range(0, 65):
+            for _ in range(12):
+                codes = rng.integers(0, ns, 64)
+                codes[nsym:] = rng.integers(0, 4, 64 - nsym)          # anything behind the query
+                if nsym and rng.random() < 0.6:
+                    codes[int(rng.integers(0, nsym))] = int(rng.integers(0, 4))
+                v = sum(int(c) << (2 * j) for j, c in enumerate(codes))
+                want = int(any(int(c) >= ns for c in codes[:nsym]))
+                got = emul.emul_packed_unsearchable(v & (2 ** 64 - 1), v >> 64, nsym, ns)
+                assert got == want, (ns, nsym, codes.tolist())

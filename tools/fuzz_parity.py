@@ -43,9 +43,12 @@ def make_text(rng, syms, kind, max_len):
     return bytes(rng.choice(syms) for _ in range(rng.randrange(0, 4)))  # tiny
 
 
-def one_case(seed):
+def one_case(seed, alph=None):
+    """One random case; `alph` fixes the alphabet (any name gdx_testutil knows), the rest is drawn from the seed as
+    it would be otherwise."""
     rng = random.Random(seed)
-    alph = rng.choice(ALPHABETS)
+    drawn = rng.choice(ALPHABETS)
+    alph = alph or drawn
     oa = util.oracle_alphabet(alph)
     syms, search = util.all_io_symbols(oa), util.searchable_io_symbols(oa)
     texts = [make_text(rng, syms, rng.choice(["random", "random", "runs", "periodic", "tiny"]),
