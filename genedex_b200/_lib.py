@@ -26,6 +26,8 @@ GDX_QUERIES_IO_BYTES, GDX_QUERIES_PACKED_2BIT = 0, 1
 GDX_RANK_CONDENSED, GDX_RANK_FLAT = 0, 1
 GDX_NCCL_UNIQUE_ID_BYTES = 128
 GDX_ABI_VERSION = 2
+GDX_HAMMING_MAX_MISMATCHES = 3
+GDX_HAMMING_MAX_QUERY_LEN = 256
 
 
 class gdx_alphabet(C.Structure):
@@ -42,6 +44,10 @@ class gdx_config(C.Structure):
 
 class gdx_hit(C.Structure):
     _fields_ = [("text_id", C.c_uint64), ("position", C.c_uint64)]
+
+
+class gdx_hamming_interval(C.Structure):
+    _fields_ = [("start", C.c_uint64), ("end", C.c_uint64), ("mismatches", C.c_uint32), ("reserved", C.c_uint32)]
 
 
 class gdx_queries(C.Structure):
@@ -131,6 +137,9 @@ PROTOTYPES = {
     "gdx_locate_intervals": (C.c_int, [_vp, _vp, _vp, _u64, _vp, _P(_vp), _P(_u64)]),
     "gdx_free_hits": (None, [_vp, _vp]),
     "gdx_extend_many": (C.c_int, [_vp, _vp, _vp, _vp, _u64]),
+    "gdx_count_many_hamming": (C.c_int, [_vp, _P(gdx_queries), _u32, _vp]),
+    "gdx_cursors_many_hamming": (C.c_int, [_vp, _P(gdx_queries), _u32, _vp, _P(_vp), _P(_u64)]),
+    "gdx_locate_many_hamming": (C.c_int, [_vp, _P(gdx_queries), _u32, _vp, _P(_vp), _P(_u64)]),
     "gdx_cursor_for_query": (C.c_int, [_vp, _vp, _u64, _P(_u64), _P(_u64)]),
     "gdx_cursors_many_device": (C.c_int, [_vp, _P(gdx_queries), _vp, _vp, _vp, _vp]),
     "gdx_count_many_device": (C.c_int, [_vp, _P(gdx_queries), _vp, _vp, _vp]),

@@ -23,6 +23,7 @@
 
 #include <cub/device/device_radix_sort.cuh>
 #include <cub/device/device_scan.cuh>
+#include <cub/device/device_segmented_sort.cuh>
 
 #include "../../include/genedex_b200.h"
 #include "device_build.h"
@@ -3128,6 +3129,342 @@ extern "C" gdx_status gdx_cursor_for_query(const gdx_index *idx, const uint8_t *
             }
         }
         return GDX_OK;
+    });
+}
+
+// ================================================================================================
+// Hamming search (no counterpart in the reference; semantics in include/genedex_b200.h, search in hamming.h)
+// ================================================================================================
+namespace {
+
+static_assert(sizeof(HammingInterval) == sizeof(gdx_hamming_interval), "HammingInterval mirrors gdx_hamming_interval");
+static_assert(GDX_HAMMING_MAX_MISMATCHES == kHammingMaxMismatches && GDX_HAMMING_MAX_QUERY_LEN == kHammingMaxQueryLen,
+              "hamming.h and the header agree on the limits");
+
+// queries per chunk: bounds the workspace (query bytes, per-query counts and offsets) whatever the batch size,
+// while one chunk still puts a thread on every slot of the device
+constexpr uint64_t kHammingChunkQueries = 1ull << 20;
+
+enum HammingMode { kHammingCount = 0, kHammingCursors = 1, kHammingLocate = 2 };
+
+// The first query the host refuses, nq if none: offsets that decrease or leave [offsets[0], offsets[nq]]
+// (GDX_ERR_BAD_ARG) or a query longer than GDX_HAMMING_MAX_QUERY_LEN (GDX_ERR_UNSUPPORTED).  One pass over the
+// offsets, which is cheap next to a search that may branch at every symbol.
+uint64_t hamming_host_check(const gdx_queries *q, gdx_status *st) {
+    *st = GDX_OK;
+    if (q->nq == 0) return 0;
+    if (!q->offsets) {
+        if (q->fixed_len <= kHammingMaxQueryLen) return q->nq;
+        *st = GDX_ERR_UNSUPPORTED;
+        return 0;
+    }
+    const uint64_t lo = q->offsets[0], hi = q->offsets[q->nq];
+    for (uint64_t i = 0; i < q->nq; ++i) {
+        const uint64_t b = q->offsets[i], e = q->offsets[i + 1];
+        if (e < b || b < lo || e > hi) {
+            *st = GDX_ERR_BAD_ARG;
+            return i;
+        }
+        if (e - b > kHammingMaxQueryLen) {
+            *st = GDX_ERR_UNSUPPORTED;
+            return i;
+        }
+    }
+    return q->nq;
+}
+
+// error word of k_hamming<.., 1>: smallest failing query (kBadOffsetFlag: its offsets leave the uploaded chunk)
+gdx_status hamming_error(uint64_t bad) {
+    if (bad == kNoError) return GDX_OK;
+    t_error_query = bad & ~kBadOffsetFlag;
+    if (bad & kBadOffsetFlag)
+        return fail(GDX_ERR_BAD_ARG, "query %llu: queries->offsets must not decrease and must stay inside the batch",
+                    (unsigned long long)t_error_query);
+    return fail(GDX_ERR_INVALID_SYMBOL, "query %llu: every byte of a Hamming query must be a searchable symbol",
+                (unsigned long long)t_error_query);
+}
+
+// the library-owned pinned buffer the results of all chunks are copied into (grows; the stream is idle then)
+struct HammingResult {
+    const gdx_index *idx;
+    void *p = nullptr;
+    uint64_t cap = 0, used = 0;  // bytes
+    gdx_status reserve(uint64_t bytes) {
+        if (bytes <= cap) return GDX_OK;
+        void *bigger = nullptr;
+        uint64_t c = 0;
+        GDX_TRY(acquire_pinned_hits(idx, std::max<uint64_t>(2 * bytes, 4096), &bigger, &c));
+        if (p) {
+            memcpy(bigger, p, used);
+            release_pinned_hits(idx, p);
+        }
+        p = bigger;
+        cap = c;
+        return GDX_OK;
+    }
+};
+
+// Chunks of kHammingChunkQueries over the queries [0, n_ok) on slot 0's stream: upload -> pass 1 (checks + counts)
+// -> [scan -> pass 2 (intervals) -> locate] -> results to the caller.  counts == NULL in kHammingCount mode: only
+// check the queries (an error is then looked for in front of a query the host refused).
+gdx_status hamming_run(const gdx_index *idx, Workspace *ws, const gdx_queries *qs, uint32_t k, int mode, uint64_t n_ok,
+                       uint64_t *counts, uint64_t *offsets_out, HammingResult &res) {
+    Slot &sl = ws->slot[0];
+    cudaStream_t st = sl.stream;
+    sl.ev_used = 0;
+    const uint64_t strata = k + 1;
+    const uint64_t elem = mode == kHammingCursors ? sizeof(gdx_hamming_interval) : sizeof(gdx_hit);
+    uint64_t *d_err = ws->small.d, *d_exp = ws->small.d + 1;  // (locate_device_intervals owns words 4..15)
+    CUDA_TRY(cudaMemsetAsync(d_err, 0xff, 8, st));
+    CUDA_TRY(cudaMemsetAsync(d_exp, 0, 8, st));
+    const bool src_pinned = n_ok && is_pinned(qs->bytes);
+    uint64_t h2d = 0, d2h = 0, launches = 0;
+    double ms_loc = 0;
+    for (uint64_t q0 = 0; q0 < n_ok; q0 += kHammingChunkQueries) {
+        const uint64_t cq = std::min<uint64_t>(kHammingChunkQueries, n_ok - q0);
+        const uint64_t sym0 = query_bytes_end(qs, q0), nsym = query_bytes_end(qs, q0 + cq) - sym0;
+        // the chunk's IO bytes (+ offsets) through pinned staging; the previous chunk's copies are done
+        CUDA_TRY(sl.bytes.reserve(nsym + 8));
+        if (nsym) {
+            const uint8_t *src = qs->bytes + sym0;
+            if (!src_pinned) {
+                CUDA_TRY(sl.h_in.reserve(nsym));
+                HostPool::get().copy(sl.h_in.p, src, nsym);
+                src = (const uint8_t *)sl.h_in.p;
+            }
+            CUDA_TRY(cudaMemcpyAsync(sl.bytes.p, src, nsym, cudaMemcpyHostToDevice, st));
+            h2d += nsym;
+        }
+        DevQueries dq = {};
+        dq.bytes = sl.bytes.as<uint8_t>();
+        dq.fixed_len = qs->fixed_len;
+        dq.nq = cq;
+        dq.limit = nsym;
+        if (qs->offsets) {
+            CUDA_TRY(sl.offsets.reserve((cq + 1) * 8));
+            CUDA_TRY(sl.h_off.reserve((cq + 1) * 8));
+            HostPool::get().copy(sl.h_off.p, qs->offsets + q0, (cq + 1) * 8);
+            CUDA_TRY(cudaMemcpyAsync(sl.offsets.p, sl.h_off.p, (cq + 1) * 8, cudaMemcpyHostToDevice, st));
+            h2d += (cq + 1) * 8;
+            dq.offsets = sl.offsets.as<uint64_t>();
+            dq.base = sym0;
+        }
+        // pass 1: checks, per-stratum counts, intervals per query
+        const bool intervals = mode != kHammingCount;
+        CUDA_TRY(sl.out_a.reserve(cq * strata * 8));
+        if (intervals) {
+            CUDA_TRY(sl.counts.reserve((cq + 1) * 8));
+            CUDA_TRY(sl.local_off.reserve((cq + 1) * 8));
+            CUDA_TRY(cudaMemsetAsync(sl.counts.as<uint64_t>() + cq, 0, 8, st));
+        }
+        const unsigned grid = (unsigned)div_up(cq, 256);
+        cudaEvent_t e0 = ws->next_event(sl), e1 = ws->next_event(sl);
+        CUDA_TRY(cudaEventRecord(e0, st));
+        GDX_TRY(dispatch_layout(idx->h.layout, [&](auto L) -> gdx_status {
+            k_hamming<decltype(L), 1><<<grid, 256, 0, st>>>(idx->dev, dq, k, q0, d_err, sl.out_a.as<uint64_t>(),
+                                                             intervals ? sl.counts.as<uint64_t>() : nullptr, nullptr,
+                                                             nullptr, nullptr, reinterpret_cast<unsigned long long *>(d_exp));
+            return GDX_OK;
+        }));
+        CUDA_TRY(cudaGetLastError());
+        CUDA_TRY(cudaEventRecord(e1, st));
+        ++launches;
+        if (!intervals) {
+            if (counts) {
+                CUDA_TRY(sl.h_out_a.reserve(cq * strata * 8));
+                CUDA_TRY(cudaMemcpyAsync(sl.h_out_a.p, sl.out_a.p, cq * strata * 8, cudaMemcpyDeviceToHost, st));
+                d2h += cq * strata * 8;
+            }
+            CUDA_TRY(cudaMemcpyAsync(ws->small.h, d_err, 8, cudaMemcpyDeviceToHost, st));
+            CUDA_TRY(cudaStreamSynchronize(st));
+            GDX_TRY(hamming_error(ws->small.h[0]));
+            if (counts) HostPool::get().copy(counts + q0 * strata, sl.h_out_a.p, cq * strata * 8);
+            continue;
+        }
+        // CSR of the chunk's intervals
+        size_t tmp = 0;
+        CUDA_TRY(cub::DeviceScan::ExclusiveSum(nullptr, tmp, sl.counts.as<uint64_t>(), sl.local_off.as<uint64_t>(), cq + 1,
+                                               st));
+        CUDA_TRY(sl.scan_tmp.reserve(tmp));
+        CUDA_TRY(cub::DeviceScan::ExclusiveSum(sl.scan_tmp.p, tmp, sl.counts.as<uint64_t>(), sl.local_off.as<uint64_t>(),
+                                               cq + 1, st));
+        CUDA_TRY(cudaMemcpyAsync(ws->small.h, d_err, 8, cudaMemcpyDeviceToHost, st));
+        CUDA_TRY(cudaMemcpyAsync(ws->small.h + 1, sl.local_off.as<uint64_t>() + cq, 8, cudaMemcpyDeviceToHost, st));
+        CUDA_TRY(cudaStreamSynchronize(st));
+        ++launches;
+        GDX_TRY(hamming_error(ws->small.h[0]));
+        const uint64_t niv = ws->small.h[1];
+        // pass 2: the intervals at their CSR offsets in search order, a sort by start within every query, then records
+        // (cursors) or starts / ends (the locate path)
+        const uint64_t rec_bytes = mode == kHammingCursors ? sizeof(HammingInterval) : 8;
+        const uint64_t held = sl.rows.cap + sl.big.cap + ws->starts.cap + sl.xbuf.cap +
+                              (mode == kHammingCursors ? sl.hits.cap : ws->ends.cap);
+        const uint64_t need = niv * (32 + rec_bytes);
+        bool fits = niv <= 0x7fffffffull;  // (the segmented sort counts items in an int)
+        if (fits && need > held) {
+            size_t free_b = 0, total_b = 0;
+            CUDA_TRY(cudaMemGetInfo(&free_b, &total_b));
+            fits = need <= free_b + held;
+        }
+        if (!fits)
+            return fail(GDX_ERR_OOM, "%llu intervals of one chunk do not fit into device memory; split the batch",
+                        (unsigned long long)niv);
+        const uint64_t nr = std::max<uint64_t>(niv, 1);
+        CUDA_TRY(sl.rows.reserve(nr * 8));
+        CUDA_TRY(sl.big.reserve(nr * 8));
+        CUDA_TRY(ws->starts.reserve(nr * 8));
+        CUDA_TRY(sl.xbuf.reserve(nr * 8));
+        CUDA_TRY(mode == kHammingCursors ? sl.hits.reserve(nr * rec_bytes) : ws->ends.reserve(nr * 8));
+        if (niv) {
+            cudaEvent_t f0 = ws->next_event(sl), f1 = ws->next_event(sl);
+            CUDA_TRY(cudaEventRecord(f0, st));
+            GDX_TRY(dispatch_layout(idx->h.layout, [&](auto L) -> gdx_status {
+                k_hamming<decltype(L), 2><<<grid, 256, 0, st>>>(idx->dev, dq, k, q0, nullptr, nullptr, nullptr,
+                                                                 sl.local_off.as<uint64_t>(), sl.rows.as<uint64_t>(),
+                                                                 sl.big.as<uint64_t>(), nullptr);
+                return GDX_OK;
+            }));
+            CUDA_TRY(cudaGetLastError());
+            size_t sort_tmp = 0;
+            const uint64_t *seg = sl.local_off.as<uint64_t>();
+            CUDA_TRY(cub::DeviceSegmentedSort::SortPairs(nullptr, sort_tmp, sl.rows.as<uint64_t>(), ws->starts.as<uint64_t>(),
+                                                         sl.big.as<uint64_t>(), sl.xbuf.as<uint64_t>(), (int)niv, (int)cq,
+                                                         seg, seg + 1, st));
+            CUDA_TRY(sl.sort.reserve(sort_tmp));
+            CUDA_TRY(cub::DeviceSegmentedSort::SortPairs(sl.sort.p, sort_tmp, sl.rows.as<uint64_t>(), ws->starts.as<uint64_t>(),
+                                                         sl.big.as<uint64_t>(), sl.xbuf.as<uint64_t>(), (int)niv, (int)cq,
+                                                         seg, seg + 1, st));
+            k_hamming_decode<<<(unsigned)div_up(niv, 256), 256, 0, st>>>(
+                ws->starts.as<uint64_t>(), sl.xbuf.as<uint64_t>(), niv,
+                mode == kHammingCursors ? sl.hits.as<HammingInterval>() : nullptr,
+                mode == kHammingCursors ? nullptr : ws->ends.as<uint64_t>());
+            CUDA_TRY(cudaGetLastError());
+            CUDA_TRY(cudaEventRecord(f1, st));
+            launches += 3;
+        }
+        // results of the chunk: records (cursors) or hits (locate, the walk of gdx_locate_intervals) + per-query offsets
+        uint64_t n_out = niv;
+        const uint64_t *d_query_off = sl.local_off.as<uint64_t>();
+        if (mode == kHammingLocate) {
+            GDX_TRY(locate_device_intervals(idx, ws, ws->starts.as<uint64_t>(), ws->ends.as<uint64_t>(), niv, &n_out));
+            CUDA_TRY(sl.out_b.reserve(cq * 8));
+            k_gather_u64<<<grid, 256, 0, st>>>(sl.local_off.as<uint64_t>(), ws->hit_offsets.as<uint64_t>(), cq,
+                                               sl.out_b.as<uint64_t>());
+            CUDA_TRY(cudaGetLastError());
+            ++launches;
+            d_query_off = sl.out_b.as<uint64_t>();
+        }
+        const uint64_t base = res.used / elem;
+        GDX_TRY(res.reserve(res.used + n_out * elem));
+        if (n_out) {
+            const void *d_src = mode == kHammingCursors ? sl.hits.p : ws->hits.p;
+            CUDA_TRY(cudaMemcpyAsync((uint8_t *)res.p + res.used, d_src, n_out * elem, cudaMemcpyDeviceToHost, st));
+            d2h += n_out * elem;
+        }
+        CUDA_TRY(sl.h_out_a.reserve(cq * 8));
+        CUDA_TRY(cudaMemcpyAsync(sl.h_out_a.p, d_query_off, cq * 8, cudaMemcpyDeviceToHost, st));
+        d2h += cq * 8;
+        CUDA_TRY(cudaStreamSynchronize(st));
+        if (mode == kHammingLocate) {
+            float ms = 0;
+            if (cudaEventElapsedTime(&ms, ws->ev_a, ws->ev_b) == cudaSuccess) ms_loc += ms;
+        }
+        const uint64_t *h_off = (const uint64_t *)sl.h_out_a.p;
+        for (uint64_t i = 0; i < cq; ++i) offsets_out[q0 + i] = base + h_off[i];
+        res.used += n_out * elem;
+    }
+    CUDA_TRY(cudaMemcpyAsync(ws->small.h + 2, d_exp, 8, cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(cudaStreamSynchronize(st));
+    double ms = 0;
+    for (size_t i = 0; i + 1 < sl.ev_used; i += 2) {
+        float t = 0;
+        cudaEventElapsedTime(&t, sl.ev[i], sl.ev[i + 1]);
+        ms += t;
+    }
+    t_stats.queries = qs->nq;
+    t_stats.lf_steps = ws->small.h[2];
+    t_stats.kernel_ms_search = ms;
+    t_stats.kernel_ms_locate = ms_loc;
+    t_stats.kernel_launches += launches;
+    t_stats.h2d_bytes = h2d;
+    t_stats.d2h_bytes = d2h;
+    if (mode == kHammingLocate) t_stats.hits = res.used / elem;
+    return GDX_OK;
+}
+
+gdx_status hamming_many_impl(const gdx_index *idx, const gdx_queries *queries, uint32_t k, int mode, uint64_t *counts,
+                             uint64_t *offsets_out, void **result, uint64_t *num_out, const char *what) {
+    GDX_TRY(begin_call(idx, what));
+    GDX_TRY(check_queries(idx, queries));
+    if (k > GDX_HAMMING_MAX_MISMATCHES)
+        return fail(GDX_ERR_BAD_ARG, "%s: max_mismatches %u is larger than GDX_HAMMING_MAX_MISMATCHES (%d)", what, k,
+                    GDX_HAMMING_MAX_MISMATCHES);
+    if (queries->encoding != GDX_QUERIES_IO_BYTES)
+        return fail(GDX_ERR_UNSUPPORTED, "%s takes IO-byte queries (GDX_QUERIES_IO_BYTES) only", what);
+    if (mode == kHammingCount ? (queries->nq && !counts) : (!offsets_out || !result || !num_out))
+        return fail(GDX_ERR_BAD_ARG, "output is NULL");
+    if (result) {
+        *result = nullptr;
+        *num_out = 0;
+    }
+    gdx_status host_st = GDX_OK;
+    const uint64_t n_ok = hamming_host_check(queries, &host_st);
+    std::shared_lock<std::shared_mutex> cfg(idx->cfg_mu);
+    DeviceGuard guard(idx->device);
+    WsLease lease(idx);
+    Workspace *ws = lease.w;
+    if (!ws) return fail(GDX_ERR_CUDA, "could not create a CUDA workspace: %s", cudaGetErrorString(cudaGetLastError()));
+    HammingResult res{idx};
+    gdx_status st = mode == kHammingCount ? GDX_OK : res.reserve(4096);
+    if (st == GDX_OK) {
+        // with a query the host refuses, the queries in front of it are only checked: a smaller offender wins
+        st = host_st == GDX_OK ? hamming_run(idx, ws, queries, k, mode, n_ok, counts, offsets_out, res)
+                               : hamming_run(idx, ws, queries, k, kHammingCount, n_ok, nullptr, nullptr, res);
+    }
+    if (st == GDX_OK && host_st != GDX_OK) {
+        t_error_query = n_ok;
+        st = host_st == GDX_ERR_BAD_ARG
+                 ? fail(GDX_ERR_BAD_ARG, "query %llu: queries->offsets must not decrease and must stay inside the batch",
+                        (unsigned long long)n_ok)
+                 : fail(GDX_ERR_UNSUPPORTED, "query %llu is longer than GDX_HAMMING_MAX_QUERY_LEN (%d symbols)",
+                        (unsigned long long)n_ok, GDX_HAMMING_MAX_QUERY_LEN);
+    }
+    if (st != GDX_OK) {
+        drain(ws);
+        if (res.p) release_pinned_hits(idx, res.p);
+        return st;
+    }
+    if (mode != kHammingCount) {
+        const uint64_t elem = mode == kHammingCursors ? sizeof(gdx_hamming_interval) : sizeof(gdx_hit);
+        offsets_out[queries->nq] = res.used / elem;
+        *result = res.p;
+        *num_out = res.used / elem;
+    }
+    return GDX_OK;
+}
+
+}  // namespace
+
+extern "C" gdx_status gdx_count_many_hamming(const gdx_index *idx, const gdx_queries *queries, uint32_t max_mismatches,
+                                             uint64_t *counts) {
+    return guarded([&] {
+        return hamming_many_impl(idx, queries, max_mismatches, kHammingCount, counts, nullptr, nullptr, nullptr,
+                                 "gdx_count_many_hamming");
+    });
+}
+extern "C" gdx_status gdx_cursors_many_hamming(const gdx_index *idx, const gdx_queries *queries, uint32_t max_mismatches,
+                                               uint64_t *interval_offsets, gdx_hamming_interval **intervals,
+                                               uint64_t *num_intervals) {
+    return guarded([&] {
+        return hamming_many_impl(idx, queries, max_mismatches, kHammingCursors, nullptr, interval_offsets,
+                                 reinterpret_cast<void **>(intervals), num_intervals, "gdx_cursors_many_hamming");
+    });
+}
+extern "C" gdx_status gdx_locate_many_hamming(const gdx_index *idx, const gdx_queries *queries, uint32_t max_mismatches,
+                                              uint64_t *hit_offsets, gdx_hit **hits, uint64_t *num_hits) {
+    return guarded([&] {
+        return hamming_many_impl(idx, queries, max_mismatches, kHammingLocate, nullptr, hit_offsets,
+                                 reinterpret_cast<void **>(hits), num_hits, "gdx_locate_many_hamming");
     });
 }
 

@@ -8,6 +8,8 @@
 //                   <.., VERIFY>: one-row intervals are finished by resolving SA[row] and comparing the
 //                   rest of the query with the text section (count / locate only, identical results)
 //   k_extend        one LF pair per cursor                   (cursor.rs:34-51)
+//   k_hamming       backtracking backward search with up to k substitutions, one thread per query (hamming.h;
+//                   no counterpart in the reference)
 //   k_interval_counts / k_expand_rows / k_expand_big_rows / k_add_base    rows of every hit (CSR)
 //   k_locate_walk   K3+K4: LF-walk to the next SA sample + text-id mapping, one thread per hit
 //                                                             (sampled_suffix_array.rs:110-138,
@@ -40,6 +42,7 @@
 #include <cub/block/block_scan.cuh>
 
 #include "device_index.h"
+#include "hamming.h"
 #include "row_context.h"
 
 namespace gdx {
@@ -854,6 +857,150 @@ k_extend(const __grid_constant__ DevIndex ix, uint64_t *__restrict__ starts, uin
         starts[q] = s;
         ends[q] = e;
     }
+}
+
+// ---- Hamming search: rank sources of hamming_search (hamming.h) ---------------------------------------
+// LF of the derived symbol (K32, sigma 6) from the sum of LF(c, i) over c = 1..4 (see K32::lf_derived)
+__device__ __forceinline__ uint64_t k32_lf_derived_from_sum(const DevIndex &ix, uint64_t i, uint64_t lf_sum) {
+    uint64_t counts = 0;
+#pragma unroll
+    for (uint32_t c = 1; c <= 4; ++c) counts += __ldg(ix.count + c);
+    const uint64_t rank0 = lower_bound_u64(ix.border_rows, ix.n_border, i);
+    return __ldg(ix.count + 5) + (i - rank0 - (lf_sum - counts));
+}
+
+// K32: an expansion fetches the record of each border once (one record when both share it) and derives the child
+// of every searchable symbol from them, the derived symbol (sigma 6 with `N` searchable) included
+struct HammingK32Source {
+    const DevIndex &ix;
+    uint32_t ns;
+    uint64_t n;
+    struct Node {
+        uint64_t s[5], e[5];
+    };
+    __device__ __forceinline__ void expand(uint64_t s, uint64_t e, Node &nd) const {
+        const K32::Rec rs = K32::load(ix, s, 0);
+        const K32::Rec re = (s >> 6) == (e >> 6) ? rs : K32::load(ix, e, 0);
+        uint64_t sum_s = 0, sum_e = 0;
+#pragma unroll
+        for (uint32_t c = 1; c <= 4; ++c) {
+            if (c > ns) break;
+            nd.s[c - 1] = sbc_load(ix, s, c) + K32::local_rank(rs, c, s);
+            nd.e[c - 1] = sbc_load(ix, e, c) + K32::local_rank(re, c, e);
+            sum_s += nd.s[c - 1];
+            sum_e += nd.e[c - 1];
+        }
+        if (ns > 4) {
+            nd.s[4] = k32_lf_derived_from_sum(ix, s, sum_s);
+            nd.e[4] = k32_lf_derived_from_sum(ix, e, sum_e);
+        }
+    }
+    __device__ __forceinline__ void child(const Node &nd, uint32_t c, uint64_t &s, uint64_t &e) const {
+        s = nd.s[c - 1];
+        e = nd.e[c - 1];
+    }
+    __device__ __forceinline__ void step(uint32_t c, uint64_t &s, uint64_t &e) const { lf_pair<K32>(ix, c, s, e); }
+};
+
+// KG<B> (up to 255 searchable symbols): a node keeps its interval, each child costs one LF pair when it is tried
+template <class L>
+struct HammingLazySource {
+    const DevIndex &ix;
+    uint32_t ns;
+    uint64_t n;
+    struct Node {
+        uint64_t s, e;
+    };
+    __device__ __forceinline__ void expand(uint64_t s, uint64_t e, Node &nd) const {
+        nd.s = s;
+        nd.e = e;
+    }
+    __device__ __forceinline__ void child(const Node &nd, uint32_t c, uint64_t &s, uint64_t &e) const {
+        s = nd.s;
+        e = nd.e;
+        lf_pair<L>(ix, c, s, e);
+    }
+    __device__ __forceinline__ void step(uint32_t c, uint64_t &s, uint64_t &e) const { lf_pair<L>(ix, c, s, e); }
+};
+
+template <class L>
+struct HammingSourceOf {
+    using type = HammingLazySource<L>;
+};
+template <>
+struct HammingSourceOf<K32> {
+    using type = HammingK32Source;
+};
+
+// dense symbol of query position j (IO bytes through the shared translation table)
+struct HammingQuery {
+    const uint8_t *tab, *p;
+    __device__ __forceinline__ uint32_t operator()(uint32_t j) const { return tab[__ldg(p + j)]; }
+};
+
+// PASS 1: checks every query in full (every byte must be a searchable symbol), then writes occ[q * (k + 1) + d]
+// (occurrences with exactly d mismatches) and, with n_iv, the number of intervals of query q; counts the node
+// expansions into *stat_expansions.  PASS 2: runs the same search again and writes the intervals of query q from
+// iv_off[q] on as sort keys and values (HammingWriter).  One thread per query; the frame stack (hamming.h) lives in
+// local memory.
+template <class L, int PASS>
+__global__ void __launch_bounds__(256)
+k_hamming(const __grid_constant__ DevIndex ix, const DevQueries qs, uint32_t k, uint64_t q_index_base, uint64_t *err,
+          uint64_t *__restrict__ occ, uint64_t *__restrict__ n_iv, const uint64_t *__restrict__ iv_off,
+          uint64_t *__restrict__ keys, uint64_t *__restrict__ vals, unsigned long long *stat_expansions) {
+    __shared__ uint8_t tab[256];
+    for (int i = threadIdx.x; i < 256; i += blockDim.x) tab[i] = ix.io_to_dense[i];
+    __syncthreads();
+    using S = typename HammingSourceOf<L>::type;
+    const uint64_t q = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    uint64_t expansions = 0;
+    if (q < qs.nq) {
+        uint64_t begin, len;
+        query_extent(qs, q, begin, len);
+        const S rs{ix, ix.ns, ix.n};
+        const HammingQuery sym{tab, qs.bytes + begin};
+        HammingFrame<typename S::Node> stack[kHammingMaxQueryLen];
+        if constexpr (PASS == 1) {
+            // (the host refuses broken offsets and long queries before the search; this keeps such a query from
+            // being read out of bounds all the same)
+            const bool broken = begin > qs.limit || len > qs.limit - begin;
+            bool bad = broken || len > kHammingMaxQueryLen;
+            for (uint32_t j = 0; !bad && j < len; ++j) {
+                const uint32_t c = sym(j);
+                bad = c == 0 || c > ix.ns;
+            }
+            HammingCounter cnt;
+            if (bad) report_error(err, (broken ? kBadOffsetFlag : 0ull) | (q_index_base + q));
+            else expansions = hamming_search(rs, sym, (uint32_t)len, k, stack, cnt);
+            for (uint32_t d = 0; d <= k; ++d) occ[q * (k + 1) + d] = cnt.occ[d];
+            if (n_iv) n_iv[q] = cnt.intervals;
+        } else {
+            HammingWriter w{keys, vals, iv_off[q]};
+            hamming_search(rs, sym, (uint32_t)len, k, stack, w);
+        }
+    }
+    if (PASS == 1 && stat_expansions) {
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) expansions += __shfl_down_sync(0xffffffffu, expansions, o);
+        if ((threadIdx.x & 31) == 0 && expansions) atomicAdd(stat_expansions, (unsigned long long)expansions);
+    }
+}
+
+// the pairs of pass 2, sorted by start per query -> records (iv) or interval ends (the starts are the keys)
+__global__ void k_hamming_decode(const uint64_t *__restrict__ keys, const uint64_t *__restrict__ vals, uint64_t n,
+                                 HammingInterval *__restrict__ iv, uint64_t *__restrict__ ends) {
+    const uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const HammingInterval h = hamming_decode(keys[i], vals[i]);
+    if (iv) iv[i] = h;
+    else ends[i] = h.end;
+}
+
+// out[i] = src[idx[i]], i < n (hit offsets of a query = those of its first interval)
+__global__ void k_gather_u64(const uint64_t *__restrict__ idx, const uint64_t *__restrict__ src, uint64_t n,
+                             uint64_t *__restrict__ out) {
+    const uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < n) out[i] = src[idx[i]];
 }
 
 // ---- CSR plumbing for locate --------------------------------------------------------------------------

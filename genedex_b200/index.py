@@ -344,6 +344,59 @@ class FmIndex:
         finally:
             self._lib.gdx_free_hits(self._h, hp)
 
+    # -- approximate search (no counterpart in the reference): up to k substitutions, semantics in genedex_b200.h
+    def count_many_hamming_packed(self, data: np.ndarray, offsets: np.ndarray | None, k: int, fixed_len: int = 0,
+                                  nq: int | None = None) -> np.ndarray:
+        """-> uint64 array (nq, k + 1): [i, d] = occurrences of query i with exactly d mismatches."""
+        nq = (offsets.size - 1) if offsets is not None else nq
+        counts = np.zeros((max(nq, 1), k + 1), dtype=np.uint64)
+        q = _queries_struct(data, offsets, fixed_len, nq)
+        _check(self._lib.gdx_count_many_hamming(self._h, C.byref(q), k, counts.ctypes.data))
+        return counts[:nq]
+
+    def cursors_many_hamming_packed(self, data: np.ndarray, offsets: np.ndarray | None, k: int, fixed_len: int = 0,
+                                    nq: int | None = None):
+        """-> (interval_offsets[nq + 1], starts, ends, mismatches): the intervals of query i are the entries
+        interval_offsets[i] .. interval_offsets[i + 1], sorted by start."""
+        nq = (offsets.size - 1) if offsets is not None else nq
+        iv_offsets = np.empty(nq + 1, dtype=np.uint64)
+        ip, n = C.c_void_p(), C.c_uint64()
+        q = _queries_struct(data, offsets, fixed_len, nq)
+        _check(self._lib.gdx_cursors_many_hamming(self._h, C.byref(q), k, iv_offsets.ctypes.data, C.byref(ip),
+                                                  C.byref(n)))
+        try:
+            rec = np.zeros((n.value, 3), dtype=np.uint64)
+            if n.value:
+                buf = (_lib.gdx_hamming_interval * n.value).from_address(ip.value)
+                raw = np.frombuffer(buf, dtype=np.uint64).reshape(n.value, 3)
+                rec[:, :2] = raw[:, :2]
+                rec[:, 2] = raw[:, 2] & 0xFFFFFFFF
+        finally:
+            self._lib.gdx_free_hits(self._h, ip)
+        return iv_offsets, rec[:, 0], rec[:, 1], rec[:, 2].astype(np.uint32)
+
+    def locate_many_hamming_packed(self, data: np.ndarray, offsets: np.ndarray | None, k: int, fixed_len: int = 0,
+                                   nq: int | None = None):
+        """-> (hit_offsets[nq + 1], hits[n, 2] = (text_id, position)); hits of a query in ascending SA-row order."""
+        nq = (offsets.size - 1) if offsets is not None else nq
+        hit_offsets = np.empty(nq + 1, dtype=np.uint64)
+        hp, nh = C.c_void_p(), C.c_uint64()
+        q = _queries_struct(data, offsets, fixed_len, nq)
+        _check(self._lib.gdx_locate_many_hamming(self._h, C.byref(q), k, hit_offsets.ctypes.data, C.byref(hp),
+                                                 C.byref(nh)))
+        return hit_offsets, self._take_hits(hp, nh.value)
+
+    def count_many_hamming(self, queries: Iterable[bytes], k: int) -> np.ndarray:
+        return self.count_many_hamming_packed(*pack_queries(queries), k)
+
+    def cursors_many_hamming(self, queries: Iterable[bytes], k: int) -> list[list[tuple["Cursor", int]]]:
+        off, starts, ends, mism = self.cursors_many_hamming_packed(*pack_queries(queries), k)
+        return [[(Cursor(self, int(starts[j]), int(ends[j])), int(mism[j])) for j in range(int(off[i]), int(off[i + 1]))]
+                for i in range(off.size - 1)]
+
+    def locate_many_hamming(self, queries: Iterable[bytes], k: int) -> list[list[Hit]]:
+        return _split_hits(*self.locate_many_hamming_packed(*pack_queries(queries), k))
+
     def locate_intervals_packed(self, starts: np.ndarray, ends: np.ndarray):
         starts = np.ascontiguousarray(starts, dtype=np.uint64)
         ends = np.ascontiguousarray(ends, dtype=np.uint64)

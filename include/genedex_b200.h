@@ -433,6 +433,46 @@ gdx_status gdx_locate_many_sharded_compact(gdx_index *const *replicas, uint32_t 
 gdx_status gdx_extend_many(const gdx_index *idx, uint64_t *starts, uint64_t *ends,
                            const uint8_t *io_symbols, uint64_t n);
 
+/* ---- approximate search, no counterpart in the reference -----------------------------------------
+ * Hamming-distance search with up to max_mismatches substitutions, IO-byte batches (GDX_QUERIES_IO_BYTES) only.
+ *   - A query of length m matches at text position p with d mismatches when the window [p, p + m) lies inside one
+ *     text, every symbol of it is a searchable dense symbol, and it differs from the query in exactly d <= k
+ *     positions, compared in the dense representation (case folding and ambiguity groups apply as everywhere else).
+ *     A window holding `N`, another symbol that is not searchable or a sentinel never matches.
+ *   - Every distinct matching window string is one non-empty SA interval [start, end); its mismatch count is its
+ *     Hamming distance to the query.  The intervals of a query are pairwise disjoint and sorted by start.
+ *   - k = 0 gives what gdx_cursors_many / gdx_count_many / gdx_locate_many give for a query of searchable symbols
+ *     (no interval when that interval is empty).  The empty query gives [0, text_len) with 0 mismatches.
+ *   - Errors are checked before any result is produced, and gdx_last_error_query() names the smallest offending
+ *     query: a byte that is not a searchable symbol (not in the alphabet, or valid but not searchable such as `N`):
+ *     GDX_ERR_INVALID_SYMBOL; a query longer than GDX_HAMMING_MAX_QUERY_LEN: GDX_ERR_UNSUPPORTED; offsets that
+ *     decrease or leave the batch: GDX_ERR_BAD_ARG.  max_mismatches > GDX_HAMMING_MAX_MISMATCHES: GDX_ERR_BAD_ARG;
+ *     GDX_QUERIES_PACKED_2BIT: GDX_ERR_UNSUPPORTED.  Results that do not fit into device memory: GDX_ERR_OOM
+ *     (split the batch).  Nothing is truncated.
+ *   - Results do not depend on the lookup depth, the storage type, the construction route, GDX_FLAG_NO_TEXT, the
+ *     accelerators or gdx_index_set_text_verification.
+ * gdx_stats: lf_steps counts search-node expansions (one per node that may still branch, one per exact LF pair). */
+#define GDX_HAMMING_MAX_MISMATCHES 3
+#define GDX_HAMMING_MAX_QUERY_LEN 256
+typedef struct gdx_hamming_interval {
+    uint64_t start, end;     /* SA interval of one matching window string */
+    uint32_t mismatches;     /* its Hamming distance to the query */
+    uint32_t reserved;       /* 0 */
+} gdx_hamming_interval;
+
+/* counts[i * (k + 1) + d] = occurrences of query i with exactly d mismatches */
+gdx_status gdx_count_many_hamming(const gdx_index *idx, const gdx_queries *queries, uint32_t max_mismatches,
+                                  uint64_t *counts);
+/* CSR: the intervals of query i are intervals[interval_offsets[i] .. interval_offsets[i+1]), sorted by start;
+ * interval_offsets has nq + 1 entries; library-allocated pinned memory, release with
+ * gdx_free_hits(idx, (gdx_hit *)intervals) */
+gdx_status gdx_cursors_many_hamming(const gdx_index *idx, const gdx_queries *queries, uint32_t max_mismatches,
+                                    uint64_t *interval_offsets, gdx_hamming_interval **intervals,
+                                    uint64_t *num_intervals);
+/* CSR as gdx_locate_many; hits of a query in ascending SA-row order over all its intervals */
+gdx_status gdx_locate_many_hamming(const gdx_index *idx, const gdx_queries *queries, uint32_t max_mismatches,
+                                   uint64_t *hit_offsets, gdx_hit **hits, uint64_t *num_hits);
+
 /* single-query forms (src/lib.rs:147-149,169-173,217-235); these follow the single-query code path
  * of the reference (the symbol left of an empty lookup interval is still translated). */
 gdx_status gdx_cursor_for_query(const gdx_index *idx, const uint8_t *query, uint64_t len,

@@ -189,6 +189,39 @@ public:
     template <class Range>
     std::vector<Cursor> cursors_for_many_queries(const Range &queries) const;             // lib.rs:241-246
 
+    // approximate search with up to k substitutions (no counterpart in the crate; semantics in genedex_b200.h)
+    // [i][d] = occurrences of query i with exactly d mismatches
+    template <class Range>
+    std::vector<std::vector<size_t>> count_many_hamming(const Range &queries, uint32_t k) const {
+        detail::Packed p(queries);
+        const size_t nq = p.offsets.size() - 1;
+        std::vector<uint64_t> c(nq * (k + 1) + 1);
+        gdx_queries q = p.view();
+        check(gdx_count_many_hamming(h_->p, &q, k, c.data()));
+        std::vector<std::vector<size_t>> out(nq);
+        for (size_t i = 0; i < nq; ++i) out[i].assign(c.begin() + i * (k + 1), c.begin() + (i + 1) * (k + 1));
+        return out;
+    }
+    // per query: (interval, mismatches) of every matching window string, sorted by start
+    template <class Range>
+    std::vector<std::vector<std::pair<Cursor, uint32_t>>> cursors_many_hamming(const Range &queries, uint32_t k) const;
+    // per query: the hits of all its intervals in ascending SA-row order
+    template <class Range>
+    std::vector<std::vector<Hit>> locate_many_hamming(const Range &queries, uint32_t k) const {
+        detail::Packed p(queries);
+        const size_t nq = p.offsets.size() - 1;
+        std::vector<uint64_t> off(nq + 1);
+        gdx_hit *hits = nullptr;
+        uint64_t n = 0;
+        gdx_queries q = p.view();
+        check(gdx_locate_many_hamming(h_->p, &q, k, off.data(), &hits, &n));
+        std::vector<std::vector<Hit>> out(nq);
+        for (size_t i = 0; i < nq; ++i)
+            for (uint64_t j = off[i]; j < off[i + 1]; ++j) out[i].push_back(Hit{hits[j].text_id, hits[j].position});
+        gdx_free_hits(h_->p, hits);
+        return out;
+    }
+
     const Alphabet &alphabet() const { return alphabet_; }                                // lib.rs:283-285
     size_t num_texts() const { return info().num_texts; }                                 // lib.rs:287-289
     size_t total_text_len() const { return info().text_len; }                             // lib.rs:292-294
@@ -252,6 +285,21 @@ std::vector<Cursor> FmIndex::cursors_for_many_queries(const Range &queries) cons
     check(gdx_cursors_many(h_->p, &q, s.data(), e.data()));
     std::vector<Cursor> out;
     for (size_t i = 0; i < nq; ++i) out.emplace_back(this, s[i], e[i]);
+    return out;
+}
+template <class Range>
+std::vector<std::vector<std::pair<Cursor, uint32_t>>> FmIndex::cursors_many_hamming(const Range &queries, uint32_t k) const {
+    detail::Packed p(queries);
+    const size_t nq = p.offsets.size() - 1;
+    std::vector<uint64_t> off(nq + 1);
+    gdx_hamming_interval *iv = nullptr;
+    uint64_t n = 0;
+    gdx_queries q = p.view();
+    check(gdx_cursors_many_hamming(h_->p, &q, k, off.data(), &iv, &n));
+    std::vector<std::vector<std::pair<Cursor, uint32_t>>> out(nq);
+    for (size_t i = 0; i < nq; ++i)
+        for (uint64_t j = off[i]; j < off[i + 1]; ++j) out[i].emplace_back(Cursor(this, iv[j].start, iv[j].end), iv[j].mismatches);
+    gdx_free_hits(h_->p, (gdx_hit *)iv);
     return out;
 }
 
