@@ -8,6 +8,7 @@
 #include <atomic>
 #include <chrono>
 #include <condition_variable>
+#include <cstddef>
 #include <deque>
 #include <thread>
 #include <cstdarg>
@@ -199,52 +200,114 @@ constexpr uint64_t kChunkMaxQueries = 64ull << 20;
 // first guess of the host-to-device link rate for the hybrid upload of pinned IO bytes (search_host)
 constexpr double kLinkGuessBytesPerMs = 50e6;  // 50 GB/s
 
+// (begin, end) event pairs around the kernels of the current call, created on first use and kept for later calls
+struct EventPairs {
+    struct Pair {
+        cudaEvent_t begin, end;
+    };
+    std::vector<cudaEvent_t> ev;
+    size_t used = 0;
+    cudaEvent_t take() {
+        if (used == ev.size()) {
+            cudaEvent_t e = nullptr;
+            if (cudaEventCreate(&e) != cudaSuccess) return nullptr;  // recording on nullptr fails loudly later
+            ev.push_back(e);
+        }
+        return ev[used++];
+    }
+    Pair next() { return Pair{take(), take()}; }
+    // the kernel time of every completed pair of the call
+    double elapsed_ms() const {
+        double ms = 0;
+        for (size_t i = 0; i + 1 < used; i += 2) {
+            float t = 0;
+            cudaEventElapsedTime(&t, ev[i], ev[i + 1]);
+            ms += t;
+        }
+        return ms;
+    }
+    void reset() { used = 0; }
+    void destroy() {
+        for (auto e : ev) cudaEventDestroy(e);
+    }
+};
+
+// SA intervals -> hits on one stream.  count() writes the width of every interval, their exclusive scan (the CSR
+// offsets, n + 1 entries) and sends the hit total and the number of wide intervals to the pinned words; expand_walk()
+// then lists the rows of every interval (wide ones through a worklist) and walks them to text positions.
+struct IntervalHits {
+    DBuf counts, offsets, scan_tmp, rows, hits, wide;
+    struct DeviceWords {
+        unsigned long long wide, cursor;  // intervals wider than kExpandInline, worklist cursor
+    } *d = nullptr;
+    struct HostWords {
+        uint64_t hits, wide;  // pinned: hit total, intervals wider than kExpandInline
+    } *h = nullptr;
+    cudaEvent_t ev_total = nullptr;  // *h is on the host
+    EventPairs timing;               // around the locate kernels of the current call
+    bool init() {
+        return cudaMalloc(&d, sizeof *d) == cudaSuccess && cudaMallocHost(&h, sizeof *h) == cudaSuccess &&
+               cudaEventCreateWithFlags(&ev_total, cudaEventDisableTiming) == cudaSuccess;
+    }
+    void destroy() {
+        for (DBuf *b : {&counts, &offsets, &scan_tmp, &rows, &hits, &wide}) b->release();
+        if (d) cudaFree(d);
+        if (h) cudaFreeHost(h);
+        if (ev_total) cudaEventDestroy(ev_total);
+        timing.destroy();
+    }
+    gdx_status count(cudaStream_t st, const uint64_t *starts, const uint64_t *ends, uint64_t n);
+    gdx_status expand_walk(const gdx_index *idx, cudaStream_t st, const uint64_t *starts, const uint64_t *ends, uint64_t n,
+                           uint64_t n_hits, uint64_t n_wide, unsigned long long *walk_steps, bool hit32);
+};
+
 struct Slot {
     cudaStream_t stream = nullptr;
     DBuf bytes, offsets, out_a, out_b, sort;
-    // pipelined locate: per-chunk CSR + rows + hits
-    DBuf counts, local_off, scan_tmp, rows, hits, big;
-    uint64_t *d_words = nullptr;  // device: [0] number of wide intervals, [1] worklist cursor
-    uint64_t *h_words = nullptr;  // pinned: [0] hits of the chunk, [1] number of wide intervals
-    cudaEvent_t ev_total = nullptr;
+    IntervalHits locate;  // pipelined locate: the chunk's CSR, rows and hits
     // staging for pageable caller buffers / packed queries / narrow results
     HBuf h_in, h_off, h_out_a, h_out_b;
     // queries of a packed chunk that hold a byte without a 2-bit code: offsets + slots + IO bytes, re-run raw
     HBuf h_x;
     DBuf xbuf;
-    std::vector<cudaEvent_t> ev_loc;  // pairs (begin, end) around the locate kernels of the current call
-    size_t ev_loc_used = 0;
     cudaEvent_t ev_h2d = nullptr, ev_out = nullptr;
     cudaEvent_t ev_link = nullptr;  // the chunk's query upload has left the PCIe link
     bool h2d_pending = false;
-    std::vector<cudaEvent_t> ev;  // pairs (begin, end) around the kernels of the current call
-    size_t ev_used = 0;
+    EventPairs timing;  // around the search kernels of the current call
 };
 
-struct Small {  // pinned + device words shared by one call
-    uint64_t *h = nullptr;  // pinned host, 16 words
-    uint64_t *d = nullptr;  // device, 16 words: [0..2] err per slot, [4] steps, [5] walk steps,
-                            //                   [6] big count, [7] big cursor, [8] total
+// The words one call shares with its kernels, in pinned host memory and on the device.  Error words hold the smallest
+// failing index (atomicMin), kNoError if there is none; the counters are sums (atomicAdd).
+struct Counters {
+    uint64_t err[kSlots];         // k_search per slot stream; k_hamming pass 1 on slot 0
+    uint64_t extend_bad_symbol;   // k_extend: err[0]
+    uint64_t extend_bad_cursor;   // k_extend: err[1]
+    SearchCounters search;        // k_search
+    unsigned long long locate_walk_steps;   // k_locate_walk, k_locate_walk_compact
+    unsigned long long hamming_expansions;  // k_hamming pass 1
 };
+static_assert(offsetof(Counters, extend_bad_cursor) == offsetof(Counters, extend_bad_symbol) + 8,
+              "k_extend reports a bad cursor in the word after its error word");
 
 struct Workspace {
     Slot slot[kSlots];
-    Small small;
-    DBuf starts, ends, counts, hit_offsets, rows, big_list, hits, scan_tmp, symbols;
-    cudaEvent_t ev_a = nullptr, ev_b = nullptr;
+    Counters *cnt_h = nullptr;  // pinned
+    Counters *cnt_d = nullptr;  // device
+    DBuf starts, ends, symbols;
+    IntervalHits locate;  // gdx_locate_intervals and the Hamming locate
+    cudaEvent_t ev_a = nullptr;  // orders the slot streams behind the reset of the counters (search_host)
     bool init() {
         for (auto &s : slot) {
             if (cudaStreamCreateWithFlags(&s.stream, cudaStreamNonBlocking) != cudaSuccess) return false;
-            if (cudaMalloc(&s.d_words, 4 * sizeof(uint64_t)) != cudaSuccess) return false;
-            if (cudaMallocHost(&s.h_words, 4 * sizeof(uint64_t)) != cudaSuccess) return false;
-            if (cudaEventCreateWithFlags(&s.ev_total, cudaEventDisableTiming) != cudaSuccess) return false;
+            if (!s.locate.init()) return false;
             if (cudaEventCreateWithFlags(&s.ev_h2d, cudaEventDisableTiming) != cudaSuccess) return false;
             if (cudaEventCreateWithFlags(&s.ev_out, cudaEventDisableTiming) != cudaSuccess) return false;
             if (cudaEventCreateWithFlags(&s.ev_link, cudaEventDisableTiming) != cudaSuccess) return false;
         }
-        if (cudaMallocHost(&small.h, 16 * sizeof(uint64_t)) != cudaSuccess) return false;
-        if (cudaMalloc(&small.d, 16 * sizeof(uint64_t)) != cudaSuccess) return false;
-        if (cudaEventCreate(&ev_a) != cudaSuccess || cudaEventCreate(&ev_b) != cudaSuccess) return false;
+        if (cudaMallocHost(&cnt_h, sizeof(Counters)) != cudaSuccess) return false;
+        if (cudaMalloc(&cnt_d, sizeof(Counters)) != cudaSuccess) return false;
+        if (!locate.init()) return false;
+        if (cudaEventCreate(&ev_a) != cudaSuccess) return false;
         return true;
     }
     void destroy() {
@@ -255,40 +318,35 @@ struct Workspace {
             s.out_a.release();
             s.out_b.release();
             s.sort.release();
-            for (DBuf *b : {&s.counts, &s.local_off, &s.scan_tmp, &s.rows, &s.hits, &s.big}) b->release();
-            if (s.d_words) cudaFree(s.d_words);
-            if (s.h_words) cudaFreeHost(s.h_words);
-            if (s.ev_total) cudaEventDestroy(s.ev_total);
+            s.locate.destroy();
             if (s.ev_h2d) cudaEventDestroy(s.ev_h2d);
             if (s.ev_out) cudaEventDestroy(s.ev_out);
             if (s.ev_link) cudaEventDestroy(s.ev_link);
             for (HBuf *b : {&s.h_in, &s.h_off, &s.h_out_a, &s.h_out_b, &s.h_x}) b->release();
             s.xbuf.release();
-            for (auto e : s.ev) cudaEventDestroy(e);
-            for (auto e : s.ev_loc) cudaEventDestroy(e);
+            s.timing.destroy();
         }
-        if (small.h) cudaFreeHost(small.h);
-        if (small.d) cudaFree(small.d);
-        for (DBuf *b : {&starts, &ends, &counts, &hit_offsets, &rows, &big_list, &hits, &scan_tmp, &symbols})
-            b->release();
+        if (cnt_h) cudaFreeHost(cnt_h);
+        if (cnt_d) cudaFree(cnt_d);
+        for (DBuf *b : {&starts, &ends, &symbols}) b->release();
+        locate.destroy();
         if (ev_a) cudaEventDestroy(ev_a);
-        if (ev_b) cudaEventDestroy(ev_b);
     }
-    cudaEvent_t next_event(Slot &s) {
-        if (s.ev_used == s.ev.size()) {
-            cudaEvent_t e = nullptr;
-            if (cudaEventCreate(&e) != cudaSuccess) return nullptr;  // recording on nullptr fails loudly later
-            s.ev.push_back(e);
-        }
-        return s.ev[s.ev_used++];
+    // error words to kNoError, counters to zero
+    cudaError_t reset_counters(cudaStream_t st) {
+        constexpr size_t kErrBytes = offsetof(Counters, search);
+        const cudaError_t e = cudaMemsetAsync(cnt_d, 0xff, kErrBytes, st);
+        return e != cudaSuccess ? e : cudaMemsetAsync((uint8_t *)cnt_d + kErrBytes, 0, sizeof(Counters) - kErrBytes, st);
     }
-    cudaEvent_t next_locate_event(Slot &s) {
-        if (s.ev_loc_used == s.ev_loc.size()) {
-            cudaEvent_t e = nullptr;
-            if (cudaEventCreate(&e) != cudaSuccess) return nullptr;
-            s.ev_loc.push_back(e);
+    cudaError_t read_counters(cudaStream_t st) {
+        return cudaMemcpyAsync(cnt_h, cnt_d, sizeof(Counters), cudaMemcpyDeviceToHost, st);
+    }
+    void reset_timing() {
+        for (auto &s : slot) {
+            s.timing.reset();
+            s.locate.timing.reset();
         }
-        return s.ev_loc[s.ev_loc_used++];
+        locate.timing.reset();
     }
 };
 
@@ -353,6 +411,27 @@ struct WsLease {
         if (w) release_ws(idx, w);
     }
 };
+
+// a failed call must not return while one of its streams still reads or writes the caller's buffers; the error that
+// made it fail stays the reported one
+void drain(Workspace *ws) {
+    for (int s = 0; s < kSlots; ++s) cudaStreamSynchronize(ws->slot[s].stream);
+    cudaGetLastError();
+}
+
+// runs f(ws) on a workspace leased for one host-buffer call, with the configuration held shared and idx's device
+// current; drains the workspace when f fails
+template <class F>
+gdx_status with_workspace(const gdx_index *idx, F &&f) {
+    std::shared_lock<std::shared_mutex> cfg(idx->cfg_mu);
+    DeviceGuard guard(idx->device);
+    WsLease lease(idx);
+    if (!lease.w) return fail(GDX_ERR_CUDA, "could not create a CUDA workspace: %s", cudaGetErrorString(cudaGetLastError()));
+    lease.w->reset_timing();
+    const gdx_status st = f(lease.w);
+    if (st != GDX_OK) drain(lease.w);
+    return st;
+}
 
 // ---- layout dispatch -----------------------------------------------------------------------------------
 template <class F>
@@ -1783,13 +1862,13 @@ bool verify_enabled() {
 // narrow: results are written as uint32 (modes 0 and 1, texts shorter than 2^32)
 template <class L>
 void launch_search(const gdx_index *idx, const DevQueries &dq, uint64_t *a, uint64_t *b, int mode, bool narrow,
-                   uint64_t qbase, uint64_t *err, unsigned long long *steps, const uint32_t *perm,
+                   uint64_t qbase, uint64_t *err, SearchCounters *stats, const uint32_t *perm,
                    const uint32_t *slot_map, cudaStream_t stream) {
     if (dq.nq == 0) return;
     const unsigned grid = (unsigned)div_up(dq.nq, 256);
     const bool verify = idx->dev.text && idx->verify;
     const int mf = mode | (narrow ? kModeNarrow : 0);
-#define GDX_LAUNCH(V, C, P) k_search<L, V, C, P><<<grid, 256, 0, stream>>>(idx->dev, dq, a, b, mf, qbase, err, steps, perm, slot_map)
+#define GDX_LAUNCH(V, C, P) k_search<L, V, C, P><<<grid, 256, 0, stream>>>(idx->dev, dq, a, b, mf, qbase, err, stats, perm, slot_map)
     if (dq.packed) {
         if (verify && mode != 0) GDX_LAUNCH(true, false, true);
         else if (verify && idx->dev.isa) GDX_LAUNCH(true, true, true);
@@ -1901,6 +1980,40 @@ const uint64_t kPackMinBytes = env_bytes("GDX_PACK_MIN_BYTES", 1ull << 20);
 gdx_status acquire_pinned_hits(const gdx_index *idx, uint64_t bytes, void **out, uint64_t *cap_out);
 void release_pinned_hits(const gdx_index *idx, void *p);
 
+// a library-owned pinned buffer the results of a call are appended to.  It grows to twice the size asked for (at least
+// 4096 bytes) and keeps what it holds; no copy into it may be in flight then.
+struct PinnedResult {
+    const gdx_index *idx;
+    void *p = nullptr;
+    uint64_t cap = 0, used = 0;  // bytes
+    gdx_status reserve(uint64_t bytes) {
+        if (bytes <= cap) return GDX_OK;
+        void *bigger = nullptr;
+        uint64_t c = 0;
+        GDX_TRY(acquire_pinned_hits(idx, std::max<uint64_t>(2 * bytes, 4096), &bigger, &c));
+        if (p) {
+            memcpy(bigger, p, used);
+            release_pinned_hits(idx, p);
+        }
+        p = bigger;
+        cap = c;
+        return GDX_OK;
+    }
+    void release() {
+        if (p) release_pinned_hits(idx, p);
+        p = nullptr;
+    }
+};
+
+// the two-call CUB exclusive scan (size query, then the scan) with its temporary storage in tmp
+gdx_status exclusive_sum(DBuf &tmp, uint64_t *in, uint64_t *out, uint64_t n, cudaStream_t st) {
+    size_t bytes = 0;
+    CUDA_TRY(cub::DeviceScan::ExclusiveSum(nullptr, bytes, in, out, n, st));
+    CUDA_TRY(tmp.reserve(bytes));
+    CUDA_TRY(cub::DeviceScan::ExclusiveSum(tmp.p, bytes, in, out, n, st));
+    return GDX_OK;
+}
+
 // K3 + K4 over `n_hits` rows.  With a sampled suffix array (walks of geometric length) the compacting kernel
 // keeps every lane busy; with the dense array (one load per row) the plain one-thread-per-hit kernel is the
 // shorter program.
@@ -1914,18 +2027,61 @@ void launch_locate_walk(const gdx_index *idx, const uint64_t *rows, uint64_t n_h
         k_locate_walk<L><<<(unsigned)div_up(n_hits, 256), 256, 0, stream>>>(idx->dev, rows, n_hits, hits, d_walk, hit32 ? 1 : 0);
 }
 
+// widths -> CSR offsets -> totals to the host (ev_total); does not wait for them
+gdx_status IntervalHits::count(cudaStream_t st, const uint64_t *starts, const uint64_t *ends, uint64_t n) {
+    CUDA_TRY(counts.reserve((n + 1) * 8));
+    CUDA_TRY(offsets.reserve((n + 1) * 8));
+    CUDA_TRY(cudaMemsetAsync(d, 0, sizeof *d, st));
+    CUDA_TRY(cudaMemsetAsync(counts.as<uint64_t>() + n, 0, 8, st));
+    if (n) k_interval_counts<<<(unsigned)div_up(n, 256), 256, 0, st>>>(starts, ends, n, counts.as<uint64_t>(), &d->wide);
+    GDX_TRY(exclusive_sum(scan_tmp, counts.as<uint64_t>(), offsets.as<uint64_t>(), n + 1, st));
+    CUDA_TRY(cudaMemcpyAsync(&h->hits, offsets.as<uint64_t>() + n, 8, cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(cudaMemcpyAsync(&h->wide, &d->wide, 8, cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(cudaEventRecord(ev_total, st));
+    t_stats.kernel_launches += 2;
+    return GDX_OK;
+}
+
+// once the totals of count() are known (n_hits > 0): rows of every interval, then the walk to the hits
+gdx_status IntervalHits::expand_walk(const gdx_index *idx, cudaStream_t st, const uint64_t *starts, const uint64_t *ends,
+                                     uint64_t n, uint64_t n_hits, uint64_t n_wide, unsigned long long *walk_steps,
+                                     bool hit32) {
+    if (n_hits * 24 > rows.cap + hits.cap) {  // 8 B of rows + 16 B of hits per hit
+        size_t free_b = 0, total_b = 0;
+        CUDA_TRY(cudaMemGetInfo(&free_b, &total_b));
+        if (n_hits * 24 > free_b + rows.cap + hits.cap)
+            return fail(GDX_ERR_OOM, "%llu hits of one chunk do not fit into device memory; split the batch",
+                        (unsigned long long)n_hits);
+    }
+    CUDA_TRY(rows.reserve(n_hits * 8));
+    CUDA_TRY(hits.reserve(n_hits * 16));
+    CUDA_TRY(wide.reserve((n_wide + 1) * 8));
+    k_expand_rows<<<(unsigned)div_up(n, 256), 256, 0, st>>>(starts, ends, offsets.as<uint64_t>(), n, rows.as<uint64_t>(),
+                                                           wide.as<uint64_t>(), &d->cursor);
+    if (n_wide) {
+        dim3 grid((unsigned)n_wide, 32);
+        k_expand_big_rows<<<grid, 256, 0, st>>>(starts, ends, offsets.as<uint64_t>(), wide.as<uint64_t>(),
+                                                rows.as<uint64_t>());
+    }
+    GDX_TRY(dispatch_layout(idx->h.layout, [&](auto L) -> gdx_status {
+        launch_locate_walk<decltype(L)>(idx, rows.as<uint64_t>(), n_hits, hits.as<ulonglong2>(), walk_steps, st, hit32);
+        return GDX_OK;
+    }));
+    CUDA_TRY(cudaGetLastError());
+    t_stats.kernel_launches += 2 + (n_wide ? 1 : 0);
+    return GDX_OK;
+}
+
 // State of a pipelined gdx_locate_many: every chunk of the search pipeline continues, on its own
 // stream, with counts -> scan -> expand -> walk -> D2H of its hits, so that the locate kernels and the
 // hit copies of chunk k overlap the query upload of the later chunks.
 struct LocatePipe {
     const gdx_index *idx;
     Workspace *ws;
+    PinnedResult &res;      // the hits of all finished chunks
     uint64_t *hit_offsets;  // caller's array, nq + 1 entries (NULL in the compact form)
     uint32_t *hit_counts = nullptr;  // compact form: hits per query, nq entries, instead of the CSR offsets
     uint64_t hit_bytes = sizeof(gdx_hit);  // 16, or 8 for gdx_hit32
-    void *pinned = nullptr; // library-owned pinned hit buffer (grows)
-    uint64_t pinned_cap = 0;
-    uint64_t total = 0;     // hits of all finished chunks
     struct Pending {
         int slot;
         uint64_t q0, cq;
@@ -1950,24 +2106,8 @@ struct LocatePipe {
 
     // after k_search(mode 2) of a chunk: widths, exclusive scan, totals to the host
     gdx_status stage_counts(Slot &sl, int slot, uint64_t q0, uint64_t cq) {
-        CUDA_TRY(sl.counts.reserve((cq + 1) * 8));
-        CUDA_TRY(sl.local_off.reserve((cq + 1) * 8));
-        CUDA_TRY(cudaMemsetAsync(sl.d_words, 0, 4 * sizeof(uint64_t), sl.stream));
-        CUDA_TRY(cudaMemsetAsync(sl.counts.as<uint64_t>() + cq, 0, 8, sl.stream));
-        k_interval_counts<<<(unsigned)div_up(cq, 256), 256, 0, sl.stream>>>(
-            sl.out_a.as<uint64_t>(), sl.out_b.as<uint64_t>(), cq, sl.counts.as<uint64_t>(),
-            reinterpret_cast<unsigned long long *>(sl.d_words));
-        size_t tmp = 0;
-        CUDA_TRY(cub::DeviceScan::ExclusiveSum(nullptr, tmp, sl.counts.as<uint64_t>(), sl.local_off.as<uint64_t>(),
-                                               cq + 1, sl.stream));
-        CUDA_TRY(sl.scan_tmp.reserve(tmp));
-        CUDA_TRY(cub::DeviceScan::ExclusiveSum(sl.scan_tmp.p, tmp, sl.counts.as<uint64_t>(),
-                                               sl.local_off.as<uint64_t>(), cq + 1, sl.stream));
-        CUDA_TRY(cudaMemcpyAsync(sl.h_words, sl.local_off.as<uint64_t>() + cq, 8, cudaMemcpyDeviceToHost, sl.stream));
-        CUDA_TRY(cudaMemcpyAsync(sl.h_words + 1, sl.d_words, 8, cudaMemcpyDeviceToHost, sl.stream));
-        CUDA_TRY(cudaEventRecord(sl.ev_total, sl.stream));
+        GDX_TRY(sl.locate.count(sl.stream, sl.out_a.as<uint64_t>(), sl.out_b.as<uint64_t>(), cq));
         pending.push_back(Pending{slot, q0, cq, true});
-        t_stats.kernel_launches += 2;
         return GDX_OK;
     }
 
@@ -1985,75 +2125,44 @@ struct LocatePipe {
     gdx_status finish(const Pending &p) {
         if (!p.valid) return GDX_OK;
         Slot &sl = ws->slot[p.slot];
+        IntervalHits &ih = sl.locate;
         const uint64_t cq = p.cq, q0 = p.q0;
-        CUDA_TRY(cudaEventSynchronize(sl.ev_total));
-        const uint64_t n_hits = sl.h_words[0], nbig = sl.h_words[1], base = total;
+        CUDA_TRY(cudaEventSynchronize(ih.ev_total));
+        const uint64_t n_hits = ih.h->hits, base = res.used / hit_bytes;
         if (n_hits) {
-            if ((base + n_hits) * hit_bytes > pinned_cap) {  // grow the pinned result buffer (rare)
+            if ((base + n_hits) * hit_bytes > res.cap) {  // grow the pinned result buffer (rare)
+                // the hits of earlier chunks may still be on their way into it, on any slot stream
                 for (int s2 = 0; s2 < kSlots; ++s2) CUDA_TRY(cudaStreamSynchronize(ws->slot[s2].stream));
-                void *bigger = nullptr;
-                uint64_t cap = 0;
-                GDX_TRY(acquire_pinned_hits(idx, 2 * (base + n_hits) * hit_bytes, &bigger, &cap));
-                if (pinned) {
-                    memcpy(bigger, pinned, base * hit_bytes);
-                    release_pinned_hits(idx, pinned);
-                }
-                pinned = bigger;
-                pinned_cap = cap;
+                GDX_TRY(res.reserve((base + n_hits) * hit_bytes));
             }
-            size_t free_b = 0, total_b = 0;
-            if (n_hits * 24 > sl.rows.cap + sl.hits.cap) {
-                CUDA_TRY(cudaMemGetInfo(&free_b, &total_b));
-                if (n_hits * 24 > free_b + sl.rows.cap + sl.hits.cap)
-                    return fail(GDX_ERR_OOM, "%llu hits of one chunk do not fit into device memory; split the batch",
-                                (unsigned long long)n_hits);
-            }
-            CUDA_TRY(sl.rows.reserve(n_hits * 8));
-            CUDA_TRY(sl.hits.reserve(n_hits * 16));
-            CUDA_TRY(sl.big.reserve((nbig + 1) * 8));
-            cudaEvent_t ev_begin = ws->next_locate_event(sl), ev_end = ws->next_locate_event(sl);
-            CUDA_TRY(cudaEventRecord(ev_begin, sl.stream));
-            k_expand_rows<<<(unsigned)div_up(cq, 256), 256, 0, sl.stream>>>(
-                sl.out_a.as<uint64_t>(), sl.out_b.as<uint64_t>(), sl.local_off.as<uint64_t>(), cq,
-                sl.rows.as<uint64_t>(), sl.big.as<uint64_t>(), reinterpret_cast<unsigned long long *>(sl.d_words + 1));
-            if (nbig) {
-                dim3 grid((unsigned)nbig, 32);
-                k_expand_big_rows<<<grid, 256, 0, sl.stream>>>(sl.out_a.as<uint64_t>(), sl.out_b.as<uint64_t>(),
-                                                               sl.local_off.as<uint64_t>(), sl.big.as<uint64_t>(),
-                                                               sl.rows.as<uint64_t>());
-            }
-            unsigned long long *d_walk = reinterpret_cast<unsigned long long *>(ws->small.d + 10);
-            GDX_TRY(dispatch_layout(idx->h.layout, [&](auto L) -> gdx_status {
-                launch_locate_walk<decltype(L)>(idx, sl.rows.as<uint64_t>(), n_hits, sl.hits.as<ulonglong2>(), d_walk, sl.stream,
-                                                hit_bytes == 8);
-                return GDX_OK;
-            }));
-            CUDA_TRY(cudaGetLastError());
-            CUDA_TRY(cudaEventRecord(ev_end, sl.stream));
-            CUDA_TRY(cudaMemcpyAsync((uint8_t *)pinned + base * hit_bytes, sl.hits.p, n_hits * hit_bytes,
-                                     cudaMemcpyDeviceToHost, sl.stream));
+            const EventPairs::Pair ev = ih.timing.next();
+            CUDA_TRY(cudaEventRecord(ev.begin, sl.stream));
+            GDX_TRY(ih.expand_walk(idx, sl.stream, sl.out_a.as<uint64_t>(), sl.out_b.as<uint64_t>(), cq, n_hits, ih.h->wide,
+                                   &ws->cnt_d->locate_walk_steps, hit_bytes == 8));
+            CUDA_TRY(cudaEventRecord(ev.end, sl.stream));
+            CUDA_TRY(cudaMemcpyAsync((uint8_t *)res.p + res.used, ih.hits.p, n_hits * hit_bytes, cudaMemcpyDeviceToHost,
+                                     sl.stream));
             t_stats.d2h_bytes += n_hits * hit_bytes;
-            t_stats.kernel_launches += 2 + (nbig ? 1 : 0);
         }
         // per query: global CSR offsets (u64), or in the compact form just the number of hits (u32; the counts are
         // narrowed into the offsets buffer, which the expansion above no longer needs)
         const uint64_t per_q = hit_counts ? 4 : 8;
-        if (hit_counts) k_narrow_u64<<<(unsigned)div_up(cq, 256), 256, 0, sl.stream>>>(sl.counts.as<uint64_t>(), cq, sl.local_off.as<uint32_t>());
-        else k_add_base<<<(unsigned)div_up(cq, 256), 256, 0, sl.stream>>>(sl.local_off.as<uint64_t>(), cq, base);
+        if (hit_counts) k_narrow_u64<<<(unsigned)div_up(cq, 256), 256, 0, sl.stream>>>(ih.counts.as<uint64_t>(), cq, ih.offsets.as<uint32_t>());
+        else k_add_base<<<(unsigned)div_up(cq, 256), 256, 0, sl.stream>>>(ih.offsets.as<uint64_t>(), cq, base);
         CUDA_TRY(cudaGetLastError());
         void *dst = hit_counts ? (void *)(hit_counts + q0) : (void *)(hit_offsets + q0);
         if (stage_offsets) {
             GDX_TRY(flush_offsets());  // frees the staging of the chunk before
             CUDA_TRY(sl.h_out_a.reserve(cq * per_q));
-            CUDA_TRY(cudaMemcpyAsync(sl.h_out_a.p, sl.local_off.p, cq * per_q, cudaMemcpyDeviceToHost, sl.stream));
+            CUDA_TRY(cudaMemcpyAsync(sl.h_out_a.p, ih.offsets.p, cq * per_q, cudaMemcpyDeviceToHost, sl.stream));
             CUDA_TRY(cudaEventRecord(sl.ev_out, sl.stream));
             pending_offsets = Pending{p.slot, q0, cq, true};
         } else {
-            CUDA_TRY(cudaMemcpyAsync(dst, sl.local_off.p, cq * per_q, cudaMemcpyDeviceToHost, sl.stream));
+            CUDA_TRY(cudaMemcpyAsync(dst, ih.offsets.p, cq * per_q, cudaMemcpyDeviceToHost, sl.stream));
         }
         t_stats.d2h_bytes += cq * per_q;
         t_stats.kernel_launches += 1;
-        total += n_hits;
+        res.used += n_hits * hit_bytes;
         return GDX_OK;
     }
 };
@@ -2065,14 +2174,11 @@ gdx_status search_host(const gdx_index *idx, Workspace *ws, const gdx_queries *q
                        uint32_t out_elem, int mode, LocatePipe *lp = nullptr) {
     const uint64_t nq = qs->nq;
     uint8_t *out_a = (uint8_t *)out_a_v, *out_b = (uint8_t *)out_b_v;
-    for (int s = 0; s < kSlots; ++s) ws->slot[s].ev_used = ws->slot[s].ev_loc_used = 0;
     // error words / counters are reset on slot 0's stream; the other slot streams (non-blocking: no implicit
     // ordering with anything) wait for that before their first kernel
-    CUDA_TRY(cudaMemsetAsync(ws->small.d, 0xff, 4 * sizeof(uint64_t), ws->slot[0].stream));
-    CUDA_TRY(cudaMemsetAsync(ws->small.d + 4, 0, 12 * sizeof(uint64_t), ws->slot[0].stream));
+    CUDA_TRY(ws->reset_counters(ws->slot[0].stream));
     CUDA_TRY(cudaEventRecord(ws->ev_a, ws->slot[0].stream));
     for (int s = 1; s < kSlots; ++s) CUDA_TRY(cudaStreamWaitEvent(ws->slot[s].stream, ws->ev_a, 0));
-    unsigned long long *d_steps = reinterpret_cast<unsigned long long *>(ws->small.d + 4);
     static const bool trace = getenv("GDX_TRACE") && atoi(getenv("GDX_TRACE")) != 0;
     struct TraceRow {
         int k;
@@ -2394,9 +2500,9 @@ gdx_status search_host(const gdx_index *idx, Workspace *ws, const gdx_queries *q
             CUDA_TRY(cudaEventRecord(sl.ev_h2d, sl.stream));
             sl.h2d_pending = true;
         }
-        cudaEvent_t e0 = ws->next_event(sl), e1 = ws->next_event(sl);
-        CUDA_TRY(cudaEventRecord(e0, sl.stream));
-        if (trace) trace_rows.push_back(TraceRow{k, cq, chunk_packed || prepacked ? (nsym + 3) / 4 : nsym, ev_h2d, e0, e1, nullptr, stage_ms});
+        const EventPairs::Pair ev = sl.timing.next();
+        CUDA_TRY(cudaEventRecord(ev.begin, sl.stream));
+        if (trace) trace_rows.push_back(TraceRow{k, cq, chunk_packed || prepacked ? (nsym + 3) / 4 : nsym, ev_h2d, ev.begin, ev.end, nullptr, stage_ms});
         const uint32_t *perm = nullptr;
         if (sp.use) {
             CUDA_TRY(sl.sort.reserve(sp.total_bytes));
@@ -2404,16 +2510,16 @@ gdx_status search_host(const gdx_index *idx, Workspace *ws, const gdx_queries *q
             t_stats.kernel_launches += 2;
         }
         gdx_status st = dispatch_layout(idx->h.layout, [&](auto L) -> gdx_status {
-            launch_search<decltype(L)>(idx, dq, a, b, mode, narrow, q0, ws->small.d + (k % kSlots), d_steps, perm, nullptr,
-                                       sl.stream);
+            launch_search<decltype(L)>(idx, dq, a, b, mode, narrow, q0, &ws->cnt_d->err[k % kSlots], &ws->cnt_d->search, perm,
+                                       nullptr, sl.stream);
             if (nx)  // overwrites the slots of the queries the packed kernel could not see correctly
-                launch_search<decltype(L)>(idx, xq, a, b, mode, narrow, q0, ws->small.d + (k % kSlots), d_steps, nullptr,
-                                           x_slots, sl.stream);
+                launch_search<decltype(L)>(idx, xq, a, b, mode, narrow, q0, &ws->cnt_d->err[k % kSlots], &ws->cnt_d->search,
+                                           nullptr, x_slots, sl.stream);
             return GDX_OK;
         });
         GDX_TRY(st);
         CUDA_TRY(cudaGetLastError());
-        CUDA_TRY(cudaEventRecord(e1, sl.stream));
+        CUDA_TRY(cudaEventRecord(ev.end, sl.stream));
         if (chunk_packed || prepacked) packed_queries += cq;
         exception_queries += nx;
         if (lp) {  // locate continues per chunk; the previous chunk is finished while this one runs
@@ -2469,25 +2575,19 @@ gdx_status search_host(const gdx_index *idx, Workspace *ws, const gdx_queries *q
             cudaEventDestroy(r.d2h_end);
         }
     }
-    CUDA_TRY(cudaMemcpy(ws->small.h, ws->small.d, 16 * sizeof(uint64_t), cudaMemcpyDeviceToHost));
+    CUDA_TRY(ws->read_counters(ws->slot[0].stream));
+    CUDA_TRY(cudaStreamSynchronize(ws->slot[0].stream));
+    const Counters &c = *ws->cnt_h;
     double ms = 0, ms_loc = 0;
     for (int s = 0; s < kSlots; ++s) {
-        for (size_t i = 0; i + 1 < ws->slot[s].ev_used; i += 2) {
-            float t = 0;
-            cudaEventElapsedTime(&t, ws->slot[s].ev[i], ws->slot[s].ev[i + 1]);
-            ms += t;
-        }
-        for (size_t i = 0; i + 1 < ws->slot[s].ev_loc_used; i += 2) {
-            float t = 0;
-            cudaEventElapsedTime(&t, ws->slot[s].ev_loc[i], ws->slot[s].ev_loc[i + 1]);
-            ms_loc += t;
-        }
+        ms += ws->slot[s].timing.elapsed_ms();
+        ms_loc += ws->slot[s].locate.timing.elapsed_ms();
     }
     t_stats.queries = nq;
-    t_stats.lf_steps = ws->small.h[4];
-    t_stats.walk_steps = ws->small.h[5] + ws->small.h[10];
-    t_stats.locate_walk_steps = ws->small.h[10];
-    t_stats.verified_queries = ws->small.h[9];
+    t_stats.lf_steps = c.search.lf_steps;
+    t_stats.walk_steps = c.search.verify_walk_steps + c.locate_walk_steps;
+    t_stats.locate_walk_steps = c.locate_walk_steps;
+    t_stats.verified_queries = c.search.verified_rows;
     t_stats.kernel_ms_search = ms;
     t_stats.kernel_ms_locate = ms_loc;
     t_stats.packed_queries = packed_queries;
@@ -2495,7 +2595,7 @@ gdx_status search_host(const gdx_index *idx, Workspace *ws, const gdx_queries *q
     t_stats.h2d_bytes = h2d_bytes;
     t_stats.d2h_bytes += d2h_bytes;
     uint64_t bad = kNoError;
-    for (int s = 0; s < kSlots; ++s) bad = std::min(bad, ws->small.h[s]);
+    for (int s = 0; s < kSlots; ++s) bad = std::min(bad, c.err[s]);
     if (bad != kNoError && (bad & kBadOffsetFlag)) {
         t_error_query = bad & ~kBadOffsetFlag;
         return fail(GDX_ERR_BAD_ARG, "query %llu: queries->offsets must not decrease and must stay inside the batch",
@@ -2516,59 +2616,20 @@ gdx_status begin_call(const gdx_index *idx, const char *what) {
     return GDX_OK;
 }
 
-// CSR + expand + walk on device-resident intervals; results in ws->hit_offsets (n+1) and ws->hits.
+// CSR + expand + walk on device-resident intervals, on slot 0's stream; results in ws->locate (offsets: n + 1, hits)
 gdx_status locate_device_intervals(const gdx_index *idx, Workspace *ws, const uint64_t *d_starts,
                                    const uint64_t *d_ends, uint64_t n, uint64_t *total_out) {
     cudaStream_t st = ws->slot[0].stream;
-    CUDA_TRY(ws->counts.reserve((n + 1) * 8));
-    CUDA_TRY(ws->hit_offsets.reserve((n + 1) * 8));
-    CUDA_TRY(cudaMemsetAsync(ws->small.d + 4, 0, 12 * sizeof(uint64_t), st));
-    CUDA_TRY(cudaMemsetAsync(ws->counts.as<uint64_t>() + n, 0, 8, st));
-    unsigned long long *d_big = reinterpret_cast<unsigned long long *>(ws->small.d + 6);
-    CUDA_TRY(cudaEventRecord(ws->ev_a, st));
-    if (n) k_interval_counts<<<(unsigned)div_up(n, 256), 256, 0, st>>>(d_starts, d_ends, n, ws->counts.as<uint64_t>(), d_big);
-    size_t tmp_bytes = 0;
-    CUDA_TRY(cub::DeviceScan::ExclusiveSum(nullptr, tmp_bytes, ws->counts.as<uint64_t>(),
-                                           ws->hit_offsets.as<uint64_t>(), n + 1, st));
-    CUDA_TRY(ws->scan_tmp.reserve(tmp_bytes));
-    CUDA_TRY(cub::DeviceScan::ExclusiveSum(ws->scan_tmp.p, tmp_bytes, ws->counts.as<uint64_t>(),
-                                           ws->hit_offsets.as<uint64_t>(), n + 1, st));
-    CUDA_TRY(cudaMemcpyAsync(ws->small.h + 8, ws->hit_offsets.as<uint64_t>() + n, 8, cudaMemcpyDeviceToHost, st));
-    CUDA_TRY(cudaMemcpyAsync(ws->small.h + 6, d_big, 8, cudaMemcpyDeviceToHost, st));
-    CUDA_TRY(cudaStreamSynchronize(st));
-    const uint64_t total = ws->small.h[8], nbig = ws->small.h[6];
+    IntervalHits &ih = ws->locate;
+    const EventPairs::Pair ev = ih.timing.next();
+    CUDA_TRY(cudaEventRecord(ev.begin, st));
+    GDX_TRY(ih.count(st, d_starts, d_ends, n));
+    CUDA_TRY(cudaEventSynchronize(ih.ev_total));
+    const uint64_t total = ih.h->hits;
     *total_out = total;
-    t_stats.kernel_launches += 2;
-    if (total) {
-        size_t free_b = 0, total_b = 0;
-        CUDA_TRY(cudaMemGetInfo(&free_b, &total_b));
-        const uint64_t need = (total > ws->rows.cap / 8 ? total * 8 : 0) + (total > ws->hits.cap / 16 ? total * 16 : 0);
-        if (need > free_b + ws->rows.cap + ws->hits.cap)
-            return fail(GDX_ERR_OOM, "%llu hits do not fit into device memory; split the batch",
-                        (unsigned long long)total);
-        CUDA_TRY(ws->rows.reserve(total * 8));
-        CUDA_TRY(ws->hits.reserve(total * 16));
-        CUDA_TRY(ws->big_list.reserve((nbig + 1) * 8));
-        unsigned long long *d_cursor = reinterpret_cast<unsigned long long *>(ws->small.d + 7);
-        k_expand_rows<<<(unsigned)div_up(n, 256), 256, 0, st>>>(d_starts, d_ends, ws->hit_offsets.as<uint64_t>(), n,
-                                                               ws->rows.as<uint64_t>(), ws->big_list.as<uint64_t>(),
-                                                               d_cursor);
-        if (nbig) {
-            dim3 grid((unsigned)nbig, 32);
-            k_expand_big_rows<<<grid, 256, 0, st>>>(d_starts, d_ends, ws->hit_offsets.as<uint64_t>(),
-                                                    ws->big_list.as<uint64_t>(), ws->rows.as<uint64_t>());
-            t_stats.kernel_launches += 1;
-        }
-        unsigned long long *d_walk = reinterpret_cast<unsigned long long *>(ws->small.d + 10);
-        gdx_status s2 = dispatch_layout(idx->h.layout, [&](auto L) -> gdx_status {
-            launch_locate_walk<decltype(L)>(idx, ws->rows.as<uint64_t>(), total, ws->hits.as<ulonglong2>(), d_walk, st);
-            return GDX_OK;
-        });
-        GDX_TRY(s2);
-        CUDA_TRY(cudaGetLastError());
-        t_stats.kernel_launches += 2;
-    }
-    CUDA_TRY(cudaEventRecord(ws->ev_b, st));
+    if (total)
+        GDX_TRY(ih.expand_walk(idx, st, d_starts, d_ends, n, total, ih.h->wide, &ws->cnt_d->locate_walk_steps, false));
+    CUDA_TRY(cudaEventRecord(ev.end, st));
     return GDX_OK;
 }
 
@@ -2616,9 +2677,9 @@ gdx_status finish_locate(const gdx_index *idx, Workspace *ws, uint64_t n, uint64
     void *h = nullptr;
     GDX_TRY(acquire_pinned_hits(idx, total * sizeof(gdx_hit), &h));
     const gdx_status copied = [&]() -> gdx_status {
-        if (total) CUDA_TRY(cudaMemcpyAsync(h, ws->hits.p, total * sizeof(gdx_hit), cudaMemcpyDeviceToHost, st));
-        CUDA_TRY(cudaMemcpyAsync(hit_offsets, ws->hit_offsets.p, (n + 1) * 8, cudaMemcpyDeviceToHost, st));
-        CUDA_TRY(cudaMemcpyAsync(ws->small.h, ws->small.d, 16 * sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
+        if (total) CUDA_TRY(cudaMemcpyAsync(h, ws->locate.hits.p, total * sizeof(gdx_hit), cudaMemcpyDeviceToHost, st));
+        CUDA_TRY(cudaMemcpyAsync(hit_offsets, ws->locate.offsets.p, (n + 1) * 8, cudaMemcpyDeviceToHost, st));
+        CUDA_TRY(ws->read_counters(st));
         CUDA_TRY(cudaStreamSynchronize(st));
         return GDX_OK;
     }();
@@ -2627,12 +2688,10 @@ gdx_status finish_locate(const gdx_index *idx, Workspace *ws, uint64_t n, uint64
         release_pinned_hits(idx, h);
         return copied;
     }
-    float ms = 0;
-    cudaEventElapsedTime(&ms, ws->ev_a, ws->ev_b);
-    t_stats.kernel_ms_locate = ms;
+    t_stats.kernel_ms_locate = ws->locate.timing.elapsed_ms();
     t_stats.hits = total;
-    t_stats.walk_steps += ws->small.h[10];
-    t_stats.locate_walk_steps = ws->small.h[10];
+    t_stats.walk_steps += ws->cnt_h->locate_walk_steps;
+    t_stats.locate_walk_steps = ws->cnt_h->locate_walk_steps;
     *hits = (gdx_hit *)h;
     *num_hits = total;
     return GDX_OK;
@@ -2642,13 +2701,6 @@ gdx_status finish_locate(const gdx_index *idx, Workspace *ws, uint64_t n, uint64
 
 namespace {
 
-// a failed call must not return while one of its streams still reads or writes the caller's buffers; the error that
-// made it fail stays the reported one
-void drain(Workspace *ws) {
-    for (int s = 0; s < kSlots; ++s) cudaStreamSynchronize(ws->slot[s].stream);
-    cudaGetLastError();
-}
-
 // mode 0: cursors, 1: counts; elem: bytes per element of the caller's arrays
 gdx_status search_many_impl(const gdx_index *idx, const gdx_queries *queries, void *a, void *b, uint32_t elem, int mode,
                             const char *what) {
@@ -2656,13 +2708,7 @@ gdx_status search_many_impl(const gdx_index *idx, const gdx_queries *queries, vo
     GDX_TRY(check_queries(idx, queries));
     if (queries->nq && (!a || (mode == 0 && !b))) return fail(GDX_ERR_BAD_ARG, "output is NULL");
     if (elem == 4 && idx->h.wide) return fail(GDX_ERR_UNSUPPORTED, "32-bit results need a text shorter than 2^32 symbols");
-    std::shared_lock<std::shared_mutex> cfg(idx->cfg_mu);
-    DeviceGuard guard(idx->device);
-    WsLease lease(idx);
-    if (!lease.w) return fail(GDX_ERR_CUDA, "could not create a CUDA workspace: %s", cudaGetErrorString(cudaGetLastError()));
-    const gdx_status st = search_host(idx, lease.w, queries, a, b, elem, mode);
-    if (st != GDX_OK) drain(lease.w);  // copies into the caller's arrays may still be in flight
-    return st;
+    return with_workspace(idx, [&](Workspace *ws) { return search_host(idx, ws, queries, a, b, elem, mode); });
 }
 
 // write_last = false: hit_offsets[nq] is left alone (it is the first entry of the next shard's range)
@@ -2676,28 +2722,28 @@ gdx_status locate_many_impl(const gdx_index *idx, const gdx_queries *queries, ui
     *num_hits = 0;
     if (hit_counts && (idx->h.wide || idx->h.ntexts > 0xffffffffull))
         return fail(GDX_ERR_UNSUPPORTED, "32-bit hits need a text shorter than 2^32 symbols");
-    std::shared_lock<std::shared_mutex> cfg(idx->cfg_mu);
-    DeviceGuard guard(idx->device);
-    WsLease lease(idx);
-    Workspace *ws = lease.w;
-    if (!ws) return fail(GDX_ERR_CUDA, "could not create a CUDA workspace: %s", cudaGetErrorString(cudaGetLastError()));
     const uint64_t n = queries->nq;
-    // every chunk of the search pipeline carries on with counts -> scan -> expand -> walk -> D2H
-    LocatePipe lp{idx, ws, hit_offsets};
-    lp.hit_counts = hit_counts;
-    lp.hit_bytes = hit_counts ? 8 : sizeof(gdx_hit);
-    lp.stage_offsets = n * 8 >= kStageMinBytes && !is_pinned(hit_counts ? (const void *)hit_counts : (const void *)hit_offsets);
-    GDX_TRY(acquire_pinned_hits(idx, std::max<uint64_t>(n, 4096) * lp.hit_bytes, &lp.pinned, &lp.pinned_cap));
-    gdx_status st = search_host(idx, ws, queries, nullptr, nullptr, 8, 2, &lp);
+    const uint64_t hit_bytes = hit_counts ? 8 : sizeof(gdx_hit);
+    PinnedResult res{idx};
+    const gdx_status st = with_workspace(idx, [&](Workspace *ws) -> gdx_status {
+        // every chunk of the search pipeline carries on with counts -> scan -> expand -> walk -> D2H
+        LocatePipe lp{idx, ws, res, hit_offsets};
+        lp.hit_counts = hit_counts;
+        lp.hit_bytes = hit_bytes;
+        lp.stage_offsets =
+            n * 8 >= kStageMinBytes && !is_pinned(hit_counts ? (const void *)hit_counts : (const void *)hit_offsets);
+        GDX_TRY(acquire_pinned_hits(idx, std::max<uint64_t>(n, 4096) * hit_bytes, &res.p, &res.cap));
+        return search_host(idx, ws, queries, nullptr, nullptr, 8, 2, &lp);
+    });
     if (st != GDX_OK) {
-        drain(ws);
-        release_pinned_hits(idx, lp.pinned);
+        res.release();  // after with_workspace drained the streams: hit copies into it may have been in flight
         return st;
     }
-    if (write_last && hit_offsets) hit_offsets[n] = lp.total;
-    t_stats.hits = lp.total;
-    *hits = (gdx_hit *)lp.pinned;
-    *num_hits = lp.total;
+    const uint64_t total = res.used / hit_bytes;
+    if (write_last && hit_offsets) hit_offsets[n] = total;
+    t_stats.hits = total;
+    *hits = (gdx_hit *)res.p;
+    *num_hits = total;
     return GDX_OK;
 }
 
@@ -2995,23 +3041,19 @@ extern "C" gdx_status gdx_locate_intervals(const gdx_index *idx, const uint64_t 
         for (uint64_t i = 0; i < n; ++i)
             if (starts[i] > ends[i] || ends[i] > idx->h.n)
                 return fail(GDX_ERR_BAD_ARG, "interval %llu is not inside [0, text_len]", (unsigned long long)i);
-        std::shared_lock<std::shared_mutex> cfg(idx->cfg_mu);
-        DeviceGuard guard(idx->device);
-        WsLease lease(idx);
-        Workspace *ws = lease.w;
-        if (!ws) return fail(GDX_ERR_CUDA, "could not create a CUDA workspace: %s", cudaGetErrorString(cudaGetLastError()));
-        cudaStream_t st = ws->slot[0].stream;
-        CUDA_TRY(ws->starts.reserve((n + 1) * 8));
-        CUDA_TRY(ws->ends.reserve((n + 1) * 8));
-        if (n) {
-            CUDA_TRY(cudaMemcpyAsync(ws->starts.p, starts, n * 8, cudaMemcpyHostToDevice, st));
-            CUDA_TRY(cudaMemcpyAsync(ws->ends.p, ends, n * 8, cudaMemcpyHostToDevice, st));
-        }
-        uint64_t total = 0;
-        gdx_status rc = locate_device_intervals(idx, ws, ws->starts.as<uint64_t>(), ws->ends.as<uint64_t>(), n, &total);
-        if (rc == GDX_OK) rc = finish_locate(idx, ws, n, total, hit_offsets, hits, num_hits);
-        if (rc != GDX_OK) drain(ws);
-        return rc;
+        return with_workspace(idx, [&](Workspace *ws) -> gdx_status {
+            cudaStream_t st = ws->slot[0].stream;
+            CUDA_TRY(ws->starts.reserve((n + 1) * 8));
+            CUDA_TRY(ws->ends.reserve((n + 1) * 8));
+            CUDA_TRY(ws->reset_counters(st));
+            if (n) {
+                CUDA_TRY(cudaMemcpyAsync(ws->starts.p, starts, n * 8, cudaMemcpyHostToDevice, st));
+                CUDA_TRY(cudaMemcpyAsync(ws->ends.p, ends, n * 8, cudaMemcpyHostToDevice, st));
+            }
+            uint64_t total = 0;
+            GDX_TRY(locate_device_intervals(idx, ws, ws->starts.as<uint64_t>(), ws->ends.as<uint64_t>(), n, &total));
+            return finish_locate(idx, ws, n, total, hit_offsets, hits, num_hits);
+        });
     });
 }
 
@@ -3031,14 +3073,7 @@ extern "C" gdx_status gdx_extend_many(const gdx_index *idx, uint64_t *starts, ui
         GDX_TRY(begin_call(idx, "gdx_extend_many"));
         if (n == 0) return GDX_OK;
         if (!starts || !ends || !io_symbols) return fail(GDX_ERR_BAD_ARG, "NULL argument");
-        std::shared_lock<std::shared_mutex> cfg(idx->cfg_mu);
-        DeviceGuard guard(idx->device);
-        WsLease lease(idx);
-        Workspace *ws = lease.w;
-        if (!ws) return fail(GDX_ERR_CUDA, "could not create a CUDA workspace: %s", cudaGetErrorString(cudaGetLastError()));
-        const gdx_status rc = extend_many_on(idx, ws, starts, ends, io_symbols, n);
-        if (rc != GDX_OK) drain(ws);
-        return rc;
+        return with_workspace(idx, [&](Workspace *ws) { return extend_many_on(idx, ws, starts, ends, io_symbols, n); });
     });
 }
 
@@ -3049,7 +3084,7 @@ static gdx_status extend_many_on(const gdx_index *idx, Workspace *ws, uint64_t *
         CUDA_TRY(ws->starts.reserve(n * 8));
         CUDA_TRY(ws->ends.reserve(n * 8));
         CUDA_TRY(ws->symbols.reserve(n));
-        CUDA_TRY(cudaMemsetAsync(ws->small.d, 0xff, 16, st));  // [0] invalid symbol, [1] cursor out of bounds
+        CUDA_TRY(ws->reset_counters(st));
         CUDA_TRY(cudaStreamSynchronize(st));
         // large pageable cursor arrays go through pinned staging (see search_host)
         Slot &sl0 = ws->slot[0];
@@ -3079,7 +3114,7 @@ static gdx_status extend_many_on(const gdx_index *idx, Workspace *ws, uint64_t *
             CUDA_TRY(cudaMemcpyAsync(d_c + off, io_symbols + off, cn, cudaMemcpyHostToDevice, cs));
             GDX_TRY(dispatch_layout(idx->h.layout, [&](auto L) -> gdx_status {
                 k_extend<decltype(L)><<<(unsigned)div_up(cn, 256), 256, 0, cs>>>(idx->dev, d_s + off, d_e + off, d_c + off, cn,
-                                                                               ws->small.d, off);
+                                                                               &ws->cnt_d->extend_bad_symbol, off);
                 return GDX_OK;
             }));
             CUDA_TRY(cudaGetLastError());
@@ -3089,15 +3124,16 @@ static gdx_status extend_many_on(const gdx_index *idx, Workspace *ws, uint64_t *
             CUDA_TRY(cudaMemcpyAsync(dst_e + off, d_e + off, cn * 8, cudaMemcpyDeviceToHost, cs));
         }
         for (int s2 = 0; s2 < kSlots; ++s2) CUDA_TRY(cudaStreamSynchronize(ws->slot[s2].stream));
-        CUDA_TRY(cudaMemcpyAsync(ws->small.h, ws->small.d, 16, cudaMemcpyDeviceToHost, st));
+        CUDA_TRY(ws->read_counters(st));
         CUDA_TRY(cudaStreamSynchronize(st));
         t_stats.kernel_launches = launches;
-        if (ws->small.h[1] != kNoError)  // checked on the device: text_with_rank_support/mod.rs:106-110
-            return fail(GDX_ERR_BAD_ARG, "cursor %llu is outside [0, text_len]", (unsigned long long)ws->small.h[1]);
-        if (ws->small.h[0] != kNoError) {
-            t_error_query = ws->small.h[0];
+        const Counters &c = *ws->cnt_h;
+        if (c.extend_bad_cursor != kNoError)  // checked on the device: text_with_rank_support/mod.rs:106-110
+            return fail(GDX_ERR_BAD_ARG, "cursor %llu is outside [0, text_len]", (unsigned long long)c.extend_bad_cursor);
+        if (c.extend_bad_symbol != kNoError) {
+            t_error_query = c.extend_bad_symbol;
             return fail(GDX_ERR_INVALID_SYMBOL, "cursor %llu: symbol in io representation should be valid (alphabet.rs:195-198)",
-                        (unsigned long long)ws->small.h[0]);
+                        (unsigned long long)c.extend_bad_symbol);
         }
         if (stage) {
             HostPool::get().copy(starts, sl0.h_out_a.p, n * 8);
@@ -3184,42 +3220,21 @@ gdx_status hamming_error(uint64_t bad) {
                 (unsigned long long)t_error_query);
 }
 
-// the library-owned pinned buffer the results of all chunks are copied into (grows; the stream is idle then)
-struct HammingResult {
-    const gdx_index *idx;
-    void *p = nullptr;
-    uint64_t cap = 0, used = 0;  // bytes
-    gdx_status reserve(uint64_t bytes) {
-        if (bytes <= cap) return GDX_OK;
-        void *bigger = nullptr;
-        uint64_t c = 0;
-        GDX_TRY(acquire_pinned_hits(idx, std::max<uint64_t>(2 * bytes, 4096), &bigger, &c));
-        if (p) {
-            memcpy(bigger, p, used);
-            release_pinned_hits(idx, p);
-        }
-        p = bigger;
-        cap = c;
-        return GDX_OK;
-    }
-};
-
 // Chunks of kHammingChunkQueries over the queries [0, n_ok) on slot 0's stream: upload -> pass 1 (checks + counts)
 // -> [scan -> pass 2 (intervals) -> locate] -> results to the caller.  counts == NULL in kHammingCount mode: only
-// check the queries (an error is then looked for in front of a query the host refused).
+// check the queries (an error is then looked for in front of a query the host refused).  The per-query CSR lives in
+// slot 0's IntervalHits (used as scratch only), the locate of the intervals in the workspace's.
 gdx_status hamming_run(const gdx_index *idx, Workspace *ws, const gdx_queries *qs, uint32_t k, int mode, uint64_t n_ok,
-                       uint64_t *counts, uint64_t *offsets_out, HammingResult &res) {
+                       uint64_t *counts, uint64_t *offsets_out, PinnedResult &res) {
     Slot &sl = ws->slot[0];
+    IntervalHits &csr = sl.locate;
     cudaStream_t st = sl.stream;
-    sl.ev_used = 0;
     const uint64_t strata = k + 1;
     const uint64_t elem = mode == kHammingCursors ? sizeof(gdx_hamming_interval) : sizeof(gdx_hit);
-    uint64_t *d_err = ws->small.d, *d_exp = ws->small.d + 1;  // (locate_device_intervals owns words 4..15)
-    CUDA_TRY(cudaMemsetAsync(d_err, 0xff, 8, st));
-    CUDA_TRY(cudaMemsetAsync(d_exp, 0, 8, st));
+    uint64_t *d_err = &ws->cnt_d->err[0];
+    CUDA_TRY(ws->reset_counters(st));
     const bool src_pinned = n_ok && is_pinned(qs->bytes);
     uint64_t h2d = 0, d2h = 0, launches = 0;
-    double ms_loc = 0;
     for (uint64_t q0 = 0; q0 < n_ok; q0 += kHammingChunkQueries) {
         const uint64_t cq = std::min<uint64_t>(kHammingChunkQueries, n_ok - q0);
         const uint64_t sym0 = query_bytes_end(qs, q0), nsym = query_bytes_end(qs, q0 + cq) - sym0;
@@ -3253,21 +3268,21 @@ gdx_status hamming_run(const gdx_index *idx, Workspace *ws, const gdx_queries *q
         const bool intervals = mode != kHammingCount;
         CUDA_TRY(sl.out_a.reserve(cq * strata * 8));
         if (intervals) {
-            CUDA_TRY(sl.counts.reserve((cq + 1) * 8));
-            CUDA_TRY(sl.local_off.reserve((cq + 1) * 8));
-            CUDA_TRY(cudaMemsetAsync(sl.counts.as<uint64_t>() + cq, 0, 8, st));
+            CUDA_TRY(csr.counts.reserve((cq + 1) * 8));
+            CUDA_TRY(csr.offsets.reserve((cq + 1) * 8));
+            CUDA_TRY(cudaMemsetAsync(csr.counts.as<uint64_t>() + cq, 0, 8, st));
         }
         const unsigned grid = (unsigned)div_up(cq, 256);
-        cudaEvent_t e0 = ws->next_event(sl), e1 = ws->next_event(sl);
-        CUDA_TRY(cudaEventRecord(e0, st));
+        const EventPairs::Pair ev = sl.timing.next();
+        CUDA_TRY(cudaEventRecord(ev.begin, st));
         GDX_TRY(dispatch_layout(idx->h.layout, [&](auto L) -> gdx_status {
             k_hamming<decltype(L), 1><<<grid, 256, 0, st>>>(idx->dev, dq, k, q0, d_err, sl.out_a.as<uint64_t>(),
-                                                             intervals ? sl.counts.as<uint64_t>() : nullptr, nullptr,
-                                                             nullptr, nullptr, reinterpret_cast<unsigned long long *>(d_exp));
+                                                             intervals ? csr.counts.as<uint64_t>() : nullptr, nullptr,
+                                                             nullptr, nullptr, &ws->cnt_d->hamming_expansions);
             return GDX_OK;
         }));
         CUDA_TRY(cudaGetLastError());
-        CUDA_TRY(cudaEventRecord(e1, st));
+        CUDA_TRY(cudaEventRecord(ev.end, st));
         ++launches;
         if (!intervals) {
             if (counts) {
@@ -3275,30 +3290,25 @@ gdx_status hamming_run(const gdx_index *idx, Workspace *ws, const gdx_queries *q
                 CUDA_TRY(cudaMemcpyAsync(sl.h_out_a.p, sl.out_a.p, cq * strata * 8, cudaMemcpyDeviceToHost, st));
                 d2h += cq * strata * 8;
             }
-            CUDA_TRY(cudaMemcpyAsync(ws->small.h, d_err, 8, cudaMemcpyDeviceToHost, st));
+            CUDA_TRY(ws->read_counters(st));
             CUDA_TRY(cudaStreamSynchronize(st));
-            GDX_TRY(hamming_error(ws->small.h[0]));
+            GDX_TRY(hamming_error(ws->cnt_h->err[0]));
             if (counts) HostPool::get().copy(counts + q0 * strata, sl.h_out_a.p, cq * strata * 8);
             continue;
         }
         // CSR of the chunk's intervals
-        size_t tmp = 0;
-        CUDA_TRY(cub::DeviceScan::ExclusiveSum(nullptr, tmp, sl.counts.as<uint64_t>(), sl.local_off.as<uint64_t>(), cq + 1,
-                                               st));
-        CUDA_TRY(sl.scan_tmp.reserve(tmp));
-        CUDA_TRY(cub::DeviceScan::ExclusiveSum(sl.scan_tmp.p, tmp, sl.counts.as<uint64_t>(), sl.local_off.as<uint64_t>(),
-                                               cq + 1, st));
-        CUDA_TRY(cudaMemcpyAsync(ws->small.h, d_err, 8, cudaMemcpyDeviceToHost, st));
-        CUDA_TRY(cudaMemcpyAsync(ws->small.h + 1, sl.local_off.as<uint64_t>() + cq, 8, cudaMemcpyDeviceToHost, st));
+        GDX_TRY(exclusive_sum(csr.scan_tmp, csr.counts.as<uint64_t>(), csr.offsets.as<uint64_t>(), cq + 1, st));
+        CUDA_TRY(ws->read_counters(st));
+        CUDA_TRY(cudaMemcpyAsync(&csr.h->hits, csr.offsets.as<uint64_t>() + cq, 8, cudaMemcpyDeviceToHost, st));
         CUDA_TRY(cudaStreamSynchronize(st));
         ++launches;
-        GDX_TRY(hamming_error(ws->small.h[0]));
-        const uint64_t niv = ws->small.h[1];
+        GDX_TRY(hamming_error(ws->cnt_h->err[0]));
+        const uint64_t niv = csr.h->hits;
         // pass 2: the intervals at their CSR offsets in search order, a sort by start within every query, then records
         // (cursors) or starts / ends (the locate path)
         const uint64_t rec_bytes = mode == kHammingCursors ? sizeof(HammingInterval) : 8;
-        const uint64_t held = sl.rows.cap + sl.big.cap + ws->starts.cap + sl.xbuf.cap +
-                              (mode == kHammingCursors ? sl.hits.cap : ws->ends.cap);
+        const uint64_t held = csr.rows.cap + csr.wide.cap + ws->starts.cap + sl.xbuf.cap +
+                              (mode == kHammingCursors ? csr.hits.cap : ws->ends.cap);
         const uint64_t need = niv * (32 + rec_bytes);
         bool fits = niv <= 0x7fffffffull;  // (the segmented sort counts items in an int)
         if (fits && need > held) {
@@ -3310,45 +3320,45 @@ gdx_status hamming_run(const gdx_index *idx, Workspace *ws, const gdx_queries *q
             return fail(GDX_ERR_OOM, "%llu intervals of one chunk do not fit into device memory; split the batch",
                         (unsigned long long)niv);
         const uint64_t nr = std::max<uint64_t>(niv, 1);
-        CUDA_TRY(sl.rows.reserve(nr * 8));
-        CUDA_TRY(sl.big.reserve(nr * 8));
+        CUDA_TRY(csr.rows.reserve(nr * 8));
+        CUDA_TRY(csr.wide.reserve(nr * 8));
         CUDA_TRY(ws->starts.reserve(nr * 8));
         CUDA_TRY(sl.xbuf.reserve(nr * 8));
-        CUDA_TRY(mode == kHammingCursors ? sl.hits.reserve(nr * rec_bytes) : ws->ends.reserve(nr * 8));
+        CUDA_TRY(mode == kHammingCursors ? csr.hits.reserve(nr * rec_bytes) : ws->ends.reserve(nr * 8));
         if (niv) {
-            cudaEvent_t f0 = ws->next_event(sl), f1 = ws->next_event(sl);
-            CUDA_TRY(cudaEventRecord(f0, st));
+            const EventPairs::Pair ev2 = sl.timing.next();
+            CUDA_TRY(cudaEventRecord(ev2.begin, st));
             GDX_TRY(dispatch_layout(idx->h.layout, [&](auto L) -> gdx_status {
                 k_hamming<decltype(L), 2><<<grid, 256, 0, st>>>(idx->dev, dq, k, q0, nullptr, nullptr, nullptr,
-                                                                 sl.local_off.as<uint64_t>(), sl.rows.as<uint64_t>(),
-                                                                 sl.big.as<uint64_t>(), nullptr);
+                                                                 csr.offsets.as<uint64_t>(), csr.rows.as<uint64_t>(),
+                                                                 csr.wide.as<uint64_t>(), nullptr);
                 return GDX_OK;
             }));
             CUDA_TRY(cudaGetLastError());
             size_t sort_tmp = 0;
-            const uint64_t *seg = sl.local_off.as<uint64_t>();
-            CUDA_TRY(cub::DeviceSegmentedSort::SortPairs(nullptr, sort_tmp, sl.rows.as<uint64_t>(), ws->starts.as<uint64_t>(),
-                                                         sl.big.as<uint64_t>(), sl.xbuf.as<uint64_t>(), (int)niv, (int)cq,
+            const uint64_t *seg = csr.offsets.as<uint64_t>();
+            CUDA_TRY(cub::DeviceSegmentedSort::SortPairs(nullptr, sort_tmp, csr.rows.as<uint64_t>(), ws->starts.as<uint64_t>(),
+                                                         csr.wide.as<uint64_t>(), sl.xbuf.as<uint64_t>(), (int)niv, (int)cq,
                                                          seg, seg + 1, st));
             CUDA_TRY(sl.sort.reserve(sort_tmp));
-            CUDA_TRY(cub::DeviceSegmentedSort::SortPairs(sl.sort.p, sort_tmp, sl.rows.as<uint64_t>(), ws->starts.as<uint64_t>(),
-                                                         sl.big.as<uint64_t>(), sl.xbuf.as<uint64_t>(), (int)niv, (int)cq,
+            CUDA_TRY(cub::DeviceSegmentedSort::SortPairs(sl.sort.p, sort_tmp, csr.rows.as<uint64_t>(), ws->starts.as<uint64_t>(),
+                                                         csr.wide.as<uint64_t>(), sl.xbuf.as<uint64_t>(), (int)niv, (int)cq,
                                                          seg, seg + 1, st));
             k_hamming_decode<<<(unsigned)div_up(niv, 256), 256, 0, st>>>(
                 ws->starts.as<uint64_t>(), sl.xbuf.as<uint64_t>(), niv,
-                mode == kHammingCursors ? sl.hits.as<HammingInterval>() : nullptr,
+                mode == kHammingCursors ? csr.hits.as<HammingInterval>() : nullptr,
                 mode == kHammingCursors ? nullptr : ws->ends.as<uint64_t>());
             CUDA_TRY(cudaGetLastError());
-            CUDA_TRY(cudaEventRecord(f1, st));
+            CUDA_TRY(cudaEventRecord(ev2.end, st));
             launches += 3;
         }
         // results of the chunk: records (cursors) or hits (locate, the walk of gdx_locate_intervals) + per-query offsets
         uint64_t n_out = niv;
-        const uint64_t *d_query_off = sl.local_off.as<uint64_t>();
+        const uint64_t *d_query_off = csr.offsets.as<uint64_t>();
         if (mode == kHammingLocate) {
             GDX_TRY(locate_device_intervals(idx, ws, ws->starts.as<uint64_t>(), ws->ends.as<uint64_t>(), niv, &n_out));
             CUDA_TRY(sl.out_b.reserve(cq * 8));
-            k_gather_u64<<<grid, 256, 0, st>>>(sl.local_off.as<uint64_t>(), ws->hit_offsets.as<uint64_t>(), cq,
+            k_gather_u64<<<grid, 256, 0, st>>>(csr.offsets.as<uint64_t>(), ws->locate.offsets.as<uint64_t>(), cq,
                                                sl.out_b.as<uint64_t>());
             CUDA_TRY(cudaGetLastError());
             ++launches;
@@ -3357,7 +3367,7 @@ gdx_status hamming_run(const gdx_index *idx, Workspace *ws, const gdx_queries *q
         const uint64_t base = res.used / elem;
         GDX_TRY(res.reserve(res.used + n_out * elem));
         if (n_out) {
-            const void *d_src = mode == kHammingCursors ? sl.hits.p : ws->hits.p;
+            const void *d_src = mode == kHammingCursors ? csr.hits.p : ws->locate.hits.p;
             CUDA_TRY(cudaMemcpyAsync((uint8_t *)res.p + res.used, d_src, n_out * elem, cudaMemcpyDeviceToHost, st));
             d2h += n_out * elem;
         }
@@ -3365,26 +3375,16 @@ gdx_status hamming_run(const gdx_index *idx, Workspace *ws, const gdx_queries *q
         CUDA_TRY(cudaMemcpyAsync(sl.h_out_a.p, d_query_off, cq * 8, cudaMemcpyDeviceToHost, st));
         d2h += cq * 8;
         CUDA_TRY(cudaStreamSynchronize(st));
-        if (mode == kHammingLocate) {
-            float ms = 0;
-            if (cudaEventElapsedTime(&ms, ws->ev_a, ws->ev_b) == cudaSuccess) ms_loc += ms;
-        }
         const uint64_t *h_off = (const uint64_t *)sl.h_out_a.p;
         for (uint64_t i = 0; i < cq; ++i) offsets_out[q0 + i] = base + h_off[i];
         res.used += n_out * elem;
     }
-    CUDA_TRY(cudaMemcpyAsync(ws->small.h + 2, d_exp, 8, cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(ws->read_counters(st));
     CUDA_TRY(cudaStreamSynchronize(st));
-    double ms = 0;
-    for (size_t i = 0; i + 1 < sl.ev_used; i += 2) {
-        float t = 0;
-        cudaEventElapsedTime(&t, sl.ev[i], sl.ev[i + 1]);
-        ms += t;
-    }
     t_stats.queries = qs->nq;
-    t_stats.lf_steps = ws->small.h[2];
-    t_stats.kernel_ms_search = ms;
-    t_stats.kernel_ms_locate = ms_loc;
+    t_stats.lf_steps = ws->cnt_h->hamming_expansions;
+    t_stats.kernel_ms_search = sl.timing.elapsed_ms();
+    t_stats.kernel_ms_locate = ws->locate.timing.elapsed_ms();
     t_stats.kernel_launches += launches;
     t_stats.h2d_bytes = h2d;
     t_stats.d2h_bytes = d2h;
@@ -3409,29 +3409,21 @@ gdx_status hamming_many_impl(const gdx_index *idx, const gdx_queries *queries, u
     }
     gdx_status host_st = GDX_OK;
     const uint64_t n_ok = hamming_host_check(queries, &host_st);
-    std::shared_lock<std::shared_mutex> cfg(idx->cfg_mu);
-    DeviceGuard guard(idx->device);
-    WsLease lease(idx);
-    Workspace *ws = lease.w;
-    if (!ws) return fail(GDX_ERR_CUDA, "could not create a CUDA workspace: %s", cudaGetErrorString(cudaGetLastError()));
-    HammingResult res{idx};
-    gdx_status st = mode == kHammingCount ? GDX_OK : res.reserve(4096);
-    if (st == GDX_OK) {
+    PinnedResult res{idx};
+    const gdx_status st = with_workspace(idx, [&](Workspace *ws) -> gdx_status {
+        if (mode != kHammingCount) GDX_TRY(res.reserve(4096));
         // with a query the host refuses, the queries in front of it are only checked: a smaller offender wins
-        st = host_st == GDX_OK ? hamming_run(idx, ws, queries, k, mode, n_ok, counts, offsets_out, res)
-                               : hamming_run(idx, ws, queries, k, kHammingCount, n_ok, nullptr, nullptr, res);
-    }
-    if (st == GDX_OK && host_st != GDX_OK) {
+        if (host_st == GDX_OK) return hamming_run(idx, ws, queries, k, mode, n_ok, counts, offsets_out, res);
+        GDX_TRY(hamming_run(idx, ws, queries, k, kHammingCount, n_ok, nullptr, nullptr, res));
         t_error_query = n_ok;
-        st = host_st == GDX_ERR_BAD_ARG
-                 ? fail(GDX_ERR_BAD_ARG, "query %llu: queries->offsets must not decrease and must stay inside the batch",
-                        (unsigned long long)n_ok)
-                 : fail(GDX_ERR_UNSUPPORTED, "query %llu is longer than GDX_HAMMING_MAX_QUERY_LEN (%d symbols)",
-                        (unsigned long long)n_ok, GDX_HAMMING_MAX_QUERY_LEN);
-    }
+        return host_st == GDX_ERR_BAD_ARG
+                   ? fail(GDX_ERR_BAD_ARG, "query %llu: queries->offsets must not decrease and must stay inside the batch",
+                          (unsigned long long)n_ok)
+                   : fail(GDX_ERR_UNSUPPORTED, "query %llu is longer than GDX_HAMMING_MAX_QUERY_LEN (%d symbols)",
+                          (unsigned long long)n_ok, GDX_HAMMING_MAX_QUERY_LEN);
+    });
     if (st != GDX_OK) {
-        drain(ws);
-        if (res.p) release_pinned_hits(idx, res.p);
+        res.release();  // after with_workspace drained the stream: a copy into it may have been in flight
         return st;
     }
     if (mode != kHammingCount) {

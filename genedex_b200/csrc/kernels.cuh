@@ -602,11 +602,18 @@ constexpr int kModeNarrow = 8;  // mode flag: results are written as uint32
 // reference, which cannot express broken offsets at all)
 constexpr uint64_t kBadOffsetFlag = 1ull << 62;
 
+// what k_search adds up over its queries (warp totals, atomicAdd)
+struct SearchCounters {
+    unsigned long long lf_steps;           // LF steps of the search
+    unsigned long long verify_walk_steps;  // walk steps of the rows verified through the text section
+    unsigned long long verified_rows;      // rows verified through the text section
+};
+
 template <class L, bool VERIFY, bool CURSORS, bool PACKED>
 __global__ void __launch_bounds__(256, VERIFY ? L::kVerifyMinBlocks : L::kSearchMinBlocks)
 k_search(const __grid_constant__ DevIndex ix, const DevQueries qs, uint64_t *__restrict__ out_a,
          uint64_t *__restrict__ out_b, int mode_flags, uint64_t q_index_base, uint64_t *err,
-         unsigned long long *stat_steps, const uint32_t *__restrict__ perm,
+         SearchCounters *stats, const uint32_t *__restrict__ perm,
          const uint32_t *__restrict__ slot_map) {
     constexpr uint32_t kTabBytes = PACKED ? 4 : 256;
     constexpr uint32_t kStageWords = PACKED ? 1 : 256 * kQuerySlotWords;
@@ -823,14 +830,14 @@ k_search(const __grid_constant__ DevIndex ix, const DevQueries qs, uint64_t *__r
             out_b[slot_q] = direct ? kDirectHit : e;
         }
     }
-    if (stat_steps) {  // [0] LF steps of the search, [1] walk steps of verified rows, [5] verified rows
+    if (stats) {
         uint32_t tot = __reduce_add_sync(0xffffffffu, steps);
-        if ((threadIdx.x & 31) == 0 && tot) atomicAdd(stat_steps, (unsigned long long)tot);
+        if ((threadIdx.x & 31) == 0 && tot) atomicAdd(&stats->lf_steps, (unsigned long long)tot);
         if (VERIFY) {
             tot = __reduce_add_sync(0xffffffffu, vsteps);
-            if ((threadIdx.x & 31) == 0 && tot) atomicAdd(stat_steps + 1, (unsigned long long)tot);
+            if ((threadIdx.x & 31) == 0 && tot) atomicAdd(&stats->verify_walk_steps, (unsigned long long)tot);
             tot = __reduce_add_sync(0xffffffffu, vrows);
-            if ((threadIdx.x & 31) == 0 && tot) atomicAdd(stat_steps + 5, (unsigned long long)tot);
+            if ((threadIdx.x & 31) == 0 && tot) atomicAdd(&stats->verified_rows, (unsigned long long)tot);
         }
     }
 }
