@@ -19,7 +19,9 @@
 #include <mutex>
 #include <shared_mutex>
 #include <new>
+#include <numeric>
 #include <string>
+#include <utility>
 #include <vector>
 
 #include <cub/device/device_radix_sort.cuh>
@@ -27,6 +29,7 @@
 #include <cub/device/device_segmented_sort.cuh>
 
 #include "../../include/genedex_b200.h"
+#include "chunk_plan.h"
 #include "device_build.h"
 #include "device_index.h"
 #include "host_build.h"
@@ -185,10 +188,8 @@ uint64_t env_bytes(const char *name, uint64_t dflt) {
 const uint64_t kStageMinBytes = env_bytes("GDX_STAGE_MIN_BYTES", 4ull << 20);
 
 constexpr int kSlots = 3;
-// Pipeline chunking (defaults 4 / 32 / 4 MB, profiles/r1_ab_pipeline_chunks.txt): the byte budget of
-// successive chunks doubles from kChunkFirst to kChunkMax
-// (fast pipeline fill, then few large launches: less launch overhead and deeper shared suffixes for the
-// per-chunk query sort) and the batch ends with a chunk of about kChunkTail (short drain).
+// Pipeline chunking (defaults 4 / 32 / 4 MB, profiles/r1_ab_pipeline_chunks.txt; the schedule is gdx::ChunkPlan): large
+// launches give less launch overhead and deeper shared suffixes for the per-chunk query sort.
 uint64_t env_mb(const char *name, uint64_t dflt) {
     const char *e = getenv(name);
     return (uint64_t)(e && atoi(e) > 0 ? atoi(e) : dflt) << 20;
@@ -197,8 +198,6 @@ const uint64_t kChunkFirst = env_mb("GDX_CHUNK_FIRST_MB", 4);
 const uint64_t kChunkMax = env_mb("GDX_CHUNK_MAX_MB", 32);
 const uint64_t kChunkTail = env_mb("GDX_CHUNK_TAIL_MB", 4);
 constexpr uint64_t kChunkMaxQueries = 64ull << 20;
-// first guess of the host-to-device link rate for the hybrid upload of pinned IO bytes (search_host)
-constexpr double kLinkGuessBytesPerMs = 50e6;  // 50 GB/s
 
 // (begin, end) event pairs around the kernels of the current call, created on first use and kept for later calls
 struct EventPairs {
@@ -2072,59 +2071,108 @@ gdx_status IntervalHits::expand_walk(const gdx_index *idx, cudaStream_t st, cons
     return GDX_OK;
 }
 
+// host -> device copies on one stream: the bytes they put on the link, and whether one read pinned staging (busy till done)
+struct Uploads {
+    cudaStream_t st = nullptr;
+    uint64_t bytes = 0;
+    bool staged = false;
+    // through the pinned buffer `stage` (filled by the pool) unless stage is NULL or src already lies in it
+    cudaError_t copy(void *dst, const void *src, uint64_t n, HBuf *stage = nullptr) {
+        if (stage && src != stage->p) {
+            const cudaError_t e = stage->reserve(n);
+            if (e != cudaSuccess) return e;
+            HostPool::get().copy(stage->p, src, n);
+            src = stage->p;
+        }
+        staged |= stage != nullptr;
+        bytes += n;
+        return cudaMemcpyAsync(dst, src, n, cudaMemcpyHostToDevice, st);
+    }
+};
+
+// grow device buffers of one stream; growing one frees the old buffer, which is only safe once the stream has drained
+gdx_status reserve_drained(cudaStream_t st, std::initializer_list<std::pair<DBuf *, uint64_t>> bufs) {
+    if (std::any_of(bufs.begin(), bufs.end(), [](const std::pair<DBuf *, uint64_t> &b) { return b.first->cap < b.second; }))
+        CUDA_TRY(cudaStreamSynchronize(st));
+    for (const auto &b : bufs) CUDA_TRY(b.first->reserve(b.second));
+    return GDX_OK;
+}
+
+gdx_status bad_offsets(uint64_t q) {
+    t_error_query = q;
+    return fail(GDX_ERR_BAD_ARG, "query %llu: queries->offsets must not decrease and must stay inside the batch",
+                (unsigned long long)q);
+}
+
+// The error word of k_search / k_hamming: kNoError, or the smallest failing query -- with kBadOffsetFlag when its offsets
+// leave the uploaded chunk, else it holds a symbol the kernel refuses (message `invalid`).
+gdx_status kernel_error(uint64_t bad, const char *invalid) {
+    if (bad == kNoError) return GDX_OK;
+    if (bad & kBadOffsetFlag) return bad_offsets(bad & ~kBadOffsetFlag);
+    t_error_query = bad;
+    return fail(GDX_ERR_INVALID_SYMBOL, "query %llu: %s", (unsigned long long)bad, invalid);
+}
+
+// A chunk [q0, q0 + cq) of a slot.  As a handover: its results are on their way into the slot's pinned staging (until
+// ev_out), and the sink hands them to the caller one chunk later, while the copy of the next chunk is in flight.
+struct Handover {
+    Slot *sl = nullptr;
+    uint64_t q0 = 0, cq = 0;
+    // after the D2H of a chunk into s's staging: mark its end, hand the chunk before over (sink.hand_over)
+    template <class Sink>
+    gdx_status defer(Slot &s, uint64_t q0_, uint64_t cq_, Sink &sink) {
+        CUDA_TRY(cudaEventRecord(s.ev_out, s.stream));
+        return std::exchange(*this, Handover{&s, q0_, cq_}).flush(sink);
+    }
+    template <class Sink>
+    gdx_status flush(Sink &sink) {
+        Slot *s = std::exchange(sl, nullptr);
+        if (!s) return GDX_OK;
+        CUDA_TRY(cudaEventSynchronize(s->ev_out));
+        sink.hand_over(*s, q0, cq);
+        return GDX_OK;
+    }
+};
+
 // State of a pipelined gdx_locate_many: every chunk of the search pipeline continues, on its own
 // stream, with counts -> scan -> expand -> walk -> D2H of its hits, so that the locate kernels and the
 // hit copies of chunk k overlap the query upload of the later chunks.
 struct LocatePipe {
+    static constexpr int mode = 2;  // k_search: interval, or resolved text position for verified queries
+    static constexpr bool narrow = false, writes_b = true;
+    static constexpr uint32_t stage_elem = 0;
+    static constexpr uint64_t d2h = 0;  // (the locate chain counts its copies in t_stats itself)
     const gdx_index *idx;
     Workspace *ws;
     PinnedResult &res;      // the hits of all finished chunks
     uint64_t *hit_offsets;  // caller's array, nq + 1 entries (NULL in the compact form)
     uint32_t *hit_counts = nullptr;  // compact form: hits per query, nq entries, instead of the CSR offsets
     uint64_t hit_bytes = sizeof(gdx_hit);  // 16, or 8 for gdx_hit32
-    struct Pending {
-        int slot;
-        uint64_t q0, cq;
-        bool valid = false;
-    } pending_offsets;
+    bool stage_offsets = false;  // the caller's hit_offsets array is pageable
     // chunks whose hit totals are on their way to the host, oldest first.  A chunk is finished two chunks after
     // it was issued (kSlots - 1): by then its total has long arrived, so the issuing thread never waits for a
     // search kernel -- and its slot is only reused by the chunk after that.
-    std::deque<Pending> pending;
-    bool stage_offsets = false;  // the caller's hit_offsets array is pageable
-
-    // hand the previous chunk's CSR offsets from the slot's pinned staging to the caller
-    gdx_status flush_offsets() {
-        if (!pending_offsets.valid) return GDX_OK;
-        pending_offsets.valid = false;
-        Slot &ps = ws->slot[pending_offsets.slot];
-        CUDA_TRY(cudaEventSynchronize(ps.ev_out));
-        if (hit_counts) HostPool::get().copy(hit_counts + pending_offsets.q0, ps.h_out_a.p, pending_offsets.cq * 4);
-        else HostPool::get().copy(hit_offsets + pending_offsets.q0, ps.h_out_a.p, pending_offsets.cq * 8);
-        return GDX_OK;
-    }
-
-    // after k_search(mode 2) of a chunk: widths, exclusive scan, totals to the host
-    gdx_status stage_counts(Slot &sl, int slot, uint64_t q0, uint64_t cq) {
+    std::deque<Handover> pending;
+    Handover staged;  // offsets (or counts) of the last finished chunk
+    // widths, exclusive scan, totals to the host; the oldest chunk is finished meanwhile
+    gdx_status chunk(Slot &sl, uint64_t q0, uint64_t cq) {
         GDX_TRY(sl.locate.count(sl.stream, sl.out_a.as<uint64_t>(), sl.out_b.as<uint64_t>(), cq));
-        pending.push_back(Pending{slot, q0, cq, true});
-        return GDX_OK;
+        pending.push_back(Handover{&sl, q0, cq});
+        return pending.size() < (size_t)kSlots ? GDX_OK : finish_oldest();
     }
-
-    // the oldest chunk once more than `keep` are waiting (keep = 0: the oldest one, if any)
-    Pending take_pending(size_t keep) {
-        Pending p;
-        if (pending.size() > keep) {
-            p = pending.front();
-            pending.pop_front();
-        }
-        return p;
+    gdx_status finish() {
+        while (!pending.empty()) GDX_TRY(finish_oldest());
+        return staged.flush(*this);
     }
-
+    // per query: global CSR offsets (u64), or in the compact form just the number of hits (u32)
+    uint64_t per_q() const { return hit_counts ? 4 : 8; }
+    void *dst(uint64_t q0) const { return hit_counts ? (void *)(hit_counts + q0) : (void *)(hit_offsets + q0); }
+    void hand_over(Slot &s, uint64_t q0, uint64_t cq) { HostPool::get().copy(dst(q0), s.h_out_a.p, cq * per_q()); }
     // once the chunk's number of hits is known: expand, walk, copy hits + global offsets out
-    gdx_status finish(const Pending &p) {
-        if (!p.valid) return GDX_OK;
-        Slot &sl = ws->slot[p.slot];
+    gdx_status finish_oldest() {
+        const Handover p = pending.front();
+        pending.pop_front();
+        Slot &sl = *p.sl;
         IntervalHits &ih = sl.locate;
         const uint64_t cq = p.cq, q0 = p.q0;
         CUDA_TRY(cudaEventSynchronize(ih.ev_total));
@@ -2144,21 +2192,17 @@ struct LocatePipe {
                                      sl.stream));
             t_stats.d2h_bytes += n_hits * hit_bytes;
         }
-        // per query: global CSR offsets (u64), or in the compact form just the number of hits (u32; the counts are
-        // narrowed into the offsets buffer, which the expansion above no longer needs)
-        const uint64_t per_q = hit_counts ? 4 : 8;
+        // (compact form: the counts are narrowed into the offsets buffer, which the expansion above no longer needs)
+        const uint64_t per_q = this->per_q();
         if (hit_counts) k_narrow_u64<<<(unsigned)div_up(cq, 256), 256, 0, sl.stream>>>(ih.counts.as<uint64_t>(), cq, ih.offsets.as<uint32_t>());
         else k_add_base<<<(unsigned)div_up(cq, 256), 256, 0, sl.stream>>>(ih.offsets.as<uint64_t>(), cq, base);
         CUDA_TRY(cudaGetLastError());
-        void *dst = hit_counts ? (void *)(hit_counts + q0) : (void *)(hit_offsets + q0);
         if (stage_offsets) {
-            GDX_TRY(flush_offsets());  // frees the staging of the chunk before
             CUDA_TRY(sl.h_out_a.reserve(cq * per_q));
             CUDA_TRY(cudaMemcpyAsync(sl.h_out_a.p, ih.offsets.p, cq * per_q, cudaMemcpyDeviceToHost, sl.stream));
-            CUDA_TRY(cudaEventRecord(sl.ev_out, sl.stream));
-            pending_offsets = Pending{p.slot, q0, cq, true};
+            GDX_TRY(staged.defer(sl, q0, cq, *this));
         } else {
-            CUDA_TRY(cudaMemcpyAsync(dst, ih.offsets.p, cq * per_q, cudaMemcpyDeviceToHost, sl.stream));
+            CUDA_TRY(cudaMemcpyAsync(dst(q0), ih.offsets.p, cq * per_q, cudaMemcpyDeviceToHost, sl.stream));
         }
         t_stats.d2h_bytes += cq * per_q;
         t_stats.kernel_launches += 1;
@@ -2167,447 +2211,329 @@ struct LocatePipe {
     }
 };
 
-// Chunked pipeline over kSlots streams: stage / pack -> H2D(queries) -> k_search -> D2H(results) per chunk.
-// With lp (locate, mode 2) the results stay on the device and every chunk continues in the LocatePipe.
-// out_elem: bytes per element of the caller's result arrays (8, or 4 for the *_u32 entry points).
-gdx_status search_host(const gdx_index *idx, Workspace *ws, const gdx_queries *qs, void *out_a_v, void *out_b_v,
-                       uint32_t out_elem, int mode, LocatePipe *lp = nullptr) {
+// Counts (mode 1) or cursors (mode 0: out_a and out_b) of gdx_count_many / gdx_cursors_many: D2H straight into the
+// caller's arrays, or into the slots' pinned staging, handed over by the pool one chunk later.  The results are uint32
+// on the device for the u32 entry points and for large batches of the u64 ones (widened on the way out); pinned uint64
+// result arrays are filled by DMA without any CPU work, so they stay 64-bit on the wire.
+struct CountSink {
+    uint8_t *out_a, *out_b;
+    uint32_t out_elem;  // bytes per element of the caller's arrays: 8, or 4 for the *_u32 entry points
+    int mode;
+    bool writes_b, narrow, widen, stage;
+    uint32_t dev_elem, stage_elem;  // bytes per result on the device (and on the wire); in staging (0: none)
+    uint64_t d2h = 0;  // bytes of the D2H copies
+    Handover staged;
+    CountSink(const gdx_index *idx, uint64_t nq, void *a, void *b, uint32_t elem, int mode_)
+        : out_a((uint8_t *)a), out_b((uint8_t *)b), out_elem(elem), mode(mode_), writes_b(mode_ == 0) {
+        const bool large = nq * 8 >= kStageMinBytes;
+        narrow = nq && !idx->h.wide &&
+                 (out_elem == 4 || (large && narrow_enabled() && !(is_pinned(out_a) && (mode != 0 || is_pinned(out_b)))));
+        widen = narrow && out_elem == 8;
+        stage = nq && (widen || (large && !is_pinned(out_a)));
+        dev_elem = narrow ? 4 : 8;  // (= out_elem unless the results are staged: widening implies staging)
+        stage_elem = stage ? dev_elem : 0;
+    }
+    gdx_status chunk(Slot &sl, uint64_t q0, uint64_t cq) {
+        const uint64_t n = cq * dev_elem;
+        CUDA_TRY(sl.h_out_a.reserve(cq * stage_elem));
+        CUDA_TRY(sl.h_out_b.reserve(writes_b ? cq * stage_elem : 0));
+        CUDA_TRY(cudaMemcpyAsync(stage ? sl.h_out_a.p : out_a + q0 * out_elem, sl.out_a.p, n, cudaMemcpyDeviceToHost, sl.stream));
+        if (writes_b)
+            CUDA_TRY(cudaMemcpyAsync(stage ? sl.h_out_b.p : out_b + q0 * out_elem, sl.out_b.p, n, cudaMemcpyDeviceToHost, sl.stream));
+        d2h += n * (writes_b ? 2 : 1);
+        return stage ? staged.defer(sl, q0, cq, *this) : GDX_OK;
+    }
+    gdx_status finish() { return staged.flush(*this); }
+    void hand_over(Slot &s, uint64_t q0, uint64_t cq) {
+        if (widen) {
+            HostPool::get().widen_u32((uint64_t *)out_a + q0, (const uint32_t *)s.h_out_a.p, cq);
+            if (writes_b) HostPool::get().widen_u32((uint64_t *)out_b + q0, (const uint32_t *)s.h_out_b.p, cq);
+        } else {
+            HostPool::get().copy(out_a + q0 * out_elem, s.h_out_a.p, cq * out_elem);
+            if (writes_b) HostPool::get().copy(out_b + q0 * out_elem, s.h_out_b.p, cq * out_elem);
+        }
+    }
+};
+
+// GDX_TRACE=1: the timeline of search_host's chunks (start of the upload, kernels, end of the D2H) on stderr
+struct Trace {
+    struct Row {
+        int k;
+        uint64_t nq, bytes;
+        EventPairs::Pair link, kernels;  // start of the upload .. end of the D2H; the kernels
+        double host_stage_ms;
+    };
+    const bool on = [] {
+        static const bool v = env_flag("GDX_TRACE", false);
+        return v;
+    }();
+    const std::chrono::steady_clock::time_point t0 = std::chrono::steady_clock::now();
+    EventPairs ev;
+    EventPairs::Pair link = {};  // of the current chunk
+    std::vector<Row> rows;
+    void chunk_begins(cudaStream_t st) { if (on) cudaEventRecord((link = ev.next()).begin, st); }
+    void kernels_recorded(int k, uint64_t nq, uint64_t bytes, const EventPairs::Pair &kernels, double stage_ms) {
+        if (on) rows.push_back(Row{k, nq, bytes, link, kernels, stage_ms});
+    }
+    void d2h_recorded(cudaStream_t st) { if (on) cudaEventRecord(rows.back().link.end, st); }
+    double ms() const {
+        return on ? std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count() : 0;
+    }
+    // once the streams have drained; t_issue: when the last chunk was issued
+    void print(double t_issue) {
+        if (rows.empty()) return;
+        fprintf(stderr, "[gdx trace] host: all chunks issued at %.3f ms, streams drained at %.3f ms (%u pool threads)\n", t_issue,
+                ms(), HostPool::get().threads());
+        cudaEvent_t base = rows[0].link.begin;
+        for (auto &r : rows) {
+            float a = 0, b = 0, c = 0, d = 0;
+            cudaError_t te = cudaEventElapsedTime(&a, base, r.link.begin);
+            if (te != cudaSuccess) fprintf(stderr, "[gdx trace] elapsed: %s\n", cudaGetErrorString(te));
+            cudaEventElapsedTime(&b, base, r.kernels.begin);
+            cudaEventElapsedTime(&c, base, r.kernels.end);
+            cudaEventElapsedTime(&d, base, r.link.end);
+            fprintf(stderr, "[gdx trace] chunk %2d slot %d nq %8llu h2d bytes %10llu host stage %.3f ms | h2d %.3f..%.3f | kernels %.3f..%.3f | d2h ..%.3f\n",
+                    r.k, r.k % kSlots, (unsigned long long)r.nq, (unsigned long long)r.bytes, r.host_stage_ms, a, b, b, c, d);
+        }
+        ev.destroy();
+    }
+};
+
+// uploads of a hybrid batch that may still be on the link, oldest first; each has left it once its slot's ev_link fired
+struct LinkQueue {
+    std::vector<std::pair<const Slot *, uint64_t>> q;  // (slot, bytes)
+    cudaError_t push(Slot &sl, uint64_t bytes) {
+        // this slot's event is about to be re-recorded: its older upload has long left the link
+        q.erase(std::remove_if(q.begin(), q.end(), [&](const auto &u) { return u.first == &sl; }), q.end());
+        q.emplace_back(&sl, bytes);
+        return cudaEventRecord(sl.ev_link, sl.stream);
+    }
+    uint64_t backlog() {
+        while (!q.empty() && cudaEventQuery(q.front().first->ev_link) == cudaSuccess) q.erase(q.begin());
+        return std::accumulate(q.begin(), q.end(), 0ull, [](uint64_t b, const auto &u) { return b + u.second; });
+    }
+};
+
+// The staging of search_host: per call, which caller buffers go through pinned staging and the packer's exception
+// lists; per chunk, what stage_chunk made of it.
+struct Staging {
+    bool in, off;  // the symbols, the u64 offsets: pageable memory of a large batch
+    bool off32;    // large variable-length batch: offsets cross chunk relative as u32 (chunks of < 2^32 symbols)
+    std::vector<uint64_t> exc;    // symbol positions (chunk relative) the packer could not encode
+    std::vector<uint32_t> exc_q;  // the queries (chunk relative) that hold them
+    DevQueries dq, xq;  // the chunk; its queries with a byte without a 2-bit code (IO bytes, re-run into x_slots)
+    const uint32_t *x_slots;
+    bool packed;  // packed by the host
+    double stage_ms;
+    Uploads up;
+};
+
+// The uploads of one chunk on its slot's stream: its symbols (host-packed, pre-packed or IO bytes), its offsets (u32
+// chunk relative or u64) and, for a host-packed chunk, the queries with a byte the packer has no code for.
+gdx_status stage_chunk(const gdx_index *idx, const gdx_queries *qs, const gdx::Chunk &c, gdx::ChunkPlan &plan,
+                       Slot &sl, Staging &u) {
+    if (sl.h2d_pending) {  // the slot's staging buffers are free again once their last upload is done
+        CUDA_TRY(cudaEventSynchronize(sl.ev_h2d));
+        sl.h2d_pending = false;
+    }
+    const auto t0 = std::chrono::steady_clock::now();
+    const uint64_t q0 = c.q0, cq = c.cq(), sym0 = c.sym0, nsym = c.nsym();
+    u.xq = DevQueries{};
+    u.packed = false;
+    u.up = Uploads{sl.stream};
+    if (nsym && c.pack) {
+        CUDA_TRY(sl.h_in.reserve((nsym + 3) / 4 + 8));
+        pack2_parallel(idx->pack, qs->bytes + sym0, nsym, (uint8_t *)sl.h_in.p, u.exc);
+        gdx::exception_queries(qs->offsets, qs->fixed_len, q0, c.q1, sym0, u.exc, u.exc_q);
+        u.packed = u.exc_q.size() * 16 <= cq;
+        if (u.packed) CUDA_TRY(u.up.copy(sl.bytes.p, sl.h_in.p, (nsym + 3) / 4, &sl.h_in));
+        else plan.packing_failed();
+    }
+    const bool words = u.packed || plan.prepacked;  // the kernel reads 2-bit words
+    DevQueries &dq = u.dq = DevQueries{words ? nullptr : sl.bytes.as<uint8_t>(), nullptr, nullptr, qs->fixed_len, cq, 0, 0,
+                                       words ? sl.bytes.as<uint32_t>() : nullptr, nsym};
+    if (nsym && plan.prepacked) {  // the caller's stream, from the byte that holds the chunk's first symbol
+        const uint64_t b0 = sym0 / 4, b1 = (c.sym1 + 3) / 4;
+        CUDA_TRY(u.up.copy(sl.bytes.p, qs->bytes + b0, b1 - b0, u.in ? &sl.h_in : nullptr));
+        dq.shift = sym0 & 3;
+        dq.limit = nsym + dq.shift;
+    } else if (nsym && !u.packed) {
+        CUDA_TRY(u.up.copy(sl.bytes.p, qs->bytes + sym0, nsym, u.in ? &sl.h_in : nullptr));
+    }
+    if (qs->offsets && u.off32 && nsym + 4 < 0xffffffffull) {
+        // chunk-relative 32-bit offsets, narrowed by the pool into pinned staging: half the PCIe bytes
+        CUDA_TRY(sl.h_off.reserve((cq + 1) * 4));
+        const uint64_t *osrc = qs->offsets + q0;
+        uint32_t *o32 = (uint32_t *)sl.h_off.p;
+        const uint64_t rel = sym0 - dq.shift, cnt = cq + 1;
+        constexpr uint64_t kPiece = 1ull << 18;
+        HostPool::get().parallel_for(div_up(cnt, kPiece), [&](uint64_t piece) {
+            const uint64_t lo = piece * kPiece, hi = std::min(cnt, lo + kPiece);
+            for (uint64_t i = lo; i < hi; ++i) o32[i] = (uint32_t)(osrc[i] - rel);
+        });
+        CUDA_TRY(u.up.copy(sl.offsets.p, o32, cnt * 4, &sl.h_off));
+        dq.offsets32 = sl.offsets.as<uint32_t>();
+        dq.shift = 0;
+    } else if (qs->offsets) {
+        CUDA_TRY(u.up.copy(sl.offsets.p, qs->offsets + q0, (cq + 1) * 8, u.off ? &sl.h_off : nullptr));
+        dq.offsets = sl.offsets.as<uint64_t>();
+        dq.base = sym0 - dq.shift;
+        dq.shift = 0;
+    }
+    // queries with an exception byte: their offsets, result slots and IO bytes in one upload
+    const uint64_t nx = u.packed ? u.exc_q.size() : 0;
+    if (nx) {
+        uint64_t xbytes = 0;
+        for (uint32_t q : u.exc_q) xbytes += query_bytes_end(qs, q0 + q + 1) - query_bytes_end(qs, q0 + q);
+        const uint64_t off_slots = (nx + 1) * 8, off_bytes = align_up(off_slots + nx * 4, 8), tot = off_bytes + xbytes + 8;
+        GDX_TRY(reserve_drained(sl.stream, {{&sl.xbuf, tot}}));
+        CUDA_TRY(sl.h_x.reserve(tot));
+        uint64_t *xo = (uint64_t *)sl.h_x.p;
+        uint32_t *xs = (uint32_t *)((uint8_t *)sl.h_x.p + off_slots);
+        uint8_t *xb = (uint8_t *)sl.h_x.p + off_bytes;
+        uint64_t acc = 0;
+        for (uint64_t i = 0; i < nx; ++i) {
+            xo[i] = acc;
+            xs[i] = u.exc_q[i];
+            acc += query_bytes_end(qs, q0 + xs[i] + 1) - query_bytes_end(qs, q0 + xs[i]);
+        }
+        xo[nx] = acc;
+        constexpr uint64_t kPiece = 4096;  // queries per piece
+        HostPool::get().parallel_for(div_up(nx, kPiece), [&](uint64_t piece) {
+            const uint64_t lo = piece * kPiece, hi = std::min(nx, lo + kPiece);
+            for (uint64_t i = lo; i < hi; ++i) {
+                const uint64_t b0 = query_bytes_end(qs, q0 + xs[i]);
+                memcpy(xb + xo[i], qs->bytes + b0, xo[i + 1] - xo[i]);
+            }
+        });
+        CUDA_TRY(u.up.copy(sl.xbuf.p, sl.h_x.p, off_bytes + xbytes, &sl.h_x));
+        u.xq = DevQueries{sl.xbuf.as<uint8_t>() + off_bytes, sl.xbuf.as<uint64_t>(), nullptr, 0, nx, 0, 0, nullptr, xbytes};
+        u.x_slots = reinterpret_cast<const uint32_t *>(sl.xbuf.as<uint8_t>() + off_slots);
+    }
+    u.stage_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
+    if (u.up.staged) {
+        CUDA_TRY(cudaEventRecord(sl.ev_h2d, sl.stream));
+        sl.h2d_pending = true;
+    }
+    return GDX_OK;
+}
+
+// once search_host's streams have drained: its counters (device and host: io) into t_stats, error words into status
+gdx_status search_result(Workspace *ws, const gdx_stats &io) {
+    CUDA_TRY(ws->read_counters(ws->slot[0].stream));
+    CUDA_TRY(cudaStreamSynchronize(ws->slot[0].stream));
+    const Counters &cnt = *ws->cnt_h;
+    t_stats.queries = io.queries;
+    t_stats.packed_queries = io.packed_queries;
+    t_stats.exception_queries = io.exception_queries;
+    t_stats.h2d_bytes = io.h2d_bytes;
+    t_stats.d2h_bytes += io.d2h_bytes;
+    for (const Slot &s : ws->slot) {
+        t_stats.kernel_ms_search += s.timing.elapsed_ms();
+        t_stats.kernel_ms_locate += s.locate.timing.elapsed_ms();
+    }
+    t_stats.lf_steps = cnt.search.lf_steps;
+    t_stats.walk_steps = cnt.search.verify_walk_steps + cnt.locate_walk_steps;
+    t_stats.locate_walk_steps = cnt.locate_walk_steps;
+    t_stats.verified_queries = cnt.search.verified_rows;
+    return kernel_error(*std::min_element(cnt.err, cnt.err + kSlots),
+                        "symbol in io representation should be valid (alphabet.rs:195-198)");
+}
+
+// Chunked pipeline over kSlots streams: stage / pack -> H2D(queries) -> k_search -> sink per chunk.  The sink (CountSink
+// for counts and cursors, or LocatePipe) takes a chunk's results from the slot's out_a (out_b) in chunk() and completes
+// the call in finish(); the slots' pinned h_out_a (h_out_b) are sized for sink.stage_elem bytes per result.
+template <class Sink>
+gdx_status search_host(const gdx_index *idx, Workspace *ws, const gdx_queries *qs, Sink &sink) {
     const uint64_t nq = qs->nq;
-    uint8_t *out_a = (uint8_t *)out_a_v, *out_b = (uint8_t *)out_b_v;
     // error words / counters are reset on slot 0's stream; the other slot streams (non-blocking: no implicit
     // ordering with anything) wait for that before their first kernel
     CUDA_TRY(ws->reset_counters(ws->slot[0].stream));
     CUDA_TRY(cudaEventRecord(ws->ev_a, ws->slot[0].stream));
     for (int s = 1; s < kSlots; ++s) CUDA_TRY(cudaStreamWaitEvent(ws->slot[s].stream, ws->ev_a, 0));
-    static const bool trace = getenv("GDX_TRACE") && atoi(getenv("GDX_TRACE")) != 0;
-    struct TraceRow {
-        int k;
-        uint64_t nq, bytes;
-        cudaEvent_t h2d_begin, k_begin, k_end, d2h_end;
-        double host_stage_ms;
-    };
-    std::vector<TraceRow> trace_rows;
-    const auto t_host0 = std::chrono::steady_clock::now();
-    const uint64_t sym_end = query_bytes_end(qs, nq);
-    const uint64_t total_syms = sym_end - query_bytes_end(qs, 0);
+    Trace trace;
     const bool prepacked = qs->encoding == GDX_QUERIES_PACKED_2BIT;
+    const uint64_t total_syms = query_bytes_end(qs, nq) - query_bytes_end(qs, 0);
     const uint64_t total_in = prepacked ? (total_syms + 3) / 4 : total_syms;
     // Ordinary (pageable) caller memory would make every cudaMemcpyAsync a blocking, driver-staged copy at
     // 8-14 GB/s.  Large batches are staged through the slots' own pinned buffers instead, filled by the host
     // thread pool; while they are staged, IO bytes of a <= 4-symbol alphabet are packed to 2 bits (a quarter
     // of the PCIe bytes) -- that pays for pinned caller buffers too.
-    bool pack_on = nq && !prepacked && idx->pack.usable && pack_enabled() && total_in >= kPackMinBytes;
+    const bool pack = nq && !prepacked && idx->pack.usable && pack_enabled() && total_in >= kPackMinBytes;
     const bool src_pinned = nq && is_pinned(qs->bytes);
-    const bool stage_in = nq && total_in >= kStageMinBytes && !src_pinned;
-    // Pinned IO bytes can also cross the link as they are, by DMA, without any CPU work.  The host packer and
-    // the link then share the batch: before the pool starts on a packed chunk (which keeps the CPU busy for
-    // t_pack), a raw chunk is put on the link that is just large enough to keep it busy for that long on top of
-    // what is still queued there.  The queue is observed (events behind every upload), so a wrong guess of
-    // either rate corrects itself: too much raw data -> the backlog grows -> the next raw chunks shrink.
-    const bool hybrid = pack_on && src_pinned;
-    struct Upload {
-        int slot;
-        uint64_t bytes;
-    };
-    std::vector<Upload> on_link;  // uploads issued, oldest first; retired when their event has fired
-    auto link_backlog = [&]() -> uint64_t {
-        size_t done = 0;
-        while (done < on_link.size() && cudaEventQuery(ws->slot[on_link[done].slot].ev_link) == cudaSuccess) ++done;
-        on_link.erase(on_link.begin(), on_link.begin() + done);
-        uint64_t b = 0;
-        for (const Upload &u : on_link) b += u.bytes;
-        return b;
-    };
-    double pack_rate = 4.0e6 * HostPool::get().threads();  // symbols per ms, refined from every packed chunk
-    bool raw_next = hybrid;                                  // the link is idle at the start: open with a raw chunk
-    uint64_t raw_want = kChunkFirst;
-
-    const bool stage_off = nq && qs->offsets && nq * 8 >= kStageMinBytes && !is_pinned(qs->offsets);
-    const bool to_host = nq && !lp;
-    const bool large_out = nq * 8 >= kStageMinBytes;
-    // results as uint32 on the device: always for the u32 entry points, for large batches of the u64 ones
-    // (widened by the pool while they are handed to the caller)
-    // (pinned uint64 result arrays are filled by DMA without any CPU work: they stay 64-bit on the wire)
-    const bool narrow = to_host && !idx->h.wide &&
-                        (out_elem == 4 || (large_out && narrow_enabled() && !(is_pinned(out_a) && (mode != 0 || is_pinned(out_b)))));
-    const bool widen = narrow && out_elem == 8;
-    const bool stage_out = to_host && (widen || (large_out && !is_pinned(out_a)));
-    const uint32_t dev_elem = narrow ? 4 : 8;
-    struct PendingOut {
-        int slot = 0;
-        uint64_t q0 = 0, cq = 0;
-        bool valid = false;
-    } pend_out;
-    auto finish_out = [&](PendingOut &p) -> gdx_status {
-        if (!p.valid) return GDX_OK;
-        p.valid = false;
-        Slot &ps = ws->slot[p.slot];
-        CUDA_TRY(cudaEventSynchronize(ps.ev_out));
-        if (widen) {
-            HostPool::get().widen_u32((uint64_t *)out_a + p.q0, (const uint32_t *)ps.h_out_a.p, p.cq);
-            if (mode == 0) HostPool::get().widen_u32((uint64_t *)out_b + p.q0, (const uint32_t *)ps.h_out_b.p, p.cq);
-        } else {
-            HostPool::get().copy(out_a + p.q0 * out_elem, ps.h_out_a.p, p.cq * out_elem);
-            if (mode == 0) HostPool::get().copy(out_b + p.q0 * out_elem, ps.h_out_b.p, p.cq * out_elem);
-        }
-        return GDX_OK;
-    };
-    for (int s2 = 0; s2 < kSlots; ++s2) ws->slot[s2].h2d_pending = false;
+    Staging u{nq && total_in >= kStageMinBytes && !src_pinned,
+              nq && qs->offsets && nq * 8 >= kStageMinBytes && !is_pinned(qs->offsets),
+              qs->offsets && nq * 8 >= kStageMinBytes && narrow_enabled()};
+    gdx::ChunkPlan plan{qs->offsets, qs->fixed_len, qs->first_symbol, nq, prepacked, pack, pack && src_pinned,
+                        kChunkFirst, kChunkMax, kChunkTail, kChunkMaxQueries, 4.0e6 * HostPool::get().threads()};
+    LinkQueue link;
+    for (Slot &sl : ws->slot) sl.h2d_pending = false;
     // Large batches: size every slot once for the largest chunk this call can cut (the adaptive schedule cuts
     // different chunks in every call; growing a buffer in mid-flight means cudaFree / cudaFreeHost + a new
     // allocation, milliseconds each, with the streams drained).  The streams are idle here.
     if (nq && total_in >= kStageMinBytes) {
-        const uint64_t max_sym = std::min<uint64_t>(total_syms, 4 * kChunkMax) + 64;
+        const uint64_t max_sym = plan.max_chunk_symbols() + 64;
         const uint64_t max_q = qs->fixed_len ? std::min<uint64_t>(nq, max_sym / qs->fixed_len + 1) : 0;
-        for (int s2 = 0; s2 < kSlots; ++s2) {
-            Slot &sl = ws->slot[s2];
+        for (Slot &sl : ws->slot) {
             CUDA_TRY(sl.bytes.reserve(max_sym));
-            if (pack_on) CUDA_TRY(sl.h_in.reserve(max_sym / 4 + 8));
-            else if (stage_in) CUDA_TRY(sl.h_in.reserve(std::min<uint64_t>(total_in, kChunkMax) + 64));
-            if (max_q) {
-                CUDA_TRY(sl.out_a.reserve(max_q * 8));
-                if (mode == 0 || lp) CUDA_TRY(sl.out_b.reserve(max_q * 8));
-                if (stage_out) {
-                    CUDA_TRY(sl.h_out_a.reserve(max_q * dev_elem));
-                    if (mode == 0) CUDA_TRY(sl.h_out_b.reserve(max_q * dev_elem));
-                }
-            }
+            if (pack) CUDA_TRY(sl.h_in.reserve(max_sym / 4 + 8));
+            else if (u.in) CUDA_TRY(sl.h_in.reserve(std::min<uint64_t>(total_in, kChunkMax) + 64));
+            CUDA_TRY(sl.out_a.reserve(max_q * 8));
+            CUDA_TRY(sl.out_b.reserve(sink.writes_b ? max_q * 8 : 0));
+            CUDA_TRY(sl.h_out_a.reserve(max_q * sink.stage_elem));
+            CUDA_TRY(sl.h_out_b.reserve(sink.writes_b ? max_q * sink.stage_elem : 0));
         }
     }
-    std::vector<uint64_t> exc;       // symbol positions (chunk relative) the packer could not encode
-    std::vector<uint32_t> exc_q;     // the queries (chunk relative) that hold them
-    uint64_t packed_queries = 0, exception_queries = 0, h2d_bytes = 0, d2h_bytes = 0;
-    uint64_t budget = kChunkFirst;
-    uint64_t q0 = 0;
-    int k = 0;
-    while (q0 < nq) {
-        // chunk [q0, q1): about `budget` input bytes (packed bytes count four-fold: the budget is PCIe time),
-        // at least one query
-        bool pack_chunk = pack_on;
-        if (hybrid && pack_on && raw_next) pack_chunk = false;
-        const uint64_t unit = (pack_chunk || prepacked) ? 4 : 1;
-        const uint64_t remaining = sym_end - query_bytes_end(qs, q0);
-        uint64_t want = (hybrid && pack_on && !pack_chunk) ? raw_want : budget * unit;
-        if (remaining <= want) want = remaining > 2 * kChunkTail * unit ? remaining - kChunkTail * unit : remaining;
-        uint64_t q1;
-        if (qs->offsets) {
-            const uint64_t *ob = qs->offsets + q0 + 1, *oe = qs->offsets + nq + 1;
-            const uint64_t *it = std::upper_bound(ob, oe, qs->offsets[q0] + want);
-            q1 = q0 + (uint64_t)(it - ob);
-            if (q1 == q0) q1 = q0 + 1;
-        } else {
-            q1 = q0 + (qs->fixed_len ? std::max<uint64_t>(1, want / qs->fixed_len) : kChunkMaxQueries);
-        }
-        q1 = std::min<uint64_t>(q1, std::min<uint64_t>(nq, q0 + kChunkMaxQueries));
-        if (pack_chunk || !(hybrid && pack_on)) budget = std::min<uint64_t>(budget * 2, kChunkMax);
-        const uint64_t cq = q1 - q0;
-        const uint64_t sym0 = query_bytes_end(qs, q0), sym1 = query_bytes_end(qs, q1), nsym = sym1 - sym0;
-        if (sym1 < sym0 || sym1 > sym_end) {  // (inside a chunk the kernel checks every query against the chunk's extent)
-            t_error_query = q0;
-            return fail(GDX_ERR_BAD_ARG, "queries->offsets must not decrease and must stay inside the batch (near query %llu)",
-                        (unsigned long long)q0);
-        }
+    gdx_stats io = {nq};  // (queries)
+    gdx::Chunk c;
+    for (int k = 0; plan.next(c); ++k) {
+        if (c.bad_offsets) return bad_offsets(c.q0);
+        const uint64_t cq = c.cq();
         Slot &sl = ws->slot[k % kSlots];
         const SortPlan sp = plan_sort(idx, cq, qs->offsets ? 0 : qs->fixed_len);
-        // growing a slot buffer frees the old one: only safe once the slot's stream has drained
-        const uint64_t in_cap = nsym + 64;  // enough for either representation of the chunk
-        if (sl.bytes.cap < in_cap || (qs->offsets && sl.offsets.cap < (cq + 1) * 8) ||
-            sl.out_a.cap < cq * 8 || ((mode == 0 || lp) && sl.out_b.cap < cq * 8) ||
-            (sp.use && sl.sort.cap < sp.total_bytes))
-            CUDA_TRY(cudaStreamSynchronize(sl.stream));
-        CUDA_TRY(sl.bytes.reserve(in_cap));
-        cudaEvent_t ev_h2d = nullptr;
-        if (trace) {
-            cudaEventCreate(&ev_h2d);
-            cudaEventRecord(ev_h2d, sl.stream);
+        GDX_TRY(reserve_drained(sl.stream, {{&sl.bytes, c.nsym() + 64}, {&sl.offsets, qs->offsets ? (cq + 1) * 8 : 0},
+                                            {&sl.out_a, cq * 8}, {&sl.out_b, sink.writes_b ? cq * 8 : 0},
+                                            {&sl.sort, sp.use ? sp.total_bytes : 0}}));
+        trace.chunk_begins(sl.stream);
+        GDX_TRY(stage_chunk(idx, qs, c, plan, sl, u));
+        const uint64_t sym_bytes = u.packed || prepacked ? (c.nsym() + 3) / 4 : c.nsym();
+        if (plan.hybrid) {
+            CUDA_TRY(link.push(sl, sym_bytes));
+            plan.after_upload(u.packed, c.nsym(), u.stage_ms, u.packed ? link.backlog() : 0);
         }
-        if (sl.h2d_pending) {  // the slot's staging buffers are free again once their last upload is done
-            CUDA_TRY(cudaEventSynchronize(sl.ev_h2d));
-            sl.h2d_pending = false;
-        }
-        const auto t_stage0 = std::chrono::steady_clock::now();
-        DevQueries dq;
-        dq.bytes = sl.bytes.as<uint8_t>();
-        dq.packed = nullptr;
-        dq.offsets = nullptr;
-        dq.offsets32 = nullptr;
-        dq.fixed_len = qs->fixed_len;
-        dq.nq = cq;
-        dq.base = 0;
-        dq.shift = 0;
-        dq.limit = nsym;  // (+ shift once a packed chunk decides it)
-        // large variable-length batches: offsets cross PCIe chunk relative as uint32
-        const bool narrow_off = qs->offsets && nq * 8 >= kStageMinBytes && nsym + 4 < 0xffffffffull && narrow_enabled();
-        bool used_staging = false;
-        uint64_t nx = 0;  // queries of this chunk that go through the IO-byte kernel after the packed one
-        bool chunk_packed = false;
-        if (nsym && pack_chunk) {
-            CUDA_TRY(sl.h_in.reserve((nsym + 3) / 4 + 8));
-            pack2_parallel(idx->pack, qs->bytes + sym0, nsym, (uint8_t *)sl.h_in.p, exc);
-            exc_q.clear();
-            for (uint64_t pos : exc) {
-                uint64_t q;
-                if (qs->offsets) {
-                    const uint64_t *ob = qs->offsets + q0, *oe = qs->offsets + q1 + 1;
-                    q = (uint64_t)(std::upper_bound(ob, oe, sym0 + pos) - ob) - 1;
-                    q = std::min(q, cq - 1);  // (offsets that are not sorted are reported by the kernel; stay in the chunk)
-                } else {
-                    q = pos / qs->fixed_len;
-                }
-                if (exc_q.empty() || exc_q.back() != (uint32_t)q) exc_q.push_back((uint32_t)q);
-            }
-            if (exc_q.size() * 16 > cq) {
-                // this is not a batch of plain searchable symbols: IO bytes from here on
-                pack_on = false;
-            } else {
-                chunk_packed = true;
-                nx = exc_q.size();
-                CUDA_TRY(cudaMemcpyAsync(sl.bytes.p, sl.h_in.p, (nsym + 3) / 4, cudaMemcpyHostToDevice, sl.stream));
-                h2d_bytes += (nsym + 3) / 4;
-                dq.bytes = nullptr;
-                dq.packed = sl.bytes.as<uint32_t>();
-                used_staging = true;
-            }
-        }
-        if (nsym && !chunk_packed) {
-            if (prepacked) {  // the caller's stream, from the byte that holds the chunk's first symbol
-                const uint64_t b0 = sym0 / 4, b1 = (sym1 + 3) / 4;
-                const uint8_t *src = qs->bytes + b0;
-                if (stage_in) {
-                    CUDA_TRY(sl.h_in.reserve(b1 - b0));
-                    HostPool::get().copy(sl.h_in.p, src, b1 - b0);
-                    src = (const uint8_t *)sl.h_in.p;
-                    used_staging = true;
-                }
-                CUDA_TRY(cudaMemcpyAsync(sl.bytes.p, src, b1 - b0, cudaMemcpyHostToDevice, sl.stream));
-                h2d_bytes += b1 - b0;
-                dq.bytes = nullptr;
-                dq.packed = sl.bytes.as<uint32_t>();
-                dq.shift = sym0 & 3;
-                dq.limit = nsym + dq.shift;
-            } else {
-                const uint8_t *src = qs->bytes + sym0;
-                if (stage_in) {
-                    CUDA_TRY(sl.h_in.reserve(nsym));
-                    HostPool::get().copy(sl.h_in.p, src, nsym);
-                    src = (const uint8_t *)sl.h_in.p;
-                    used_staging = true;
-                }
-                CUDA_TRY(cudaMemcpyAsync(sl.bytes.p, src, nsym, cudaMemcpyHostToDevice, sl.stream));
-                h2d_bytes += nsym;
-            }
-        } else if (!nsym && prepacked) {
-            dq.bytes = nullptr;
-            dq.packed = sl.bytes.as<uint32_t>();
-        }
-        if (qs->offsets && narrow_off) {
-            // chunk-relative 32-bit offsets, narrowed by the pool into pinned staging: half the PCIe bytes
-            CUDA_TRY(sl.offsets.reserve((cq + 1) * 8));
-            CUDA_TRY(sl.h_off.reserve((cq + 1) * 4));
-            const uint64_t *osrc = qs->offsets + q0;
-            uint32_t *o32 = (uint32_t *)sl.h_off.p;
-            const uint64_t rel = sym0 - dq.shift, cnt = cq + 1;
-            constexpr uint64_t kPiece = 1ull << 18;
-            HostPool::get().parallel_for(div_up(cnt, kPiece), [&](uint64_t piece) {
-                const uint64_t lo = piece * kPiece, hi = std::min(cnt, lo + kPiece);
-                for (uint64_t i = lo; i < hi; ++i) o32[i] = (uint32_t)(osrc[i] - rel);
-            });
-            used_staging = true;
-            CUDA_TRY(cudaMemcpyAsync(sl.offsets.p, o32, cnt * 4, cudaMemcpyHostToDevice, sl.stream));
-            h2d_bytes += cnt * 4;
-            dq.offsets32 = sl.offsets.as<uint32_t>();
-            dq.shift = 0;
-        } else if (qs->offsets) {
-            CUDA_TRY(sl.offsets.reserve((cq + 1) * 8));
-            const uint64_t *osrc = qs->offsets + q0;
-            if (stage_off) {
-                CUDA_TRY(sl.h_off.reserve((cq + 1) * 8));
-                HostPool::get().copy(sl.h_off.p, osrc, (cq + 1) * 8);
-                osrc = (const uint64_t *)sl.h_off.p;
-                used_staging = true;
-            }
-            CUDA_TRY(cudaMemcpyAsync(sl.offsets.p, osrc, (cq + 1) * 8, cudaMemcpyHostToDevice, sl.stream));
-            h2d_bytes += (cq + 1) * 8;
-            dq.offsets = sl.offsets.as<uint64_t>();
-            dq.base = sym0 - dq.shift;
-            dq.shift = 0;
-        }
-        // queries with an exception byte: their offsets, result slots and IO bytes in one upload
-        DevQueries xq = {};
-        const uint32_t *x_slots = nullptr;
-        if (nx) {
-            uint64_t xbytes = 0;
-            for (uint32_t q : exc_q) xbytes += query_bytes_end(qs, q0 + q + 1) - query_bytes_end(qs, q0 + q);
-            const uint64_t off_slots = (nx + 1) * 8, off_bytes = align_up(off_slots + nx * 4, 8), tot = off_bytes + xbytes + 8;
-            if (sl.xbuf.cap < tot) CUDA_TRY(cudaStreamSynchronize(sl.stream));
-            CUDA_TRY(sl.xbuf.reserve(tot));
-            CUDA_TRY(sl.h_x.reserve(tot));
-            uint64_t *xo = (uint64_t *)sl.h_x.p;
-            uint32_t *xs = (uint32_t *)((uint8_t *)sl.h_x.p + off_slots);
-            uint8_t *xb = (uint8_t *)sl.h_x.p + off_bytes;
-            uint64_t acc = 0;
-            for (uint64_t i = 0; i < nx; ++i) {
-                xo[i] = acc;
-                xs[i] = exc_q[i];
-                acc += query_bytes_end(qs, q0 + exc_q[i] + 1) - query_bytes_end(qs, q0 + exc_q[i]);
-            }
-            xo[nx] = acc;
-            constexpr uint64_t kPiece = 4096;  // queries per piece
-            HostPool::get().parallel_for(div_up(nx, kPiece), [&](uint64_t piece) {
-                const uint64_t lo = piece * kPiece, hi = std::min(nx, lo + kPiece);
-                for (uint64_t i = lo; i < hi; ++i) {
-                    const uint64_t b0 = query_bytes_end(qs, q0 + exc_q[i]);
-                    memcpy(xb + xo[i], qs->bytes + b0, xo[i + 1] - xo[i]);
-                }
-            });
-            CUDA_TRY(cudaMemcpyAsync(sl.xbuf.p, sl.h_x.p, off_bytes + xbytes, cudaMemcpyHostToDevice, sl.stream));
-            h2d_bytes += off_bytes + xbytes;
-            xq.bytes = sl.xbuf.as<uint8_t>() + off_bytes;
-            xq.offsets = sl.xbuf.as<uint64_t>();
-            xq.nq = nx;
-            xq.limit = xbytes;
-            x_slots = reinterpret_cast<const uint32_t *>(sl.xbuf.as<uint8_t>() + off_slots);
-            used_staging = true;
-        }
-        const double stage_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t_stage0).count();
-        if (hybrid) {
-            // this slot's event is about to be re-recorded: its older upload has long left the link
-            for (size_t i = 0; i < on_link.size();)
-                if (on_link[i].slot == k % kSlots) on_link.erase(on_link.begin() + i);
-                else ++i;
-            CUDA_TRY(cudaEventRecord(sl.ev_link, sl.stream));
-            on_link.push_back(Upload{k % kSlots, chunk_packed ? (nsym + 3) / 4 : nsym});
-            if (chunk_packed && stage_ms > 0.02) pack_rate = 0.5 * pack_rate + 0.5 * (double)nsym / stage_ms;
-            if (chunk_packed) {
-                // how long will the pool need for the next packed chunk, and will the link last that long?
-                const double t_pack = (double)(budget * 4) / pack_rate;
-                const double have = (double)link_backlog();
-                const double need = t_pack * kLinkGuessBytesPerMs;
-                raw_next = pack_on && need - have >= (double)(2ull << 20);
-                raw_want = raw_next ? std::min<uint64_t>((uint64_t)(need - have), 4 * kChunkMax) : 0;
-            } else {
-                raw_next = false;  // a raw chunk is always followed by a packed one
-            }
-        }
-
-        CUDA_TRY(sl.out_a.reserve(cq * 8));
-        uint64_t *a = sl.out_a.as<uint64_t>(), *b = nullptr;
-        if (mode == 0 || lp) {
-            CUDA_TRY(sl.out_b.reserve(cq * 8));
-            b = sl.out_b.as<uint64_t>();
-        }
-        if (used_staging) {
-            CUDA_TRY(cudaEventRecord(sl.ev_h2d, sl.stream));
-            sl.h2d_pending = true;
-        }
+        uint64_t *a = sl.out_a.as<uint64_t>(), *b = sink.writes_b ? sl.out_b.as<uint64_t>() : nullptr;
         const EventPairs::Pair ev = sl.timing.next();
         CUDA_TRY(cudaEventRecord(ev.begin, sl.stream));
-        if (trace) trace_rows.push_back(TraceRow{k, cq, chunk_packed || prepacked ? (nsym + 3) / 4 : nsym, ev_h2d, ev.begin, ev.end, nullptr, stage_ms});
+        trace.kernels_recorded(k, cq, sym_bytes, ev, u.stage_ms);
         const uint32_t *perm = nullptr;
         if (sp.use) {
-            CUDA_TRY(sl.sort.reserve(sp.total_bytes));
-            GDX_TRY(sort_queries(idx, dq, sp, sl.sort.p, sl.stream, &perm));
+            GDX_TRY(sort_queries(idx, u.dq, sp, sl.sort.p, sl.stream, &perm));
             t_stats.kernel_launches += 2;
         }
-        gdx_status st = dispatch_layout(idx->h.layout, [&](auto L) -> gdx_status {
-            launch_search<decltype(L)>(idx, dq, a, b, mode, narrow, q0, &ws->cnt_d->err[k % kSlots], &ws->cnt_d->search, perm,
+        uint64_t *err = &ws->cnt_d->err[k % kSlots];
+        GDX_TRY(dispatch_layout(idx->h.layout, [&](auto L) -> gdx_status {
+            launch_search<decltype(L)>(idx, u.dq, a, b, sink.mode, sink.narrow, c.q0, err, &ws->cnt_d->search, perm,
                                        nullptr, sl.stream);
-            if (nx)  // overwrites the slots of the queries the packed kernel could not see correctly
-                launch_search<decltype(L)>(idx, xq, a, b, mode, narrow, q0, &ws->cnt_d->err[k % kSlots], &ws->cnt_d->search,
-                                           nullptr, x_slots, sl.stream);
+            if (u.xq.nq)  // overwrites the slots of the queries the packed kernel could not see correctly
+                launch_search<decltype(L)>(idx, u.xq, a, b, sink.mode, sink.narrow, c.q0, err, &ws->cnt_d->search,
+                                           nullptr, u.x_slots, sl.stream);
             return GDX_OK;
-        });
-        GDX_TRY(st);
+        }));
         CUDA_TRY(cudaGetLastError());
         CUDA_TRY(cudaEventRecord(ev.end, sl.stream));
-        if (chunk_packed || prepacked) packed_queries += cq;
-        exception_queries += nx;
-        if (lp) {  // locate continues per chunk; the previous chunk is finished while this one runs
-            GDX_TRY(lp->stage_counts(sl, k % kSlots, q0, cq));
-            GDX_TRY(lp->finish(lp->take_pending(kSlots - 1)));
-        } else if (stage_out) {  // results go to pinned staging; the previous chunk's are handed over meanwhile
-            PendingOut prev = pend_out;
-            CUDA_TRY(sl.h_out_a.reserve(cq * dev_elem));
-            CUDA_TRY(cudaMemcpyAsync(sl.h_out_a.p, a, cq * dev_elem, cudaMemcpyDeviceToHost, sl.stream));
-            if (mode == 0) {
-                CUDA_TRY(sl.h_out_b.reserve(cq * dev_elem));
-                CUDA_TRY(cudaMemcpyAsync(sl.h_out_b.p, b, cq * dev_elem, cudaMemcpyDeviceToHost, sl.stream));
-            }
-            CUDA_TRY(cudaEventRecord(sl.ev_out, sl.stream));
-            pend_out = PendingOut{k % kSlots, q0, cq, true};
-            d2h_bytes += cq * dev_elem * (mode == 0 ? 2 : 1);
-            GDX_TRY(finish_out(prev));
-        } else {
-            d2h_bytes += cq * out_elem * (mode == 0 ? 2 : 1);
-            CUDA_TRY(cudaMemcpyAsync(out_a + q0 * out_elem, a, cq * out_elem, cudaMemcpyDeviceToHost, sl.stream));
-            if (mode == 0) CUDA_TRY(cudaMemcpyAsync(out_b + q0 * out_elem, b, cq * out_elem, cudaMemcpyDeviceToHost, sl.stream));
-        }
-        if (trace) {
-            cudaEventCreate(&trace_rows.back().d2h_end);
-            cudaEventRecord(trace_rows.back().d2h_end, sl.stream);
-        }
-        t_stats.kernel_launches += 1 + (nx ? 1 : 0);
-        q0 = q1;
-        ++k;
+        if (u.packed || prepacked) io.packed_queries += cq;
+        io.exception_queries += u.xq.nq;
+        io.h2d_bytes += u.up.bytes;
+        GDX_TRY(sink.chunk(sl, c.q0, cq));
+        trace.d2h_recorded(sl.stream);
+        t_stats.kernel_launches += 1 + (u.xq.nq ? 1 : 0);
     }
-    while (lp && !lp->pending.empty()) GDX_TRY(lp->finish(lp->take_pending(0)));
-    if (lp) GDX_TRY(lp->flush_offsets());
-    GDX_TRY(finish_out(pend_out));
-    const double t_issue = trace ? std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t_host0).count() : 0;
+    GDX_TRY(sink.finish());
+    const double t_issue = trace.ms();
     for (int s = 0; s < kSlots; ++s) CUDA_TRY(cudaStreamSynchronize(ws->slot[s].stream));
-    if (trace && !trace_rows.empty()) {
-        const double t_sync = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t_host0).count();
-        fprintf(stderr, "[gdx trace] host: all chunks issued at %.3f ms, streams drained at %.3f ms (%u pool threads)\n", t_issue,
-                t_sync, HostPool::get().threads());
-        cudaEvent_t base = trace_rows[0].h2d_begin;
-        for (auto &r : trace_rows) {
-            float a = 0, b = 0, c = 0, d = 0;
-            cudaError_t te = cudaEventElapsedTime(&a, base, r.h2d_begin);
-            if (te != cudaSuccess) fprintf(stderr, "[gdx trace] elapsed: %s\n", cudaGetErrorString(te));
-            cudaEventElapsedTime(&b, base, r.k_begin);
-            cudaEventElapsedTime(&c, base, r.k_end);
-            cudaEventElapsedTime(&d, base, r.d2h_end);
-            fprintf(stderr, "[gdx trace] chunk %2d slot %d nq %8llu h2d bytes %10llu host stage %.3f ms | h2d %.3f..%.3f | kernels %.3f..%.3f | d2h ..%.3f\n",
-                    r.k, r.k % kSlots, (unsigned long long)r.nq, (unsigned long long)r.bytes, r.host_stage_ms, a, b, b, c, d);
-        }
-        for (auto &r : trace_rows) {
-            cudaEventDestroy(r.h2d_begin);
-            cudaEventDestroy(r.d2h_end);
-        }
-    }
-    CUDA_TRY(ws->read_counters(ws->slot[0].stream));
-    CUDA_TRY(cudaStreamSynchronize(ws->slot[0].stream));
-    const Counters &c = *ws->cnt_h;
-    double ms = 0, ms_loc = 0;
-    for (int s = 0; s < kSlots; ++s) {
-        ms += ws->slot[s].timing.elapsed_ms();
-        ms_loc += ws->slot[s].locate.timing.elapsed_ms();
-    }
-    t_stats.queries = nq;
-    t_stats.lf_steps = c.search.lf_steps;
-    t_stats.walk_steps = c.search.verify_walk_steps + c.locate_walk_steps;
-    t_stats.locate_walk_steps = c.locate_walk_steps;
-    t_stats.verified_queries = c.search.verified_rows;
-    t_stats.kernel_ms_search = ms;
-    t_stats.kernel_ms_locate = ms_loc;
-    t_stats.packed_queries = packed_queries;
-    t_stats.exception_queries = exception_queries;
-    t_stats.h2d_bytes = h2d_bytes;
-    t_stats.d2h_bytes += d2h_bytes;
-    uint64_t bad = kNoError;
-    for (int s = 0; s < kSlots; ++s) bad = std::min(bad, c.err[s]);
-    if (bad != kNoError && (bad & kBadOffsetFlag)) {
-        t_error_query = bad & ~kBadOffsetFlag;
-        return fail(GDX_ERR_BAD_ARG, "query %llu: queries->offsets must not decrease and must stay inside the batch",
-                    (unsigned long long)t_error_query);
-    }
-    if (bad != kNoError) {
-        t_error_query = bad;
-        return fail(GDX_ERR_INVALID_SYMBOL,
-                    "query %llu: symbol in io representation should be valid (alphabet.rs:195-198)",
-                    (unsigned long long)bad);
-    }
-    return GDX_OK;
+    trace.print(t_issue);
+    io.d2h_bytes = sink.d2h;
+    return search_result(ws, io);
 }
 
 gdx_status begin_call(const gdx_index *idx, const char *what) {
@@ -2708,7 +2634,10 @@ gdx_status search_many_impl(const gdx_index *idx, const gdx_queries *queries, vo
     GDX_TRY(check_queries(idx, queries));
     if (queries->nq && (!a || (mode == 0 && !b))) return fail(GDX_ERR_BAD_ARG, "output is NULL");
     if (elem == 4 && idx->h.wide) return fail(GDX_ERR_UNSUPPORTED, "32-bit results need a text shorter than 2^32 symbols");
-    return with_workspace(idx, [&](Workspace *ws) { return search_host(idx, ws, queries, a, b, elem, mode); });
+    return with_workspace(idx, [&](Workspace *ws) {
+        CountSink sink(idx, queries->nq, a, b, elem, mode);
+        return search_host(idx, ws, queries, sink);
+    });
 }
 
 // write_last = false: hit_offsets[nq] is left alone (it is the first entry of the next shard's range)
@@ -2733,7 +2662,7 @@ gdx_status locate_many_impl(const gdx_index *idx, const gdx_queries *queries, ui
         lp.stage_offsets =
             n * 8 >= kStageMinBytes && !is_pinned(hit_counts ? (const void *)hit_counts : (const void *)hit_offsets);
         GDX_TRY(acquire_pinned_hits(idx, std::max<uint64_t>(n, 4096) * hit_bytes, &res.p, &res.cap));
-        return search_host(idx, ws, queries, nullptr, nullptr, 8, 2, &lp);
+        return search_host(idx, ws, queries, lp);
     });
     if (st != GDX_OK) {
         res.release();  // after with_workspace drained the streams: hit copies into it may have been in flight
@@ -2800,8 +2729,7 @@ extern "C" gdx_status gdx_pack_queries(const gdx_index *idx, const gdx_queries *
         for (uint64_t pos : exc) {
             const uint64_t sym = a0 + pos;
             if (sym < s0) continue;
-            first = q->offsets ? (uint64_t)(std::upper_bound(q->offsets, q->offsets + q->nq + 1, sym) - q->offsets) - 1
-                               : (sym - q->first_symbol) / q->fixed_len;
+            first = q->offsets ? query_of_symbol(q->offsets, 0, q->nq + 1, sym) : (sym - q->first_symbol) / q->fixed_len;
             break;
         }
         if (first_unencodable) *first_unencodable = first;
@@ -3209,16 +3137,7 @@ uint64_t hamming_host_check(const gdx_queries *q, gdx_status *st) {
     return q->nq;
 }
 
-// error word of k_hamming<.., 1>: smallest failing query (kBadOffsetFlag: its offsets leave the uploaded chunk)
-gdx_status hamming_error(uint64_t bad) {
-    if (bad == kNoError) return GDX_OK;
-    t_error_query = bad & ~kBadOffsetFlag;
-    if (bad & kBadOffsetFlag)
-        return fail(GDX_ERR_BAD_ARG, "query %llu: queries->offsets must not decrease and must stay inside the batch",
-                    (unsigned long long)t_error_query);
-    return fail(GDX_ERR_INVALID_SYMBOL, "query %llu: every byte of a Hamming query must be a searchable symbol",
-                (unsigned long long)t_error_query);
-}
+constexpr const char *kHammingBadSymbol = "every byte of a Hamming query must be a searchable symbol";
 
 // Chunks of kHammingChunkQueries over the queries [0, n_ok) on slot 0's stream: upload -> pass 1 (checks + counts)
 // -> [scan -> pass 2 (intervals) -> locate] -> results to the caller.  counts == NULL in kHammingCount mode: only
@@ -3234,22 +3153,14 @@ gdx_status hamming_run(const gdx_index *idx, Workspace *ws, const gdx_queries *q
     uint64_t *d_err = &ws->cnt_d->err[0];
     CUDA_TRY(ws->reset_counters(st));
     const bool src_pinned = n_ok && is_pinned(qs->bytes);
-    uint64_t h2d = 0, d2h = 0, launches = 0;
+    Uploads up{st};
+    uint64_t d2h = 0, launches = 0;
     for (uint64_t q0 = 0; q0 < n_ok; q0 += kHammingChunkQueries) {
         const uint64_t cq = std::min<uint64_t>(kHammingChunkQueries, n_ok - q0);
         const uint64_t sym0 = query_bytes_end(qs, q0), nsym = query_bytes_end(qs, q0 + cq) - sym0;
-        // the chunk's IO bytes (+ offsets) through pinned staging; the previous chunk's copies are done
+        // the chunk's IO bytes (pageable: through pinned staging) + offsets (staged); the previous chunk's copies are done
         CUDA_TRY(sl.bytes.reserve(nsym + 8));
-        if (nsym) {
-            const uint8_t *src = qs->bytes + sym0;
-            if (!src_pinned) {
-                CUDA_TRY(sl.h_in.reserve(nsym));
-                HostPool::get().copy(sl.h_in.p, src, nsym);
-                src = (const uint8_t *)sl.h_in.p;
-            }
-            CUDA_TRY(cudaMemcpyAsync(sl.bytes.p, src, nsym, cudaMemcpyHostToDevice, st));
-            h2d += nsym;
-        }
+        if (nsym) CUDA_TRY(up.copy(sl.bytes.p, qs->bytes + sym0, nsym, src_pinned ? nullptr : &sl.h_in));
         DevQueries dq = {};
         dq.bytes = sl.bytes.as<uint8_t>();
         dq.fixed_len = qs->fixed_len;
@@ -3257,10 +3168,7 @@ gdx_status hamming_run(const gdx_index *idx, Workspace *ws, const gdx_queries *q
         dq.limit = nsym;
         if (qs->offsets) {
             CUDA_TRY(sl.offsets.reserve((cq + 1) * 8));
-            CUDA_TRY(sl.h_off.reserve((cq + 1) * 8));
-            HostPool::get().copy(sl.h_off.p, qs->offsets + q0, (cq + 1) * 8);
-            CUDA_TRY(cudaMemcpyAsync(sl.offsets.p, sl.h_off.p, (cq + 1) * 8, cudaMemcpyHostToDevice, st));
-            h2d += (cq + 1) * 8;
+            CUDA_TRY(up.copy(sl.offsets.p, qs->offsets + q0, (cq + 1) * 8, &sl.h_off));
             dq.offsets = sl.offsets.as<uint64_t>();
             dq.base = sym0;
         }
@@ -3292,7 +3200,7 @@ gdx_status hamming_run(const gdx_index *idx, Workspace *ws, const gdx_queries *q
             }
             CUDA_TRY(ws->read_counters(st));
             CUDA_TRY(cudaStreamSynchronize(st));
-            GDX_TRY(hamming_error(ws->cnt_h->err[0]));
+            GDX_TRY(kernel_error(ws->cnt_h->err[0], kHammingBadSymbol));
             if (counts) HostPool::get().copy(counts + q0 * strata, sl.h_out_a.p, cq * strata * 8);
             continue;
         }
@@ -3302,7 +3210,7 @@ gdx_status hamming_run(const gdx_index *idx, Workspace *ws, const gdx_queries *q
         CUDA_TRY(cudaMemcpyAsync(&csr.h->hits, csr.offsets.as<uint64_t>() + cq, 8, cudaMemcpyDeviceToHost, st));
         CUDA_TRY(cudaStreamSynchronize(st));
         ++launches;
-        GDX_TRY(hamming_error(ws->cnt_h->err[0]));
+        GDX_TRY(kernel_error(ws->cnt_h->err[0], kHammingBadSymbol));
         const uint64_t niv = csr.h->hits;
         // pass 2: the intervals at their CSR offsets in search order, a sort by start within every query, then records
         // (cursors) or starts / ends (the locate path)
@@ -3386,7 +3294,7 @@ gdx_status hamming_run(const gdx_index *idx, Workspace *ws, const gdx_queries *q
     t_stats.kernel_ms_search = sl.timing.elapsed_ms();
     t_stats.kernel_ms_locate = ws->locate.timing.elapsed_ms();
     t_stats.kernel_launches += launches;
-    t_stats.h2d_bytes = h2d;
+    t_stats.h2d_bytes = up.bytes;
     t_stats.d2h_bytes = d2h;
     if (mode == kHammingLocate) t_stats.hits = res.used / elem;
     return GDX_OK;
@@ -3415,12 +3323,10 @@ gdx_status hamming_many_impl(const gdx_index *idx, const gdx_queries *queries, u
         // with a query the host refuses, the queries in front of it are only checked: a smaller offender wins
         if (host_st == GDX_OK) return hamming_run(idx, ws, queries, k, mode, n_ok, counts, offsets_out, res);
         GDX_TRY(hamming_run(idx, ws, queries, k, kHammingCount, n_ok, nullptr, nullptr, res));
+        if (host_st == GDX_ERR_BAD_ARG) return bad_offsets(n_ok);
         t_error_query = n_ok;
-        return host_st == GDX_ERR_BAD_ARG
-                   ? fail(GDX_ERR_BAD_ARG, "query %llu: queries->offsets must not decrease and must stay inside the batch",
-                          (unsigned long long)n_ok)
-                   : fail(GDX_ERR_UNSUPPORTED, "query %llu is longer than GDX_HAMMING_MAX_QUERY_LEN (%d symbols)",
-                          (unsigned long long)n_ok, GDX_HAMMING_MAX_QUERY_LEN);
+        return fail(GDX_ERR_UNSUPPORTED, "query %llu is longer than GDX_HAMMING_MAX_QUERY_LEN (%d symbols)",
+                    (unsigned long long)n_ok, GDX_HAMMING_MAX_QUERY_LEN);
     });
     if (st != GDX_OK) {
         res.release();  // after with_workspace drained the stream: a copy into it may have been in flight
