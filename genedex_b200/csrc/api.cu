@@ -29,6 +29,7 @@
 #include <cub/device/device_segmented_sort.cuh>
 
 #include "../../include/genedex_b200.h"
+#include "accel_policy.h"
 #include "chunk_plan.h"
 #include "device_build.h"
 #include "device_index.h"
@@ -145,6 +146,34 @@ struct DBuf {
         p = nullptr;
         cap = 0;
     }
+    template <class T>
+    T *as() const { return reinterpret_cast<T *>(p); }
+};
+
+// one device allocation with one owner: an accelerator table, an image under construction, a temporary of a build
+struct DevMem {
+    void *p = nullptr;
+    uint64_t bytes = 0;
+    DevMem() = default;
+    DevMem(DevMem &&o) noexcept : p(std::exchange(o.p, nullptr)), bytes(std::exchange(o.bytes, 0)) {}
+    DevMem &operator=(DevMem &&o) noexcept {
+        std::swap(p, o.p);
+        std::swap(bytes, o.bytes);
+        return *this;
+    }
+    ~DevMem() {
+        if (p) cudaFree(p);
+    }
+    cudaError_t alloc(uint64_t nbytes) {
+        const cudaError_t e = cudaMalloc(&p, nbytes);
+        bytes = e == cudaSuccess ? nbytes : 0;
+        return e;
+    }
+    void *release() {
+        bytes = 0;
+        return std::exchange(p, nullptr);
+    }
+    explicit operator bool() const { return p != nullptr; }
     template <class T>
     T *as() const { return reinterpret_cast<T *>(p); }
 };
@@ -362,13 +391,10 @@ struct gdx_index {
     void *image = nullptr;
     bool own_image = false;
     int device = 0;
-    DevIndex dev;
-    void *dense_sa = nullptr;      // accelerator outside the image (gdx_index_set_dense_suffix_array)
-    uint64_t dense_sa_bytes = 0;
-    void *seed_lut = nullptr;      // accelerator outside the image (gdx_index_set_seed_table_depth)
-    uint64_t seed_lut_bytes = 0;
-    void *row_ctx = nullptr;       // accelerator outside the image (gdx_index_set_row_context_table)
-    uint64_t row_ctx_bytes = 0;
+    DevIndex dev;                  // written by refresh_dev only
+    // accelerators outside the image (gdx_index_set_dense_suffix_array / _seed_table_depth / _row_context_table)
+    DevMem dense_sa, seed_table, row_context;
+    uint32_t seed_depth = 0;
     bool verify = true;            // finish one-row intervals through the text section (gdx_index_set_text_verification)
     PackTable pack;                // io byte -> 2-bit code (host packer, host_pack.h)
     // host-buffer queries hold this shared for the whole call; (re)building or freeing an accelerator needs it
@@ -432,6 +458,19 @@ gdx_status with_workspace(const gdx_index *idx, F &&f) {
     return st;
 }
 
+// runs f() with the configuration of idx held exclusively and idx's device current; busy is the GDX_ERR_BUSY message
+// while host-buffer queries hold the configuration
+template <class F>
+gdx_status with_config(gdx_index *idx, const char *busy, F &&f) {
+    return guarded([&]() -> gdx_status {
+        if (!idx) return fail(GDX_ERR_BAD_ARG, "NULL argument");
+        std::unique_lock<std::shared_mutex> cfg(idx->cfg_mu, std::try_to_lock);
+        if (!cfg.owns_lock()) return fail(GDX_ERR_BUSY, "%s", busy);
+        DeviceGuard guard(idx->device);
+        return f();
+    });
+}
+
 // ---- layout dispatch -----------------------------------------------------------------------------------
 template <class F>
 gdx_status dispatch_layout(const RankLayout &L, F &&f) {
@@ -450,6 +489,15 @@ gdx_status dispatch_layout(const RankLayout &L, F &&f) {
 }
 
 // ---- device image construction -------------------------------------------------------------------------
+// u32 or u64 words on the host or on the device (at most one of the pointers is set)
+struct Words {
+    const uint64_t *h64 = nullptr;
+    const uint32_t *h32 = nullptr;
+    const void *d = nullptr;
+    bool d_wide = false;
+    bool any() const { return h64 || h32 || d; }
+};
+
 struct ImageSources {
     const gdx_alphabet *alphabet;
     uint32_t storage, sampling_rate, lookup_depth;
@@ -462,14 +510,8 @@ struct ImageSources {
     uint64_t n_border;
     const uint8_t *d_bwt;              // device, n bytes
     const uint8_t *d_text = nullptr;   // device, n bytes dense text (optional: enables the text section)
-    // exactly one of the sample sources
-    const uint64_t *h_samples64 = nullptr;  // host
-    const void *d_samples = nullptr;        // device, element width given by d_samples_wide
-    bool d_samples_wide = false;
-    // optional sampled inverse suffix array (one of them, only together with d_text)
-    const uint64_t *h_isa64 = nullptr;      // host
-    const uint32_t *d_isa32 = nullptr;      // device
-    const uint32_t *h_samples32 = nullptr;  // host, the crate's own Vec<u32> for 32-bit storage
+    Words samples;                     // the sampled suffix array (set when n > 0)
+    Words isa;                         // optional sampled inverse suffix array, only together with d_text
     // accelerator policy of the index (travels with the image)
     uint32_t accel_flags = 0;
     uint64_t accel_budget = 0;
@@ -556,7 +598,7 @@ gdx_status plan_header(const ImageSources &src, ImageHeader &h, int wide_overrid
     }
     h.has_isa = 0;
     h.off_isa = off;
-    if (h.text_bits && (src.h_isa64 || src.d_isa32)) {
+    if (h.text_bits && src.isa.any()) {
         h.has_isa = 1;
         h.off_isa = place(h.n_samples * esz);
     }
@@ -588,7 +630,7 @@ gdx_status validate_header(const ImageHeader &h) {
     src.ntexts = h.ntexts;
     src.n_border = h.n_border;
     src.d_text = h.text_bits ? reinterpret_cast<const uint8_t *>(&a) : nullptr;            // presence only
-    src.d_isa32 = h.has_isa ? reinterpret_cast<const uint32_t *>(&a) : nullptr;            // presence only
+    src.isa.d = h.has_isa ? &a : nullptr;                                                 // presence only
     src.accel_flags = h.accel_flags;
     src.accel_budget = h.accel_budget;
     ImageHeader want;
@@ -598,119 +640,106 @@ gdx_status validate_header(const ImageHeader &h) {
     return GDX_OK;
 }
 
-// run-time overrides of kernel parameters (measurements only)
+// ---- accelerators outside the image (include/genedex_b200.h, policy in accel_policy.h) ---------------------
 bool verify_enabled();
-gdx_status init_policies(gdx_index *idx) {
-    build_pack_table(idx->h.io_to_dense, idx->h.ns, idx->pack);
-    idx->verify = verify_enabled();
-    if (const char *vm = getenv("GDX_VERIFY_MIN"))
-        if (atoi(vm) > 0) idx->dev.verify_min_remaining = (uint32_t)atoi(vm);
+
+// idx->dev from the image and the accelerators the index holds; nothing else writes idx->dev
+void refresh_dev(gdx_index *idx) {
+    DevIndex d = make_dev_index(idx->h, idx->image);
+    if (idx->dense_sa) {  // resolve_row / k_locate_walk see a suffix array with sampling rate 1
+        d.samples = idx->dense_sa.p;
+        d.sampling_rate = 1;
+        d.sampling_shift = 0;
+    }
+    if (idx->seed_table) {
+        d.seed_lookup = idx->seed_table.p;
+        d.seed_depth = idx->seed_depth;
+    }
+    d.row_context = idx->row_context.p;
+    d.verify_min_remaining = verify_min_remaining((bool)idx->dense_sa, getenv("GDX_VERIFY_MIN"));
+    idx->dev = d;
+}
+
+gdx_status table_oom(const char *what, uint64_t bytes) {
+    cudaGetLastError();
+    return fail(GDX_ERR_OOM, "%s: %llu bytes of device memory not available", what, (unsigned long long)bytes);
+}
+
+// table := `bytes` of device memory filled by launch(L, p) for the rank layout L of the index, once the kernel is done
+template <class F>
+gdx_status fill_table(gdx_index *idx, DevMem &table, uint64_t bytes, const char *what, F &&launch) {
+    DevMem d;
+    if (d.alloc(bytes) != cudaSuccess) return table_oom(what, bytes);
+    GDX_TRY(dispatch_layout(idx->h.layout, [&](auto L) -> gdx_status {
+        launch(L, d.p);
+        return GDX_OK;
+    }));
+    const cudaError_t e = cudaDeviceSynchronize();
+    if (e != cudaSuccess) return fail(GDX_ERR_CUDA, "%s: %s", what, cudaGetErrorString(e));
+    table = std::move(d);
+    refresh_dev(idx);
     return GDX_OK;
 }
 
-// ---- dense suffix array accelerator (include/genedex_b200.h: gdx_index_set_dense_suffix_array) ----------
+void drop_table(gdx_index *idx, DevMem &table) {
+    table = DevMem();
+    refresh_dev(idx);
+}
+
+AccelPolicy accel_policy(const ImageHeader &h) {
+    return AccelPolicy{h.n, h.accel_budget, h.ns, h.lookup_depth, h.wide != 0, h.text_bits != 0,
+                       (h.accel_flags & kAccelNoDenseSA) != 0, (h.accel_flags & kAccelNoSeedTable) != 0,
+                       (h.accel_flags & kAccelNoRowContext) != 0};
+}
+
 gdx_status build_dense_sa(gdx_index *idx) {
     if (idx->dense_sa || idx->h.n == 0) return GDX_OK;
-    const uint64_t n = idx->h.n, bytes = n * (idx->h.wide ? 8 : 4);
-    void *d = nullptr;
-    if (cudaMalloc(&d, bytes) != cudaSuccess) {
-        cudaGetLastError();
-        return fail(GDX_ERR_OOM, "dense suffix array: %llu bytes of device memory not available", (unsigned long long)bytes);
-    }
-    gdx_status st = dispatch_layout(idx->h.layout, [&](auto L) -> gdx_status {
+    const uint64_t n = idx->h.n;
+    return fill_table(idx, idx->dense_sa, n * (idx->h.wide ? 8 : 4), "dense suffix array", [&](auto L, void *d) {
         k_densify<decltype(L)><<<(unsigned)div_up(n, 256), 256>>>(idx->dev, d, n);
-        return GDX_OK;
     });
-    cudaError_t e = st == GDX_OK ? cudaDeviceSynchronize() : cudaSuccess;
-    if (st != GDX_OK || e != cudaSuccess) {
-        cudaFree(d);
-        return st != GDX_OK ? st : fail(GDX_ERR_CUDA, "dense suffix array: %s", cudaGetErrorString(e));
-    }
-    idx->dense_sa = d;
-    idx->dense_sa_bytes = bytes;
-    idx->dev.samples = d;  // resolve_row / k_locate_walk now see a suffix array with sampling rate 1
-    idx->dev.sampling_rate = 1;
-    idx->dev.sampling_shift = 0;
-    // resolving a row is now one load: the text comparison pays off from 4 remaining symbols on (measured on the
-    // protein config, 12-symbol queries: 2.58 -> 1.23 ms per 10 M queries; no effect on 50-symbol DNA queries)
-    if (!getenv("GDX_VERIFY_MIN")) idx->dev.verify_min_remaining = 4;
-    return GDX_OK;
-}
-
-void drop_dense_sa(gdx_index *idx) {
-    if (!idx->dense_sa) return;
-    const DevIndex fresh = make_dev_index(idx->h, idx->image);
-    idx->dev.samples = fresh.samples;
-    idx->dev.sampling_rate = fresh.sampling_rate;
-    idx->dev.sampling_shift = fresh.sampling_shift;
-    if (!getenv("GDX_VERIFY_MIN")) idx->dev.verify_min_remaining = fresh.verify_min_remaining;
-    cudaFree(idx->dense_sa);
-    idx->dense_sa = nullptr;
-    idx->dense_sa_bytes = 0;
-}
-
-// ---- row context table accelerator (include/genedex_b200.h: gdx_index_set_row_context_table) ------------
-void drop_row_context(gdx_index *idx) {
-    if (!idx->row_ctx) return;
-    idx->dev.row_context = nullptr;
-    cudaFree(idx->row_ctx);
-    idx->row_ctx = nullptr;
-    idx->row_ctx_bytes = 0;
-}
-
-bool row_context_possible(const gdx_index *idx) {
-    const ImageHeader &h = idx->h;
-    return h.n > 0 && !h.wide && h.n < (1ull << 32) && h.ns >= 1 && h.ns <= 4 && h.text_bits != 0;
 }
 
 gdx_status build_row_context(gdx_index *idx) {
-    if (idx->row_ctx) return GDX_OK;
-    if (!row_context_possible(idx))
+    if (idx->row_context) return GDX_OK;
+    if (!accel_policy(idx->h).row_context_possible())
         return fail(GDX_ERR_UNSUPPORTED, "the row context table needs the text section, at most 4 searchable symbols and a "
                                          "text shorter than 2^32 symbols");
-    const uint64_t n = idx->h.n, bytes = n * 16;
-    void *d = nullptr;
-    if (cudaMalloc(&d, bytes) != cudaSuccess) {
-        cudaGetLastError();
-        return fail(GDX_ERR_OOM, "row context table: %llu bytes of device memory not available", (unsigned long long)bytes);
-    }
-    gdx_status st = dispatch_layout(idx->h.layout, [&](auto L) -> gdx_status {
+    const uint64_t n = idx->h.n;
+    return fill_table(idx, idx->row_context, n * 16, "row context table", [&](auto L, void *d) {
         k_build_row_context<decltype(L)><<<(unsigned)div_up(n, 256), 256>>>(idx->dev, reinterpret_cast<uint4 *>(d), n);
-        return GDX_OK;
     });
-    cudaError_t e = st == GDX_OK ? cudaDeviceSynchronize() : cudaSuccess;
-    if (st != GDX_OK || e != cudaSuccess) {
-        cudaFree(d);
-        return st != GDX_OK ? st : fail(GDX_ERR_CUDA, "row context table: %s", cudaGetErrorString(e));
-    }
-    idx->row_ctx = d;
-    idx->row_ctx_bytes = bytes;
-    idx->dev.row_context = d;
-    return GDX_OK;
 }
 
-// ---- seed table accelerator (include/genedex_b200.h: gdx_index_set_seed_table_depth) -------------------
-void drop_seed_table(gdx_index *idx) {
-    if (!idx->seed_lut) return;
-    idx->dev.seed_lookup = nullptr;
-    idx->dev.seed_depth = 0;
-    cudaFree(idx->seed_lut);
-    idx->seed_lut = nullptr;
-    idx->seed_lut_bytes = 0;
+// count words to dst as u64 (wide) or u32, converted on the host or on the device where the source has the other width
+cudaError_t put_words(void *dst, uint64_t count, bool wide, const Words &w) {
+    const uint64_t esz = wide ? 8 : 4;
+    if (w.d && w.d_wide == wide) return cudaMemcpy(dst, w.d, count * esz, cudaMemcpyDeviceToDevice);
+    if (w.d) {
+        const unsigned g = (unsigned)div_up(count, 256);
+        if (wide) k_widen_u32<<<g, 256>>>((const uint32_t *)w.d, count, (uint64_t *)dst);
+        else k_narrow_u64<<<g, 256>>>((const uint64_t *)w.d, count, (uint32_t *)dst);
+        return cudaGetLastError();
+    }
+    if (wide ? w.h64 != nullptr : w.h32 != nullptr)
+        return cudaMemcpy(dst, wide ? (const void *)w.h64 : w.h32, count * esz, cudaMemcpyHostToDevice);
+    if (!w.any()) return cudaSuccess;
+    auto convert = [&](auto zero) {
+        std::vector<decltype(zero)> v(count);
+        for (uint64_t i = 0; i < count; ++i) v[i] = (decltype(zero))(w.h64 ? w.h64[i] : w.h32[i]);
+        return cudaMemcpy(dst, v.data(), count * esz, cudaMemcpyHostToDevice);
+    };
+    return wide ? convert(uint64_t{}) : convert(uint32_t{});
 }
 
-// entries of level d, 0 if ns^d exceeds 2^36 (grid and memory limits)
-uint64_t seed_entries(uint32_t ns, uint32_t d) {
-    uint64_t e = 1;
-    for (uint32_t i = 0; i < d; ++i) {
-        e *= ns;
-        if (e > (1ull << 36)) return 0;
-    }
-    return e;
+// level 0 of a lookup table: [(0, n)] (lookup_table.rs:205-209)
+cudaError_t put_lookup_level0(void *dst, uint64_t n, bool wide) {
+    const uint64_t e0[2] = {0, n};
+    return put_words(dst, 2, wide, Words{e0});
 }
 
 gdx_status build_seed_table(gdx_index *idx, uint32_t depth) {
-    drop_seed_table(idx);
+    drop_table(idx, idx->seed_table);
     const ImageHeader &h = idx->h;
     // a level no deeper than the configured table would change nothing for the better and would move the
     // eager translation of the configured suffix (lookup_table.rs:154-157): not built
@@ -718,137 +747,93 @@ gdx_status build_seed_table(gdx_index *idx, uint32_t depth) {
     const uint64_t esz = h.wide ? 16 : 8, last = seed_entries(h.ns, depth), prev = seed_entries(h.ns, depth - 1);
     if (last == 0 || depth > 40) return fail(GDX_ERR_UNSUPPORTED, "seed table of depth %u is too large", depth);
     // levels alternate between the final buffer and a temporary one of the size of level depth - 1
-    void *fin = nullptr, *tmp = nullptr;
-    if (cudaMalloc(&fin, last * esz) != cudaSuccess || cudaMalloc(&tmp, prev * esz) != cudaSuccess) {
-        cudaGetLastError();
-        if (fin) cudaFree(fin);
-        return fail(GDX_ERR_OOM, "seed table of depth %u: %llu bytes of device memory not available", depth,
-                    (unsigned long long)((last + prev) * esz));
+    DevMem fin, tmp;
+    if (fin.alloc(last * esz) != cudaSuccess || tmp.alloc(prev * esz) != cudaSuccess) {
+        char what[40];
+        snprintf(what, sizeof what, "seed table of depth %u", depth);
+        return table_oom(what, (last + prev) * esz);
     }
-    void *cur = (depth % 2 == 0) ? fin : tmp;  // level 0 lives where level `depth` will not collide: parity of depth
-    cudaError_t e;
-    if (h.wide) {
-        const uint64_t e0[2] = {0, h.n};
-        e = cudaMemcpy(cur, e0, sizeof e0, cudaMemcpyHostToDevice);
-    } else {
-        const uint32_t e0[2] = {0, (uint32_t)h.n};
-        e = cudaMemcpy(cur, e0, sizeof e0, cudaMemcpyHostToDevice);
-    }
-    gdx_status st = GDX_OK;
-    for (uint32_t d = 1; d <= depth && e == cudaSuccess && st == GDX_OK; ++d) {
-        void *nxt = cur == fin ? tmp : fin;
+    // level 0 lives where level `depth` will not collide: parity of depth
+    void *cur = (depth % 2 == 0) ? fin.p : tmp.p;
+    cudaError_t e = put_lookup_level0(cur, h.n, h.wide);
+    for (uint32_t d = 1; d <= depth && e == cudaSuccess; ++d) {
+        void *nxt = cur == fin.p ? tmp.p : fin.p;
         const uint64_t entries = seed_entries(h.ns, d);
-        st = dispatch_layout(h.layout, [&](auto L) -> gdx_status {
+        GDX_TRY(dispatch_layout(h.layout, [&](auto L) -> gdx_status {
             k_lut_extend<decltype(L)><<<(unsigned)div_up(entries, 256), 256>>>(idx->dev, cur, nxt, entries);
             return GDX_OK;
-        });
+        }));
         e = cudaGetLastError();
         cur = nxt;
     }
-    if (e == cudaSuccess && st == GDX_OK) e = cudaDeviceSynchronize();
-    cudaFree(tmp);
-    if (st != GDX_OK || e != cudaSuccess || cur != fin) {
-        cudaFree(fin);
-        return st != GDX_OK ? st : fail(GDX_ERR_CUDA, "seed table: %s", cudaGetErrorString(e));
-    }
-    idx->seed_lut = fin;
-    idx->seed_lut_bytes = last * esz;
-    idx->dev.seed_lookup = fin;
-    idx->dev.seed_depth = depth;
+    if (e == cudaSuccess) e = cudaDeviceSynchronize();
+    if (e != cudaSuccess || cur != fin.p) return fail(GDX_ERR_CUDA, "seed table: %s", cudaGetErrorString(e));
+    idx->seed_table = std::move(fin);
+    idx->seed_depth = depth;
+    refresh_dev(idx);
     return GDX_OK;
 }
 
-// Accelerator policy (include/genedex_b200.h): flags and byte budget live in the image header, so every way of
-// making a replica follows the same rule.  Without a budget an accelerator may take a quarter of the memory
-// that is free right now.  GDX_DENSE_SA / GDX_SEED_TABLE override the policy for measurements.
-uint64_t accel_room(const gdx_index *idx) {
-    if (idx->h.accel_budget) {
-        const uint64_t used = idx->dense_sa_bytes + idx->seed_lut_bytes + idx->row_ctx_bytes;
-        return idx->h.accel_budget > used ? idx->h.accel_budget - used : 0;
-    }
+uint64_t free_device_bytes() {
     size_t free_b = 0, total_b = 0;
-    if (cudaMemGetInfo(&free_b, &total_b) != cudaSuccess) return 0;
-    return free_b / 4;
+    return cudaMemGetInfo(&free_b, &total_b) == cudaSuccess ? free_b : kFreeUnknown;
 }
 
-void auto_seed_table(gdx_index *idx) {
-    if (!idx || idx->h.n == 0 || idx->h.ns < 2) return;
-    const char *e = getenv("GDX_SEED_TABLE");
-    uint32_t depth = 0;
-    if (e) {
-        if (atoi(e) <= 0) return;
-        depth = (uint32_t)atoi(e);
-    } else {
-        if (idx->h.accel_flags & kAccelNoSeedTable) return;
-        // the deepest level with at most four entries per text position (then most k-mers of the text have one row
-        // and almost no LF step is left): 3.1 Gbp DNA -> depth 16 (34 GB; 0.82 instead of 0.97 ms per 7.5 M queries
-        // against depth 15), 500 M residues of protein -> depth 7 (10 GB); the budget below has the last word
-        while (seed_entries(idx->h.ns, depth + 1) && seed_entries(idx->h.ns, depth + 1) <= 4 * idx->h.n) ++depth;
-        const uint64_t esz = idx->h.wide ? 16 : 8, room = accel_room(idx);
-        size_t free_b = 0, total_b = 0;
-        if (cudaMemGetInfo(&free_b, &total_b) != cudaSuccess) return;
-        // the finished level must fit the budget; the temporary previous level only has to fit the device
-        while (depth > 0 && (seed_entries(idx->h.ns, depth) * esz > room ||
-                             (seed_entries(idx->h.ns, depth) + seed_entries(idx->h.ns, depth - 1)) * esz > free_b))
-            --depth;
-    }
-    if (depth <= idx->h.lookup_depth) return;  // the configured table is at least as deep
-    if (build_seed_table(idx, depth) != GDX_OK) t_error.clear();  // optional: not an error of the call
+// what the policy of the index allows, in this order; each table is optional, so a failed build is no error of the call
+void build_accelerators(gdx_index *idx) {
+    const AccelPolicy p = accel_policy(idx->h);
+    auto used = [&] { return idx->dense_sa.bytes + idx->seed_table.bytes + idx->row_context.bytes; };
+    if (p.dense_sa(used(), free_device_bytes(), getenv("GDX_DENSE_SA")) && build_dense_sa(idx) != GDX_OK)
+        t_error.clear();
+    const uint32_t depth = p.seed_depth(used(), free_device_bytes(), getenv("GDX_SEED_TABLE"));
+    if (depth && build_seed_table(idx, depth) != GDX_OK) t_error.clear();
+    if (p.row_context(used(), free_device_bytes(), getenv("GDX_ROW_CONTEXT")) && build_row_context(idx) != GDX_OK)
+        t_error.clear();
 }
 
-// best effort after every way of creating a replica; the caller holds a DeviceGuard and has freed its temporaries
-void auto_dense_sa(gdx_index *idx) {
-    if (!idx || idx->h.n == 0) return;
-    const char *e = getenv("GDX_DENSE_SA");
-    if (e && atoi(e) == 0) return;
-    if (!(e && atoi(e) != 0)) {
-        if (idx->h.accel_flags & kAccelNoDenseSA) return;
-        if (idx->h.n * (idx->h.wide ? 8ull : 4ull) > accel_room(idx)) return;
-    }
-    if (build_dense_sa(idx) != GDX_OK) t_error.clear();  // optional: not an error of the call
-}
-
-// built last (it is the largest: 16 B per text position) and only from what the other two left: the budget when
-// one is set, else up to half of the memory that is still free
-void auto_row_context(gdx_index *idx) {
-    if (!idx || !row_context_possible(idx)) return;
-    const char *e = getenv("GDX_ROW_CONTEXT");
-    if (e && atoi(e) == 0) return;
-    if (!(e && atoi(e) != 0)) {
-        if (idx->h.accel_flags & kAccelNoRowContext) return;
-        const uint64_t room = idx->h.accel_budget ? accel_room(idx) : 2 * accel_room(idx);
-        if (idx->h.n * 16 > room) return;
-    }
-    if (build_row_context(idx) != GDX_OK) t_error.clear();  // optional: not an error of the call
-}
-
-gdx_status build_image(const ImageSources &src, int device, gdx_index **out) {
-    std::unique_ptr<gdx_index> idx(new gdx_index());
-    GDX_TRY(plan_header(src, idx->h));
-    ImageHeader &h = idx->h;
+// Every way of creating an index ends here, with a finished image.  The caller has the device current and has released
+// its device temporaries, so that the policy sees what the index leaves free.  On failure the image stays the caller's.
+gdx_status open_index(const ImageHeader &h, void *image, bool own_image, int device, gdx_index **out) {
+    gdx_index *idx = new (std::nothrow) gdx_index();
+    if (!idx) return fail(GDX_ERR_OOM, "out of host memory");
+    idx->h = h;
+    idx->image = image;
+    idx->own_image = own_image;
     idx->device = device;
-    CUDA_TRY(cudaMalloc(&idx->image, h.image_bytes));
-    idx->own_image = true;
-    auto cleanup = [&](gdx_status st) {
-        cudaFree(idx->image);
-        idx->image = nullptr;
-        return st;
-    };
-#define IMG_TRY(expr)                                                                             \
-    do {                                                                                          \
-        cudaError_t _e = (expr);                                                                  \
-        if (_e != cudaSuccess)                                                                    \
-            return cleanup(fail(GDX_ERR_CUDA, "%s failed: %s (%s:%d)", #expr,                     \
-                                cudaGetErrorString(_e), __FILE__, __LINE__));                     \
-    } while (0)
-    uint8_t *base = (uint8_t *)idx->image;
-    IMG_TRY(cudaMemset(base, 0, h.image_bytes));
-    IMG_TRY(cudaMemcpy(base + h.off_sentinels, src.sentinels, h.ntexts * 8, cudaMemcpyHostToDevice));
+    build_pack_table(h.io_to_dense, h.ns, idx->pack);
+    idx->verify = verify_enabled();
+    refresh_dev(idx);
+    build_accelerators(idx);
+    *out = idx;
+    return GDX_OK;
+}
+
+// an image built here: the index owns it once it is open
+gdx_status open_index(const ImageHeader &h, DevMem &image, int device, gdx_index **out) {
+    GDX_TRY(open_index(h, image.p, true, device, out));
+    image.release();
+    return GDX_OK;
+}
+
+// the host BWT (n bytes) on the device
+gdx_status upload_bwt(const uint8_t *bwt, uint64_t n, DevMem &d_bwt) {
+    CUDA_TRY(d_bwt.alloc(n ? n : 1));
+    const cudaError_t e = cudaMemcpy(d_bwt.p, bwt, n, cudaMemcpyHostToDevice);
+    return e == cudaSuccess ? GDX_OK : fail(GDX_ERR_CUDA, "BWT upload failed: %s", cudaGetErrorString(e));
+}
+
+// fills h and a new image from src; the caller releases its temporaries and then opens the index over the image
+gdx_status build_image(const ImageSources &src, ImageHeader &h, DevMem &image) {
+    GDX_TRY(plan_header(src, h));
+    CUDA_TRY(image.alloc(h.image_bytes));
+    uint8_t *base = image.as<uint8_t>();
+    CUDA_TRY(cudaMemset(base, 0, h.image_bytes));
+    CUDA_TRY(cudaMemcpy(base + h.off_sentinels, src.sentinels, h.ntexts * 8, cudaMemcpyHostToDevice));
     if (h.n_border) {
-        IMG_TRY(cudaMemcpy(base + h.off_border_rows, src.border_rows, h.n_border * 8, cudaMemcpyHostToDevice));
-        IMG_TRY(cudaMemcpy(base + h.off_border_pos, src.border_pos, h.n_border * 8, cudaMemcpyHostToDevice));
+        CUDA_TRY(cudaMemcpy(base + h.off_border_rows, src.border_rows, h.n_border * 8, cudaMemcpyHostToDevice));
+        CUDA_TRY(cudaMemcpy(base + h.off_border_pos, src.border_pos, h.n_border * 8, cudaMemcpyHostToDevice));
     }
-    IMG_TRY(cudaMemcpy(base + h.off_count, src.count, (uint64_t)(h.sigma + 1) * 8, cudaMemcpyHostToDevice));
+    CUDA_TRY(cudaMemcpy(base + h.off_count, src.count, (uint64_t)(h.sigma + 1) * 8, cudaMemcpyHostToDevice));
 
     // rank records + superblock table
     uint64_t *sbc = (uint64_t *)(base + h.off_sbc);
@@ -856,7 +841,7 @@ gdx_status build_image(const ImageSources &src, int device, gdx_index **out) {
         k_pack_k32<<<(unsigned)h.n_superblocks, 1024>>>(src.d_bwt, h.n, h.layout.noff, base + h.off_records,
                                                         h.n_records, sbc);
     } else {
-        gdx_status st = dispatch_layout(h.layout, [&](auto L) -> gdx_status {
+        GDX_TRY(dispatch_layout(h.layout, [&](auto L) -> gdx_status {
             using LT = decltype(L);
             if constexpr (!std::is_same<LT, K32>::value) {
                 constexpr int B = LT::kPlanes;
@@ -864,97 +849,33 @@ gdx_status build_image(const ImageSources &src, int device, gdx_index **out) {
                                                                  base + h.off_records, h.n_records, sbc);
             }
             return GDX_OK;
-        });
-        if (st != GDX_OK) return cleanup(st);
+        }));
     }
-    IMG_TRY(cudaGetLastError());
+    CUDA_TRY(cudaGetLastError());
     k_sb_scan<<<div_up(h.layout.noff, 64), 64>>>(sbc, h.n_superblocks, h.layout.noff,
                                                  (const uint64_t *)(base + h.off_count));
-    IMG_TRY(cudaGetLastError());
+    CUDA_TRY(cudaGetLastError());
 
-    // SA samples
-    if (h.n_samples) {
-        void *dst = base + h.off_samples;
-        if (src.h_samples64) {
-            if (h.wide) {
-                IMG_TRY(cudaMemcpy(dst, src.h_samples64, h.n_samples * 8, cudaMemcpyHostToDevice));
-            } else {
-                std::vector<uint32_t> narrow(h.n_samples);
-                for (uint64_t i = 0; i < h.n_samples; ++i) narrow[i] = (uint32_t)src.h_samples64[i];
-                IMG_TRY(cudaMemcpy(dst, narrow.data(), h.n_samples * 4, cudaMemcpyHostToDevice));
-            }
-        } else if (src.h_samples32) {
-            if (!h.wide) {
-                IMG_TRY(cudaMemcpy(dst, src.h_samples32, h.n_samples * 4, cudaMemcpyHostToDevice));
-            } else {
-                std::vector<uint64_t> wide(h.n_samples);
-                for (uint64_t i = 0; i < h.n_samples; ++i) wide[i] = src.h_samples32[i];
-                IMG_TRY(cudaMemcpy(dst, wide.data(), h.n_samples * 8, cudaMemcpyHostToDevice));
-            }
-        } else if (src.d_samples) {
-            const unsigned g = (unsigned)div_up(h.n_samples, 256);
-            if (src.d_samples_wide == (h.wide != 0))
-                IMG_TRY(cudaMemcpy(dst, src.d_samples, h.n_samples * (h.wide ? 8 : 4), cudaMemcpyDeviceToDevice));
-            else if (h.wide)
-                k_widen_u32<<<g, 256>>>((const uint32_t *)src.d_samples, h.n_samples, (uint64_t *)dst);
-            else
-                k_narrow_u64<<<g, 256>>>((const uint64_t *)src.d_samples, h.n_samples, (uint32_t *)dst);
-            IMG_TRY(cudaGetLastError());
-        }
-    }
-
-    if (h.has_isa && h.n_samples) {  // same element width as the SA samples
-        void *dst = base + h.off_isa;
-        if (src.h_isa64) {
-            if (h.wide) {
-                IMG_TRY(cudaMemcpy(dst, src.h_isa64, h.n_samples * 8, cudaMemcpyHostToDevice));
-            } else {
-                std::vector<uint32_t> narrow(h.n_samples);
-                for (uint64_t i = 0; i < h.n_samples; ++i) narrow[i] = (uint32_t)src.h_isa64[i];
-                IMG_TRY(cudaMemcpy(dst, narrow.data(), h.n_samples * 4, cudaMemcpyHostToDevice));
-            }
-        } else if (h.wide) {
-            k_widen_u32<<<(unsigned)div_up(h.n_samples, 256), 256>>>(src.d_isa32, h.n_samples, (uint64_t *)dst);
-            IMG_TRY(cudaGetLastError());
-        } else {
-            IMG_TRY(cudaMemcpy(dst, src.d_isa32, h.n_samples * 4, cudaMemcpyDeviceToDevice));
-        }
-    }
+    if (h.n_samples) CUDA_TRY(put_words(base + h.off_samples, h.n_samples, h.wide, src.samples));
+    if (h.has_isa && h.n_samples) CUDA_TRY(put_words(base + h.off_isa, h.n_samples, h.wide, src.isa));
     if (h.text_bits && h.n) {
         const uint64_t items = h.text_bits == 4 ? (h.n + 1) / 2 : h.n;
         k_pack_text<<<(unsigned)div_up(items, 256), 256>>>(src.d_text, h.n, h.text_bits, base + h.off_text);
-        IMG_TRY(cudaGetLastError());
+        CUDA_TRY(cudaGetLastError());
     }
 
-    idx->dev = make_dev_index(h, idx->image);
-    {
-        gdx_status ps = init_policies(idx.get());
-        if (ps != GDX_OK) return cleanup(ps);
+    // lookup tables: level d from level d-1
+    const DevIndex dev = make_dev_index(h, base);
+    void *lut = base + h.off_lookup;
+    CUDA_TRY(put_lookup_level0(lut, h.n, h.wide));
+    for (uint32_t d = 1; d <= h.lookup_depth; ++d) {
+        GDX_TRY(dispatch_layout(h.layout, [&](auto L) -> gdx_status {
+            k_lut_fill<decltype(L)><<<(unsigned)div_up(h.lut_pow[d], 256), 256>>>(dev, lut, d);
+            return GDX_OK;
+        }));
+        CUDA_TRY(cudaGetLastError());
     }
-
-    // lookup tables: level 0 = [(0, n)] (lookup_table.rs:205-209), level d from level d-1
-    {
-        void *lut = base + h.off_lookup;
-        if (h.wide) {
-            uint64_t e0[2] = {0, h.n};
-            IMG_TRY(cudaMemcpy(lut, e0, sizeof e0, cudaMemcpyHostToDevice));
-        } else {
-            uint32_t e0[2] = {0, (uint32_t)h.n};
-            IMG_TRY(cudaMemcpy(lut, e0, sizeof e0, cudaMemcpyHostToDevice));
-        }
-        for (uint32_t d = 1; d <= h.lookup_depth; ++d) {
-            gdx_status st = dispatch_layout(h.layout, [&](auto L) -> gdx_status {
-                using LT = decltype(L);
-                k_lut_fill<LT><<<(unsigned)div_up(h.lut_pow[d], 256), 256>>>(idx->dev, lut, d);
-                return GDX_OK;
-            });
-            if (st != GDX_OK) return cleanup(st);
-            IMG_TRY(cudaGetLastError());
-        }
-    }
-    IMG_TRY(cudaDeviceSynchronize());
-#undef IMG_TRY
-    *out = idx.release();
+    CUDA_TRY(cudaDeviceSynchronize());
     return GDX_OK;
 }
 
@@ -1069,12 +990,6 @@ extern "C" gdx_status gdx_index_build(const uint8_t *texts, const uint64_t *text
         // optional text section of the image
         const bool keep_text = (config->flags & GDX_FLAG_NO_TEXT) == 0;
         const bool keep_isa = keep_text && (config->flags & GDX_FLAG_NO_INVERSE_SAMPLES) == 0;
-        struct DevText {
-            uint8_t *p = nullptr;
-            ~DevText() {
-                if (p) cudaFree(p);
-            }
-        } d_text;
         uint32_t construction = config->construction;
         if (construction == GDX_CONSTRUCT_AUTO) {  // device suffix sort when the text and its scratch fit
             size_t free_b = 0, total_b = 0;
@@ -1082,63 +997,47 @@ extern "C" gdx_status gdx_index_build(const uint8_t *texts, const uint64_t *text
             if (n < 0xffffffffull && cudaMemGetInfo(&free_b, &total_b) == cudaSuccess && free_b > 36 * n + (1ull << 30))
                 construction = GDX_CONSTRUCT_DEVICE;
         }
-        if (keep_text || construction == GDX_CONSTRUCT_DEVICE) {
-            CUDA_TRY(cudaMalloc(&d_text.p, n ? n : 1));
-            CUDA_TRY(cudaMemcpy(d_text.p, ct.text.data(), n, cudaMemcpyHostToDevice));
-            if (keep_text) src.d_text = d_text.p;
-        }
-    
-        if (construction == GDX_CONSTRUCT_DEVICE) {
-            DeviceBuildResult r;
-            const bool verify = (config->flags & GDX_FLAG_VERIFY_SUFFIX_ARRAY) != 0;
-            st = device_build_from_text(nullptr, d_text.p, n, alphabet->num_dense_symbols,
-                                        config->suffix_array_sampling_rate, r, t_error, false, verify, keep_isa);
-            if (st != GDX_OK) return st;
-            if (verify && r.verify_violations) {
-                r.release();
-                return fail(GDX_ERR_CUDA, "device suffix array failed verification (%llu violations)",
-                            (unsigned long long)r.verify_violations);
+        ImageHeader h;
+        DevMem image;
+        {
+            DevMem d_text;
+            if (keep_text || construction == GDX_CONSTRUCT_DEVICE) {
+                CUDA_TRY(d_text.alloc(n ? n : 1));
+                CUDA_TRY(cudaMemcpy(d_text.p, ct.text.data(), n, cudaMemcpyHostToDevice));
+                if (keep_text) src.d_text = d_text.as<uint8_t>();
             }
-            src.border_rows = r.border_rows.data();
-            src.border_pos = r.border_pos.data();
-            src.n_border = r.border_rows.size();
-            src.d_bwt = r.d_bwt;
-            src.d_samples = r.d_samples;
-            src.d_samples_wide = false;
-            src.d_isa32 = r.d_isa_samples;
-            st = build_image(src, device, out);
-            r.release();
-            if (st == GDX_OK) {
-                auto_dense_sa(*out);
-                auto_seed_table(*out);
-                auto_row_context(*out);
+            if (construction == GDX_CONSTRUCT_DEVICE) {
+                DeviceBuildResult r;
+                const bool verify = (config->flags & GDX_FLAG_VERIFY_SUFFIX_ARRAY) != 0;
+                const uint32_t rate = config->suffix_array_sampling_rate;
+                GDX_TRY(device_build_from_text(nullptr, d_text.as<uint8_t>(), n, alphabet->num_dense_symbols, rate, r,
+                                               t_error, false, verify, keep_isa));
+                if (verify && r.verify_violations)
+                    return fail(GDX_ERR_CUDA, "device suffix array failed verification (%llu violations)",
+                                (unsigned long long)r.verify_violations);
+                src.border_rows = r.border_rows.data();
+                src.border_pos = r.border_pos.data();
+                src.n_border = r.border_rows.size();
+                src.d_bwt = r.d_bwt;
+                src.samples.d = r.d_samples;
+                src.isa.d = r.d_isa_samples;
+                GDX_TRY(build_image(src, h, image));
+            } else {
+                HostParts hp;
+                host_parts_from_text(ct.text.data(), n, alphabet->num_dense_symbols,
+                                     config->suffix_array_sampling_rate, hp);
+                DevMem d_bwt;
+                GDX_TRY(upload_bwt(hp.bwt.data(), n, d_bwt));
+                src.border_rows = hp.border_rows.data();
+                src.border_pos = hp.border_pos.data();
+                src.n_border = hp.border_rows.size();
+                src.d_bwt = d_bwt.as<uint8_t>();
+                src.samples.h64 = hp.samples.data();
+                if (keep_isa) src.isa.h64 = hp.isa_samples.data();
+                GDX_TRY(build_image(src, h, image));
             }
-            return st;
         }
-    
-        HostParts hp;
-        host_parts_from_text(ct.text.data(), n, alphabet->num_dense_symbols, config->suffix_array_sampling_rate, hp);
-        uint8_t *d_bwt = nullptr;
-        CUDA_TRY(cudaMalloc(&d_bwt, n ? n : 1));
-        cudaError_t e = cudaMemcpy(d_bwt, hp.bwt.data(), n, cudaMemcpyHostToDevice);
-        if (e != cudaSuccess) {
-            cudaFree(d_bwt);
-            return fail(GDX_ERR_CUDA, "BWT upload failed: %s", cudaGetErrorString(e));
-        }
-        src.border_rows = hp.border_rows.data();
-        src.border_pos = hp.border_pos.data();
-        src.n_border = hp.border_rows.size();
-        src.d_bwt = d_bwt;
-        src.h_samples64 = hp.samples.data();
-        if (keep_isa) src.h_isa64 = hp.isa_samples.data();
-        st = build_image(src, device, out);
-        cudaFree(d_bwt);
-        if (st == GDX_OK) {
-            auto_dense_sa(*out);
-            auto_seed_table(*out);
-            auto_row_context(*out);
-        }
-        return st;
+        return open_index(h, image, device, out);
     });
 }
 
@@ -1174,8 +1073,8 @@ static gdx_status sources_from_parts(const gdx_parts *parts, ImageSources &src,
     src.n_border = rows.size();
     if ((parts->sampled_suffix_array != nullptr) == (parts->sampled_suffix_array_u32 != nullptr) && parts->text_len)
         return fail(GDX_ERR_BAD_ARG, "exactly one of sampled_suffix_array / sampled_suffix_array_u32 must be set");
-    src.h_samples64 = parts->sampled_suffix_array;
-    src.h_samples32 = parts->sampled_suffix_array_u32;
+    src.samples.h64 = parts->sampled_suffix_array;
+    src.samples.h32 = parts->sampled_suffix_array_u32;
     src.accel_flags = accel_flags_from_config(parts->flags);
     src.accel_budget = parts->accelerator_budget_bytes;
     return GDX_OK;
@@ -1193,22 +1092,15 @@ extern "C" gdx_status gdx_index_create_from_bwt(const uint8_t *bwt, const gdx_pa
         int device;
         GDX_TRY(resolve_device(device_req, &device));
         DeviceGuard guard(device);
-        uint8_t *d_bwt = nullptr;
-        CUDA_TRY(cudaMalloc(&d_bwt, src.n ? src.n : 1));
-        cudaError_t e = cudaMemcpy(d_bwt, bwt, src.n, cudaMemcpyHostToDevice);
-        if (e != cudaSuccess) {
-            cudaFree(d_bwt);
-            return fail(GDX_ERR_CUDA, "BWT upload failed: %s", cudaGetErrorString(e));
+        ImageHeader h;
+        DevMem image;
+        {
+            DevMem d_bwt;
+            GDX_TRY(upload_bwt(bwt, src.n, d_bwt));
+            src.d_bwt = d_bwt.as<uint8_t>();
+            GDX_TRY(build_image(src, h, image));
         }
-        src.d_bwt = d_bwt;
-        gdx_status st = build_image(src, device, out);
-        cudaFree(d_bwt);
-        if (st == GDX_OK) {
-            auto_dense_sa(*out);
-            auto_seed_table(*out);
-            auto_row_context(*out);
-        }
-        return st;
+        return open_index(h, image, device, out);
     });
 }
 
@@ -1231,29 +1123,27 @@ extern "C" gdx_status gdx_index_create_from_parts(const gdx_parts *parts, int32_
         const uint32_t words = block_bits / 64, used = block_bits - (flat ? 16 : 0);
         const uint32_t units = flat ? parts->alphabet.num_dense_symbols : choose_layout(parts->alphabet.num_dense_symbols).planes;
         const uint64_t nwords = div_up(src.n + 1, used) * units * words;
-        uint64_t *d_blocks = nullptr;
-        uint8_t *d_bwt = nullptr;
-        CUDA_TRY(cudaMalloc(&d_blocks, nwords * 8));
-        cudaError_t e = cudaMalloc(&d_bwt, src.n ? src.n : 1);
-        if (e == cudaSuccess) e = cudaMemcpy(d_blocks, parts->interleaved_blocks, nwords * 8, cudaMemcpyHostToDevice);
-        if (e == cudaSuccess && src.n) {
-            k_ref_blocks_to_bwt<<<(unsigned)div_up(src.n, 256), 256>>>(d_blocks, flat ? 1u : 0u, words, units, src.n, d_bwt);
-            e = cudaGetLastError();
+        ImageHeader h;
+        DevMem image;
+        {
+            DevMem d_bwt;
+            {
+                DevMem d_blocks;
+                CUDA_TRY(d_blocks.alloc(nwords * 8));
+                cudaError_t e = d_bwt.alloc(src.n ? src.n : 1);
+                if (e == cudaSuccess)
+                    e = cudaMemcpy(d_blocks.p, parts->interleaved_blocks, nwords * 8, cudaMemcpyHostToDevice);
+                if (e == cudaSuccess && src.n) {
+                    k_ref_blocks_to_bwt<<<(unsigned)div_up(src.n, 256), 256>>>(
+                        d_blocks.as<uint64_t>(), flat ? 1u : 0u, words, units, src.n, d_bwt.as<uint8_t>());
+                    e = cudaGetLastError();
+                }
+                if (e != cudaSuccess) return fail(GDX_ERR_CUDA, "block upload failed: %s", cudaGetErrorString(e));
+            }
+            src.d_bwt = d_bwt.as<uint8_t>();
+            GDX_TRY(build_image(src, h, image));
         }
-        cudaFree(d_blocks);
-        if (e != cudaSuccess) {
-            if (d_bwt) cudaFree(d_bwt);
-            return fail(GDX_ERR_CUDA, "block upload failed: %s", cudaGetErrorString(e));
-        }
-        src.d_bwt = d_bwt;
-        gdx_status st = build_image(src, device, out);
-        cudaFree(d_bwt);
-        if (st == GDX_OK) {
-            auto_dense_sa(*out);
-            auto_seed_table(*out);
-            auto_row_context(*out);
-        }
-        return st;
+        return open_index(h, image, device, out);
     });
 }
 
@@ -1377,11 +1267,8 @@ extern "C" void gdx_index_destroy(gdx_index *idx) {
     }
     for (auto &p : idx->pinned)
         if (p.p) cudaFreeHost(p.p);
-    if (idx->dense_sa) cudaFree(idx->dense_sa);
-    if (idx->seed_lut) cudaFree(idx->seed_lut);
-    if (idx->row_ctx) cudaFree(idx->row_ctx);
     if (idx->own_image && idx->image) cudaFree(idx->image);
-    delete idx;
+    delete idx;  // and its accelerators
 }
 
 extern "C" gdx_status gdx_index_get_info(const gdx_index *idx, gdx_index_info *out) {
@@ -1406,10 +1293,10 @@ extern "C" gdx_status gdx_index_get_info(const gdx_index *idx, gdx_index_info *o
     out->num_text_borders = h.n_border;
     out->text_bytes = h.text_bits ? h.off_isa - h.off_text : 0;
     out->inverse_sample_bytes = h.has_isa ? h.image_bytes - h.off_isa : 0;
-    out->dense_suffix_array_bytes = idx->dense_sa_bytes;
-    out->seed_table_bytes = idx->seed_lut_bytes;
-    out->seed_table_depth = idx->dev.seed_depth;
-    out->row_context_entry_bytes = idx->row_ctx ? 16 : 0;
+    out->dense_suffix_array_bytes = idx->dense_sa.bytes;
+    out->seed_table_bytes = idx->seed_table.bytes;
+    out->seed_table_depth = idx->seed_table ? idx->seed_depth : 0;
+    out->row_context_entry_bytes = idx->row_context ? 16 : 0;
     return GDX_OK;
 }
 
@@ -1532,73 +1419,41 @@ extern "C" gdx_status gdx_index_adopt_image(const void *header, void *device_ima
         GDX_TRY(validate_header(h));
         int device;
         GDX_TRY(resolve_device(device_req, &device));
-        gdx_index *idx = new (std::nothrow) gdx_index();
-        if (!idx) return fail(GDX_ERR_OOM, "out of host memory");
-        idx->h = h;
-        idx->image = device_image;
-        idx->own_image = own_image != 0;
-        idx->device = device;
-        idx->dev = make_dev_index(h, device_image);
-        {
-            DeviceGuard guard(device);
-            gdx_status st = init_policies(idx);
-            if (st != GDX_OK) {
-                delete idx;
-                return st;
-            }
-            auto_dense_sa(idx);
-            auto_seed_table(idx);
-            auto_row_context(idx);
-        }
-        *out = idx;
-        return GDX_OK;
+        DeviceGuard guard(device);
+        return open_index(h, device_image, own_image != 0, device, out);
     });
 }
 
 extern "C" gdx_status gdx_index_set_seed_table_depth(gdx_index *idx, int32_t depth) {
-    return guarded([&]() -> gdx_status {
-        if (!idx) return fail(GDX_ERR_BAD_ARG, "NULL argument");
-        std::unique_lock<std::shared_mutex> cfg(idx->cfg_mu, std::try_to_lock);
-        if (!cfg.owns_lock()) return fail(GDX_ERR_BUSY, "queries are running on this index: the seed table cannot change now");
-        DeviceGuard guard(idx->device);
-        if (depth <= 0) {
-            drop_seed_table(idx);
-            return GDX_OK;
-        }
-        return build_seed_table(idx, (uint32_t)depth);
+    const char *busy = "queries are running on this index: the seed table cannot change now";
+    return with_config(idx, busy, [&]() -> gdx_status {
+        if (depth > 0) return build_seed_table(idx, (uint32_t)depth);
+        drop_table(idx, idx->seed_table);
+        return GDX_OK;
     });
 }
 
 extern "C" gdx_status gdx_index_set_row_context_table(gdx_index *idx, int32_t on) {
-    return guarded([&]() -> gdx_status {
-        if (!idx) return fail(GDX_ERR_BAD_ARG, "NULL argument");
-        std::unique_lock<std::shared_mutex> cfg(idx->cfg_mu, std::try_to_lock);
-        if (!cfg.owns_lock()) return fail(GDX_ERR_BUSY, "queries are running on this index: the row context table cannot change now");
-        DeviceGuard guard(idx->device);
+    const char *busy = "queries are running on this index: the row context table cannot change now";
+    return with_config(idx, busy, [&]() -> gdx_status {
         if (on) return build_row_context(idx);
-        drop_row_context(idx);
+        drop_table(idx, idx->row_context);
         return GDX_OK;
     });
 }
 
 extern "C" gdx_status gdx_index_set_text_verification(gdx_index *idx, int32_t on) {
-    return guarded([&]() -> gdx_status {
-        if (!idx) return fail(GDX_ERR_BAD_ARG, "NULL argument");
-        std::unique_lock<std::shared_mutex> cfg(idx->cfg_mu, std::try_to_lock);
-        if (!cfg.owns_lock()) return fail(GDX_ERR_BUSY, "queries are running on this index");
+    return with_config(idx, "queries are running on this index", [&]() -> gdx_status {
         idx->verify = on != 0;
         return GDX_OK;
     });
 }
 
 extern "C" gdx_status gdx_index_set_dense_suffix_array(gdx_index *idx, int32_t on) {
-    return guarded([&]() -> gdx_status {
-        if (!idx) return fail(GDX_ERR_BAD_ARG, "NULL argument");
-        std::unique_lock<std::shared_mutex> cfg(idx->cfg_mu, std::try_to_lock);
-        if (!cfg.owns_lock()) return fail(GDX_ERR_BUSY, "queries are running on this index: the dense suffix array cannot change now");
-        DeviceGuard guard(idx->device);
+    const char *busy = "queries are running on this index: the dense suffix array cannot change now";
+    return with_config(idx, busy, [&]() -> gdx_status {
         if (on) return build_dense_sa(idx);
-        drop_dense_sa(idx);
+        drop_table(idx, idx->dense_sa);
         return GDX_OK;
     });
 }

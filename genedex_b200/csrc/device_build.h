@@ -26,6 +26,10 @@ struct DeviceBuildResult {
     std::vector<uint64_t> border_rows, border_pos;  // sorted by row (bwt.rs:108-116)
     uint64_t verify_violations = 0;                 // only meaningful when verify was requested
     uint32_t rounds = 0;
+    DeviceBuildResult() = default;
+    DeviceBuildResult(const DeviceBuildResult &) = delete;
+    DeviceBuildResult &operator=(const DeviceBuildResult &) = delete;
+    ~DeviceBuildResult() { release(); }
     void release();
 };
 

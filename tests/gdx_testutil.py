@@ -1,4 +1,5 @@
 """Shared helpers of the parity tests: the same texts / alphabets / configs for oracle and product."""
+import ctypes as C
 import random
 
 import numpy as np
@@ -103,3 +104,38 @@ def assert_same_results(oidx, pidx, queries, check_locate=True):
         poff, phits = pidx.locate_many_packed(data, offsets)
         assert np.array_equal(ooff, poff), "hit offsets differ"
         assert np.array_equal(ohits, phits), "hits differ (same SA-row order expected)"
+
+
+def reference_parts(gdx, oidx, oa, sampling_rate, lookup_depth, blocks=None, samples_u32=False):
+    """gdx_parts of an index constructed by the reference crate (here: by the oracle, in the reference's own three-array
+    layout) for gdx_index_create_from_parts / _from_bwt.  blocks: another rank variant's interleaved_blocks instead of
+    the oracle's own (with their offsets).  Returns (parts, keep): keep holds the arrays the struct points into."""
+    L = gdx._lib
+    parts = L.gdx_parts()
+    C.memmove(parts.alphabet.io_to_dense, oa.io_to_dense.tobytes(), 256)
+    parts.alphabet.num_dense_symbols = oa.sigma
+    parts.alphabet.num_searchable_dense_symbols = oa.num_searchable
+    parts.storage = L.GDX_U32
+    parts.text_len = oidx.text_len
+    keep = dict(count=oidx.count_array(), blocks=oidx.blocks() if blocks is None else blocks,
+                sent=oidx.sentinel_indices())
+    keep["rows"], keep["pos"] = oidx.border()
+    parts.count = keep["count"].ctypes.data
+    parts.interleaved_blocks = keep["blocks"].ctypes.data
+    if blocks is None:
+        keep["bo"] = oidx.block_offsets()
+        parts.interleaved_block_offsets = keep["bo"].ctypes.data
+    if samples_u32:
+        keep["ssa32"] = oidx.samples().astype(np.uint32)
+        parts.sampled_suffix_array_u32 = keep["ssa32"].ctypes.data
+    else:
+        keep["ssa"] = oidx.samples()
+        parts.sampled_suffix_array = keep["ssa"].ctypes.data
+    parts.sampling_rate = sampling_rate
+    parts.text_border_rows = keep["rows"].ctypes.data
+    parts.text_border_positions = keep["pos"].ctypes.data
+    parts.num_text_borders = keep["rows"].size
+    parts.sentinel_indices = keep["sent"].ctypes.data
+    parts.num_texts = keep["sent"].size
+    parts.lookup_table_depth = lookup_depth
+    return parts, keep

@@ -213,26 +213,7 @@ def test_from_reference_parts(gdx):
         texts = util.random_texts(rng, oa, 3, 5000)
         oidx = O.OracleIndex.build(texts, oa, "u32", sampling_rate=4, lookup_depth=2)
         L = gdx._lib
-        parts = L.gdx_parts()
-        C.memmove(parts.alphabet.io_to_dense, oa.io_to_dense.tobytes(), 256)
-        parts.alphabet.num_dense_symbols = oa.sigma
-        parts.alphabet.num_searchable_dense_symbols = oa.num_searchable
-        parts.storage = L.GDX_U32
-        parts.text_len = oidx.text_len
-        keep = dict(count=oidx.count_array(), blocks=oidx.blocks(), bo=oidx.block_offsets(), ssa=oidx.samples(),
-                    sent=oidx.sentinel_indices())
-        keep["rows"], keep["pos"] = oidx.border()
-        parts.count = keep["count"].ctypes.data
-        parts.interleaved_blocks = keep["blocks"].ctypes.data
-        parts.interleaved_block_offsets = keep["bo"].ctypes.data
-        parts.sampled_suffix_array = keep["ssa"].ctypes.data
-        parts.sampling_rate = 4
-        parts.text_border_rows = keep["rows"].ctypes.data
-        parts.text_border_positions = keep["pos"].ctypes.data
-        parts.num_text_borders = keep["rows"].size
-        parts.sentinel_indices = keep["sent"].ctypes.data
-        parts.num_texts = keep["sent"].size
-        parts.lookup_table_depth = 2
+        parts, keep = util.reference_parts(gdx, oidx, oa, 4, 2)
         qs = util.random_queries(rng, oa, texts, 200, 100, 16, searchable_only=True)
         h = C.c_void_p()
         assert L.load().gdx_index_create_from_parts(C.byref(parts), -1, C.byref(h)) == 0
@@ -255,25 +236,7 @@ def test_from_reference_parts_all_rank_variants(gdx, variant, block_bits):
         texts = util.random_texts(rng, oa, 3, 70_000 if alph == "ascii_dna" else 6000)
         oidx = O.OracleIndex.build(texts, oa, "u32", sampling_rate=3, lookup_depth=1)
         vr = O.OracleVariantRank(oidx.bwt(), oa.sigma, "u32", variant, block_bits)
-        parts = L.gdx_parts()
-        C.memmove(parts.alphabet.io_to_dense, oa.io_to_dense.tobytes(), 256)
-        parts.alphabet.num_dense_symbols = oa.sigma
-        parts.alphabet.num_searchable_dense_symbols = oa.num_searchable
-        parts.storage = L.GDX_U32
-        parts.text_len = oidx.text_len
-        keep = dict(count=oidx.count_array(), blocks=vr.blocks(), ssa32=oidx.samples().astype(np.uint32),
-                    sent=oidx.sentinel_indices())
-        keep["rows"], keep["pos"] = oidx.border()
-        parts.count = keep["count"].ctypes.data
-        parts.interleaved_blocks = keep["blocks"].ctypes.data
-        parts.sampled_suffix_array_u32 = keep["ssa32"].ctypes.data
-        parts.sampling_rate = 3
-        parts.text_border_rows = keep["rows"].ctypes.data
-        parts.text_border_positions = keep["pos"].ctypes.data
-        parts.num_text_borders = keep["rows"].size
-        parts.sentinel_indices = keep["sent"].ctypes.data
-        parts.num_texts = keep["sent"].size
-        parts.lookup_table_depth = 1
+        parts, keep = util.reference_parts(gdx, oidx, oa, 3, 1, blocks=vr.blocks(), samples_u32=True)
         parts.rank_variant = L.GDX_RANK_FLAT if variant == "flat" else L.GDX_RANK_CONDENSED
         parts.block_bits = block_bits
         parts.flags = L.GDX_FLAG_NO_SEED_TABLE
