@@ -1,7 +1,10 @@
 """GPU tests of the Hamming search (gdx_count_many_hamming / gdx_cursors_many_hamming / gdx_locate_many_hamming) against a
 naive scan of every window and the oracle, on every rank layout, storage type, construction route, with and without the
 text section and the accelerators; its k = 0 form against the exact entry points; its errors; batches of several
-chunks; concurrent calls; the C++ mirror."""
+chunks; concurrent calls; the C++ mirror.  On indexes of several rank superblocks (where a superblock's counts differ
+from `count`), a homopolymer run, a repeat-rich genome slice and long queries: against the references of
+tests/hamming_ref.py, and the node expansions (gdx_stats.lf_steps) against the host emulation of the same search, which
+ties the device-only K32 expansion to the CPU-tested core.  Exact search on the same indexes against the oracle."""
 import ctypes as C
 import os
 import random
@@ -15,7 +18,9 @@ import pytest
 
 from oracle import oracle as O
 import gdx_testutil as util
-from hamming_ref import Naive, hamming_queries, hamming_texts
+from hamming_ref import (SUPERBLOCK, Cheapest, Naive, hamming_queries, hamming_texts, multi_superblock_texts,
+                         window_queries)
+from test_hamming_host import EmulIndex, build_emul
 
 pytestmark = pytest.mark.gpu
 
@@ -330,6 +335,237 @@ def test_wide_path():
     # the 64-bit sample / lookup paths, on a subset of this file in a process of its own
     env = dict(os.environ, GDX_FORCE_WIDE="1")
     out = subprocess.run([sys.executable, "-m", "pytest", os.path.abspath(__file__), "-m", "gpu", "-q", "-x",
-                          "-p", "no:cacheprovider", "-k", "parity_with_naive_scan and (u32 or i32) or long_queries or errors"],
+                          "-p", "no:cacheprovider", "-k",
+                          "parity_with_naive_scan and (u32 or i32) or long_queries or errors or configurations or "
+                          "boundary_lengths"],
                          env=env, capture_output=True, text=True, cwd=ROOT)
     assert out.returncode == 0, out.stdout[-3000:] + out.stderr[-2000:]
+
+
+# ---- indexes of several rank superblocks -----------------------------------------------------------------------
+
+@pytest.fixture(scope="module")
+def emul(tmp_path_factory):
+    return build_emul(tmp_path_factory.mktemp("emul_hamming"))
+
+
+# (rank_layout, rank_record_bytes): 0 = K32 (32-byte records of 64 positions), 1 = KG<B> (128 positions)
+LAYOUTS = {
+    "u8_until_0": (0, 32), "u8_until_2": (0, 32), "ascii_dna": (0, 32), "acg_n": (0, 32),
+    "ascii_dna_with_n": (0, 32), "dna_n_searchable": (0, 32),
+    "dna_rny": (1, 64),                     # KG<3>
+    "dna_iupac_kept": (1, 96),              # KG<4>
+    "protein20": (1, 128),                  # KG<5>
+    "u8_until_40": (1, 192),                # KG<6>
+    "ascii_printable": (1, 320),            # KG<7>
+    "u8_ns4": (1, 640), "u8_until_254": (1, 640),  # KG<8>
+}
+LONG = (64, 65, 127, 128, 200, 255, 256)
+
+
+def expect_layout(pidx, oidx, name):
+    info = pidx.info()
+    assert (info.rank_layout, info.rank_record_bytes) == LAYOUTS[name], name
+    assert info.text_len == oidx.text_len
+    return info
+
+
+def check_with_steps(gdx, pidx, oidx, ref, ex, qs, k):
+    """check_against_naive with another reference, and the node expansions of the locate call against the host
+    emulation of the same search"""
+    check_against_naive(gdx, pidx, oidx, ref, qs, k)
+    assert pidx.stats().lf_steps == sum(ex.search(q, k)[2] for q in qs), k
+
+
+def check_exact(pidx, oidx, oa, texts, seed):
+    """exact search against the oracle, and extend_many on intervals that straddle each superblock boundary"""
+    rng = random.Random(seed)
+    util.assert_same_results(oidx, pidx, util.random_queries(rng, oa, texts, 300, 100, 40))
+    syms = util.searchable_io_symbols(oa)
+    n = oidx.text_len
+    iv = []
+    for b in range(SUPERBLOCK, n + 1, SUPERBLOCK):
+        iv += [(b - 1, min(b + 1, n)), (b, min(b + 64, n)), (b - 128, b)]
+        iv += [(b - rng.randrange(1, 5000), min(n, b + rng.randrange(1, 5000))) for _ in range(6)]
+    sym = [rng.choice(syms) for _ in iv]
+    s, e = pidx.extend_many_packed(np.array([a for a, _ in iv], dtype=np.uint64),
+                                   np.array([b for _, b in iv], dtype=np.uint64), np.frombuffer(bytes(sym), np.uint8))
+    assert list(zip(s.tolist(), e.tolist())) == [oidx.extend_query_front(x, c) for x, c in zip(iv, sym)]
+
+
+def plan_for(ns):
+    """[(k, query lengths, queries per length)] that keep the references cheap"""
+    if ns == 1:  # a homopolymer: every window matches, one interval of the whole text per query
+        return [(1, (10,), 1), (3, (40,), 1)]
+    if ns <= 5:
+        return [(1, (10, 24), 10), (2, (12, 30), 10), (3, (12, 16), 10), (3, LONG, 2)]
+    if ns < 255:
+        return [(1, (6, 12), 10), (2, (9,), 10), (3, (12,), 10), (3, LONG, 2)]
+    return [(1, (3, 8), 10), (2, (9,), 6), (3, (12, 256), 2)]
+
+
+SUPERBLOCK_CASES = [  # (alphabet, symbols)
+    ("u8_until_0", 300_000), ("u8_until_2", 400_000), ("ascii_dna", 400_000), ("acg_n", 400_000),
+    ("ascii_dna_with_n", 600_000), ("dna_n_searchable", 400_000), ("dna_rny", 400_000),
+    ("dna_iupac_kept", 300_000), ("protein20", 400_000), ("u8_until_40", 300_000), ("ascii_printable", 300_000),
+    ("u8_ns4", 300_000), ("u8_until_254", 400_000),
+]
+
+
+@pytest.mark.parametrize("name,total", SUPERBLOCK_CASES, ids=[c[0] for c in SUPERBLOCK_CASES])
+def test_every_layout_on_several_superblocks(gdx, emul, name, total):
+    oa = util.oracle_alphabet(name)
+    seed = zlib.crc32(b"sb-" + name.encode())
+    # (one searchable symbol: short texts, since a long homopolymer makes the oracle's suffix sort quadratic)
+    texts = multi_superblock_texts(seed, oa, total, ntexts=6 if oa.num_searchable > 1 else 300)
+    oidx = O.OracleIndex.build(texts, oa, "u32", sampling_rate=4)
+    pidx = build(gdx, texts, name, on_device=seed % 2 == 0)
+    expect_layout(pidx, oidx, name)
+    assert oidx.text_len > 4 * SUPERBLOCK
+    ref, ex = Cheapest(oidx, oa), EmulIndex(emul, oidx, oa)
+    for k, lengths, nq in plan_for(oa.num_searchable):
+        qs = [q for m in lengths for q in window_queries(seed + 31 * k + m, oa, texts, nq, m, k)]
+        check_with_steps(gdx, pidx, oidx, ref, ex, qs, k)
+    check_k0_equals_exact(pidx, window_queries(seed, oa, texts, 200 if oa.num_searchable > 1 else 4, 20, 0) + [b""])
+    if LAYOUTS[name][0] == 0:  # the K32 expansion on borders of different superblocks, the derived child past 0
+        _, derived = ex.layout()
+        assert ex.cover[0] > 0, ex.cover
+        assert (ex.cover[1] > 0) == (0 < derived <= oa.num_searchable), ex.cover
+    check_exact(pidx, oidx, oa, texts, seed)
+
+
+BOUNDARY_CASES = [(name, extra) for name in ("ascii_dna_with_n", "protein20") for extra in (-1, 0)]
+
+
+@pytest.mark.parametrize("name,extra", BOUNDARY_CASES, ids=[f"{n}-n_plus_{1 + e}" for n, e in BOUNDARY_CASES])
+def test_boundary_lengths(gdx, emul, name, extra):
+    # text_len + 1 (extra = -1) or text_len (extra = 0) a multiple of the superblock: the last superblock filled up to
+    # its end, and the record of position n alone in a superblock of its own
+    oa = util.oracle_alphabet(name)
+    seed = zlib.crc32(f"bl-{name}{extra}".encode())
+    n = 4 * SUPERBLOCK + extra
+    texts = multi_superblock_texts(seed, oa, n - 6)  # 6 texts, 6 sentinels
+    oidx = O.OracleIndex.build(texts, oa, "u32", sampling_rate=4)
+    assert oidx.text_len == n and len(texts) == 6
+    pidx = build(gdx, texts, name, on_device=extra == 0)
+    expect_layout(pidx, oidx, name)
+    ref, ex = Cheapest(oidx, oa), EmulIndex(emul, oidx, oa)
+    for k, lengths, nq in plan_for(oa.num_searchable)[:3]:
+        qs = [q for m in lengths for q in window_queries(seed + k + m, oa, texts, nq, m, k)]
+        check_with_steps(gdx, pidx, oidx, ref, ex, qs, k)
+    check_exact(pidx, oidx, oa, texts, seed)
+
+
+def test_interval_wider_than_u16(gdx, emul):
+    # A x 70 000 across a superblock boundary: in-superblock u16 offsets near their maximum, and queries A x m whose
+    # exact interval holds ~70 000 rows (the (end - start) << 2 packing and the fill of wide intervals in locate)
+    oa = util.oracle_alphabet("ascii_dna_with_n")
+    nrng = np.random.default_rng(70)
+    rand = lambda n: nrng.choice(np.frombuffer(b"ACGTN", dtype=np.uint8), n, p=[.24] * 4 + [.04]).tobytes()  # noqa
+    texts = [rand(40_000), rand(20_000) + b"A" * 70_000 + rand(50_000), b"", rand(30_000)]
+    oidx = O.OracleIndex.build(texts, oa, "u32", sampling_rate=4)
+    pidx = build(gdx, texts, "ascii_dna_with_n")
+    expect_layout(pidx, oidx, "ascii_dna_with_n")
+    ref, ex = Cheapest(oidx, oa), EmulIndex(emul, oidx, oa)
+    qs = [b"A" * m for m in (1, 2, 12, 20, 100)] + [b"A" * 30 + b"C" + b"A" * 30, b"CA" + b"A" * 40]
+    for k in range(4):
+        check_with_steps(gdx, pidx, oidx, ref, ex, qs, k)
+    assert ex.cover[2] > 0 and ex.cover[0] > 0, ex.cover
+    cnt = pidx.count_many_hamming([b"A" * 20], 1)
+    assert cnt[0, 0] > 65535
+
+
+def test_repeat_rich_index(gdx, emul):
+    # hg38-like repeat families at 6 Mbp: queries from repeat copies have hundreds of intervals (deep searches, large
+    # pass-2 sort segments, many wide intervals); one batch of more than 2^20 queries, a sample of every chunk
+    import torch
+    if os.path.join(ROOT, "tools") not in sys.path:
+        sys.path.insert(0, os.path.join(ROOT, "tools"))
+    import run_configs
+    oa = util.oracle_alphabet("ascii_dna_with_n")
+    text, _ = run_configs.make_repeat_rich_text(6_000_000, torch.device("cuda", 0))
+    host = text.cpu().numpy()
+    del text
+    texts = [host[:2_500_000].tobytes(), b"", host[2_500_000:].tobytes()]
+    oidx = O.OracleIndex.build(texts, oa, "u32", sampling_rate=4)
+    pidx = build(gdx, texts, "ascii_dna_with_n", on_device=True)
+    expect_layout(pidx, oidx, "ascii_dna_with_n")
+    ref, ex = Cheapest(oidx, oa), EmulIndex(emul, oidx, oa)
+    rng = random.Random(77)
+    # windows of repeat copies (at least 20 occurrences; 2 at m = 100, where copies diverge), 0..k substitutions
+    most = 0
+    for k, m in ((1, 20), (1, 100), (2, 20), (2, 40), (3, 20), (3, 40), (3, 100)):
+        cand = [w.replace(b"N", b"A") for w in window_queries(rng.random(), oa, texts, 2000, m, 0)]
+        c = oidx.count_many(cand, nthreads=0)
+        reps = [w for w, x in zip(cand, c.tolist()) if x >= (20 if m < 100 else 2)][:6]
+        assert len(reps) >= 3, (k, m)
+        qs = []
+        for w in reps:
+            w = bytearray(w)
+            for _ in range(rng.randrange(k + 1)):
+                w[rng.randrange(m)] = rng.choice(b"ACGT")
+            qs.append(bytes(w))
+        check_with_steps(gdx, pidx, oidx, ref, ex, qs, k)
+        data, off = O.pack(qs)
+        ioff = pidx.cursors_many_hamming_packed(data, off, k)[0]
+        most = max(most, int(np.diff(ioff).max()))
+    assert most >= 100, most
+    # more than 2^20 queries at k = 1: a sample of each chunk and the first and last query against the reference
+    nrng = np.random.default_rng(78)
+    nq, m = CHUNK + 40_000, 30
+    arr = np.frombuffer(b"".join(texts), dtype=np.uint8)
+    starts = nrng.integers(0, arr.size - m, nq)
+    qmat = arr[starts[:, None] + np.arange(m)].copy()
+    qmat[qmat == ord("N")] = ord("C")
+    flip = np.flatnonzero(nrng.random(nq) < 0.5)
+    qmat[flip, nrng.integers(0, m, flip.size)] = ord("G")
+    data = np.ascontiguousarray(qmat.reshape(-1))
+    off = np.arange(nq + 1, dtype=np.uint64) * m
+    counts = pidx.count_many_hamming_packed(data, off, 1)
+    ioff, s, e, d = pidx.cursors_many_hamming_packed(data, off, 1)
+    hoff, hits = pidx.locate_many_hamming_packed(data, off, 1)
+    assert np.array_equal(np.diff(hoff), counts.sum(axis=1))
+    sample = sorted(set(rng.sample(range(CHUNK), 40) + rng.sample(range(CHUNK, nq), 40) + [0, CHUNK - 1, CHUNK, nq - 1]))
+    for i in sample:
+        occ, ivs, _ = ref.expected(bytes(qmat[i]), 1)
+        assert counts[i].tolist() == occ, i
+        a, b = int(ioff[i]), int(ioff[i + 1])
+        assert list(zip(s[a:b].tolist(), e[a:b].tolist(), d[a:b].tolist())) == ivs, i
+        a, b = int(hoff[i]), int(hoff[i + 1])
+        assert [tuple(h) for h in hits[a:b].tolist()] == [h for x, y, _ in ivs for h in oidx.locate_interval(x, y)], i
+    # the sampled queries alone: node expansions against the host emulation
+    check_with_steps(gdx, pidx, oidx, ref, ex, [bytes(qmat[i]) for i in sample], 1)
+
+
+CONFIGS = [  # (alphabet, storage, on_device, sampling rate, dense suffix array, text section)
+    ("ascii_dna_with_n", "u32", False, 1, True, True),
+    ("ascii_dna_with_n", "i64", True, 3, False, True),
+    ("ascii_dna_with_n", "u32", True, 32, False, False),
+    ("ascii_dna_with_n", "i64", False, 4, True, False),
+    ("protein20", "u32", True, 1, False, False),
+    ("protein20", "i64", False, 3, True, True),
+    ("protein20", "u32", False, 32, True, False),
+    ("protein20", "i64", True, 4, False, True),
+]
+
+
+@pytest.mark.parametrize("name,storage,on_device,rate,dense,text", CONFIGS,
+                         ids=["-".join(str(x) for x in c) for c in CONFIGS])
+def test_configurations_on_several_superblocks(gdx, emul, name, storage, on_device, rate, dense, text):
+    oa = util.oracle_alphabet(name)
+    seed = zlib.crc32("-".join(str(x) for x in (name, storage, on_device, rate, dense, text)).encode())
+    texts = multi_superblock_texts(seed, oa, 300_000)
+    oidx = O.OracleIndex.build(texts, oa, storage, sampling_rate=rate)
+    cfg = (gdx.FmIndexConfig(storage).suffix_array_sampling_rate(rate).construct_on_device(on_device, verify=on_device)
+           .keep_text(text).dense_suffix_array(dense))
+    pidx = cfg.construct_index(texts, util.product_alphabet(gdx, name))
+    if dense:
+        pidx.set_dense_suffix_array(True)
+    info = expect_layout(pidx, oidx, name)
+    assert info.sampling_rate == rate
+    assert (info.dense_suffix_array_bytes > 0) == dense and (info.text_bytes > 0) == text
+    ref, ex = Cheapest(oidx, oa), EmulIndex(emul, oidx, oa)
+    for k, lengths, nq in plan_for(oa.num_searchable):
+        qs = [q for m in lengths for q in window_queries(seed + 7 * k + m, oa, texts, min(nq, 4), m, k)]
+        check_with_steps(gdx, pidx, oidx, ref, ex, qs, k)
+    check_exact(pidx, oidx, oa, texts, seed)
