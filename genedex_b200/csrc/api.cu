@@ -31,6 +31,7 @@
 #include "../../include/genedex_b200.h"
 #include "accel_policy.h"
 #include "chunk_plan.h"
+#include "cuda_owners.h"
 #include "device_build.h"
 #include "device_index.h"
 #include "host_build.h"
@@ -123,82 +124,6 @@ struct DeviceGuard {
     }
 };
 
-// grow-only device buffer
-struct DBuf {
-    void *p = nullptr;
-    uint64_t cap = 0;
-    cudaError_t reserve(uint64_t bytes) {
-        if (bytes <= cap) return cudaSuccess;
-        if (p) cudaFree(p);
-        p = nullptr;
-        cap = 0;
-        uint64_t want = align_up(bytes + bytes / 8, 256);
-        cudaError_t e = cudaMalloc(&p, want);
-        if (e != cudaSuccess) {
-            e = cudaMalloc(&p, want = align_up(bytes, 256));
-            if (e != cudaSuccess) return e;
-        }
-        cap = want;
-        return cudaSuccess;
-    }
-    void release() {
-        if (p) cudaFree(p);
-        p = nullptr;
-        cap = 0;
-    }
-    template <class T>
-    T *as() const { return reinterpret_cast<T *>(p); }
-};
-
-// one device allocation with one owner: an accelerator table, an image under construction, a temporary of a build
-struct DevMem {
-    void *p = nullptr;
-    uint64_t bytes = 0;
-    DevMem() = default;
-    DevMem(DevMem &&o) noexcept : p(std::exchange(o.p, nullptr)), bytes(std::exchange(o.bytes, 0)) {}
-    DevMem &operator=(DevMem &&o) noexcept {
-        std::swap(p, o.p);
-        std::swap(bytes, o.bytes);
-        return *this;
-    }
-    ~DevMem() {
-        if (p) cudaFree(p);
-    }
-    cudaError_t alloc(uint64_t nbytes) {
-        const cudaError_t e = cudaMalloc(&p, nbytes);
-        bytes = e == cudaSuccess ? nbytes : 0;
-        return e;
-    }
-    void *release() {
-        bytes = 0;
-        return std::exchange(p, nullptr);
-    }
-    explicit operator bool() const { return p != nullptr; }
-    template <class T>
-    T *as() const { return reinterpret_cast<T *>(p); }
-};
-
-// grow-only pinned host buffer (staging for callers that pass ordinary pageable memory)
-struct HBuf {
-    void *p = nullptr;
-    uint64_t cap = 0;
-    cudaError_t reserve(uint64_t bytes) {
-        if (bytes <= cap) return cudaSuccess;
-        if (p) cudaFreeHost(p);
-        p = nullptr;
-        cap = 0;
-        const uint64_t want = align_up(bytes + bytes / 8, 4096);
-        cudaError_t e = cudaMallocHost(&p, want);
-        if (e == cudaSuccess) cap = want;
-        return e;
-    }
-    void release() {
-        if (p) cudaFreeHost(p);
-        p = nullptr;
-        cap = 0;
-    }
-};
-
 // true for cudaMallocHost / cudaHostRegister'ed / managed memory, false for ordinary (pageable) host memory
 bool is_pinned(const void *p) {
     cudaPointerAttributes attr;
@@ -233,13 +158,13 @@ struct EventPairs {
     struct Pair {
         cudaEvent_t begin, end;
     };
-    std::vector<cudaEvent_t> ev;
+    std::vector<Event> ev;
     size_t used = 0;
     cudaEvent_t take() {
         if (used == ev.size()) {
-            cudaEvent_t e = nullptr;
-            if (cudaEventCreate(&e) != cudaSuccess) return nullptr;  // recording on nullptr fails loudly later
-            ev.push_back(e);
+            Event e;
+            if (e.create(cudaEventDefault) != cudaSuccess) return nullptr;  // recording on nullptr fails loudly later
+            ev.push_back(std::move(e));
         }
         return ev[used++];
     }
@@ -255,51 +180,45 @@ struct EventPairs {
         return ms;
     }
     void reset() { used = 0; }
-    void destroy() {
-        for (auto e : ev) cudaEventDestroy(e);
-    }
 };
 
 // SA intervals -> hits on one stream.  count() writes the width of every interval, their exclusive scan (the CSR
 // offsets, n + 1 entries) and sends the hit total and the number of wide intervals to the pinned words; expand_walk()
 // then lists the rows of every interval (wide ones through a worklist) and walks them to text positions.
 struct IntervalHits {
-    DBuf counts, offsets, scan_tmp, rows, hits, wide;
+    DevMem counts, offsets, scan_tmp, rows, hits, wide;
     struct DeviceWords {
         unsigned long long wide, cursor;  // intervals wider than kExpandInline, worklist cursor
-    } *d = nullptr;
+    };
     struct HostWords {
         uint64_t hits, wide;  // pinned: hit total, intervals wider than kExpandInline
-    } *h = nullptr;
-    cudaEvent_t ev_total = nullptr;  // *h is on the host
-    EventPairs timing;               // around the locate kernels of the current call
+    };
+    DevMem d_words;
+    HBuf h_words;
+    Event ev_total;     // *h() is on the host
+    EventPairs timing;  // around the locate kernels of the current call
     bool init() {
-        return cudaMalloc(&d, sizeof *d) == cudaSuccess && cudaMallocHost(&h, sizeof *h) == cudaSuccess &&
-               cudaEventCreateWithFlags(&ev_total, cudaEventDisableTiming) == cudaSuccess;
+        return d_words.alloc(sizeof(DeviceWords)) == cudaSuccess && h_words.alloc(sizeof(HostWords)) == cudaSuccess &&
+               ev_total.create(cudaEventDisableTiming) == cudaSuccess;
     }
-    void destroy() {
-        for (DBuf *b : {&counts, &offsets, &scan_tmp, &rows, &hits, &wide}) b->release();
-        if (d) cudaFree(d);
-        if (h) cudaFreeHost(h);
-        if (ev_total) cudaEventDestroy(ev_total);
-        timing.destroy();
-    }
+    DeviceWords *d() const { return d_words.as<DeviceWords>(); }
+    HostWords *h() const { return h_words.as<HostWords>(); }
     gdx_status count(cudaStream_t st, const uint64_t *starts, const uint64_t *ends, uint64_t n);
     gdx_status expand_walk(const gdx_index *idx, cudaStream_t st, const uint64_t *starts, const uint64_t *ends, uint64_t n,
                            uint64_t n_hits, uint64_t n_wide, unsigned long long *walk_steps, bool hit32);
 };
 
 struct Slot {
-    cudaStream_t stream = nullptr;
-    DBuf bytes, offsets, out_a, out_b, sort;
+    Stream stream;
+    DevMem bytes, offsets, out_a, out_b, sort;
     IntervalHits locate;  // pipelined locate: the chunk's CSR, rows and hits
     // staging for pageable caller buffers / packed queries / narrow results
     HBuf h_in, h_off, h_out_a, h_out_b;
     // queries of a packed chunk that hold a byte without a 2-bit code: offsets + slots + IO bytes, re-run raw
     HBuf h_x;
-    DBuf xbuf;
-    cudaEvent_t ev_h2d = nullptr, ev_out = nullptr;
-    cudaEvent_t ev_link = nullptr;  // the chunk's query upload has left the PCIe link
+    DevMem xbuf;
+    Event ev_h2d, ev_out;
+    Event ev_link;  // the chunk's query upload has left the PCIe link
     bool h2d_pending = false;
     EventPairs timing;  // around the search kernels of the current call
 };
@@ -319,55 +238,21 @@ static_assert(offsetof(Counters, extend_bad_cursor) == offsetof(Counters, extend
 
 struct Workspace {
     Slot slot[kSlots];
-    Counters *cnt_h = nullptr;  // pinned
-    Counters *cnt_d = nullptr;  // device
-    DBuf starts, ends, symbols;
+    HBuf cnt_host;
+    DevMem cnt_dev;
+    DevMem starts, ends, symbols;
     IntervalHits locate;  // gdx_locate_intervals and the Hamming locate
-    cudaEvent_t ev_a = nullptr;  // orders the slot streams behind the reset of the counters (search_host)
-    bool init() {
-        for (auto &s : slot) {
-            if (cudaStreamCreateWithFlags(&s.stream, cudaStreamNonBlocking) != cudaSuccess) return false;
-            if (!s.locate.init()) return false;
-            if (cudaEventCreateWithFlags(&s.ev_h2d, cudaEventDisableTiming) != cudaSuccess) return false;
-            if (cudaEventCreateWithFlags(&s.ev_out, cudaEventDisableTiming) != cudaSuccess) return false;
-            if (cudaEventCreateWithFlags(&s.ev_link, cudaEventDisableTiming) != cudaSuccess) return false;
-        }
-        if (cudaMallocHost(&cnt_h, sizeof(Counters)) != cudaSuccess) return false;
-        if (cudaMalloc(&cnt_d, sizeof(Counters)) != cudaSuccess) return false;
-        if (!locate.init()) return false;
-        if (cudaEventCreate(&ev_a) != cudaSuccess) return false;
-        return true;
-    }
-    void destroy() {
-        for (auto &s : slot) {
-            if (s.stream) cudaStreamDestroy(s.stream);
-            s.bytes.release();
-            s.offsets.release();
-            s.out_a.release();
-            s.out_b.release();
-            s.sort.release();
-            s.locate.destroy();
-            if (s.ev_h2d) cudaEventDestroy(s.ev_h2d);
-            if (s.ev_out) cudaEventDestroy(s.ev_out);
-            if (s.ev_link) cudaEventDestroy(s.ev_link);
-            for (HBuf *b : {&s.h_in, &s.h_off, &s.h_out_a, &s.h_out_b, &s.h_x}) b->release();
-            s.xbuf.release();
-            s.timing.destroy();
-        }
-        if (cnt_h) cudaFreeHost(cnt_h);
-        if (cnt_d) cudaFree(cnt_d);
-        for (DBuf *b : {&starts, &ends, &symbols}) b->release();
-        locate.destroy();
-        if (ev_a) cudaEventDestroy(ev_a);
-    }
+    Event ev_a;           // orders the slot streams behind the reset of the counters (search_host)
+    Counters *cnt_h() const { return cnt_host.as<Counters>(); }  // pinned
+    Counters *cnt_d() const { return cnt_dev.as<Counters>(); }   // device
     // error words to kNoError, counters to zero
     cudaError_t reset_counters(cudaStream_t st) {
         constexpr size_t kErrBytes = offsetof(Counters, search);
-        const cudaError_t e = cudaMemsetAsync(cnt_d, 0xff, kErrBytes, st);
-        return e != cudaSuccess ? e : cudaMemsetAsync((uint8_t *)cnt_d + kErrBytes, 0, sizeof(Counters) - kErrBytes, st);
+        const cudaError_t e = cudaMemsetAsync(cnt_d(), 0xff, kErrBytes, st);
+        return e != cudaSuccess ? e : cudaMemsetAsync((uint8_t *)cnt_d() + kErrBytes, 0, sizeof(Counters) - kErrBytes, st);
     }
     cudaError_t read_counters(cudaStream_t st) {
-        return cudaMemcpyAsync(cnt_h, cnt_d, sizeof(Counters), cudaMemcpyDeviceToHost, st);
+        return cudaMemcpyAsync(cnt_h(), cnt_d(), sizeof(Counters), cudaMemcpyDeviceToHost, st);
     }
     void reset_timing() {
         for (auto &s : slot) {
@@ -378,9 +263,23 @@ struct Workspace {
     }
 };
 
+// a workspace with its streams, events and words, or nullptr when one of them cannot be created
+std::unique_ptr<Workspace> new_workspace() {
+    auto w = std::make_unique<Workspace>();
+    for (auto &s : w->slot)
+        if (s.stream.create(cudaStreamNonBlocking) != cudaSuccess || !s.locate.init() ||
+            s.ev_h2d.create(cudaEventDisableTiming) != cudaSuccess || s.ev_out.create(cudaEventDisableTiming) != cudaSuccess ||
+            s.ev_link.create(cudaEventDisableTiming) != cudaSuccess)
+            return nullptr;
+    if (w->cnt_host.alloc(sizeof(Counters)) != cudaSuccess || w->cnt_dev.alloc(sizeof(Counters)) != cudaSuccess ||
+        !w->locate.init() || w->ev_a.create(cudaEventDefault) != cudaSuccess)
+        return nullptr;
+    return w;
+}
+
+// a pinned hit buffer of the index, lent to one call at a time
 struct PinnedHits {
-    void *p = nullptr;
-    uint64_t cap = 0;
+    HBuf buf;
     bool in_use = false;
 };
 
@@ -389,7 +288,7 @@ struct PinnedHits {
 struct gdx_index {
     ImageHeader h;
     void *image = nullptr;
-    bool own_image = false;
+    DevMem owned_image;            // holds image unless it was adopted with own_image = 0
     int device = 0;
     DevIndex dev;                  // written by refresh_dev only
     // accelerators outside the image (gdx_index_set_dense_suffix_array / _seed_table_depth / _row_context_table)
@@ -401,39 +300,31 @@ struct gdx_index {
     // exclusively and reports GDX_ERR_BUSY instead of pulling memory from under a running kernel
     mutable std::shared_mutex cfg_mu;
     mutable std::mutex mu;
-    mutable std::vector<Workspace *> free_ws;
+    mutable std::vector<std::unique_ptr<Workspace>> free_ws;
     mutable std::vector<PinnedHits> pinned;
 };
 
 namespace {
 
-Workspace *acquire_ws(const gdx_index *idx) {
+std::unique_ptr<Workspace> acquire_ws(const gdx_index *idx) {
     {
         std::lock_guard<std::mutex> lk(idx->mu);
         if (!idx->free_ws.empty()) {
-            Workspace *w = idx->free_ws.back();
+            std::unique_ptr<Workspace> w = std::move(idx->free_ws.back());
             idx->free_ws.pop_back();
             return w;
         }
     }
-    Workspace *w = new Workspace();
-    if (!w->init()) {
-        w->destroy();
-        delete w;
-        return nullptr;
-    }
-    return w;
-}
-void release_ws(const gdx_index *idx, Workspace *w) {
-    std::lock_guard<std::mutex> lk(idx->mu);
-    idx->free_ws.push_back(w);
+    return new_workspace();
 }
 struct WsLease {
     const gdx_index *idx;
-    Workspace *w;
+    std::unique_ptr<Workspace> w;
     explicit WsLease(const gdx_index *i) : idx(i), w(acquire_ws(i)) {}
     ~WsLease() {
-        if (w) release_ws(idx, w);
+        if (!w) return;
+        std::lock_guard<std::mutex> lk(idx->mu);
+        idx->free_ws.push_back(std::move(w));
     }
 };
 
@@ -453,8 +344,8 @@ gdx_status with_workspace(const gdx_index *idx, F &&f) {
     WsLease lease(idx);
     if (!lease.w) return fail(GDX_ERR_CUDA, "could not create a CUDA workspace: %s", cudaGetErrorString(cudaGetLastError()));
     lease.w->reset_timing();
-    const gdx_status st = f(lease.w);
-    if (st != GDX_OK) drain(lease.w);
+    const gdx_status st = f(lease.w.get());
+    if (st != GDX_OK) drain(lease.w.get());
     return st;
 }
 
@@ -798,7 +689,7 @@ gdx_status open_index(const ImageHeader &h, void *image, bool own_image, int dev
     if (!idx) return fail(GDX_ERR_OOM, "out of host memory");
     idx->h = h;
     idx->image = image;
-    idx->own_image = own_image;
+    if (own_image) idx->owned_image = DevMem(image, h.image_bytes);
     idx->device = device;
     build_pack_table(h.io_to_dense, h.ns, idx->pack);
     idx->verify = verify_enabled();
@@ -817,7 +708,7 @@ gdx_status open_index(const ImageHeader &h, DevMem &image, int device, gdx_index
 
 // the host BWT (n bytes) on the device
 gdx_status upload_bwt(const uint8_t *bwt, uint64_t n, DevMem &d_bwt) {
-    CUDA_TRY(d_bwt.alloc(n ? n : 1));
+    CUDA_TRY(d_bwt.alloc(n));
     const cudaError_t e = cudaMemcpy(d_bwt.p, bwt, n, cudaMemcpyHostToDevice);
     return e == cudaSuccess ? GDX_OK : fail(GDX_ERR_CUDA, "BWT upload failed: %s", cudaGetErrorString(e));
 }
@@ -1002,7 +893,7 @@ extern "C" gdx_status gdx_index_build(const uint8_t *texts, const uint64_t *text
         {
             DevMem d_text;
             if (keep_text || construction == GDX_CONSTRUCT_DEVICE) {
-                CUDA_TRY(d_text.alloc(n ? n : 1));
+                CUDA_TRY(d_text.alloc(n));
                 CUDA_TRY(cudaMemcpy(d_text.p, ct.text.data(), n, cudaMemcpyHostToDevice));
                 if (keep_text) src.d_text = d_text.as<uint8_t>();
             }
@@ -1018,9 +909,9 @@ extern "C" gdx_status gdx_index_build(const uint8_t *texts, const uint64_t *text
                 src.border_rows = r.border_rows.data();
                 src.border_pos = r.border_pos.data();
                 src.n_border = r.border_rows.size();
-                src.d_bwt = r.d_bwt;
-                src.samples.d = r.d_samples;
-                src.isa.d = r.d_isa_samples;
+                src.d_bwt = r.d_bwt.as<uint8_t>();
+                src.samples.d = r.d_samples.p;
+                src.isa.d = r.d_isa_samples.p;
                 GDX_TRY(build_image(src, h, image));
             } else {
                 HostParts hp;
@@ -1130,7 +1021,7 @@ extern "C" gdx_status gdx_index_create_from_parts(const gdx_parts *parts, int32_
             {
                 DevMem d_blocks;
                 CUDA_TRY(d_blocks.alloc(nwords * 8));
-                cudaError_t e = d_bwt.alloc(src.n ? src.n : 1);
+                cudaError_t e = d_bwt.alloc(src.n);
                 if (e == cudaSuccess)
                     e = cudaMemcpy(d_blocks.p, parts->interleaved_blocks, nwords * 8, cudaMemcpyHostToDevice);
                 if (e == cudaSuccess && src.n) {
@@ -1191,9 +1082,9 @@ extern "C" gdx_status gdx_suffix_array(const uint8_t *dense_text, uint64_t n, ui
         gdx_status st = device_build_from_text(dense_text, nullptr, n, sigma, 1, r, t_error, true, true);
         if (st != GDX_OK) return st;
         std::vector<uint32_t> sa32(n);
-        cudaError_t e = cudaMemcpy(sa32.data(), r.d_sa, n * 4, cudaMemcpyDeviceToHost);
+        cudaError_t e = cudaMemcpy(sa32.data(), r.d_sa.p, n * 4, cudaMemcpyDeviceToHost);
         const uint64_t viol = r.verify_violations;
-        r.release();
+        r = DeviceBuildResult();
         if (e != cudaSuccess) return fail(GDX_ERR_CUDA, "suffix array download failed: %s", cudaGetErrorString(e));
         for (uint64_t i = 0; i < n; ++i) sa_out[i] = sa32[i];
         if (viol) return fail(GDX_ERR_CUDA, "device suffix array failed verification (%llu violations)", (unsigned long long)viol);
@@ -1206,20 +1097,18 @@ extern "C" gdx_status gdx_index_download_bwt(const gdx_index *idx, uint8_t *bwt_
         if (!idx || !bwt_out) return fail(GDX_ERR_BAD_ARG, "NULL argument");
         DeviceGuard guard(idx->device);
         const uint64_t n = idx->h.n, chunk = 256ull << 20;
-        uint8_t *d = nullptr;
-        CUDA_TRY(cudaMalloc(&d, std::min<uint64_t>(n ? n : 1, chunk)));
-        gdx_status st = GDX_OK;
-        for (uint64_t b = 0; b < n && st == GDX_OK; b += chunk) {
+        DevMem d;
+        CUDA_TRY(d.alloc(std::min<uint64_t>(n, chunk)));
+        for (uint64_t b = 0; b < n; b += chunk) {
             const uint64_t e = std::min<uint64_t>(n, b + chunk);
-            st = dispatch_layout(idx->h.layout, [&](auto L) -> gdx_status {
-                k_records_to_bwt<decltype(L)><<<(unsigned)div_up(e - b, 256), 256>>>(idx->dev, b, e, d);
+            GDX_TRY(dispatch_layout(idx->h.layout, [&](auto L) -> gdx_status {
+                k_records_to_bwt<decltype(L)><<<(unsigned)div_up(e - b, 256), 256>>>(idx->dev, b, e, d.as<uint8_t>());
                 return GDX_OK;
-            });
-            cudaError_t ce = cudaMemcpy(bwt_out + b, d, e - b, cudaMemcpyDeviceToHost);
-            if (st == GDX_OK && ce != cudaSuccess) st = fail(GDX_ERR_CUDA, "BWT download failed: %s", cudaGetErrorString(ce));
+            }));
+            const cudaError_t ce = cudaMemcpy(bwt_out + b, d.p, e - b, cudaMemcpyDeviceToHost);
+            if (ce != cudaSuccess) return fail(GDX_ERR_CUDA, "BWT download failed: %s", cudaGetErrorString(ce));
         }
-        cudaFree(d);
-        return st;
+        return GDX_OK;
     });
 }
 
@@ -1261,14 +1150,7 @@ extern "C" gdx_status gdx_index_get_count(const gdx_index *idx, uint64_t *count_
 extern "C" void gdx_index_destroy(gdx_index *idx) {
     if (!idx) return;
     DeviceGuard guard(idx->device);
-    for (Workspace *w : idx->free_ws) {
-        w->destroy();
-        delete w;
-    }
-    for (auto &p : idx->pinned)
-        if (p.p) cudaFreeHost(p.p);
-    if (idx->own_image && idx->image) cudaFree(idx->image);
-    delete idx;  // and its accelerators
+    delete idx;
 }
 
 extern "C" gdx_status gdx_index_get_info(const gdx_index *idx, gdx_index_info *out) {
@@ -1333,17 +1215,15 @@ extern "C" gdx_status gdx_index_save_to_file(const gdx_index *idx, const char *p
             (user_bytes && fwrite(user_data, user_bytes, 1, fc.f) != 1))
             return fail(GDX_ERR_BAD_ARG, "write to %s failed", path);
         const uint64_t chunk = 64ull << 20;
-        void *stage = nullptr;
-        CUDA_TRY(cudaMallocHost(&stage, chunk));
-        gdx_status st = GDX_OK;
-        for (uint64_t off = 0; off < p.image_bytes && st == GDX_OK; off += chunk) {
+        HBuf stage;
+        CUDA_TRY(stage.alloc(chunk));
+        for (uint64_t off = 0; off < p.image_bytes; off += chunk) {
             const uint64_t nb = std::min<uint64_t>(chunk, p.image_bytes - off);
-            cudaError_t e = cudaMemcpy(stage, (const uint8_t *)idx->image + off, nb, cudaMemcpyDeviceToHost);
-            if (e != cudaSuccess) st = fail(GDX_ERR_CUDA, "image download failed: %s", cudaGetErrorString(e));
-            else if (fwrite(stage, nb, 1, fc.f) != 1) st = fail(GDX_ERR_BAD_ARG, "write to %s failed", path);
+            const cudaError_t e = cudaMemcpy(stage.p, (const uint8_t *)idx->image + off, nb, cudaMemcpyDeviceToHost);
+            if (e != cudaSuccess) return fail(GDX_ERR_CUDA, "image download failed: %s", cudaGetErrorString(e));
+            if (fwrite(stage.p, nb, 1, fc.f) != 1) return fail(GDX_ERR_BAD_ARG, "write to %s failed", path);
         }
-        cudaFreeHost(stage);
-        return st;
+        return GDX_OK;
     });
 }
 
@@ -1377,21 +1257,19 @@ extern "C" gdx_status gdx_index_load_from_file(const char *path, int32_t device_
         int device;
         GDX_TRY(resolve_device(device_req, &device));
         DeviceGuard guard(device);
-        void *image = nullptr, *stage = nullptr;
-        CUDA_TRY(cudaMalloc(&image, p.image_bytes ? p.image_bytes : 1));
+        DevMem image;
+        CUDA_TRY(image.alloc(p.image_bytes));
         const uint64_t chunk = 64ull << 20;
-        cudaError_t e = cudaMallocHost(&stage, chunk);
-        gdx_status st = e == cudaSuccess ? GDX_OK : fail(GDX_ERR_OOM, "pinned staging allocation failed");
-        for (uint64_t off = 0; off < p.image_bytes && st == GDX_OK; off += chunk) {
+        HBuf stage;
+        if (stage.alloc(chunk) != cudaSuccess) return fail(GDX_ERR_OOM, "pinned staging allocation failed");
+        for (uint64_t off = 0; off < p.image_bytes; off += chunk) {
             const uint64_t nb = std::min<uint64_t>(chunk, p.image_bytes - off);
-            if (fread(stage, nb, 1, fc.f) != 1) st = fail(GDX_ERR_BAD_ARG, "%s is truncated", path);
-            else if ((e = cudaMemcpy((uint8_t *)image + off, stage, nb, cudaMemcpyHostToDevice)) != cudaSuccess)
-                st = fail(GDX_ERR_CUDA, "image upload failed: %s", cudaGetErrorString(e));
+            if (fread(stage.p, nb, 1, fc.f) != 1) return fail(GDX_ERR_BAD_ARG, "%s is truncated", path);
+            const cudaError_t e = cudaMemcpy(image.as<uint8_t>() + off, stage.p, nb, cudaMemcpyHostToDevice);
+            if (e != cudaSuccess) return fail(GDX_ERR_CUDA, "image upload failed: %s", cudaGetErrorString(e));
         }
-        if (stage) cudaFreeHost(stage);
-        if (st == GDX_OK) st = gdx_index_adopt_image(&h, image, device, 1, out);
-        if (st != GDX_OK) cudaFree(image);
-        return st;
+        stage.reset();
+        return open_index(h, image, device, out);
     });
 }
 
@@ -1529,23 +1407,24 @@ extern "C" gdx_status gdx_index_replicate(const gdx_index *idx, const int32_t *d
         for (int i = 0; i < n_devices; ++i) out_replicas[i] = nullptr;
         std::vector<int> dev(n_devices);
         for (int i = 0; i < n_devices; ++i) GDX_TRY(resolve_device(devices[i], &dev[i]));
-        std::vector<void *> img(n_devices, nullptr);
-        auto free_images = [&] {
-            for (int i = 0; i < n_devices; ++i)
-                if (img[i]) {
-                    DeviceGuard g(dev[i]);
-                    cudaFree(img[i]);
-                    img[i] = nullptr;
-                }
-        };
+        // the images not yet opened as replicas, each freed with its device current
+        struct Images {
+            const std::vector<int> &dev;
+            std::vector<DevMem> img;
+            ~Images() {
+                for (size_t i = 0; i < img.size(); ++i)
+                    if (img[i]) {
+                        DeviceGuard g(dev[i]);
+                        img[i].reset();
+                    }
+            }
+        } images{dev, std::vector<DevMem>(n_devices)};
+        std::vector<DevMem> &img = images.img;
         const uint64_t bytes = idx->h.image_bytes;
         for (int i = 0; i < n_devices; ++i) {
             DeviceGuard g(dev[i]);
-            cudaError_t e = cudaMalloc(&img[i], bytes ? bytes : 1);
-            if (e != cudaSuccess) {
-                free_images();
-                return fail(GDX_ERR_OOM, "replica on device %d: %s", dev[i], cudaGetErrorString(e));
-            }
+            const cudaError_t e = img[i].alloc(bytes);
+            if (e != cudaSuccess) return fail(GDX_ERR_OOM, "replica on device %d: %s", dev[i], cudaGetErrorString(e));
         }
         // communicator over the source device + every distinct other target; targets on the source device (and
         // repeated targets) are filled by device-to-device copies afterwards
@@ -1562,12 +1441,12 @@ extern "C" gdx_status gdx_index_replicate(const gdx_index *idx, const int32_t *d
             const Nccl &N = nccl();
             const int world = (int)comm_dev.size();
             std::vector<Nccl::comm_t> comms(world, nullptr);
-            std::vector<cudaStream_t> streams(world, nullptr);
+            std::vector<Stream> streams(world);
             gdx_status st = [&]() -> gdx_status {
                 NCCL_TRY(N.CommInitAll(comms.data(), world, comm_dev.data()));
                 for (int r = 0; r < world; ++r) {
                     DeviceGuard g(comm_dev[r]);
-                    CUDA_TRY(cudaStreamCreateWithFlags(&streams[r], cudaStreamNonBlocking));
+                    CUDA_TRY(streams[r].create(cudaStreamNonBlocking));
                 }
                 for (uint64_t off = 0; off < bytes; off += kBroadcastPiece) {
                     const uint64_t nb = std::min(kBroadcastPiece, bytes - off);
@@ -1575,7 +1454,7 @@ extern "C" gdx_status gdx_index_replicate(const gdx_index *idx, const int32_t *d
                     for (int r = 0; r < world; ++r) {
                         void *recv = (uint8_t *)idx->image + off;  // root: in place
                         for (int i = 0; i < n_devices && r > 0; ++i)
-                            if (member[i] == r) recv = (uint8_t *)img[i] + off;
+                            if (member[i] == r) recv = img[i].as<uint8_t>() + off;
                         DeviceGuard g(comm_dev[r]);
                         NCCL_TRY(N.Broadcast((const uint8_t *)idx->image + off, recv, nb, Nccl::kUint8, 0, comms[r], streams[r]));
                     }
@@ -1589,13 +1468,10 @@ extern "C" gdx_status gdx_index_replicate(const gdx_index *idx, const int32_t *d
             }();
             for (int r = 0; r < world; ++r) {
                 DeviceGuard g(comm_dev[r]);
-                if (streams[r]) cudaStreamDestroy(streams[r]);
+                streams[r] = Stream();
                 if (comms[r]) N.CommDestroy(comms[r]);
             }
-            if (st != GDX_OK) {
-                free_images();
-                return st;
-            }
+            if (st != GDX_OK) return st;
             t_transport = "nccl";
             done = true;
         }
@@ -1608,29 +1484,24 @@ extern "C" gdx_status gdx_index_replicate(const gdx_index *idx, const int32_t *d
             if (done && member[i] < 0 && dev[i] != idx->device)
                 for (int j = 0; j < i; ++j)
                     if (dev[j] == dev[i] && member[j] >= 0) {
-                        from = img[j];
+                        from = img[j].p;
                         from_dev = dev[j];
                     }
-            cudaError_t e = cudaMemcpyPeer(img[i], dev[i], from, from_dev, bytes);
-            if (e != cudaSuccess) {
-                free_images();
-                return fail(GDX_ERR_CUDA, "copy to device %d failed: %s", dev[i], cudaGetErrorString(e));
-            }
+            const cudaError_t e = cudaMemcpyPeer(img[i].p, dev[i], from, from_dev, bytes);
+            if (e != cudaSuccess) return fail(GDX_ERR_CUDA, "copy to device %d failed: %s", dev[i], cudaGetErrorString(e));
             if (!done && *t_transport == 0) t_transport = "peer";
         }
         if (*t_transport == 0) t_transport = "peer";
         for (int i = 0; i < n_devices; ++i) {
-            gdx_status st = gdx_index_adopt_image(&idx->h, img[i], dev[i], 1, &out_replicas[i]);
+            DeviceGuard g(dev[i]);
+            const gdx_status st = open_index(idx->h, img[i], dev[i], &out_replicas[i]);
             if (st != GDX_OK) {
                 for (int j = 0; j < i; ++j) {
                     gdx_index_destroy(out_replicas[j]);
                     out_replicas[j] = nullptr;
-                    img[j] = nullptr;
                 }
-                free_images();
                 return st;
             }
-            img[i] = nullptr;  // owned by the replica now
         }
         return GDX_OK;
     });
@@ -1661,41 +1532,35 @@ extern "C" gdx_status gdx_index_broadcast(const gdx_index *src, const void *uniq
         memcpy(&id, unique_id, sizeof id);
         Nccl::comm_t comm = nullptr;
         NCCL_TRY(N.CommInitRank(&comm, world, id, rank));
-        cudaStream_t stream = nullptr;
-        void *d_hdr = nullptr, *image = nullptr;
+        DevMem image;  // of a receiving rank
         ImageHeader h;
-        gdx_status st = [&]() -> gdx_status {
-            CUDA_TRY(cudaStreamCreateWithFlags(&stream, cudaStreamNonBlocking));
-            CUDA_TRY(cudaMalloc(&d_hdr, sizeof(ImageHeader)));
-            if (rank == root) CUDA_TRY(cudaMemcpyAsync(d_hdr, &src->h, sizeof(ImageHeader), cudaMemcpyHostToDevice, stream));
-            NCCL_TRY(N.Broadcast(d_hdr, d_hdr, sizeof(ImageHeader), Nccl::kUint8, root, comm, stream));
-            CUDA_TRY(cudaMemcpyAsync(&h, d_hdr, sizeof(ImageHeader), cudaMemcpyDeviceToHost, stream));
+        const gdx_status st = [&]() -> gdx_status {
+            Stream stream;
+            DevMem d_hdr;
+            CUDA_TRY(stream.create(cudaStreamNonBlocking));
+            CUDA_TRY(d_hdr.alloc(sizeof(ImageHeader)));
+            if (rank == root) CUDA_TRY(cudaMemcpyAsync(d_hdr.p, &src->h, sizeof(ImageHeader), cudaMemcpyHostToDevice, stream));
+            NCCL_TRY(N.Broadcast(d_hdr.p, d_hdr.p, sizeof(ImageHeader), Nccl::kUint8, root, comm, stream));
+            CUDA_TRY(cudaMemcpyAsync(&h, d_hdr.p, sizeof(ImageHeader), cudaMemcpyDeviceToHost, stream));
             CUDA_TRY(cudaStreamSynchronize(stream));
             GDX_TRY(validate_header(h));
-            if (rank == root) image = src->image;
-            else CUDA_TRY(cudaMalloc(&image, h.image_bytes ? h.image_bytes : 1));
+            if (rank != root) CUDA_TRY(image.alloc(h.image_bytes));
+            uint8_t *img = rank == root ? (uint8_t *)src->image : image.as<uint8_t>();
             for (uint64_t off = 0; off < h.image_bytes; off += kBroadcastPiece) {
                 const uint64_t nb = std::min(kBroadcastPiece, h.image_bytes - off);
-                NCCL_TRY(N.Broadcast((uint8_t *)image + off, (uint8_t *)image + off, nb, Nccl::kUint8, root, comm, stream));
+                NCCL_TRY(N.Broadcast(img + off, img + off, nb, Nccl::kUint8, root, comm, stream));
             }
             CUDA_TRY(cudaStreamSynchronize(stream));
             return GDX_OK;
         }();
-        if (d_hdr) cudaFree(d_hdr);
-        if (stream) cudaStreamDestroy(stream);
         N.CommDestroy(comm);
-        if (st != GDX_OK) {
-            if (rank != root && image) cudaFree(image);
-            return st;
-        }
+        if (st != GDX_OK) return st;
         t_transport = "nccl";
         if (rank == root) {
             *out = const_cast<gdx_index *>(src);
             return GDX_OK;
         }
-        st = gdx_index_adopt_image(&h, image, device, 1, out);
-        if (st != GDX_OK) cudaFree(image);
-        return st;
+        return open_index(h, image, device, out);
     });
 }
 
@@ -1835,11 +1700,19 @@ gdx_status acquire_pinned_hits(const gdx_index *idx, uint64_t bytes, void **out,
 void release_pinned_hits(const gdx_index *idx, void *p);
 
 // a library-owned pinned buffer the results of a call are appended to.  It grows to twice the size asked for (at least
-// 4096 bytes) and keeps what it holds; no copy into it may be in flight then.
+// 4096 bytes) and keeps what it holds; no copy into it may be in flight then.  Unless it is handed over to the caller,
+// it goes back to the pool when it dies, which must be after with_workspace drained the streams of a failed call: copies
+// into it may still be in flight until then.
 struct PinnedResult {
     const gdx_index *idx;
     void *p = nullptr;
     uint64_t cap = 0, used = 0;  // bytes
+    explicit PinnedResult(const gdx_index *i) : idx(i) {}
+    PinnedResult(const PinnedResult &) = delete;
+    PinnedResult &operator=(const PinnedResult &) = delete;
+    ~PinnedResult() {
+        if (p) release_pinned_hits(idx, p);
+    }
     gdx_status reserve(uint64_t bytes) {
         if (bytes <= cap) return GDX_OK;
         void *bigger = nullptr;
@@ -1853,14 +1726,11 @@ struct PinnedResult {
         cap = c;
         return GDX_OK;
     }
-    void release() {
-        if (p) release_pinned_hits(idx, p);
-        p = nullptr;
-    }
+    void *hand_over() { return std::exchange(p, nullptr); }
 };
 
 // the two-call CUB exclusive scan (size query, then the scan) with its temporary storage in tmp
-gdx_status exclusive_sum(DBuf &tmp, uint64_t *in, uint64_t *out, uint64_t n, cudaStream_t st) {
+gdx_status exclusive_sum(DevMem &tmp, uint64_t *in, uint64_t *out, uint64_t n, cudaStream_t st) {
     size_t bytes = 0;
     CUDA_TRY(cub::DeviceScan::ExclusiveSum(nullptr, bytes, in, out, n, st));
     CUDA_TRY(tmp.reserve(bytes));
@@ -1885,12 +1755,12 @@ void launch_locate_walk(const gdx_index *idx, const uint64_t *rows, uint64_t n_h
 gdx_status IntervalHits::count(cudaStream_t st, const uint64_t *starts, const uint64_t *ends, uint64_t n) {
     CUDA_TRY(counts.reserve((n + 1) * 8));
     CUDA_TRY(offsets.reserve((n + 1) * 8));
-    CUDA_TRY(cudaMemsetAsync(d, 0, sizeof *d, st));
+    CUDA_TRY(cudaMemsetAsync(d(), 0, sizeof(DeviceWords), st));
     CUDA_TRY(cudaMemsetAsync(counts.as<uint64_t>() + n, 0, 8, st));
-    if (n) k_interval_counts<<<(unsigned)div_up(n, 256), 256, 0, st>>>(starts, ends, n, counts.as<uint64_t>(), &d->wide);
+    if (n) k_interval_counts<<<(unsigned)div_up(n, 256), 256, 0, st>>>(starts, ends, n, counts.as<uint64_t>(), &d()->wide);
     GDX_TRY(exclusive_sum(scan_tmp, counts.as<uint64_t>(), offsets.as<uint64_t>(), n + 1, st));
-    CUDA_TRY(cudaMemcpyAsync(&h->hits, offsets.as<uint64_t>() + n, 8, cudaMemcpyDeviceToHost, st));
-    CUDA_TRY(cudaMemcpyAsync(&h->wide, &d->wide, 8, cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(cudaMemcpyAsync(&h()->hits, offsets.as<uint64_t>() + n, 8, cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(cudaMemcpyAsync(&h()->wide, &d()->wide, 8, cudaMemcpyDeviceToHost, st));
     CUDA_TRY(cudaEventRecord(ev_total, st));
     t_stats.kernel_launches += 2;
     return GDX_OK;
@@ -1900,10 +1770,10 @@ gdx_status IntervalHits::count(cudaStream_t st, const uint64_t *starts, const ui
 gdx_status IntervalHits::expand_walk(const gdx_index *idx, cudaStream_t st, const uint64_t *starts, const uint64_t *ends,
                                      uint64_t n, uint64_t n_hits, uint64_t n_wide, unsigned long long *walk_steps,
                                      bool hit32) {
-    if (n_hits * 24 > rows.cap + hits.cap) {  // 8 B of rows + 16 B of hits per hit
+    if (n_hits * 24 > rows.bytes + hits.bytes) {  // 8 B of rows + 16 B of hits per hit
         size_t free_b = 0, total_b = 0;
         CUDA_TRY(cudaMemGetInfo(&free_b, &total_b));
-        if (n_hits * 24 > free_b + rows.cap + hits.cap)
+        if (n_hits * 24 > free_b + rows.bytes + hits.bytes)
             return fail(GDX_ERR_OOM, "%llu hits of one chunk do not fit into device memory; split the batch",
                         (unsigned long long)n_hits);
     }
@@ -1911,7 +1781,7 @@ gdx_status IntervalHits::expand_walk(const gdx_index *idx, cudaStream_t st, cons
     CUDA_TRY(hits.reserve(n_hits * 16));
     CUDA_TRY(wide.reserve((n_wide + 1) * 8));
     k_expand_rows<<<(unsigned)div_up(n, 256), 256, 0, st>>>(starts, ends, offsets.as<uint64_t>(), n, rows.as<uint64_t>(),
-                                                           wide.as<uint64_t>(), &d->cursor);
+                                                           wide.as<uint64_t>(), &d()->cursor);
     if (n_wide) {
         dim3 grid((unsigned)n_wide, 32);
         k_expand_big_rows<<<grid, 256, 0, st>>>(starts, ends, offsets.as<uint64_t>(), wide.as<uint64_t>(),
@@ -1946,8 +1816,8 @@ struct Uploads {
 };
 
 // grow device buffers of one stream; growing one frees the old buffer, which is only safe once the stream has drained
-gdx_status reserve_drained(cudaStream_t st, std::initializer_list<std::pair<DBuf *, uint64_t>> bufs) {
-    if (std::any_of(bufs.begin(), bufs.end(), [](const std::pair<DBuf *, uint64_t> &b) { return b.first->cap < b.second; }))
+gdx_status reserve_drained(cudaStream_t st, std::initializer_list<std::pair<DevMem *, uint64_t>> bufs) {
+    if (std::any_of(bufs.begin(), bufs.end(), [](const std::pair<DevMem *, uint64_t> &b) { return b.first->bytes < b.second; }))
         CUDA_TRY(cudaStreamSynchronize(st));
     for (const auto &b : bufs) CUDA_TRY(b.first->reserve(b.second));
     return GDX_OK;
@@ -2031,7 +1901,7 @@ struct LocatePipe {
         IntervalHits &ih = sl.locate;
         const uint64_t cq = p.cq, q0 = p.q0;
         CUDA_TRY(cudaEventSynchronize(ih.ev_total));
-        const uint64_t n_hits = ih.h->hits, base = res.used / hit_bytes;
+        const uint64_t n_hits = ih.h()->hits, base = res.used / hit_bytes;
         if (n_hits) {
             if ((base + n_hits) * hit_bytes > res.cap) {  // grow the pinned result buffer (rare)
                 // the hits of earlier chunks may still be on their way into it, on any slot stream
@@ -2040,8 +1910,8 @@ struct LocatePipe {
             }
             const EventPairs::Pair ev = ih.timing.next();
             CUDA_TRY(cudaEventRecord(ev.begin, sl.stream));
-            GDX_TRY(ih.expand_walk(idx, sl.stream, sl.out_a.as<uint64_t>(), sl.out_b.as<uint64_t>(), cq, n_hits, ih.h->wide,
-                                   &ws->cnt_d->locate_walk_steps, hit_bytes == 8));
+            GDX_TRY(ih.expand_walk(idx, sl.stream, sl.out_a.as<uint64_t>(), sl.out_b.as<uint64_t>(), cq, n_hits, ih.h()->wide,
+                                   &ws->cnt_d()->locate_walk_steps, hit_bytes == 8));
             CUDA_TRY(cudaEventRecord(ev.end, sl.stream));
             CUDA_TRY(cudaMemcpyAsync((uint8_t *)res.p + res.used, ih.hits.p, n_hits * hit_bytes, cudaMemcpyDeviceToHost,
                                      sl.stream));
@@ -2150,7 +2020,6 @@ struct Trace {
             fprintf(stderr, "[gdx trace] chunk %2d slot %d nq %8llu h2d bytes %10llu host stage %.3f ms | h2d %.3f..%.3f | kernels %.3f..%.3f | d2h ..%.3f\n",
                     r.k, r.k % kSlots, (unsigned long long)r.nq, (unsigned long long)r.bytes, r.host_stage_ms, a, b, b, c, d);
         }
-        ev.destroy();
     }
 };
 
@@ -2277,7 +2146,7 @@ gdx_status stage_chunk(const gdx_index *idx, const gdx_queries *qs, const gdx::C
 gdx_status search_result(Workspace *ws, const gdx_stats &io) {
     CUDA_TRY(ws->read_counters(ws->slot[0].stream));
     CUDA_TRY(cudaStreamSynchronize(ws->slot[0].stream));
-    const Counters &cnt = *ws->cnt_h;
+    const Counters &cnt = *ws->cnt_h();
     t_stats.queries = io.queries;
     t_stats.packed_queries = io.packed_queries;
     t_stats.exception_queries = io.exception_queries;
@@ -2324,7 +2193,7 @@ gdx_status search_host(const gdx_index *idx, Workspace *ws, const gdx_queries *q
     LinkQueue link;
     for (Slot &sl : ws->slot) sl.h2d_pending = false;
     // Large batches: size every slot once for the largest chunk this call can cut (the adaptive schedule cuts
-    // different chunks in every call; growing a buffer in mid-flight means cudaFree / cudaFreeHost + a new
+    // different chunks in every call; growing a buffer in mid-flight means freeing it and a new
     // allocation, milliseconds each, with the streams drained).  The streams are idle here.
     if (nq && total_in >= kStageMinBytes) {
         const uint64_t max_sym = plan.max_chunk_symbols() + 64;
@@ -2365,12 +2234,12 @@ gdx_status search_host(const gdx_index *idx, Workspace *ws, const gdx_queries *q
             GDX_TRY(sort_queries(idx, u.dq, sp, sl.sort.p, sl.stream, &perm));
             t_stats.kernel_launches += 2;
         }
-        uint64_t *err = &ws->cnt_d->err[k % kSlots];
+        uint64_t *err = &ws->cnt_d()->err[k % kSlots];
         GDX_TRY(dispatch_layout(idx->h.layout, [&](auto L) -> gdx_status {
-            launch_search<decltype(L)>(idx, u.dq, a, b, sink.mode, sink.narrow, c.q0, err, &ws->cnt_d->search, perm,
+            launch_search<decltype(L)>(idx, u.dq, a, b, sink.mode, sink.narrow, c.q0, err, &ws->cnt_d()->search, perm,
                                        nullptr, sl.stream);
             if (u.xq.nq)  // overwrites the slots of the queries the packed kernel could not see correctly
-                launch_search<decltype(L)>(idx, u.xq, a, b, sink.mode, sink.narrow, c.q0, err, &ws->cnt_d->search,
+                launch_search<decltype(L)>(idx, u.xq, a, b, sink.mode, sink.narrow, c.q0, err, &ws->cnt_d()->search,
                                            nullptr, u.x_slots, sl.stream);
             return GDX_OK;
         }));
@@ -2406,10 +2275,10 @@ gdx_status locate_device_intervals(const gdx_index *idx, Workspace *ws, const ui
     CUDA_TRY(cudaEventRecord(ev.begin, st));
     GDX_TRY(ih.count(st, d_starts, d_ends, n));
     CUDA_TRY(cudaEventSynchronize(ih.ev_total));
-    const uint64_t total = ih.h->hits;
+    const uint64_t total = ih.h()->hits;
     *total_out = total;
     if (total)
-        GDX_TRY(ih.expand_walk(idx, st, d_starts, d_ends, n, total, ih.h->wide, &ws->cnt_d->locate_walk_steps, false));
+        GDX_TRY(ih.expand_walk(idx, st, d_starts, d_ends, n, total, ih.h()->wide, &ws->cnt_d()->locate_walk_steps, false));
     CUDA_TRY(cudaEventRecord(ev.end, st));
     return GDX_OK;
 }
@@ -2417,38 +2286,32 @@ gdx_status locate_device_intervals(const gdx_index *idx, Workspace *ws, const ui
 void release_pinned_hits(const gdx_index *idx, void *p) {
     std::lock_guard<std::mutex> lk(idx->mu);
     for (auto &b : idx->pinned)
-        if (b.p == p) b.in_use = false;
+        if (b.buf.p == p) b.in_use = false;
 }
 
 gdx_status acquire_pinned_hits(const gdx_index *idx, uint64_t bytes, void **out, uint64_t *cap_out = nullptr) {
     std::lock_guard<std::mutex> lk(idx->mu);
     PinnedHits *best = nullptr;
     for (auto &p : idx->pinned)
-        if (!p.in_use && p.cap >= bytes && (!best || p.cap < best->cap)) best = &p;
+        if (!p.in_use && p.buf.bytes >= bytes && (!best || p.buf.bytes < best->buf.bytes)) best = &p;
     if (!best) {
         for (auto &p : idx->pinned)  // recycle the largest free but too small buffer
-            if (!p.in_use && (!best || p.cap > best->cap)) best = &p;
-        if (best) {
-            cudaFreeHost(best->p);
-            best->p = nullptr;
-            best->cap = 0;
-        } else {
-            idx->pinned.push_back(PinnedHits{});
+            if (!p.in_use && (!best || p.buf.bytes > best->buf.bytes)) best = &p;
+        if (!best) {
+            idx->pinned.emplace_back();
             best = &idx->pinned.back();
         }
         const uint64_t want = align_up(bytes + bytes / 4 + 4096, 4096);
-        cudaError_t e = cudaMallocHost(&best->p, want);
+        const cudaError_t e = best->buf.alloc(want);
         if (e != cudaSuccess) {
-            best->p = nullptr;
             cudaGetLastError();
             return fail(GDX_ERR_OOM, "pinned host allocation of %llu bytes failed: %s", (unsigned long long)want,
                         cudaGetErrorString(e));
         }
-        best->cap = want;
     }
     best->in_use = true;
-    *out = best->p;
-    if (cap_out) *cap_out = best->cap;
+    *out = best->buf.p;
+    if (cap_out) *cap_out = best->buf.bytes;
     return GDX_OK;
 }
 
@@ -2471,8 +2334,8 @@ gdx_status finish_locate(const gdx_index *idx, Workspace *ws, uint64_t n, uint64
     }
     t_stats.kernel_ms_locate = ws->locate.timing.elapsed_ms();
     t_stats.hits = total;
-    t_stats.walk_steps += ws->cnt_h->locate_walk_steps;
-    t_stats.locate_walk_steps = ws->cnt_h->locate_walk_steps;
+    t_stats.walk_steps += ws->cnt_h()->locate_walk_steps;
+    t_stats.locate_walk_steps = ws->cnt_h()->locate_walk_steps;
     *hits = (gdx_hit *)h;
     *num_hits = total;
     return GDX_OK;
@@ -2519,14 +2382,11 @@ gdx_status locate_many_impl(const gdx_index *idx, const gdx_queries *queries, ui
         GDX_TRY(acquire_pinned_hits(idx, std::max<uint64_t>(n, 4096) * hit_bytes, &res.p, &res.cap));
         return search_host(idx, ws, queries, lp);
     });
-    if (st != GDX_OK) {
-        res.release();  // after with_workspace drained the streams: hit copies into it may have been in flight
-        return st;
-    }
+    if (st != GDX_OK) return st;
     const uint64_t total = res.used / hit_bytes;
     if (write_last && hit_offsets) hit_offsets[n] = total;
     t_stats.hits = total;
-    *hits = (gdx_hit *)res.p;
+    *hits = (gdx_hit *)res.hand_over();
     *num_hits = total;
     return GDX_OK;
 }
@@ -2841,10 +2701,7 @@ extern "C" gdx_status gdx_locate_intervals(const gdx_index *idx, const uint64_t 
 }
 
 extern "C" void gdx_free_hits(const gdx_index *idx, gdx_hit *hits) {
-    if (!idx || !hits) return;
-    std::lock_guard<std::mutex> lk(idx->mu);
-    for (auto &p : idx->pinned)
-        if (p.p == hits) p.in_use = false;
+    if (idx && hits) release_pinned_hits(idx, hits);
 }
 
 static gdx_status extend_many_on(const gdx_index *idx, Workspace *ws, uint64_t *starts, uint64_t *ends,
@@ -2897,7 +2754,7 @@ static gdx_status extend_many_on(const gdx_index *idx, Workspace *ws, uint64_t *
             CUDA_TRY(cudaMemcpyAsync(d_c + off, io_symbols + off, cn, cudaMemcpyHostToDevice, cs));
             GDX_TRY(dispatch_layout(idx->h.layout, [&](auto L) -> gdx_status {
                 k_extend<decltype(L)><<<(unsigned)div_up(cn, 256), 256, 0, cs>>>(idx->dev, d_s + off, d_e + off, d_c + off, cn,
-                                                                               &ws->cnt_d->extend_bad_symbol, off);
+                                                                               &ws->cnt_d()->extend_bad_symbol, off);
                 return GDX_OK;
             }));
             CUDA_TRY(cudaGetLastError());
@@ -2910,7 +2767,7 @@ static gdx_status extend_many_on(const gdx_index *idx, Workspace *ws, uint64_t *
         CUDA_TRY(ws->read_counters(st));
         CUDA_TRY(cudaStreamSynchronize(st));
         t_stats.kernel_launches = launches;
-        const Counters &c = *ws->cnt_h;
+        const Counters &c = *ws->cnt_h();
         if (c.extend_bad_cursor != kNoError)  // checked on the device: text_with_rank_support/mod.rs:106-110
             return fail(GDX_ERR_BAD_ARG, "cursor %llu is outside [0, text_len]", (unsigned long long)c.extend_bad_cursor);
         if (c.extend_bad_symbol != kNoError) {
@@ -3005,7 +2862,7 @@ gdx_status hamming_run(const gdx_index *idx, Workspace *ws, const gdx_queries *q
     cudaStream_t st = sl.stream;
     const uint64_t strata = k + 1;
     const uint64_t elem = mode == kHammingCursors ? sizeof(gdx_hamming_interval) : sizeof(gdx_hit);
-    uint64_t *d_err = &ws->cnt_d->err[0];
+    uint64_t *d_err = &ws->cnt_d()->err[0];
     CUDA_TRY(ws->reset_counters(st));
     const bool src_pinned = n_ok && is_pinned(qs->bytes);
     Uploads up{st};
@@ -3041,7 +2898,7 @@ gdx_status hamming_run(const gdx_index *idx, Workspace *ws, const gdx_queries *q
         GDX_TRY(dispatch_layout(idx->h.layout, [&](auto L) -> gdx_status {
             k_hamming<decltype(L), 1><<<grid, 256, 0, st>>>(idx->dev, dq, k, q0, d_err, sl.out_a.as<uint64_t>(),
                                                              intervals ? csr.counts.as<uint64_t>() : nullptr, nullptr,
-                                                             nullptr, nullptr, &ws->cnt_d->hamming_expansions);
+                                                             nullptr, nullptr, &ws->cnt_d()->hamming_expansions);
             return GDX_OK;
         }));
         CUDA_TRY(cudaGetLastError());
@@ -3055,23 +2912,23 @@ gdx_status hamming_run(const gdx_index *idx, Workspace *ws, const gdx_queries *q
             }
             CUDA_TRY(ws->read_counters(st));
             CUDA_TRY(cudaStreamSynchronize(st));
-            GDX_TRY(kernel_error(ws->cnt_h->err[0], kHammingBadSymbol));
+            GDX_TRY(kernel_error(ws->cnt_h()->err[0], kHammingBadSymbol));
             if (counts) HostPool::get().copy(counts + q0 * strata, sl.h_out_a.p, cq * strata * 8);
             continue;
         }
         // CSR of the chunk's intervals
         GDX_TRY(exclusive_sum(csr.scan_tmp, csr.counts.as<uint64_t>(), csr.offsets.as<uint64_t>(), cq + 1, st));
         CUDA_TRY(ws->read_counters(st));
-        CUDA_TRY(cudaMemcpyAsync(&csr.h->hits, csr.offsets.as<uint64_t>() + cq, 8, cudaMemcpyDeviceToHost, st));
+        CUDA_TRY(cudaMemcpyAsync(&csr.h()->hits, csr.offsets.as<uint64_t>() + cq, 8, cudaMemcpyDeviceToHost, st));
         CUDA_TRY(cudaStreamSynchronize(st));
         ++launches;
-        GDX_TRY(kernel_error(ws->cnt_h->err[0], kHammingBadSymbol));
-        const uint64_t niv = csr.h->hits;
+        GDX_TRY(kernel_error(ws->cnt_h()->err[0], kHammingBadSymbol));
+        const uint64_t niv = csr.h()->hits;
         // pass 2: the intervals at their CSR offsets in search order, a sort by start within every query, then records
         // (cursors) or starts / ends (the locate path)
         const uint64_t rec_bytes = mode == kHammingCursors ? sizeof(HammingInterval) : 8;
-        const uint64_t held = csr.rows.cap + csr.wide.cap + ws->starts.cap + sl.xbuf.cap +
-                              (mode == kHammingCursors ? csr.hits.cap : ws->ends.cap);
+        const uint64_t held = csr.rows.bytes + csr.wide.bytes + ws->starts.bytes + sl.xbuf.bytes +
+                              (mode == kHammingCursors ? csr.hits.bytes : ws->ends.bytes);
         const uint64_t need = niv * (32 + rec_bytes);
         bool fits = niv <= 0x7fffffffull;  // (the segmented sort counts items in an int)
         if (fits && need > held) {
@@ -3145,7 +3002,7 @@ gdx_status hamming_run(const gdx_index *idx, Workspace *ws, const gdx_queries *q
     CUDA_TRY(ws->read_counters(st));
     CUDA_TRY(cudaStreamSynchronize(st));
     t_stats.queries = qs->nq;
-    t_stats.lf_steps = ws->cnt_h->hamming_expansions;
+    t_stats.lf_steps = ws->cnt_h()->hamming_expansions;
     t_stats.kernel_ms_search = sl.timing.elapsed_ms();
     t_stats.kernel_ms_locate = ws->locate.timing.elapsed_ms();
     t_stats.kernel_launches += launches;
@@ -3183,14 +3040,11 @@ gdx_status hamming_many_impl(const gdx_index *idx, const gdx_queries *queries, u
         return fail(GDX_ERR_UNSUPPORTED, "query %llu is longer than GDX_HAMMING_MAX_QUERY_LEN (%d symbols)",
                     (unsigned long long)n_ok, GDX_HAMMING_MAX_QUERY_LEN);
     });
-    if (st != GDX_OK) {
-        res.release();  // after with_workspace drained the stream: a copy into it may have been in flight
-        return st;
-    }
+    if (st != GDX_OK) return st;
     if (mode != kHammingCount) {
         const uint64_t elem = mode == kHammingCursors ? sizeof(gdx_hamming_interval) : sizeof(gdx_hit);
         offsets_out[queries->nq] = res.used / elem;
-        *result = res.p;
+        *result = res.hand_over();
         *num_out = res.used / elem;
     }
     return GDX_OK;
@@ -3248,17 +3102,17 @@ static gdx_status search_device(const gdx_index *idx, const gdx_queries *dq_in, 
     cudaStream_t st = (cudaStream_t)stream;
     const SortPlan sp = plan_sort(idx, dq.nq, dq.offsets ? 0 : dq.fixed_len);
     const uint32_t *perm = nullptr;
-    void *scratch = nullptr;
+    AsyncMem scratch;
     if (sp.use) {  // stream-ordered scratch from the device's memory pool
-        CUDA_TRY(cudaMallocAsync(&scratch, sp.total_bytes, st));
-        GDX_TRY(sort_queries(idx, dq, sp, scratch, st, &perm));
+        CUDA_TRY(scratch.alloc(sp.total_bytes, st));
+        GDX_TRY(sort_queries(idx, dq, sp, scratch.p, st, &perm));
     }
     GDX_TRY(dispatch_layout(idx->h.layout, [&](auto L) -> gdx_status {
         launch_search<decltype(L)>(idx, dq, a, b, mode, false, 0, d_error, nullptr, perm, nullptr, st);
         return GDX_OK;
     }));
     CUDA_TRY(cudaGetLastError());
-    if (scratch) CUDA_TRY(cudaFreeAsync(scratch, st));
+    CUDA_TRY(scratch.free());
     return GDX_OK;
 }
 
@@ -3280,9 +3134,10 @@ extern "C" gdx_status gdx_locate_intervals_device(const gdx_index *idx, const ui
     DeviceGuard guard(idx->device);
     cudaStream_t st = (cudaStream_t)stream;
     // stream-ordered scratch: rows (8 B per hit), worklist of wide intervals, two counters
-    uint64_t *rows = nullptr, *big = nullptr;
-    CUDA_TRY(cudaMallocAsync((void **)&rows, num_hits * 8, st));
-    CUDA_TRY(cudaMallocAsync((void **)&big, (n + 2) * 8, st));
+    AsyncMem rows_mem, big_mem;
+    CUDA_TRY(rows_mem.alloc(num_hits * 8, st));
+    CUDA_TRY(big_mem.alloc((n + 2) * 8, st));
+    uint64_t *rows = rows_mem.as<uint64_t>(), *big = big_mem.as<uint64_t>();
     CUDA_TRY(cudaMemsetAsync(big, 0, 16, st));
     k_expand_rows<<<(unsigned)div_up(n, 256), 256, 0, st>>>(d_starts, d_ends, d_hit_offsets, n, rows, big + 2,
                                                            reinterpret_cast<unsigned long long *>(big));
@@ -3299,8 +3154,8 @@ extern "C" gdx_status gdx_locate_intervals_device(const gdx_index *idx, const ui
         return GDX_OK;
     }));
     CUDA_TRY(cudaGetLastError());
-    CUDA_TRY(cudaFreeAsync(rows, st));
-    CUDA_TRY(cudaFreeAsync(big, st));
+    CUDA_TRY(rows_mem.free());
+    CUDA_TRY(big_mem.free());
     return GDX_OK;
 }
 
@@ -3323,11 +3178,15 @@ extern "C" gdx_status gdx_measure_random_gather(int32_t device_req, uint64_t tab
     DeviceGuard guard(device);
     uint64_t nrec = 1;
     while (nrec * 2 * record_bytes <= table_bytes) nrec *= 2;
-    uint8_t *table = nullptr;
-    uint64_t *sink = nullptr;
-    CUDA_TRY(cudaMalloc(&table, nrec * record_bytes));
-    cudaError_t e = cudaMalloc(&sink, 8);
-    cudaEvent_t e0 = nullptr, e1 = nullptr;
+    DevMem table_mem, sink_mem;
+    CUDA_TRY(table_mem.alloc(nrec * record_bytes));
+    auto check = [](cudaError_t e) {
+        return e == cudaSuccess ? GDX_OK : fail(GDX_ERR_CUDA, "gather microbenchmark failed: %s", cudaGetErrorString(e));
+    };
+    GDX_TRY(check(sink_mem.alloc(8)));
+    const uint8_t *table = table_mem.as<uint8_t>();
+    uint64_t *sink = sink_mem.as<uint64_t>();
+    Event e0, e1;
     float ms = 0;
     const unsigned blocks = 148 * 8, threads = 256;
     uint32_t rounds = (uint32_t)std::max<uint64_t>(1, loads / (2ull * blocks * threads));
@@ -3336,24 +3195,15 @@ extern "C" gdx_status gdx_measure_random_gather(int32_t device_req, uint64_t tab
         else if (record_bytes == 64) k_gather<64><<<blocks, threads>>>(table, nrec - 1, r, chained, sink);
         else k_gather<128><<<blocks, threads>>>(table, nrec - 1, r, chained, sink);
     };
-    if (e == cudaSuccess) {
-        k_fill_random<<<blocks, threads>>>((uint64_t *)table, nrec * record_bytes / 8);
-        launch(rounds / 8 + 1);  // warm-up
-        e = cudaEventCreate(&e0);
-    }
-    if (e == cudaSuccess) e = cudaEventCreate(&e1);
-    if (e == cudaSuccess) e = cudaEventRecord(e0);
-    if (e == cudaSuccess) {
-        launch(rounds);
-        e = cudaEventRecord(e1);
-    }
-    if (e == cudaSuccess) e = cudaEventSynchronize(e1);
-    if (e == cudaSuccess) e = cudaEventElapsedTime(&ms, e0, e1);
-    if (e0) cudaEventDestroy(e0);
-    if (e1) cudaEventDestroy(e1);
-    cudaFree(table);
-    if (sink) cudaFree(sink);
-    if (e != cudaSuccess) return fail(GDX_ERR_CUDA, "gather microbenchmark failed: %s", cudaGetErrorString(e));
+    k_fill_random<<<blocks, threads>>>(table_mem.as<uint64_t>(), nrec * record_bytes / 8);
+    launch(rounds / 8 + 1);  // warm-up
+    GDX_TRY(check(e0.create(cudaEventDefault)));
+    GDX_TRY(check(e1.create(cudaEventDefault)));
+    GDX_TRY(check(cudaEventRecord(e0)));
+    launch(rounds);
+    GDX_TRY(check(cudaEventRecord(e1)));
+    GDX_TRY(check(cudaEventSynchronize(e1)));
+    GDX_TRY(check(cudaEventElapsedTime(&ms, e0, e1)));
     const double nloads = 2.0 * blocks * threads * (double)rounds;
     if (gloads_out) *gloads_out = nloads / (ms * 1e-3) / 1e9;
     if (gbps_out) *gbps_out = nloads * record_bytes / (ms * 1e-3) / 1e9;

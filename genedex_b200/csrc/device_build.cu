@@ -14,38 +14,7 @@
 
 namespace gdx {
 
-void DeviceBuildResult::release() {
-    if (d_bwt) cudaFree(d_bwt);
-    if (d_samples) cudaFree(d_samples);
-    if (d_sa) cudaFree(d_sa);
-    if (d_isa_samples) cudaFree(d_isa_samples);
-    d_isa_samples = nullptr;
-    d_bwt = nullptr;
-    d_samples = nullptr;
-    d_sa = nullptr;
-}
-
 namespace {
-
-struct Dev {  // owning device pointer
-    void *p = nullptr;
-    ~Dev() { reset(); }
-    void reset() {
-        if (p) cudaFree(p);
-        p = nullptr;
-    }
-    cudaError_t alloc(uint64_t bytes) {
-        reset();
-        return cudaMalloc(&p, bytes ? bytes : 1);
-    }
-    template <class T>
-    T *as() const { return reinterpret_cast<T *>(p); }
-    void *take() {
-        void *q = p;
-        p = nullptr;
-        return q;
-    }
-};
 
 struct MaxU32 {
     __host__ __device__ uint32_t operator()(uint32_t a, uint32_t b) const { return a > b ? a : b; }
@@ -203,7 +172,7 @@ unsigned grid_for(uint64_t n, unsigned block = 256) { return (unsigned)((n + blo
             snprintf(_buf, sizeof _buf, "%s failed: %s (%s:%d)", #expr, cudaGetErrorString(_e),  \
                      __FILE__, __LINE__);                                                         \
             err = _buf;                                                                           \
-            out.release();                                                                        \
+            out = DeviceBuildResult();                                                            \
             return _e == cudaErrorMemoryAllocation ? GDX_ERR_OOM : GDX_ERR_CUDA;                  \
         }                                                                                         \
     } while (0)
@@ -219,7 +188,7 @@ gdx_status device_build_from_text(const uint8_t *h_text, const uint8_t *d_text_i
         err = "empty text or sampling rate 0";
         return GDX_ERR_BAD_ARG;
     }
-    Dev text_own;
+    DevMem text_own;
     const uint8_t *text = d_text_in;
     if (!text) {
         DB_TRY(text_own.alloc(n));
@@ -231,7 +200,7 @@ gdx_status device_build_from_text(const uint8_t *h_text, const uint8_t *d_text_i
     const uint32_t k = 64 / bits;
 
     // ---- phase 1: sort all suffixes by their first k symbols ---------------------------------------
-    Dev keyA, keyB, valA, valB, tmp;
+    DevMem keyA, keyB, valA, valB, tmp;
     DB_TRY(keyA.alloc(n * 8));
     DB_TRY(keyB.alloc(n * 8));
     DB_TRY(valA.alloc(n * 4));
@@ -246,7 +215,7 @@ gdx_status device_build_from_text(const uint8_t *h_text, const uint8_t *d_text_i
     DB_TRY(cub::DeviceRadixSort::SortPairs(tmp.p, tmp_bytes, dk, dv, (int64_t)n, 0, (int)(k * bits)));
 
     // ---- phase 2: group heads (= ranks) from the sorted keys --------------------------------------
-    Dev head, open_flags;
+    DevMem head, open_flags;
     DB_TRY(head.alloc(n * 4));
     DB_TRY(open_flags.alloc(n));
     {
@@ -264,23 +233,23 @@ gdx_status device_build_from_text(const uint8_t *h_text, const uint8_t *d_text_i
     DB_TRY(cudaGetLastError());
     DB_TRY(cudaDeviceSynchronize());
     // keep the sorted positions as SA, drop the wide key buffers before ISA is allocated
-    Dev sa;
+    DevMem sa;
     if (dv.Current() == valA.as<uint32_t>()) {
-        sa.p = valA.take();
+        sa = std::move(valA);
         valB.reset();
     } else {
-        sa.p = valB.take();
+        sa = std::move(valB);
         valA.reset();
     }
     keyA.reset();
     keyB.reset();
-    Dev isa;
+    DevMem isa;
     DB_TRY(isa.alloc(n * 4));
     k_scatter_isa<<<grid_for(n), 256>>>(sa.as<uint32_t>(), head.as<uint32_t>(), n, isa.as<uint32_t>());
     DB_TRY(cudaGetLastError());
 
     // ---- phase 3: doubling rounds over the still open suffixes -----------------------------------
-    Dev slots, slots2, d_m;
+    DevMem slots, slots2, d_m;
     DB_TRY(d_m.alloc(8));
     uint64_t m = 0;
     {
@@ -301,7 +270,7 @@ gdx_status device_build_from_text(const uint8_t *h_text, const uint8_t *d_text_i
     open_flags.reset();
     out.rounds = 0;
     if (m > 0) {
-        Dev rkA, rkB, rvA, rvB, newhead, still_open;
+        DevMem rkA, rkB, rvA, rvB, newhead, still_open;
         DB_TRY(rkA.alloc(m * 8));
         DB_TRY(rkB.alloc(m * 8));
         DB_TRY(rvA.alloc(m * 4));
@@ -349,10 +318,10 @@ gdx_status device_build_from_text(const uint8_t *h_text, const uint8_t *d_text_i
             DB_TRY(cub::DeviceSelect::Flagged(tmp.p, b6, slots.as<uint32_t>(), still_open.as<uint8_t>(),
                                               slots2.as<uint32_t>(), d_m.as<uint64_t>(), (int64_t)m));
             DB_TRY(cudaMemcpy(&m, d_m.p, 8, cudaMemcpyDeviceToHost));
-            std::swap(slots.p, slots2.p);
+            std::swap(slots, slots2);
             if (h > (1ull << 40)) {
                 err = "prefix doubling did not converge";
-                out.release();
+                out = DeviceBuildResult();
                 return GDX_ERR_CUDA;
             }
         }
@@ -364,7 +333,7 @@ gdx_status device_build_from_text(const uint8_t *h_text, const uint8_t *d_text_i
 
     // ---- optional O(n) verification ------------------------------------------------------------------
     if (verify) {
-        Dev inv, viol;
+        DevMem inv, viol;
         DB_TRY(inv.alloc(n * 4));
         DB_TRY(viol.alloc(8));
         DB_TRY(cudaMemset(inv.p, 0xff, n * 4));
@@ -377,7 +346,7 @@ gdx_status device_build_from_text(const uint8_t *h_text, const uint8_t *d_text_i
     }
 
     // ---- phase 4: BWT, samples, text borders --------------------------------------------------------
-    Dev zeros;
+    DevMem zeros;
     DB_TRY(zeros.alloc(16));
     DB_TRY(cudaMemset(zeros.p, 0, 16));
     k_count_zeros<<<148 * 8, 256>>>(text, n, zeros.as<unsigned long long>());
@@ -385,7 +354,7 @@ gdx_status device_build_from_text(const uint8_t *h_text, const uint8_t *d_text_i
     uint64_t nzero = 0;
     DB_TRY(cudaMemcpy(&nzero, zeros.p, 8, cudaMemcpyDeviceToHost));
     const uint64_t nsamp = (n + sampling_rate - 1) / sampling_rate;
-    Dev bwt, samples, brow, bpos;
+    DevMem bwt, samples, brow, bpos;
     DB_TRY(bwt.alloc(n));
     DB_TRY(samples.alloc(nsamp * 4));
     DB_TRY(brow.alloc((nzero + 1) * 8));
@@ -398,7 +367,7 @@ gdx_status device_build_from_text(const uint8_t *h_text, const uint8_t *d_text_i
     DB_TRY(cudaMemcpy(&nborder, zeros.as<uint64_t>() + 1, 8, cudaMemcpyDeviceToHost));
     if (nborder != nzero) {
         err = "internal error: number of BWT sentinels differs from the number of text sentinels";
-        out.release();
+        out = DeviceBuildResult();
         return GDX_ERR_CUDA;
     }
     std::vector<uint64_t> rows(nborder), pos(nborder);
@@ -414,15 +383,15 @@ gdx_status device_build_from_text(const uint8_t *h_text, const uint8_t *d_text_i
         out.border_pos[i] = pos[order[i]];
     }
     if (want_isa) {
-        Dev isa_s;
+        DevMem isa_s;
         DB_TRY(isa_s.alloc(nsamp * 4));
         k_sample_isa<<<grid_for(n), 256>>>(sa.as<uint32_t>(), n, sampling_rate, isa_s.as<uint32_t>());
         DB_TRY(cudaGetLastError());
-        out.d_isa_samples = (uint32_t *)isa_s.take();
+        out.d_isa_samples = std::move(isa_s);
     }
-    out.d_bwt = (uint8_t *)bwt.take();
-    out.d_samples = (uint32_t *)samples.take();
-    if (keep_sa) out.d_sa = (uint32_t *)sa.take();
+    out.d_bwt = std::move(bwt);
+    out.d_samples = std::move(samples);
+    if (keep_sa) out.d_sa = std::move(sa);
     return GDX_OK;
 }
 

@@ -15,22 +15,18 @@
 #include <vector>
 
 #include "../../include/genedex_b200.h"
+#include "cuda_owners.h"
 
 namespace gdx {
 
 struct DeviceBuildResult {
-    uint8_t *d_bwt = nullptr;       // n bytes, dense symbols
-    uint32_t *d_samples = nullptr;  // SA[0], SA[s], ... (n < 2^32 - 1)
-    uint32_t *d_sa = nullptr;       // full suffix array, only when keep_sa
-    uint32_t *d_isa_samples = nullptr;  // ISA[0], ISA[s], ... (row of every s-th text position), when want_isa
+    DevMem d_bwt;          // n bytes, dense symbols
+    DevMem d_samples;      // u32 SA[0], SA[s], ... (n < 2^32 - 1)
+    DevMem d_sa;           // u32 full suffix array, only when keep_sa
+    DevMem d_isa_samples;  // u32 ISA[0], ISA[s], ... (row of every s-th text position), when want_isa
     std::vector<uint64_t> border_rows, border_pos;  // sorted by row (bwt.rs:108-116)
     uint64_t verify_violations = 0;                 // only meaningful when verify was requested
     uint32_t rounds = 0;
-    DeviceBuildResult() = default;
-    DeviceBuildResult(const DeviceBuildResult &) = delete;
-    DeviceBuildResult &operator=(const DeviceBuildResult &) = delete;
-    ~DeviceBuildResult() { release(); }
-    void release();
 };
 
 // exactly one of h_text / d_text is non-null (dense symbols incl. sentinels)
