@@ -76,7 +76,8 @@ class gdx_index_info(C.Structure):
                 ("sample_bytes", C.c_uint64), ("lookup_bytes", C.c_uint64), ("num_samples", C.c_uint64),
                 ("num_text_borders", C.c_uint64), ("text_bytes", C.c_uint64),
                 ("inverse_sample_bytes", C.c_uint64), ("dense_suffix_array_bytes", C.c_uint64), ("seed_table_bytes", C.c_uint64),
-                ("seed_table_depth", C.c_uint32), ("row_context_entry_bytes", C.c_uint32)]
+                ("seed_table_depth", C.c_uint32), ("row_context_entry_bytes", C.c_uint32),
+                ("compact_seed_depth", C.c_uint32), ("compact_seed_bytes", C.c_uint64)]
 
 
 class gdx_stats(C.Structure):

@@ -1,10 +1,12 @@
 // Which accelerators an index builds outside its image (include/genedex_b200.h: the dense suffix array, the seed table
-// and the row context table) and the text verification threshold that follows from them.  Host only and free of CUDA,
+// with its compact seed level, and the row context table) and the text verification threshold that follows from them.  Host only and free of CUDA,
 // so that the policy runs on the CPU against a plain model (tests/test_accel_policy_host.py); api.cu observes the free
 // device memory and builds the tables.
 #pragma once
 #include <cstdint>
 #include <cstdlib>
+
+#include "compact_seed.h"
 
 namespace gdx {
 
@@ -78,6 +80,26 @@ struct AccelPolicy {
         if (!row_context_possible()) return false;
         if (env) return atoi(env) != 0;
         return !no_row_context && n * 16 <= (budget ? room(used, free) : 2 * room(used, free));
+    }
+
+    // The compact seed level (compact_seed.h) goes with a seed table of depth seed_depth: built after it (and after the
+    // row context table), dropped with it.  Rows and bases are u32 and its builder reads the text section.
+    bool compact_seed_possible(uint32_t seed_depth) const {
+        return seed_depth > 0 && !wide && n > 0 && n < (1ull << 32) && text && ns >= 2;
+    }
+    // the deepest level worth building: at most 32 d-mers per text position (3.1 Gbp DNA -> 18, 0.06 instead of 0.71 LF
+    // steps per query sampled from the text), 0 if none is deeper than the seed table
+    uint32_t compact_seed_max_depth(uint32_t seed_depth) const {
+        if (!compact_seed_possible(seed_depth)) return 0;
+        uint32_t d = seed_depth;
+        while (seed_entries(ns, d + 1) && seed_entries(ns, d + 1) <= 32 * n) ++d;
+        return d > seed_depth ? d : 0;
+    }
+    // level d with record_bytes of exception records fits what the tables built so far left: the budget when one is
+    // set, else half of the memory that is still free (the rule of the row context table)
+    bool compact_seed_fits(uint32_t d, uint64_t record_bytes, uint64_t used, uint64_t free) const {
+        const uint64_t groups = (seed_entries(ns, d) + kCsSlots - 1) / kCsSlots;
+        return groups * kCsGroupBytes + record_bytes <= (budget ? room(used, free) : 2 * room(used, free));
     }
 };
 

@@ -292,8 +292,8 @@ struct gdx_index {
     int device = 0;
     DevIndex dev;                  // written by refresh_dev only
     // accelerators outside the image (gdx_index_set_dense_suffix_array / _seed_table_depth / _row_context_table)
-    DevMem dense_sa, seed_table, row_context;
-    uint32_t seed_depth = 0;
+    DevMem dense_sa, seed_table, row_context, compact_seed;
+    uint32_t seed_depth = 0, compact_depth = 0;
     bool verify = true;            // finish one-row intervals through the text section (gdx_index_set_text_verification)
     PackTable pack;                // io byte -> 2-bit code (host packer, host_pack.h)
     // host-buffer queries hold this shared for the whole call; (re)building or freeing an accelerator needs it
@@ -547,6 +547,12 @@ void refresh_dev(gdx_index *idx) {
         d.seed_depth = idx->seed_depth;
     }
     d.row_context = idx->row_context.p;
+    if (idx->compact_seed) {
+        d.compact_seed = idx->compact_seed.as<uint8_t>();
+        d.compact_pool = reinterpret_cast<const uint32_t *>(
+            d.compact_seed + cs_groups(seed_entries(idx->h.ns, idx->compact_depth)) * kCsGroupBytes);
+        d.compact_depth = idx->compact_depth;
+    }
     d.verify_min_remaining = verify_min_remaining((bool)idx->dense_sa, getenv("GDX_VERIFY_MIN"));
     idx->dev = d;
 }
@@ -630,6 +636,7 @@ cudaError_t put_lookup_level0(void *dst, uint64_t n, bool wide) {
 }
 
 gdx_status build_seed_table(gdx_index *idx, uint32_t depth) {
+    drop_table(idx, idx->compact_seed);  // it goes with the seed table
     drop_table(idx, idx->seed_table);
     const ImageHeader &h = idx->h;
     // a level no deeper than the configured table would change nothing for the better and would move the
@@ -670,16 +677,112 @@ uint64_t free_device_bytes() {
     return cudaMemGetInfo(&free_b, &total_b) == cudaSuccess ? free_b : kFreeUnknown;
 }
 
+uint64_t accel_bytes(const gdx_index *idx) {
+    return idx->dense_sa.bytes + idx->seed_table.bytes + idx->row_context.bytes + idx->compact_seed.bytes;
+}
+
+// The compact seed level of depth d (compact_seed.h) from suffix array order and the text section.  A counting pass
+// sizes the exception records first; *fits = false (nothing built, no error) when the groups and records do not fit
+// what the policy leaves.
+gdx_status build_compact_seed_level(gdx_index *idx, uint32_t d, bool *fits) {
+    const ImageHeader &h = idx->h;
+    const AccelPolicy p = accel_policy(h);
+    *fits = false;
+    const uint64_t n = h.n, groups = cs_groups(seed_entries(h.ns, d)), group_bytes = groups * kCsGroupBytes;
+    const unsigned grid = (unsigned)div_up(n + 1, 256);
+    DevMem counters;  // n_exc, order_error
+    CUDA_TRY(counters.alloc(16));
+    CUDA_TRY(cudaMemset(counters.p, 0, 16));
+    CsBuild b{};
+    b.n_groups = groups;
+    b.d = d;
+    b.n_exc = counters.as<unsigned long long>();
+    b.order_error = reinterpret_cast<unsigned int *>(counters.as<uint8_t>() + 8);
+    auto rows_pass = [&]() -> gdx_status {
+        GDX_TRY(dispatch_layout(h.layout, [&](auto L) -> gdx_status {
+            k_cs_rows<decltype(L)><<<grid, 256>>>(idx->dev, b);
+            return GDX_OK;
+        }));
+        const cudaError_t e = cudaDeviceSynchronize();
+        return e == cudaSuccess ? GDX_OK : fail(GDX_ERR_CUDA, "compact seed level: %s", cudaGetErrorString(e));
+    };
+    GDX_TRY(rows_pass());
+    uint64_t m = 0;
+    uint32_t order_error = 0;
+    CUDA_TRY(cudaMemcpy(&m, counters.p, 8, cudaMemcpyDeviceToHost));
+    CUDA_TRY(cudaMemcpy(&order_error, b.order_error, 4, cudaMemcpyDeviceToHost));
+    if (order_error) return fail(GDX_ERR_CUDA, "compact seed level: the rows are not in suffix array order");
+    // pool: one count per group with a record (at most one per exception) + a triple per exception
+    const uint64_t pool_words = 4 * m;
+    if (m >= (1ull << 30) || !p.compact_seed_fits(d, pool_words * 4, accel_bytes(idx), free_device_bytes()))
+        return GDX_OK;
+    DevMem table, key, val, tmp;
+    if (table.alloc(group_bytes + pool_words * 4) != cudaSuccess) return table_oom("compact seed level", group_bytes + pool_words * 4);
+    int end_bit = 1;  // d-mer indices are below ns^d
+    while (end_bit < 64 && (seed_entries(h.ns, d) >> end_bit) != 0) ++end_bit;
+    size_t sort_bytes = 0, scan_bytes = 0;
+    CUDA_TRY(cub::DeviceRadixSort::SortPairs(nullptr, sort_bytes, (const uint64_t *)nullptr, (uint64_t *)nullptr,
+                                             (const uint64_t *)nullptr, (uint64_t *)nullptr, (int)m, 0, end_bit));
+    CUDA_TRY(cub::DeviceScan::InclusiveSum(nullptr, scan_bytes, (const uint32_t *)nullptr, (uint32_t *)nullptr, (int)m));
+    const uint64_t piece = align_up(m * 8 + 8, 256);
+    if (key.alloc(2 * piece) != cudaSuccess || val.alloc(2 * piece) != cudaSuccess ||
+        tmp.alloc(align_up(std::max(sort_bytes, scan_bytes), 256) + 2 * piece) != cudaSuccess)
+        return table_oom("compact seed level (build)", 4 * piece + std::max(sort_bytes, scan_bytes));
+    uint64_t *key_in = key.as<uint64_t>(), *key_out = (uint64_t *)(key.as<uint8_t>() + piece);
+    uint64_t *val_in = val.as<uint64_t>(), *val_out = (uint64_t *)(val.as<uint8_t>() + piece);
+    uint32_t *flag = (uint32_t *)tmp.p, *ord = (uint32_t *)(tmp.as<uint8_t>() + piece);
+    void *cub_tmp = tmp.as<uint8_t>() + 2 * piece;
+    CUDA_TRY(cudaMemset(table.p, 0, group_bytes));
+    CUDA_TRY(cudaMemset(counters.p, 0, 8));
+    b.groups = table.as<uint8_t>();
+    b.write = 1;
+    b.exc_cap = m;
+    b.exc_key = key_in;
+    b.exc_val = val_in;
+    GDX_TRY(rows_pass());
+    if (m) {
+        CUDA_TRY(cub::DeviceRadixSort::SortPairs(cub_tmp, sort_bytes, key_in, key_out, val_in, val_out, (int)m, 0, end_bit));
+        const unsigned g = (unsigned)div_up(m, 256);
+        k_cs_first_of_group<<<g, 256>>>(key_out, m, flag);
+        CUDA_TRY(cub::DeviceScan::InclusiveSum(cub_tmp, scan_bytes, flag, ord, (int)m));
+        k_cs_records<<<g, 256>>>(key_out, val_out, ord, m, table.as<uint8_t>(), (uint32_t *)(table.as<uint8_t>() + group_bytes));
+        const cudaError_t e = cudaDeviceSynchronize();
+        if (e != cudaSuccess) return fail(GDX_ERR_CUDA, "compact seed level: %s", cudaGetErrorString(e));
+    }
+    idx->compact_seed = std::move(table);
+    idx->compact_depth = d;
+    refresh_dev(idx);
+    *fits = true;
+    return GDX_OK;
+}
+
+// the compact seed level of the seed table the index holds now: the deepest level the policy allows whose groups and
+// records fit, or none
+gdx_status build_compact_seed(gdx_index *idx) {
+    drop_table(idx, idx->compact_seed);
+    const AccelPolicy p = accel_policy(idx->h);
+    const uint32_t seed = idx->seed_table ? idx->seed_depth : 0;
+    for (uint32_t d = p.compact_seed_max_depth(seed); d > seed; --d) {
+        if (!p.compact_seed_fits(d, 0, accel_bytes(idx), free_device_bytes())) continue;
+        bool fits = false;
+        GDX_TRY(build_compact_seed_level(idx, d, &fits));
+        if (fits) break;
+    }
+    return GDX_OK;
+}
+
 // what the policy of the index allows, in this order; each table is optional, so a failed build is no error of the call
 void build_accelerators(gdx_index *idx) {
     const AccelPolicy p = accel_policy(idx->h);
-    auto used = [&] { return idx->dense_sa.bytes + idx->seed_table.bytes + idx->row_context.bytes; };
+    auto used = [&] { return accel_bytes(idx); };
     if (p.dense_sa(used(), free_device_bytes(), getenv("GDX_DENSE_SA")) && build_dense_sa(idx) != GDX_OK)
         t_error.clear();
     const uint32_t depth = p.seed_depth(used(), free_device_bytes(), getenv("GDX_SEED_TABLE"));
     if (depth && build_seed_table(idx, depth) != GDX_OK) t_error.clear();
     if (p.row_context(used(), free_device_bytes(), getenv("GDX_ROW_CONTEXT")) && build_row_context(idx) != GDX_OK)
         t_error.clear();
+    // last: the three tables above build exactly what they would without it
+    if (build_compact_seed(idx) != GDX_OK) t_error.clear();
 }
 
 // Every way of creating an index ends here, with a finished image.  The caller has the device current and has released
@@ -1179,6 +1282,8 @@ extern "C" gdx_status gdx_index_get_info(const gdx_index *idx, gdx_index_info *o
     out->seed_table_bytes = idx->seed_table.bytes;
     out->seed_table_depth = idx->seed_table ? idx->seed_depth : 0;
     out->row_context_entry_bytes = idx->row_context ? 16 : 0;
+    out->compact_seed_depth = idx->compact_seed ? idx->compact_depth : 0;
+    out->compact_seed_bytes = idx->compact_seed.bytes;
     return GDX_OK;
 }
 
@@ -1305,7 +1410,11 @@ extern "C" gdx_status gdx_index_adopt_image(const void *header, void *device_ima
 extern "C" gdx_status gdx_index_set_seed_table_depth(gdx_index *idx, int32_t depth) {
     const char *busy = "queries are running on this index: the seed table cannot change now";
     return with_config(idx, busy, [&]() -> gdx_status {
-        if (depth > 0) return build_seed_table(idx, (uint32_t)depth);
+        if (depth > 0) {
+            GDX_TRY(build_seed_table(idx, (uint32_t)depth));
+            return build_compact_seed(idx);
+        }
+        drop_table(idx, idx->compact_seed);
         drop_table(idx, idx->seed_table);
         return GDX_OK;
     });

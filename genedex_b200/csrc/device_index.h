@@ -67,6 +67,8 @@ struct DevIndex {
     const void *isa;  // sampled inverse suffix array (same element width as samples) or nullptr
     const void *seed_lookup;  // level seed_depth of a lookup table deeper than the configured one, or nullptr
     const void *row_context;  // 16-byte entries: SA[row] + 45 symbols of text context per row (kernels.cuh: ctx_matches), or nullptr
+    const uint8_t *compact_seed;   // groups of the compact seed level (compact_seed.h), or nullptr
+    const uint32_t *compact_pool;  // its exception records
     uint64_t n, ntexts, n_border;
     uint32_t sigma, ns, sampling_rate, lookup_depth;
     uint32_t wide, noff, stride, derived_symbol;
@@ -77,6 +79,7 @@ struct DevIndex {
     uint32_t verify_min_remaining;  // text verification needs at least this many symbols left (8; 4 with the dense suffix array)
     uint32_t isa_rate;              // sampling rate of the inverse samples (= the configured rate)
     uint32_t seed_depth;
+    uint32_t compact_depth;
     uint64_t lut_level_off[kMaxLookupDepth + 1];
     uint64_t lut_pow[kMaxLookupDepth + 1];
     uint8_t io_to_dense[256];
@@ -113,6 +116,9 @@ inline DevIndex make_dev_index(const ImageHeader &h, const void *image) {
     d.seed_lookup = nullptr;
     d.seed_depth = 0;
     d.row_context = nullptr;
+    d.compact_seed = nullptr;
+    d.compact_pool = nullptr;
+    d.compact_depth = 0;
     if ((h.sampling_rate & (h.sampling_rate - 1)) == 0) {
         uint32_t s = 0;
         while ((1u << s) < h.sampling_rate) ++s;

@@ -21,6 +21,7 @@
 //   k_records_to_bwt device records -> dense BWT (export)
 //   k_densify       SA[row] for every row from the sampled suffix array (accelerator)
 //   k_build_row_context  SA[row] + 45 symbols of text context per row (accelerator)
+//   k_cs_rows / k_cs_records  the compact seed level from suffix array order and the text (accelerator, compact_seed.h)
 //   k_lut_extend    one level of the seed table (accelerator: a deeper lookup level outside the image)
 //   k_gather        random-gather ceiling microbenchmark     (SURVEY 8d)
 //
@@ -41,6 +42,7 @@
 
 #include <cub/block/block_scan.cuh>
 
+#include "compact_seed.h"
 #include "device_index.h"
 #include "hamming.h"
 #include "row_context.h"
@@ -351,6 +353,15 @@ __device__ __forceinline__ void seed_load(const DevIndex &ix, uint64_t entry, ui
         s = v.x;
         e = v.y;
     }
+}
+
+// (start, end) of d-mer k from the compact seed level: one 64 B group, exception records only where a group has one
+__device__ __forceinline__ void compact_seed_load(const DevIndex &ix, uint64_t k, uint64_t &s, uint64_t &e) {
+    const uint8_t *g = ix.compact_seed + (k / kCsSlots) * kCsGroupBytes;
+    uint64_t w[8];
+    ldg256_na(g, w);
+    ldg256_na(g + 32, w + 4);
+    cs_decode(w, (uint32_t)(k % kCsSlots), ix.compact_pool, s, e);
 }
 
 __device__ __forceinline__ void report_error(uint64_t *err, uint64_t q) {
@@ -708,13 +719,36 @@ k_search(const __grid_constant__ DevIndex ix, const DevQueries qs, uint64_t *__r
         const uint32_t depth = len < ix.lookup_depth ? (uint32_t)len : ix.lookup_depth;
         uint64_t pos = len - depth;
         uint64_t s = 0, e = 0;
+        bool seeded = false;
+        // Compact seed level (compact_seed.h, built with the seed table): the exact interval of the last compact_depth
+        // symbols when all of them are searchable.  An empty interval does not keep the value it had when it became
+        // empty, which only counts and hits may ignore: never for cursors.
+        if (!CURSORS && mode != 0 && !bad && ix.compact_seed && len >= ix.compact_depth) {
+            const uint32_t d = ix.compact_depth;
+            const uint64_t p0 = len - d;
+            bool ok = true;
+            uint64_t k = 0;
+            if (coded && ix.ns == 4 && p0 >= tail_begin) {
+                k = cs_index_from_codes(tail_bits(ptail, (uint32_t)(p0 - tail_begin), d), d);
+            } else {
+                for (uint32_t j = 0; j < d; ++j) {
+                    const uint32_t c = symbol_at(p0 + j);
+                    if (c == 0 || c > ix.ns) ok = false;
+                    k = k * ix.ns + (c - 1);
+                }
+            }
+            if (ok) {
+                compact_seed_load(ix, k, s, e);
+                pos = p0;
+                seeded = true;
+            }
+        }
         // Seed table accelerator (gdx_index_set_seed_table_depth): one level of a lookup table deeper than
         // the configured one.  Its entries are exactly what the configured table + LF steps produce (an empty
         // interval stays as it was when it became empty, k_lut_extend), so it may stand in whenever all of its
         // symbols are searchable; anything else (invalid byte, `N`, short query) takes the configured path,
         // which keeps the reference's lazy panic and the documented deviation where they were.
-        bool seeded = false;
-        if (!bad && ix.seed_lookup && len >= ix.seed_depth) {
+        if (!seeded && !bad && ix.seed_lookup && len >= ix.seed_depth) {
             const uint64_t p0 = len - ix.seed_depth;
             bool ok = true;
             const uint64_t li = lookup_index(p0, ix.seed_depth, ok);
@@ -1378,6 +1412,105 @@ k_build_row_context(const __grid_constant__ DevIndex ix, uint4 *__restrict__ out
     const uint64_t at = resolve_row<L>(ix, row, steps);
     const CtxEntry en = ctx_make_entry(at, ix.ns, [&](uint64_t p) { return text_symbol(ix, p); });
     out[row] = make_uint4(en.x, en.y, en.z, en.w);
+}
+
+// ---- compact seed level (compact_seed.h) from suffix array order and the text section --------------------------
+// 2 (key + 1) + gap of cs_row_key for a row: does not decrease from one row to the next
+template <class L>
+__device__ __forceinline__ uint64_t cs_row_code(const DevIndex &ix, uint64_t row, uint32_t d) {
+    uint32_t steps = 0;
+    const uint64_t at = resolve_row<L>(ix, row, steps);
+    bool gap;
+    const uint64_t k1 = cs_row_key([&](uint32_t j) { return at + j < ix.n ? text_symbol(ix, at + j) : 0u; }, d, ix.ns, gap);
+    return 2 * k1 + (gap ? 1 : 0);
+}
+
+// first row in [lo, n) whose code exceeds c (n if none), galloping from lo: a run of rows that share a d-mer (a repeat
+// family, the rows in front of an N run) costs its logarithm, not its length
+template <class L>
+__device__ uint64_t cs_upper(const DevIndex &ix, uint64_t lo, uint32_t d, uint64_t c) {
+    uint64_t hi = lo, step = 1;
+    while (hi < ix.n && cs_row_code<L>(ix, hi, d) <= c) {
+        lo = hi + 1;
+        hi += step;
+        step *= 2;
+    }
+    if (hi > ix.n) hi = ix.n;
+    while (lo < hi) {
+        const uint64_t mid = lo + (hi - lo) / 2;
+        if (cs_row_code<L>(ix, mid, d) <= c) lo = mid + 1;
+        else hi = mid;
+    }
+    return lo;
+}
+
+struct CsBuild {
+    uint8_t *groups;                    // write pass: zeroed groups; receives base, exc = kCsNoRecord and the fields
+    uint64_t n_groups;
+    uint32_t d;
+    int write;                          // 0: count the exception slots only
+    unsigned long long *n_exc;          // exception slots counted / placed
+    uint64_t exc_cap;
+    uint64_t *exc_key, *exc_val;        // write pass: d-mer, width | gap << 32 of every exception slot (unordered)
+    unsigned int *order_error;          // set when the codes decrease from one row to the next
+};
+
+// one thread per row r in [0, n] (r = n: the end of the last group).  Row r is the first row of the groups
+// [ceil(key1(r-1) / 224), ceil(key1(r) / 224)); a row that starts the rows of its d-mer measures its width and gap.
+template <class L>
+__global__ void __launch_bounds__(256) k_cs_rows(const __grid_constant__ DevIndex ix, const CsBuild b) {
+    const uint64_t r = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (r > ix.n) return;
+    const uint64_t code = r < ix.n ? cs_row_code<L>(ix, r, b.d) : ~0ull;
+    const uint64_t prev = r > 0 ? cs_row_code<L>(ix, r - 1, b.d) : 0;
+    if (r > 0 && code < prev) atomicOr(b.order_error, 1u);
+    const uint64_t k1 = code >> 1;
+    if (b.write) {
+        const uint64_t g_lo = r == 0 ? 0 : ((prev >> 1) + kCsSlots - 1) / kCsSlots;
+        const uint64_t g_hi = r == ix.n ? b.n_groups : (k1 + kCsSlots - 1) / kCsSlots;
+        for (uint64_t g = g_lo; g < g_hi; ++g)
+            *reinterpret_cast<uint64_t *>(b.groups + g * kCsGroupBytes) = r | ((uint64_t)kCsNoRecord << 32);
+    }
+    if (r == ix.n || k1 == 0 || (r > 0 && (prev >> 1) == k1)) return;
+    const uint64_t real_end = (code & 1) ? r : cs_upper<L>(ix, r + 1, b.d, code);
+    const uint64_t width = real_end - r, gap = cs_upper<L>(ix, real_end, b.d, 2 * k1 + 1) - real_end;
+    const uint64_t k = k1 - 1;
+    const uint32_t j = (uint32_t)(k % kCsSlots);
+    if (b.write && width)
+        atomicOr(reinterpret_cast<unsigned int *>(b.groups + (k / kCsSlots) * kCsGroupBytes + 8) + j / 16,
+                 (unsigned int)(width < 3 ? width : 3) << (2 * (j % 16)));
+    if (width >= 3 || gap > 0) {
+        const unsigned long long i = atomicAdd(b.n_exc, 1ull);
+        if (b.write && i < b.exc_cap) {
+            b.exc_key[i] = k;
+            b.exc_val[i] = width | (gap << 32);
+        }
+    }
+}
+
+// flag[i] = exception i (sorted by d-mer) is the first of its group
+__global__ void k_cs_first_of_group(const uint64_t *__restrict__ key, uint64_t m, uint32_t *__restrict__ flag) {
+    const uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < m) flag[i] = i == 0 || key[i] / kCsSlots != key[i - 1] / kCsSlots;
+}
+
+// the exception records: the group of exception i (sorted) has ordinal ord[i] - 1 among the groups with a record, so
+// its record starts at pool word 3 p + ord[i] - 1 (p = its first exception) and exception i lies at 3 i + ord[i]
+__global__ void k_cs_records(const uint64_t *__restrict__ key, const uint64_t *__restrict__ val,
+                             const uint32_t *__restrict__ ord, uint64_t m, uint8_t *__restrict__ groups,
+                             uint32_t *__restrict__ pool) {
+    const uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= m) return;
+    const uint64_t g = key[i] / kCsSlots, at = 3 * i + ord[i];
+    pool[at] = (uint32_t)(key[i] % kCsSlots);
+    pool[at + 1] = (uint32_t)val[i];
+    pool[at + 2] = (uint32_t)(val[i] >> 32);
+    if (i == 0 || key[i - 1] / kCsSlots != g) {
+        uint32_t cnt = 1;
+        while (i + cnt < m && key[i + cnt] / kCsSlots == g) ++cnt;
+        pool[at - 1] = cnt;
+        reinterpret_cast<uint32_t *>(groups + g * kCsGroupBytes)[1] = (uint32_t)(at - 1);
+    }
 }
 
 // ---- random-gather ceiling (SURVEY 8d) ----------------------------------------------------------------

@@ -132,7 +132,9 @@ class FmIndexConfig:
     def seed_table(self, allow: bool = True) -> "FmIndexConfig":
         """Allow (default) or forbid the seed table accelerator: one level of a lookup table deeper than the
         configured one (largest depth with ns^depth <= 4 * text length), built when device memory is ample
-        (`FmIndex.set_seed_table_depth` forces a depth).  Results and error behaviour are identical."""
+        (`FmIndex.set_seed_table_depth` forces a depth).  It brings a compact seed level that count and locate start
+        from (2 bits per d-mer, d the largest depth with ns^d <= 32 * text length that fits; `info().compact_seed_depth`
+        and `compact_seed_bytes`), built and dropped with it.  Results and error behaviour are identical."""
         self._flags = (self._flags & ~_lib.GDX_FLAG_NO_SEED_TABLE) | (0 if allow else _lib.GDX_FLAG_NO_SEED_TABLE)
         return self
 

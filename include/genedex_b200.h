@@ -201,6 +201,8 @@ typedef struct gdx_index_info {
     uint64_t seed_table_bytes;         /* device-only accelerator outside the image, 0 if absent */
     uint32_t seed_table_depth;         /* 0 if absent */
     uint32_t row_context_entry_bytes;  /* row context table: bytes per text position (16), 0 if absent */
+    uint32_t compact_seed_depth;       /* compact seed level of the seed table (see gdx_index_set_seed_table_depth), 0 if absent */
+    uint64_t compact_seed_bytes;       /* device-only accelerator outside the image, 0 if absent */
 } gdx_index_info;
 
 /* counters of the last search / locate call on this thread (feeds the roofline arithmetic) */
@@ -290,7 +292,13 @@ gdx_status gdx_index_set_dense_suffix_array(gdx_index *idx, int32_t on);
  * ns^d <= 4 * text length (at most four entries per text position), under the same policy as the dense suffix array (GDX_FLAG_NO_SEED_TABLE,
  * gdx_config.accelerator_budget_bytes, else a quarter of the free memory; GDX_SEED_TABLE=0 / =d overrides it
  * for measurements).  depth > configured depth (re)builds it at that depth now (GDX_ERR_OOM /
- * GDX_ERR_UNSUPPORTED if it does not fit), any smaller depth just frees it.  GDX_ERR_BUSY as above. */
+ * GDX_ERR_UNSUPPORTED if it does not fit), any smaller depth just frees it.  GDX_ERR_BUSY as above.
+ * The seed table brings a compact seed level: the interval of every d-mer two or more symbols deeper, in about
+ * 2 bits per d-mer (groups of 224 d-mers in 64 B, exception records for d-mers of more than two rows).  Count
+ * and locate queries whose last d symbols are all searchable start from it; cursors never do.  d is the largest
+ * depth with ns^d <= 32 * text length whose level fits the budget when one is set, else half of the free memory.
+ * It needs the text section, a text shorter than 2^32 symbols and 32-bit entries, is built last, and is rebuilt
+ * and freed together with the seed table (also by GDX_FLAG_NO_SEED_TABLE and GDX_SEED_TABLE=0). */
 gdx_status gdx_index_set_seed_table_depth(gdx_index *idx, int32_t depth);
 
 /* Row context table accelerator (memory for speed; alphabets with at most 4 searchable symbols, texts shorter than

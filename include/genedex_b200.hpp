@@ -376,7 +376,8 @@ public:
     FmIndexConfig &keep_inverse_samples(bool keep = true) { return flag(GDX_FLAG_NO_INVERSE_SAMPLES, !keep); }
     // dense suffix array accelerator (gdx_index_set_dense_suffix_array): default = built when memory is ample
     FmIndexConfig &dense_suffix_array(bool allow = true) { return flag(GDX_FLAG_NO_DENSE_SUFFIX_ARRAY, !allow); }
-    // seed table accelerator (gdx_index_set_seed_table_depth): default = built when memory is ample
+    // seed table accelerator and its compact seed level (gdx_index_set_seed_table_depth): default = built when memory
+    // is ample
     FmIndexConfig &seed_table(bool allow = true) { return flag(GDX_FLAG_NO_SEED_TABLE, !allow); }
     // row context table accelerator (gdx_index_set_row_context_table): default = built when memory is ample
     FmIndexConfig &row_context_table(bool allow = true) { return flag(GDX_FLAG_NO_ROW_CONTEXT_TABLE, !allow); }
